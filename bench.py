@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W                     # this framework
     python bench.py --impl reference --gpus N --steps K --warmup W    # CPU reference arm (oracle port)
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR  # also write the last timed step's ids to DIR
 
 Workload (BASELINE.json configs[2], the configuration the metric "tokens/s at 1/2/4/8 B200" is quoted on and the
 reference's production call, mmt_result_test_functions_15_4.py:504-570): config_V8 random-init weights, MULTINOMIAL
@@ -41,6 +42,7 @@ MAX_LEN = 128
 C2_SPECTRA_PER_GPU = 256        # config 2 (extra key): greedy, weak scaling
 REF_SAMPLE_CAND = 16            # CPU arms: candidates of ONE spectrum per step (the reference decodes one spectrum at a time)
 EAGER_SAMPLE_SPECTRA = 8        # gpu_eager_baseline: spectra x 128 candidates under torch eager
+DUMP_SEQUENCES = 65536          # --dump-outputs: 65,536 x 128 ids in float32 = 32 MiB (all 131,072 would be 64 MiB)
 STOI = {"<PAD>": 0, "<UNK>": 1, "<EOS>": 2, "<SOS>": 3, "<MASK>": 4}
 # algorithmic work model (SURVEY.md 8d / BASELINE.md 4)
 FLOP_ENCODE_PER_SPECTRUM = 9.50e9
@@ -63,6 +65,17 @@ def source_hash():
     for f in sorted(os.listdir(d)):
         h.update(open(os.path.join(d, f), "rb").read())
     return h.hexdigest()[:16]
+
+
+def dump_outputs(out_dir, ids):
+    """Write DIR/ids.npy: the rows of the (sequences, positions) u8 ids a caller of the timed path receives, at a fixed
+    seeded sample of DUMP_SEQUENCES sequences in ascending order, as float32 (exact for ids < 2**24)."""
+    import numpy as np
+    import torch
+    n = ids.shape[0]
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:min(n, DUMP_SEQUENCES)].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "ids.npy"), ids[rows.to(ids.device)].cpu().numpy().astype(np.float32))
 
 
 class ClockSampler:
@@ -186,8 +199,15 @@ def main():
     ap.add_argument("--precision", default=os.environ.get("MMT_BENCH_PRECISION", "auto"), choices=["auto", "fp32", "bf16"])
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the cpu / gpu-eager comparator legs")
     ap.add_argument("--no-config2", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the ids of the last timed step of the main workload to DIR/ids.npy (float32, a fixed sample "
+                         f"of {DUMP_SEQUENCES:,} of the {N_SPECTRA * N_CAND:,} sequences), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs --impl b200")
         return run_reference(args)
 
     import torch
@@ -204,7 +224,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
 
     precision = args.precision
     if precision == "auto":
@@ -232,7 +252,8 @@ def main():
         """k steps; step i's gathered ids are consumed after step i+1 has been issued, so the collective (side stream) and
         the rendezvous with the slowest rank overlap the next step.  Device time from CUDA events on the launching stream,
         barrier + synchronize on both sides, max over ranks.  With `flush` (an L2 flush between steps) every step has its
-        own event pair and the flushes fall between the pairs."""
+        own event pair and the flushes fall between the pairs.  Returns (device ms, wall s, what the last step's issue()
+        returned)."""
         barrier()
         t0 = time.perf_counter()
         evs = []
@@ -258,7 +279,7 @@ def main():
         evs[-1][1].record()
         barrier()
         wall = time.perf_counter() - t0
-        return max_over_ranks(sum(a.elapsed_time(b) for a, b in evs)), wall
+        return max_over_ranks(sum(a.elapsed_time(b) for a, b in evs)), wall, prev
 
     COPIED = ("src_1H", "mask_1H", "src_13C", "mask_13C", "src_HSQC", "src_HSQC", "mask_HSQC", "src_COSY", "src_COSY", "mask_COSY",
               "src_IR", "src_MF", "mask_MF", "trg_MW", "trg_enc_SMI")      # what run_model moves to the device (HSQC / COSY twice: it also returns them)
@@ -292,9 +313,12 @@ def main():
     if rank == 0:
         sampler.start()
     l0 = eng.launch_count()
-    ms_res, wall_res = timed_pipeline(issue_resident, consume_resident, K)
+    ms_res, wall_res, last = timed_pipeline(issue_resident, consume_resident, K)
     launches = eng.launch_count() - l0
-    ms_e2e, wall_e2e = timed_pipeline(issue_e2e, consume_e2e, K)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last.packed())
+    del last
+    ms_e2e, wall_e2e, _ = timed_pipeline(issue_e2e, consume_e2e, K)
     clocks = sampler.stop() if rank == 0 else None
     if world > 1:
         t = torch.tensor([launches], device=dev, dtype=torch.int64)
@@ -321,9 +345,9 @@ def main():
             g_res().packed()
         g_e2e().packed()
         l0 = eng.launch_count()
-        ms2, _ = timed_pipeline(g_res, lambda p: p.packed(), K2, flush=lambda: flush_buf.fill_(1))
+        ms2, _, _ = timed_pipeline(g_res, lambda p: p.packed(), K2, flush=lambda: flush_buf.fill_(1))
         launches2 = eng.launch_count() - l0
-        ms2e, _ = timed_pipeline(g_e2e, lambda p: out2.copy_(p.packed(), non_blocking=True), K2, flush=lambda: flush_buf.fill_(1))
+        ms2e, _, _ = timed_pipeline(g_e2e, lambda p: out2.copy_(p.packed(), non_blocking=True), K2, flush=lambda: flush_buf.fill_(1))
         tok2 = MAX_LEN * C2_SPECTRA_PER_GPU * world
         c2 = {"workload": f"BASELINE.json configs[1]: greedy decode, {C2_SPECTRA_PER_GPU} spectra per GPU x {MAX_LEN} tokens, weak scaling, "
                           "explicit 256 MiB L2 flush between steps (untimed)",
