@@ -282,6 +282,24 @@ int32_t mmt_ffn(mmt_engine* e, const float* d_x, const float* d_w1, const float*
                 const float* d_b2, const float* d_gamma, const float* d_beta, float* d_out,
                 int64_t M, int32_t F, int32_t splits, int32_t weight_terms, void* stream);
 
+/* The self-attention half of one decoder layer of the un-fused (large-wave) decode step, stand-alone, with the code the
+ * step runs: QKV projection of layer `layer` (bf16: tcgen05 on W_hi, K | V appended to the paged cache by the GEMM's
+ * epilogue or by the attention kernel, as the engine's MMT_KV_HEAD_MAJOR / MMT_NO_KV_EPILOGUE knobs select; fp32: SIMT
+ * GEMM) followed by the matching paged self-attention kernel, for positions t = 0 .. T-1 of N sequences in one wave
+ * (slot-major page map).  d_x (T,N,128) f32: the layer's input rows at every position (rounded to bf16 in the bf16 mode);
+ * d_out (T,N,128) f32: the attention output (before out_proj) of position t over keys 0..t, widened from bf16 in the
+ * bf16 mode.  Unwritten cache slots hold NaN. */
+int32_t mmt_decode_self_attention(mmt_engine* e, int32_t layer, const float* d_x, int64_t N, int32_t T, int32_t precision,
+                                  float* d_out, void* stream);
+
+/* The cross-attention of one decoder layer of the un-fused decode step, stand-alone: the memory of a->Bm spectra is
+ * prepared as one decode wave (memory index, K/V projection with the two-term weights), then the queries d_q
+ * (Bm*n_cand,128) f32 attend to it -- the tensor-core kernel for a->n_cand >= 8 in the bf16 mode (MMT_NO_TC_ATTENTION: the
+ * SIMT kernel), the SIMT kernel otherwise.  d_out (Bm*n_cand,128) f32: the attention output (before out_proj), widened
+ * from bf16 in the bf16 mode.  Memory, key_bias, S, Bm, n_cand and precision come from `a`; the rest of it is ignored. */
+int32_t mmt_decode_cross_attention(mmt_engine* e, const mmt_decode_args* a, int32_t layer, const float* d_q, float* d_out,
+                                   void* stream);
+
 /* launches issued by this engine since creation (bench.py's gpu_launches). */
 int64_t mmt_launch_count(const mmt_engine* e);
 

@@ -1018,6 +1018,57 @@ static int decode_prepare_wave(mmt_engine* e, const mmt_decode_args& a, int b0, 
     return 0;
 }
 
+// Un-fused step, one decoder layer: the QKV projection of the new position (x16 / x at step *b.ctl) and its self-attention
+// over the layer's cache `pool` -> att16 (bf16) | att (fp32).  bf16: tcgen05 projection whose epilogue appends K | V to the
+// token-major (default) or head-major pages, or (MMT_NO_KV_EPILOGUE) the attention kernel appends them; fp32: SIMT GEMM.
+// decode_step and the unit hook mmt_decode_self_attention both run this.
+static int decode_self_attention_layer(mmt_engine* e, const LayerW& w, const DecBuffers& b, char* pool, int pps, int64_t Nw, bool bf16,
+                                       bool pdl_u, cudaStream_t s) {
+    const int H = e->desc.n_heads, dh = D / H;
+    const float scale = 1.0f / sqrtf((float)dh);
+    const int* step = b.ctl;
+    const int M = (int)Nw;
+    if (dh != 8) MMT_FAIL("decoder head dim must be 8");
+    if (bf16) {   // K | V columns of the projection land in the cache pages directly; the fp32 row keeps only Q
+        TcGemmParams p = tc_params(M, 3 * D, D);
+        // (with the K | V columns going to the cache, the Q columns form a dense [N][D] buffer: a 512-byte row every 512
+        // bytes instead of every 1536)
+        p.bias = w.in_b; p.out_f32 = b.qkv; p.ld_f32 = e->use_kv_epilogue ? D : 3 * D;
+        p.kv_append = e->use_kv_epilogue ? (e->kv_tok_major && H % 8 == 0 ? 2 : 1) : 0; p.kv_pool = reinterpret_cast<__nv_bfloat16*>(pool); p.block_table = b.block_table; p.pps = pps; p.step = step; p.kv_heads = H;
+        MMT_TRY(launch_tc(e, p, b.x16, D, e->Wb(w.in_w), TC_EPI_STORE, s, e->dec_proj_single ? nullptr : e->Wlo(w.in_w), pdl_u));
+    } else {
+        GemmParams p = gemm_params(3 * D, D, 3 * D, 0);
+        p.g[0].A = b.x; p.g[0].lda = D; p.g[0].W = w.in_w; p.g[0].bias = w.in_b; p.g[0].C = b.qkv; p.g[0].M = M;
+        p.splits = 1; p.part_stride = Nw * D;
+        MMT_TRY(launch_gemm(e, p, 1, M, s));
+    }
+    prof_pre(e, s);
+    const unsigned sa_blocks = (unsigned)((Nw * (H / 4) + 7) / 8);     // a warp per (sequence, 4 heads)
+    if (bf16 && e->use_kv_epilogue && e->kv_tok_major && H % 8 == 0)      // token-major pages: a warp per (sequence, 8 heads)
+        launch_args(decode_self_attention_tm<8>, dim3((unsigned)((Nw * (H / 8) + 7) / 8)), dim3(256), 0, s, pdl_u, (const float*)b.qkv, (const __nv_bfloat16*)reinterpret_cast<__nv_bfloat16*>(pool), (const int*)b.block_table, pps, Nw, H, scale, step, b.att16);
+    else if (bf16 && e->use_kv_epilogue) launch_args(decode_self_attention_g8<8, __nv_bfloat16, false>, dim3(sa_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qkv, reinterpret_cast<__nv_bfloat16*>(pool), (const int*)b.block_table, pps, Nw, H, scale, step, (float*)nullptr, b.att16);
+    else if (bf16) launch_args(decode_self_attention_g8<8, __nv_bfloat16>, dim3(sa_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qkv, reinterpret_cast<__nv_bfloat16*>(pool), (const int*)b.block_table, pps, Nw, H, scale, step, (float*)nullptr, b.att16);
+    else decode_self_attention_g8<8, float><<<sa_blocks, 256, 0, s>>>(b.qkv, reinterpret_cast<float*>(pool), b.block_table, pps, Nw, H, scale, step, b.att, b.att16);
+    return check_launch(e, "decode_self_attention", s);
+}
+
+// Un-fused step, one decoder layer: cross attention of the queries qc over the layer's projected memory `ckv` -> att16 | att.
+// Candidates of a spectrum share K/V: tensor-core tiles of 16 candidates for n_cand >= 8 in the bf16 mode (MMT_NO_TC_ATTENTION:
+// the SIMT kernel).  decode_step and the unit hook mmt_decode_cross_attention both run this.
+static int decode_cross_attention_layer(mmt_engine* e, const mmt_decode_args& a, const DecBuffers& b, const char* ckv, int64_t Nw, int Bmw,
+                                        bool bf16, bool pdl_u, cudaStream_t s) {
+    const int H = e->desc.n_heads, dh = D / H;
+    const float scale = 1.0f / sqrtf((float)dh);
+    if (dh != 8) MMT_FAIL("decoder head dim must be 8");
+    const unsigned attn_blocks = (unsigned)((Nw * H + 7) / 8);
+    prof_pre(e, s);
+    if (bf16 && a.n_cand >= 8 && e->use_tc_attention)
+        launch_args(decode_cross_attention_tc, dim3(H, Bmw), dim3(256), dx_smem_bytes(a.S), s, pdl_u, (const float*)b.qc, reinterpret_cast<const __nv_bfloat16*>(ckv), (int64_t)a.S, (const int*)b.nk, (const int*)b.row_start, (const float*)b.kbias_c, (int)a.n_cand, H, scale, (float*)nullptr, b.att16);
+    else if (bf16) launch_args(decode_cross_attention<8, __nv_bfloat16>, dim3(attn_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qc, reinterpret_cast<const __nv_bfloat16*>(ckv), (int64_t)a.S, (const int*)b.nk, (const int*)b.row_start, (const float*)b.kbias_c, (int)a.n_cand, Nw, H, scale, (float*)nullptr, b.att16);
+    else decode_cross_attention<8, float><<<attn_blocks, 256, 0, s>>>(b.qc, reinterpret_cast<const float*>(ckv), a.S, b.nk, b.row_start, b.kbias_c, a.n_cand, Nw, H, scale, b.att, b.att16);
+    return check_launch(e, "decode_cross_attention", s);
+}
+
 static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw, int Bmw, DecBuffers& b, bool bf16, cudaStream_t s) {
     const mmt_model_desc& d = e->desc;
     const mmt_decode_args& a = *r.a;
@@ -1156,28 +1207,11 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
         else launch_args(decode_embed, dim3((unsigned)((Nw + 3) / 4)), dim3(128), 0, s, pdl_u, (const int64_t*)(r.tokens + n0), 1, 3, Nw, ldn, e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, step, b.x, b.x16);
         MMT_TRY(check_launch(e, "decode_embed", s));
 
-        const unsigned attn_blocks = (unsigned)((Nw * H + 7) / 8);
-        if (dh != 8) MMT_FAIL("decoder head dim must be 8");
         for (int l = 0; l < d.n_dec_layers; ++l) {
             const LayerW& w = e->dec[l];
             char* pool = b.kv_pool + (size_t)l * b.pool_pages * 2 * PAGE_TOKENS * D * b.kv_esz;
             const char* ckv = b.cross_kv + (size_t)l * 2 * R * D * b.kv_esz;
-            if (bf16) {   // K | V columns of the projection land in the cache pages directly; the fp32 row keeps only Q
-                TcGemmParams p = tc_params(M, 3 * D, D);
-                // (with the K | V columns going to the cache, the Q columns form a dense [N][D] buffer: a 512-byte row every 512
-                // bytes instead of every 1536)
-                p.bias = w.in_b; p.out_f32 = b.qkv; p.ld_f32 = e->use_kv_epilogue ? D : 3 * D;
-                p.kv_append = e->use_kv_epilogue ? (e->kv_tok_major && H % 8 == 0 ? 2 : 1) : 0; p.kv_pool = reinterpret_cast<__nv_bfloat16*>(pool); p.block_table = b.block_table; p.pps = pps; p.step = step; p.kv_heads = H;
-                MMT_TRY(launch_tc(e, p, b.x16, D, e->Wb(w.in_w), TC_EPI_STORE, s, plo(w.in_w), pdl_u));
-            } else MMT_TRY(gemm(b.x, D, w.in_w, w.in_b, b.qkv, 3 * D, D, 0, 1));
-            prof_pre(e, s);
-            const unsigned sa_blocks = (unsigned)((Nw * (H / 4) + 7) / 8);     // a warp per (sequence, 4 heads)
-            if (bf16 && e->use_kv_epilogue && e->kv_tok_major && H % 8 == 0)      // token-major pages: a warp per (sequence, 8 heads)
-                launch_args(decode_self_attention_tm<8>, dim3((unsigned)((Nw * (H / 8) + 7) / 8)), dim3(256), 0, s, pdl_u, (const float*)b.qkv, (const __nv_bfloat16*)reinterpret_cast<__nv_bfloat16*>(pool), (const int*)b.block_table, pps, Nw, H, scale, step, b.att16);
-            else if (bf16 && e->use_kv_epilogue) launch_args(decode_self_attention_g8<8, __nv_bfloat16, false>, dim3(sa_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qkv, reinterpret_cast<__nv_bfloat16*>(pool), (const int*)b.block_table, pps, Nw, H, scale, step, (float*)nullptr, b.att16);
-            else if (bf16) launch_args(decode_self_attention_g8<8, __nv_bfloat16>, dim3(sa_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qkv, reinterpret_cast<__nv_bfloat16*>(pool), (const int*)b.block_table, pps, Nw, H, scale, step, (float*)nullptr, b.att16);
-            else decode_self_attention_g8<8, float><<<sa_blocks, 256, 0, s>>>(b.qkv, reinterpret_cast<float*>(pool), b.block_table, pps, Nw, H, scale, step, b.att, b.att16);
-            MMT_TRY(check_launch(e, "decode_self_attention", s));
+            MMT_TRY(decode_self_attention_layer(e, w, b, pool, pps, Nw, bf16, pdl_u, s));
             if (bf16) {
                 // out-proj + LN1 and the cross-attention query projection as one launch -- for waves up to 24,576 rows: the chained
                 // kernel holds 192 KB of shared memory (one CTA per SM instead of three), which costs more than the saved launch
@@ -1194,12 +1228,7 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
                 MMT_TRY(ln(b.part, 1, w.out_b, w.n1_w, w.n1_b));
                 MMT_TRY(gemm(b.x, D, w.ca_in_w, w.ca_in_b, b.qc, D, D, 0, 1));
             }
-            prof_pre(e, s);
-            if (bf16 && a.n_cand >= 8 && e->use_tc_attention)   // candidates of a spectrum share K/V: tensor-core tiles of 16 candidates
-                launch_args(decode_cross_attention_tc, dim3(H, Bmw), dim3(256), dx_smem_bytes(a.S), s, pdl_u, (const float*)b.qc, reinterpret_cast<const __nv_bfloat16*>(ckv), (int64_t)a.S, (const int*)b.nk, (const int*)b.row_start, (const float*)b.kbias_c, (int)a.n_cand, H, scale, (float*)nullptr, b.att16);
-            else if (bf16) launch_args(decode_cross_attention<8, __nv_bfloat16>, dim3(attn_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qc, reinterpret_cast<const __nv_bfloat16*>(ckv), (int64_t)a.S, (const int*)b.nk, (const int*)b.row_start, (const float*)b.kbias_c, (int)a.n_cand, Nw, H, scale, (float*)nullptr, b.att16);
-            else decode_cross_attention<8, float><<<attn_blocks, 256, 0, s>>>(b.qc, reinterpret_cast<const float*>(ckv), a.S, b.nk, b.row_start, b.kbias_c, a.n_cand, Nw, H, scale, b.att, b.att16);
-            MMT_TRY(check_launch(e, "decode_cross_attention", s));
+            MMT_TRY(decode_cross_attention_layer(e, a, b, ckv, Nw, Bmw, bf16, pdl_u, s));
             if (bf16) {
                 const bool ffn_pro = e->use_ffn_prologue && M >= 2048;     // cross-attention out-projection + norm2 as the FFN kernel's prologue
                 if (!ffn_pro) MMT_TRY(tc_ln(b.att16, D, w.ca_out_w, w.ca_out_b, D, w.n2_w, w.n2_b));
@@ -2028,6 +2057,81 @@ int32_t mmt_ffn(mmt_engine* e, const float* d_x, const float* d_w1, const float*
     g.part = part; g.bias = d_b2; g.res = d_x; g.gamma = d_gamma; g.beta = d_beta; g.out = d_out; g.M = (int)M;
     g.S_in = (int)M; g.stride_b = 0; g.stride_s = 1; g.off = 0;
     return launch_ln(e, q, 1, (int)M, cs);
+}
+
+int32_t mmt_decode_self_attention(mmt_engine* e, int32_t layer, const float* d_x, int64_t N, int32_t T, int32_t precision,
+                                  float* d_out, void* stream) {
+    if (!e || !d_x || !d_out) MMT_FAIL("null argument");
+    const mmt_model_desc& d = e->desc;
+    if (layer < 0 || layer >= d.n_dec_layers) MMT_FAIL("mmt_decode_self_attention: layer out of range");
+    if (N <= 0 || N > 0x7fffffff) MMT_FAIL("mmt_decode_self_attention: N must be in [1, 2^31)");
+    if (T < 1 || T > d.max_len || T > 128) MMT_FAIL("mmt_decode_self_attention: T must be in [1, min(128, pe_trg rows)]");
+    if (precision != MMT_PREC_FP32 && precision != MMT_PREC_BF16) MMT_FAIL("bad precision");
+    const bool bf16 = precision == MMT_PREC_BF16;
+    cudaStream_t s = (cudaStream_t)stream;
+    EngineCall call(e, s);
+    // the buffers of a one-layer decode wave of N sequences, planned like run_decode's (no cross-attention memory)
+    mmt_model_desc d1 = d;
+    d1.n_dec_layers = 1;
+    Arena ar;
+    DecBuffers b;
+    plan_decoder(ar, d1, N, 1, 1, T, b, bf16, e->fused_decode_rows);
+    MMT_TRY(ensure_arena(e, ar.off));
+    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
+    plan_decoder(ar, d1, N, 1, 1, T, b, bf16, e->fused_decode_rows);
+    const int pps = (T + PAGE_TOKENS - 1) / PAGE_TOKENS;
+    // unwritten cache slots hold NaN: a key read before it was appended poisons the output instead of passing unnoticed
+    MMT_CUDA(cudaMemsetAsync(b.kv_pool, 0xff, (size_t)b.pool_pages * 2 * PAGE_TOKENS * D * b.kv_esz, s));
+    prof_pre(e, s);
+    init_block_table<<<(unsigned)((N * pps + 255) / 256), 256, 0, s>>>(b.block_table, N, pps);
+    MMT_TRY(check_launch(e, "init_block_table", s));
+    const int64_t n_el = N * D;
+    const unsigned blocks = (unsigned)((n_el + 255) / 256);
+    for (int t = 0; t < T; ++t) {
+        set_i32<<<1, 1, 0, s>>>(b.ctl, t);
+        MMT_TRY(check_launch(e, "set_i32", s));
+        if (bf16) {
+            f32_to_bf16<<<blocks, 256, 0, s>>>(d_x + t * n_el, n_el, b.x16);
+            MMT_TRY(check_launch(e, "f32_to_bf16", s));
+        } else MMT_CUDA(cudaMemcpyAsync(b.x, d_x + t * n_el, n_el * sizeof(float), cudaMemcpyDeviceToDevice, s));
+        MMT_TRY(decode_self_attention_layer(e, e->dec[layer], b, b.kv_pool, pps, N, bf16, false, s));
+        if (bf16) {
+            bf16_to_f32<<<blocks, 256, 0, s>>>(b.att16, n_el, d_out + t * n_el);
+            MMT_TRY(check_launch(e, "bf16_to_f32", s));
+        } else MMT_CUDA(cudaMemcpyAsync(d_out + t * n_el, b.att, n_el * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    }
+    return 0;
+}
+
+int32_t mmt_decode_cross_attention(mmt_engine* e, const mmt_decode_args* a, int32_t layer, const float* d_q, float* d_out, void* stream) {
+    if (!e || !a || !d_q || !d_out) MMT_FAIL("null argument");
+    const mmt_model_desc& d = e->desc;
+    if (layer < 0 || layer >= d.n_dec_layers) MMT_FAIL("mmt_decode_cross_attention: layer out of range");
+    if (a->Bm <= 0 || a->n_cand <= 0 || a->S <= 0) MMT_FAIL("mmt_decode_cross_attention: empty batch");
+    if ((a->stride_s % 4) || (a->stride_b % 4) || ((uintptr_t)a->d_memory % 16)) MMT_FAIL("mmt_decode_cross_attention: memory must be 16-byte aligned with strides that are multiples of 4 floats");
+    if (a->precision != MMT_PREC_FP32 && a->precision != MMT_PREC_BF16) MMT_FAIL("bad precision");
+    const int64_t N = (int64_t)a->Bm * a->n_cand;
+    if (N > 0x7fffffff) MMT_FAIL("mmt_decode_cross_attention: too many sequences");
+    const bool bf16 = a->precision == MMT_PREC_BF16;
+    cudaStream_t s = (cudaStream_t)stream;
+    EngineCall call(e, s);
+    // one wave of all Bm memories, planned like run_decode's (self-attention cache of a single position)
+    Arena ar;
+    DecBuffers b;
+    plan_decoder(ar, d, N, a->Bm, a->S, 1, b, bf16, e->fused_decode_rows);
+    MMT_TRY(ensure_arena(e, ar.off));
+    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
+    plan_decoder(ar, d, N, a->Bm, a->S, 1, b, bf16, e->fused_decode_rows);
+    MMT_TRY(decode_prepare_wave(e, *a, 0, a->Bm, b, bf16, s));
+    MMT_CUDA(cudaMemcpyAsync(b.qc, d_q, (size_t)N * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    const int64_t R = (int64_t)a->Bm * a->S;
+    MMT_TRY(decode_cross_attention_layer(e, *a, b, b.cross_kv + (size_t)layer * 2 * R * D * b.kv_esz, N, a->Bm, bf16, false, s));
+    if (bf16) {
+        bf16_to_f32<<<(unsigned)((N * D + 255) / 256), 256, 0, s>>>(b.att16, N * D, d_out);
+        return check_launch(e, "bf16_to_f32", s);
+    }
+    MMT_CUDA(cudaMemcpyAsync(d_out, b.att, (size_t)N * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    return 0;
 }
 
 int64_t mmt_launch_count(const mmt_engine* e) { return e ? e->launches : 0; }

@@ -1699,4 +1699,11 @@ __global__ void f32_to_bf16(const float* in, int64_t n, __nv_bfloat16* out) {
     if (i < n) out[i] = __float2bfloat16_rn(in[i]);
 }
 
+__global__ void bf16_to_f32(const __nv_bfloat16* in, int64_t n, float* out) {
+    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = __bfloat162float(in[i]);
+}
+
+__global__ void set_i32(int* dst, int v) { *dst = v; }
+
 }  // namespace mmt

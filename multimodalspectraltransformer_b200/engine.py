@@ -335,6 +335,31 @@ class Engine:
         _lib.check(self.L.mmt_ffn(self.h, *[v.data_ptr() for v in t], out.data_ptr(), M, F, splits, weight_terms, self._stream()))
         return out
 
+    def decode_self_attention(self, layer, x, precision="bf16"):
+        """x (T,N,128): input rows of decoder layer ``layer`` at positions 0..T-1 -> (T,N,128) f32 self-attention output
+        (before out_proj) of every position over keys 0..t, through the un-fused decode step's QKV projection, paged KV
+        cache and attention kernel (test hook)."""
+        x = x.to(self.device, torch.float32).contiguous()
+        T, N, _ = x.shape
+        out = torch.empty_like(x)
+        _lib.check(self.L.mmt_decode_self_attention(self.h, layer, x.data_ptr(), N, T, _PREC[precision], out.data_ptr(),
+                                                    self._stream()))
+        return out
+
+    def decode_cross_attention(self, layer, memory, key_bias, q, *, n_cand=1, precision="bf16"):
+        """q (Bm*n_cand,128) queries of decoder layer ``layer`` over memory (S,Bm,128) with the additive key_bias (Bm,S)
+        -> (Bm*n_cand,128) f32 cross-attention output (before out_proj), through the un-fused decode step's memory
+        preparation and attention kernel (test hook)."""
+        a, keep = self._decode_args(memory, key_bias, n_cand, 1, 1.0, 0, False, precision)
+        q = q.to(self.device, torch.float32).contiguous()
+        if tuple(q.shape) != (a.Bm * n_cand, self.desc.d_model):
+            raise ValueError("q must be (Bm * n_cand, 128)")
+        out = torch.empty_like(q)
+        _lib.check(self.L.mmt_decode_cross_attention(self.h, C.byref(a), layer, q.data_ptr(), out.data_ptr(), self._stream()))
+        for t in keep:
+            t.record_stream(torch.cuda.current_stream(self.dev_index))
+        return out
+
     def pack_tokens(self, tokens):
         tokens = tokens.contiguous()
         out = torch.empty(tokens.shape, device=self.device, dtype=torch.uint8)
