@@ -300,6 +300,22 @@ int32_t mmt_decode_self_attention(mmt_engine* e, int32_t layer, const float* d_x
 int32_t mmt_decode_cross_attention(mmt_engine* e, const mmt_decode_args* a, int32_t layer, const float* d_q, float* d_out,
                                    void* stream);
 
+/* Layer `layer` of encoder stack `stack` (0-4: encoder_1H / 13C / HSQC / COSY / IR, 16 heads; 5: encoder_cross, n_heads_cross
+ * heads), stand-alone, with the code the encoder runs: encoder_layer_bf16 (tcgen05 projections on the two-term weights, the
+ * fused FFN) or encoder_layer_fp32, and the encoder attention kernel the engine's MMT_NO_TC_ATTENTION / MMT_TC5_ATTENTION /
+ * MMT_TC_ATTENTION_FP32 knobs select.  d_x (rows,128) f32 input rows, B sequences in one of two layouts:
+ *   dense  (d_key_bias != NULL): rows == B*S, sequence b owns rows b*S .. b*S+S-1; d_key_bias (B,S) additive (-inf: not a
+ *          key; float masks: 0 / +1.0); the keys are compacted as the dense encoder does; row_start .. kstride ignored.
+ *   ragged (d_key_bias == NULL): sequence b owns rows row_start[b] .. row_start[b]+cnt[b]-1 (cnt[b] <= S) and attends, with
+ *          bias 0, the nk[b] rows kidx[b*kstride + j] (j < nk[b], row numbers relative to row_start[b]); all int32 on the
+ *          device.  The attention CTAs are sized by max nk and max cnt, as the ragged encoder sizes them.
+ * Outputs (rows,128) f32: d_qkv (rows,384, optional) the QKV projection the attention reads, d_att (optional) the attention
+ * output before out_proj (widened from bf16 in the bf16 mode), d_out the layer output after norm2. */
+int32_t mmt_encoder_layer(mmt_engine* e, int32_t stack, int32_t layer, const float* d_x, int64_t rows, int32_t B, int32_t S,
+                          const float* d_key_bias, const int32_t* d_row_start, const int32_t* d_cnt, const int32_t* d_kidx,
+                          const int32_t* d_nk, int32_t kstride, int32_t precision, float* d_qkv, float* d_att, float* d_out,
+                          void* stream);
+
 /* launches issued by this engine since creation (bench.py's gpu_launches). */
 int64_t mmt_launch_count(const mmt_engine* e);
 

@@ -2134,6 +2134,86 @@ int32_t mmt_decode_cross_attention(mmt_engine* e, const mmt_decode_args* a, int3
     return 0;
 }
 
+int32_t mmt_encoder_layer(mmt_engine* e, int32_t stack, int32_t layer, const float* d_x, int64_t rows, int32_t B, int32_t S,
+                          const float* d_key_bias, const int32_t* d_row_start, const int32_t* d_cnt, const int32_t* d_kidx,
+                          const int32_t* d_nk, int32_t kstride, int32_t precision, float* d_qkv, float* d_att, float* d_out,
+                          void* stream) {
+    if (!e || !d_x || !d_out) MMT_FAIL("null argument");
+    const mmt_model_desc& d = e->desc;
+    if (stack < 0 || stack > 5) MMT_FAIL("mmt_encoder_layer: stack must be in [0, 5]");
+    if (layer < 0 || layer >= d.n_enc_layers) MMT_FAIL("mmt_encoder_layer: layer out of range");
+    if (B <= 0 || B > 65535 || S <= 0 || rows <= 0 || rows > 0x7fffffff) MMT_FAIL("mmt_encoder_layer: empty or oversized batch");
+    if (precision != MMT_PREC_FP32 && precision != MMT_PREC_BF16) MMT_FAIL("bad precision");
+    const bool ragged = d_key_bias == nullptr;
+    if (ragged && (!d_row_start || !d_cnt || !d_kidx || !d_nk || kstride <= 0)) MMT_FAIL("mmt_encoder_layer: the ragged layout needs row_start, cnt, kidx, nk and kstride");
+    if (!ragged && rows != (int64_t)B * S) MMT_FAIL("mmt_encoder_layer: the dense layout has B * S rows");
+    const bool bf16 = precision == MMT_PREC_BF16;
+    const int heads = stack == 5 ? d.n_heads_cross : d.n_heads;
+    cudaStream_t s = (cudaStream_t)stream;
+    EngineCall call(e, s);
+    // the ragged encoder sizes its attention CTAs by the actual per-sequence maxima (encode_chunk_compact reads them back
+    // from the index kernels); the dense one by S (max_keys = max_rows = 0)
+    int max_keys = 0, max_rows = 0;
+    if (ragged) {
+        std::vector<int32_t> nk(B), cnt(B), rs(B);
+        MMT_CUDA(cudaMemcpyAsync(nk.data(), d_nk, B * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        MMT_CUDA(cudaMemcpyAsync(cnt.data(), d_cnt, B * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        MMT_CUDA(cudaMemcpyAsync(rs.data(), d_row_start, B * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        MMT_CUDA(cudaStreamSynchronize(s));
+        for (int b = 0; b < B; ++b) {
+            if (nk[b] < 1 || nk[b] > kstride || cnt[b] < 1 || cnt[b] > S || nk[b] > cnt[b] || rs[b] < 0 || rs[b] + (int64_t)cnt[b] > rows)
+                MMT_FAIL("mmt_encoder_layer: ragged sequence " + std::to_string(b) + " out of range");
+            max_keys = std::max(max_keys, (int)nk[b]); max_rows = std::max(max_rows, (int)cnt[b]);
+        }
+    }
+    Arena a;
+    float *X, *QKV, *ATT = nullptr, *PART = nullptr, *H = nullptr;
+    __nv_bfloat16 *X16 = nullptr, *ATT16 = nullptr;
+    int *kidx = nullptr, *nkd = nullptr;
+    auto plan = [&]() {
+        X = a.get<float>((size_t)rows * D);
+        QKV = a.get<float>((size_t)rows * 3 * D);
+        if (bf16) { X16 = a.get<__nv_bfloat16>((size_t)rows * D); ATT16 = a.get<__nv_bfloat16>((size_t)rows * D); }
+        else { ATT = a.get<float>((size_t)rows * D); PART = a.get<float>((size_t)rows * D); H = a.get<float>((size_t)rows * d.d_ff); }
+        if (!ragged) { kidx = a.get<int>((size_t)B * S); nkd = a.get<int>(B); }
+    };
+    a.plan = true; plan();
+    MMT_TRY(ensure_arena(e, a.off));
+    a.plan = false; a.base = e->arena; a.cap = e->arena_bytes; a.off = 0; plan();
+    MMT_CUDA(cudaMemcpyAsync(X, d_x, (size_t)rows * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    EncGroupRun g;
+    memset(&g, 0, sizeof(g));
+    g.X = X; g.rows = (int)rows; g.S = S; g.w = &e->enc[stack][layer];
+    g.qkv = QKV; g.att = ATT; g.part = PART; g.h = H; g.x16 = X16; g.att16 = ATT16;
+    if (ragged) {
+        g.kidx = d_kidx; g.nk = d_nk; g.row_start = d_row_start; g.cnt = d_cnt; g.kstride = kstride;
+        g.max_keys = max_keys; g.max_rows = max_rows;
+    } else {   // key compaction of the dense encoder (encode_chunk)
+        g.kbias = d_key_bias; g.kidx = kidx; g.nk = nkd;
+        KeyIndexParams p;
+        memset(&p, 0, sizeof(p));
+        p.g[0].kbias = d_key_bias; p.g[0].kidx = kidx; p.g[0].nk = nkd; p.g[0].S = S; p.B = B;
+        prof_pre(e, s);
+        build_key_index<<<dim3(B, 1), 32, 0, s>>>(p);
+        MMT_TRY(check_launch(e, "build_key_index", s));
+    }
+    if (bf16) {
+        prof_pre(e, s);
+        pack_rows_bf16<<<(unsigned)((rows + 7) / 8), 256, 0, s>>>(X, nullptr, D, rows, X16);
+        MMT_TRY(check_launch(e, "pack_rows_bf16", s));
+        MMT_TRY(encoder_layer_bf16(e, &g, 1, B, heads, d.d_ff, s));
+    } else MMT_TRY(encoder_layer_fp32(e, &g, 1, B, heads, d.d_ff, s));
+    if (d_qkv) MMT_CUDA(cudaMemcpyAsync(d_qkv, QKV, (size_t)rows * 3 * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    if (d_att) {
+        if (bf16) {
+            bf16_to_f32<<<(unsigned)((rows * D + 255) / 256), 256, 0, s>>>(ATT16, rows * D, d_att);
+            MMT_TRY(check_launch(e, "bf16_to_f32", s));
+        } else MMT_CUDA(cudaMemcpyAsync(d_att, ATT, (size_t)rows * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    }
+    MMT_CUDA(cudaMemcpyAsync(d_out, X, (size_t)rows * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    return 0;
+}
+
 int64_t mmt_launch_count(const mmt_engine* e) { return e ? e->launches : 0; }
 
 int32_t mmt_profile_enable(mmt_engine* e, int32_t on) {

@@ -360,6 +360,35 @@ class Engine:
             t.record_stream(torch.cuda.current_stream(self.dev_index))
         return out
 
+    def encoder_layer(self, stack, layer, x, *, key_bias=None, row_start=None, cnt=None, kidx=None, nk=None, S=None,
+                      precision="bf16"):
+        """Layer ``layer`` of encoder stack ``stack`` (0-4 the modality stacks, 5 encoder_cross) on the rows x (R,128),
+        through the encoder's own layer code and attention kernel (test hook).  Dense layout: key_bias (B,S) additive, x
+        holds B*S rows.  Ragged layout: row_start / cnt / nk (B,) and kidx (B,kstride) int, sequence b owns rows
+        row_start[b] .. + cnt[b] - 1 and attends rows row_start[b] + kidx[b, :nk[b]] (S: bound of cnt, default max cnt).
+        -> (qkv (R,384), attention output before out_proj (R,128), layer output after norm2 (R,128)), f32."""
+        x = x.to(self.device, torch.float32).contiguous()
+        R = x.shape[0]
+        keep = [x]
+        if key_bias is not None:
+            key_bias = key_bias.to(self.device, torch.float32).contiguous()
+            B, S = key_bias.shape
+            ptrs, kstride = [key_bias.data_ptr(), None, None, None, None], 0
+            keep.append(key_bias)
+        else:
+            ints = [t.to(self.device, torch.int32).contiguous() for t in (row_start, cnt, kidx, nk)]
+            keep += ints
+            B, kstride = ints[2].shape
+            S = S or int(ints[1].max())
+            ptrs = [None] + [t.data_ptr() for t in ints]
+        qkv = torch.empty(R, 3 * self.desc.d_model, device=self.device, dtype=torch.float32)
+        att, out = torch.empty_like(x), torch.empty_like(x)
+        _lib.check(self.L.mmt_encoder_layer(self.h, stack, layer, x.data_ptr(), R, B, S, *ptrs, kstride, _PREC[precision],
+                                            qkv.data_ptr(), att.data_ptr(), out.data_ptr(), self._stream()))
+        for t in keep:
+            t.record_stream(torch.cuda.current_stream(self.dev_index))
+        return qkv, att, out
+
     def pack_tokens(self, tokens):
         tokens = tokens.contiguous()
         out = torch.empty(tokens.shape, device=self.device, dtype=torch.uint8)

@@ -113,6 +113,8 @@ def _mha(P, prefix, nhead, x_q, x_kv, attn_bias):
     k = k.reshape(Tk, B, nhead, dh).permute(1, 2, 0, 3)
     v = v.reshape(Tk, B, nhead, dh).permute(1, 2, 0, 3)
     if attn_bias is not None:
+        # in q's dtype: torch's CPU SDPA returns wrong values, without an error, for float64 q/k/v with a float32 mask
+        attn_bias = attn_bias.to(q.dtype)
         attn_bias = attn_bias.expand(B, nhead, Tq, Tk) if attn_bias.dim() == 4 else attn_bias
     if FUSED_SDPA:
         # what the reference executes: torch's fused scaled_dot_product_attention (float additive mask)
@@ -186,17 +188,18 @@ def causal_bias(T, device):
 def encode(P, data, config):
     """validate_generate_MMT_v15_4.py:95-267 / models_MMT_v15_4.py:803-953.
 
-    Returns (memory (S,B,D) f32, src_padding_mask (B,S) bool-or-float,
+    Computes in the dtype of the weights (fp32 as the reference; float64 weights give the fp64 oracle).
+    Returns (memory (S,B,D), src_padding_mask (B,S) bool-or-float,
     fingerprint (B,512), embedding_src (S,B,D))."""
     mode = config.training_mode
-    dev = P["fc_out.weight"].device
+    dev, dt = P["fc_out.weight"].device, P["fc_out.weight"].dtype
     g = lambda k: data[k].to(dev)
     nL, H = config.num_encoder_layers, config.num_heads
     B = None
     emb, msk = {}, {}
     for m in ("1H", "13C", "HSQC", "COSY"):
         if m in mode:                                                  # :733-759
-            x = g(f"src_{m}")
+            x = g(f"src_{m}").to(dt)
             if m == "13C":
                 x = x.unsqueeze(-1)
             W, b = P[_EMBED_KEYS[m] + ".weight"], P[_EMBED_KEYS[m] + ".bias"]
@@ -205,7 +208,7 @@ def encode(P, data, config):
             msk[m] = g(f"mask_{m}").to(torch.bool)
             B = e.shape[0]
     if "IR" in mode:                                                   # :761-767, :827-828
-        x = g("src_IR").float()
+        x = g("src_IR").to(dt)
         e = F.relu(F.linear(x, P[_EMBED_KEYS["IR"] + ".weight"], P[_EMBED_KEYS["IR"] + ".bias"]))
         emb["IR"] = e.unsqueeze(0)
         msk["IR"] = torch.zeros(e.shape[0], 1, dtype=torch.bool, device=dev)
@@ -217,7 +220,7 @@ def encode(P, data, config):
         e = F.relu(F.embedding(g("src_MS"), P["linear_embedding_MS.embedding.weight"]))
         extra.append((e.permute(1, 0, 2), g("mask_MS")))
     if "MW" in mode:                                                   # :787-792, :804, :830-831
-        mw = g("trg_MW").float().unsqueeze(1)
+        mw = g("trg_MW").to(dt).unsqueeze(1)
         e = F.relu(F.linear(mw, P["linear_embedding_MW.linear_spec_embedding_MW.weight"],
                             P["linear_embedding_MW.linear_spec_embedding_MW.bias"]))
         extra.append((e.unsqueeze(0), torch.zeros(mw.shape[0], 1, dtype=torch.bool, device=dev)))
@@ -234,8 +237,8 @@ def encode(P, data, config):
             masks.append(k)
         else:                                                          # :850-858 ... :931-939
             n = {"COSY": 65, "IR": fdim_ir}.get(m, fdim)
-            mems.append(torch.zeros(n, B, D, device=dev))
-            embs.append(torch.zeros(n, B, D, device=dev))
+            mems.append(torch.zeros(n, B, D, device=dev, dtype=dt))
+            embs.append(torch.zeros(n, B, D, device=dev, dtype=dt))
             if m == "IR":
                 masks.append(torch.zeros(B, n, dtype=torch.bool, device=dev))
             else:
