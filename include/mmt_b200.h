@@ -300,6 +300,19 @@ int32_t mmt_decode_self_attention(mmt_engine* e, int32_t layer, const float* d_x
 int32_t mmt_decode_cross_attention(mmt_engine* e, const mmt_decode_args* a, int32_t layer, const float* d_q, float* d_out,
                                    void* stream);
 
+/* The rest of one decoder layer of the un-fused decode step after its two attentions, stand-alone, with the code the step
+ * runs: R sequences in one wave, the variants chosen as the step chooses them (from R and the engine's MMT_NO_GEMM_CHAIN,
+ * MMT_NO_FFN_PROLOGUE, MMT_DEC_PROJ_TWO_TERM and MMT_DEC_FFN_TWO_TERM knobs).  Inputs (R,128) f32: d_x the layer's input
+ * rows (the fp32 residual), d_att_self / d_att_cross the self- and cross-attention outputs before their out_proj (rounded
+ * to bf16 in the bf16 mode, as the step stores them).  Outputs (R,128) f32:
+ *   d_x1  = norm1(x + out_proj(att_self)),
+ *   d_qc  = the cross-attention query projection of x1,
+ *   d_x2  = norm2(x1 + ca_out_proj(att_cross)) -- optional (may be NULL), and written only where the step stores it: not
+ *           when the FFN kernel's prologue computes it (bf16 mode, R >= 2048, no MMT_NO_FFN_PROLOGUE),
+ *   d_out = norm3(x2 + FFN(x2)), the layer's output. */
+int32_t mmt_decode_layer_tail(mmt_engine* e, int32_t layer, const float* d_x, const float* d_att_self, const float* d_att_cross,
+                              int64_t R, int32_t precision, float* d_x1, float* d_qc, float* d_x2, float* d_out, void* stream);
+
 /* Layer `layer` of encoder stack `stack` (0-4: encoder_1H / 13C / HSQC / COSY / IR, 16 heads; 5: encoder_cross, n_heads_cross
  * heads), stand-alone, with the code the encoder runs: encoder_layer_bf16 (tcgen05 projections on the two-term weights, the
  * fused FFN) or encoder_layer_fp32, and the encoder attention kernel the engine's MMT_NO_TC_ATTENTION / MMT_TC5_ATTENTION /

@@ -25,7 +25,7 @@ EXPORTS = [
     "mmt_weight_offset", "mmt_weight_total", "mmt_create", "mmt_destroy", "mmt_memory_len",
     "mmt_mask_is_float", "mmt_encode", "mmt_spectra_equal", "mmt_decode", "mmt_teacher_forced", "mmt_teacher_forced_scores", "mmt_beam_search", "mmt_philox_increment",
     "mmt_pack_tokens_u8", "mmt_unpack_tokens_u8", "mmt_pack_tokens_u8_seqmajor", "mmt_unpack_tokens_u8_seqmajor", "mmt_first_eos", "mmt_ingest_peaks", "mmt_ingest_ir", "mmt_sample", "mmt_exponential", "mmt_sample_probs", "mmt_linear", "mmt_ffn",
-    "mmt_decode_self_attention", "mmt_decode_cross_attention", "mmt_encoder_layer", "mmt_launch_count",
+    "mmt_decode_self_attention", "mmt_decode_cross_attention", "mmt_decode_layer_tail", "mmt_encoder_layer", "mmt_launch_count",
     "mmt_profile_enable", "mmt_profile_report",
 ]
 
@@ -171,6 +171,7 @@ def lib():
     L.mmt_ffn.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, i32, i32, i32, vp]; L.mmt_ffn.restype = i32
     L.mmt_decode_self_attention.argtypes = [vp, i32, vp, i64, i32, i32, vp, vp]; L.mmt_decode_self_attention.restype = i32
     L.mmt_decode_cross_attention.argtypes = [vp, C.POINTER(DecodeArgs), i32, vp, vp, vp]; L.mmt_decode_cross_attention.restype = i32
+    L.mmt_decode_layer_tail.argtypes = [vp, i32, vp, vp, vp, i64, i32, vp, vp, vp, vp, vp]; L.mmt_decode_layer_tail.restype = i32
     L.mmt_encoder_layer.argtypes = [vp, i32, i32, vp, i64, i32, i32, vp, vp, vp, vp, vp, i32, i32, vp, vp, vp, vp]
     L.mmt_encoder_layer.restype = i32
     L.mmt_launch_count.argtypes = [vp]; L.mmt_launch_count.restype = i64

@@ -1069,6 +1069,122 @@ static int decode_cross_attention_layer(mmt_engine* e, const mmt_decode_args& a,
     return check_launch(e, "decode_cross_attention", s);
 }
 
+// Launches of the decode step over the Nw rows of one wave; the residual stream is b.x (fp32) with its bf16 copy b.x16.
+struct DecOps {
+    mmt_engine* e; const DecBuffers& b; int64_t Nw; bool pdl_u; cudaStream_t s;
+    // x = LN(x + bias + sum_s part[s]) (separate kernel; fp32 mode and split-K FFN2)
+    int ln(const float* part, int splits, const float* bias, const float* gamma, const float* beta) const {
+        LnParams q;
+        memset(&q, 0, sizeof(q));
+        q.splits = splits; q.part_stride = Nw * D; q.eps = 1e-5f;
+        LnGroup& g = q.g[0];
+        g.part = part; g.bias = bias; g.res = b.x; g.gamma = gamma; g.beta = beta; g.out = b.x; g.out_bf16 = b.x16; g.M = (int)Nw;
+        g.S_in = (int)Nw; g.stride_b = 0; g.stride_s = 1; g.off = 0;
+        return launch_ln(e, q, 1, (int)Nw, s);
+    }
+    int gemm(const float* A, int64_t lda, const float* W, const float* bias, float* C, int N, int K, int act, int splits) const {
+        GemmParams p = gemm_params(N, K, N, act);
+        p.g[0].A = A; p.g[0].lda = lda; p.g[0].W = W; p.g[0].bias = bias; p.g[0].C = C; p.g[0].M = (int)Nw;
+        p.splits = splits; p.part_stride = Nw * D;
+        return launch_gemm(e, p, 1, (int)Nw, s);
+    }
+    // The four attention projections of the un-fused step run on the hi term of the bf16 weight split alone, like the small-wave
+    // kernel's (decode_attn keeps only the hi terms in shared memory): one weight slab per stage -> 68 KB instead of 100 KB of
+    // shared memory per CTA (three resident tiles per SM instead of two), half the weight TMA bytes and MMAs.  At every wave
+    // size, so that a shard decoded alone reproduces its rows of the full call bit for bit.  Measured on the golden cases:
+    // worst logit error 6.37e-3 -> 6.20e-3 of the row scale, mean +12 % (profiles/r02_bf16_error_dec_proj_terms.txt).
+    // MMT_DEC_PROJ_TWO_TERM=1 restores both terms.
+    const __nv_bfloat16* plo(const float* w) const { return e->dec_proj_single ? nullptr : e->Wlo(w); }
+    // The decoder FFN runs on the hi term of the bf16 weight split alone: measured on the 12 golden cases the lo term changes
+    // the worst logit error from 5.75e-3 to 5.76e-3 of the row scale (profiles/r02_bf16_error.md) for twice the tensor work.
+    // MMT_DEC_FFN_TWO_TERM=1 restores it.
+    const __nv_bfloat16* dlo(const float* w) const { return e->dec_ffn_single ? nullptr : e->Wlo(w); }
+    // tensor-core variants: plain projection (fp32 or bf16 out) and projection + residual + LN in place on x / x16
+    int tc(const __nv_bfloat16* A, int64_t lda, const float* W, const float* bias, float* C32, __nv_bfloat16* C16, int N, int K, int act, int splits) const {
+        TcGemmParams p = tc_params((int)Nw, N, K);
+        p.bias = bias; p.act = act; p.out_f32 = C32; p.ld_f32 = N; p.out_b16 = C16; p.ld_b16 = N;
+        p.splits = splits; p.part_stride = Nw * D;
+        return launch_tc(e, p, A, lda, e->Wb(W), TC_EPI_STORE, s, plo(W), pdl_u);
+    }
+    int tc_ln(const __nv_bfloat16* A, int64_t lda, const float* W, const float* bias, int K, const float* gamma, const float* beta,
+              const TcChain* chain = nullptr) const {
+        TcGemmParams p = tc_params((int)Nw, D, K);
+        p.bias = bias; p.res = b.x; p.gamma = gamma; p.beta = beta;
+        p.out_f32 = b.x; p.ld_f32 = D; p.out_b16 = b.x16; p.ld_b16 = D;
+        return launch_tc(e, p, A, lda, e->Wb(W), TC_EPI_LN, s, plo(W), pdl_u, chain);
+    }
+};
+
+// Un-fused step, one decoder layer after its self-attention (att16 | att): x = norm1(x + out_proj(att)), then the
+// cross-attention query projection of x -> qc.  decode_step and the unit hook mmt_decode_layer_tail both run this.
+static int decode_self_tail_layer(const DecOps& o, const LayerW& w, bool bf16) {
+    const DecBuffers& b = o.b;
+    if (bf16) {
+        // out-proj + LN1 and the cross-attention query projection as one launch -- for waves up to 24,576 rows: the chained
+        // kernel holds 192 KB of shared memory (one CTA per SM instead of three), which costs more than the saved launch
+        // once there are several tiles per SM (measured: 1383 -> 1357 us per position at 16,384 rows, 4851 -> 4901 at 65,536)
+        if (o.e->use_gemm_chain && o.Nw <= 24576) {
+            const TcChain ch{o.e->Wb(w.ca_in_w), o.plo(w.ca_in_w), w.ca_in_b, b.qc, D};
+            MMT_TRY(o.tc_ln(b.att16, D, w.out_w, w.out_b, D, w.n1_w, w.n1_b, &ch));
+        } else {
+            MMT_TRY(o.tc_ln(b.att16, D, w.out_w, w.out_b, D, w.n1_w, w.n1_b));
+            MMT_TRY(o.tc(b.x16, D, w.ca_in_w, w.ca_in_b, b.qc, nullptr, D, D, 0, 1));
+        }
+    } else {
+        MMT_TRY(o.gemm(b.att, D, w.out_w, nullptr, b.part, D, D, 0, 1));
+        MMT_TRY(o.ln(b.part, 1, w.out_b, w.n1_w, w.n1_b));
+        MMT_TRY(o.gemm(b.x, D, w.ca_in_w, w.ca_in_b, b.qc, D, D, 0, 1));
+    }
+    return 0;
+}
+
+// Un-fused step, layer l after its cross attention (att16 | att): x = norm2(x + ca_out_proj(att)), then
+// x = norm3(x + FFN(x)).  x2 (unit hook only; decode_step passes nullptr): receives x after norm2 where the variant stores it,
+// i.e. not with the FFN prologue, which keeps it inside the FFN kernel.  decode_step and mmt_decode_layer_tail both run this.
+static int decode_cross_tail_layer(const DecOps& o, const LayerW& w, int l, bool bf16, float* x2 = nullptr) {
+    mmt_engine* e = o.e;
+    const DecBuffers& b = o.b;
+    const int M = (int)o.Nw, F = e->desc.d_ff;
+    cudaStream_t s = o.s;
+    auto keep_x2 = [&]() -> int {
+        if (x2) MMT_CUDA(cudaMemcpyAsync(x2, b.x, (size_t)M * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+        return 0;
+    };
+    if (bf16) {
+        const bool ffn_pro = e->use_ffn_prologue && M >= 2048;     // cross-attention out-projection + norm2 as the FFN kernel's prologue
+        if (!ffn_pro) { MMT_TRY(o.tc_ln(b.att16, D, w.ca_out_w, w.ca_out_b, D, w.n2_w, w.n2_b)); MMT_TRY(keep_x2()); }
+        if (M >= 2048) {
+            FfnParams f = ffn_params(M, F);
+            f.b1 = w.l1_b; f.bias = w.l2_b; f.res = b.x; f.gamma = w.n3_w; f.beta = w.n3_b; f.out_f32 = b.x; f.out_b16 = b.x16;
+            if (getenv("MMT_FFN_DEBUG")) {     // phase stamps of the layer-3 FFN launch (printed by run_decode)
+                if (!e->ffn_dbg) { MMT_CUDA(cudaMallocManaged(&e->ffn_dbg, 4096 * 16 * sizeof(long long))); memset(e->ffn_dbg, 0, 4096 * 16 * sizeof(long long)); }
+                f.dbg = l == 3 ? e->ffn_dbg : nullptr;
+            }
+            if (ffn_pro) {
+                const FfnPro pr{e->Wb(w.ca_out_w), o.plo(w.ca_out_w), w.ca_out_b, w.n2_w, w.n2_b, b.x};
+                MMT_TRY(launch_ffn(e, f, b.att16, D, e->Wb(w.l1_w), o.dlo(w.l1_w), e->Wb(w.l2_w), o.dlo(w.l2_w), TC_EPI_LN, s, o.pdl_u, &pr));
+            } else
+            MMT_TRY(launch_ffn(e, f, b.x16, D, e->Wb(w.l1_w), o.dlo(w.l1_w), e->Wb(w.l2_w), o.dlo(w.l2_w), TC_EPI_LN, s, o.pdl_u));
+        } else {   // few rows: split F over the grid, reduce the partials in the LayerNorm kernel
+            FfnParams f = ffn_params(M, F);
+            f.b1 = w.l1_b; f.splits = MAX_SPLITS; f.out_f32 = b.part; f.part_stride = o.Nw * D;
+            if ((int64_t)f.splits * o.Nw > b.part_rows) MMT_FAIL("decode: FFN partial buffer too small for this wave (plan_decoder)");
+            MMT_TRY(launch_ffn(e, f, b.x16, D, e->Wb(w.l1_w), o.dlo(w.l1_w), e->Wb(w.l2_w), o.dlo(w.l2_w), TC_EPI_STORE, s, o.pdl_u));
+            MMT_TRY(o.ln(b.part, f.splits, w.l2_b, w.n3_w, w.n3_b));
+        }
+    } else {
+        MMT_TRY(o.gemm(b.att, D, w.ca_out_w, nullptr, b.part, D, D, 0, 1));
+        MMT_TRY(o.ln(b.part, 1, w.ca_out_b, w.n2_w, w.n2_b));
+        MMT_TRY(keep_x2());
+        MMT_TRY(o.gemm(b.x, D, w.l1_w, w.l1_b, b.h, F, D, 1, 1));
+        int splits = pick_splits(M, D, F);
+        if ((int64_t)splits * o.Nw > b.part_rows) MMT_FAIL("decode: FFN partial buffer too small for this wave (plan_decoder)");
+        MMT_TRY(o.gemm(b.h, F, w.l2_w, nullptr, b.part, D, F, 0, splits));
+        MMT_TRY(o.ln(b.part, splits, w.l2_b, w.n3_w, w.n3_b));
+    }
+    return 0;
+}
+
 static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw, int Bmw, DecBuffers& b, bool bf16, cudaStream_t s) {
     const mmt_model_desc& d = e->desc;
     const mmt_decode_args& a = *r.a;
@@ -1092,47 +1208,7 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
     // Only for moderate waves: measured 50.2 -> 45.2 ms for a beam search over 2560 slots, but 1426 -> 1473 us per position at
     // 16,384 sequences, where the early-scheduled CTAs take SM resources from a predecessor that is throughput-bound.
     const bool pdl_u = !fused && bf16 && e->use_pdl && !e->profiling && Nw <= e->pdl_rows;
-    // x = LN(x + bias + sum_s part[s]) (separate kernel; fp32 mode and split-K FFN2)
-    auto ln = [&](const float* part, int splits, const float* bias, const float* gamma, const float* beta) -> int {
-        LnParams q;
-        memset(&q, 0, sizeof(q));
-        q.splits = splits; q.part_stride = Nw * D; q.eps = 1e-5f;
-        LnGroup& g = q.g[0];
-        g.part = part; g.bias = bias; g.res = b.x; g.gamma = gamma; g.beta = beta; g.out = b.x; g.out_bf16 = b.x16; g.M = M;
-        g.S_in = M; g.stride_b = 0; g.stride_s = 1; g.off = 0;
-        return launch_ln(e, q, 1, M, s);
-    };
-    auto gemm = [&](const float* A, int64_t lda, const float* W, const float* bias, float* C, int N, int K, int act, int splits) -> int {
-        GemmParams p = gemm_params(N, K, N, act);
-        p.g[0].A = A; p.g[0].lda = lda; p.g[0].W = W; p.g[0].bias = bias; p.g[0].C = C; p.g[0].M = M;
-        p.splits = splits; p.part_stride = Nw * D;
-        return launch_gemm(e, p, 1, M, s);
-    };
-    // The four attention projections of the un-fused step run on the hi term of the bf16 weight split alone, like the small-wave
-    // kernel's (decode_attn keeps only the hi terms in shared memory): one weight slab per stage -> 68 KB instead of 100 KB of
-    // shared memory per CTA (three resident tiles per SM instead of two), half the weight TMA bytes and MMAs.  At every wave
-    // size, so that a shard decoded alone reproduces its rows of the full call bit for bit.  Measured on the golden cases:
-    // worst logit error 6.37e-3 -> 6.20e-3 of the row scale, mean +12 % (profiles/r02_bf16_error_dec_proj_terms.txt).
-    // MMT_DEC_PROJ_TWO_TERM=1 restores both terms.
-    auto plo = [&](const float* w) -> const __nv_bfloat16* { return e->dec_proj_single ? nullptr : e->Wlo(w); };
-    // tensor-core variants: plain projection (fp32 or bf16 out) and projection + residual + LN in place on x / x16
-    auto tc = [&](const __nv_bfloat16* A, int64_t lda, const float* W, const float* bias, float* C32, __nv_bfloat16* C16, int N, int K, int act, int splits) -> int {
-        TcGemmParams p = tc_params(M, N, K);
-        p.bias = bias; p.act = act; p.out_f32 = C32; p.ld_f32 = N; p.out_b16 = C16; p.ld_b16 = N;
-        p.splits = splits; p.part_stride = Nw * D;
-        return launch_tc(e, p, A, lda, e->Wb(W), TC_EPI_STORE, s, plo(W), pdl_u);
-    };
-    auto tc_ln = [&](const __nv_bfloat16* A, int64_t lda, const float* W, const float* bias, int K, const float* gamma, const float* beta,
-                     const TcChain* chain = nullptr) -> int {
-        TcGemmParams p = tc_params(M, D, K);
-        p.bias = bias; p.res = b.x; p.gamma = gamma; p.beta = beta;
-        p.out_f32 = b.x; p.ld_f32 = D; p.out_b16 = b.x16; p.ld_b16 = D;
-        return launch_tc(e, p, A, lda, e->Wb(W), TC_EPI_LN, s, plo(W), pdl_u, chain);
-    };
-    // The decoder FFN runs on the hi term of the bf16 weight split alone: measured on the 12 golden cases the lo term changes
-    // the worst logit error from 5.75e-3 to 5.76e-3 of the row scale (profiles/r02_bf16_error.md) for twice the tensor work.
-    // MMT_DEC_FFN_TWO_TERM=1 restores it.
-    auto dlo = [&](const float* w) -> const __nv_bfloat16* { return e->dec_ffn_single ? nullptr : e->Wlo(w); };
+    const DecOps o{e, b, Nw, pdl_u, s};
     int ffn_splits = 1;
     if (fused) {
         if (dh != 8 || H != DA_H) MMT_FAIL("decoder must have 16 heads of dim 8");
@@ -1195,10 +1271,10 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
                 FfnParams f = ffn_params(M, d.d_ff);
                 f.b1 = w.l1_b; f.splits = ffn_splits; f.out_f32 = b.part; f.part_stride = Nw * D;
                 f.dbg = (e->da_dbg && l == 3) ? e->da_dbg + 2048 * 16 : nullptr;
-                MMT_TRY(launch_ffn(e, f, b.x16, D, e->Wb(w.l1_w), dlo(w.l1_w), e->Wb(w.l2_w), dlo(w.l2_w), TC_EPI_STORE, s, pdl));
+                MMT_TRY(launch_ffn(e, f, b.x16, D, e->Wb(w.l1_w), o.dlo(w.l1_w), e->Wb(w.l2_w), o.dlo(w.l2_w), TC_EPI_STORE, s, pdl));
             } else {
-                MMT_TRY(gemm(b.x, D, w.l1_w, w.l1_b, b.h, d.d_ff, D, 1, 1));
-                MMT_TRY(gemm(b.h, d.d_ff, w.l2_w, nullptr, b.part, D, d.d_ff, 0, ffn_splits));
+                MMT_TRY(o.gemm(b.x, D, w.l1_w, w.l1_b, b.h, d.d_ff, D, 1, 1));
+                MMT_TRY(o.gemm(b.h, d.d_ff, w.l2_w, nullptr, b.part, D, d.d_ff, 0, ffn_splits));
             }
         }
     } else {
@@ -1212,54 +1288,9 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
             char* pool = b.kv_pool + (size_t)l * b.pool_pages * 2 * PAGE_TOKENS * D * b.kv_esz;
             const char* ckv = b.cross_kv + (size_t)l * 2 * R * D * b.kv_esz;
             MMT_TRY(decode_self_attention_layer(e, w, b, pool, pps, Nw, bf16, pdl_u, s));
-            if (bf16) {
-                // out-proj + LN1 and the cross-attention query projection as one launch -- for waves up to 24,576 rows: the chained
-                // kernel holds 192 KB of shared memory (one CTA per SM instead of three), which costs more than the saved launch
-                // once there are several tiles per SM (measured: 1383 -> 1357 us per position at 16,384 rows, 4851 -> 4901 at 65,536)
-                if (e->use_gemm_chain && Nw <= 24576) {
-                    const TcChain ch{e->Wb(w.ca_in_w), plo(w.ca_in_w), w.ca_in_b, b.qc, D};
-                    MMT_TRY(tc_ln(b.att16, D, w.out_w, w.out_b, D, w.n1_w, w.n1_b, &ch));
-                } else {
-                    MMT_TRY(tc_ln(b.att16, D, w.out_w, w.out_b, D, w.n1_w, w.n1_b));
-                    MMT_TRY(tc(b.x16, D, w.ca_in_w, w.ca_in_b, b.qc, nullptr, D, D, 0, 1));
-                }
-            } else {
-                MMT_TRY(gemm(b.att, D, w.out_w, nullptr, b.part, D, D, 0, 1));
-                MMT_TRY(ln(b.part, 1, w.out_b, w.n1_w, w.n1_b));
-                MMT_TRY(gemm(b.x, D, w.ca_in_w, w.ca_in_b, b.qc, D, D, 0, 1));
-            }
+            MMT_TRY(decode_self_tail_layer(o, w, bf16));
             MMT_TRY(decode_cross_attention_layer(e, a, b, ckv, Nw, Bmw, bf16, pdl_u, s));
-            if (bf16) {
-                const bool ffn_pro = e->use_ffn_prologue && M >= 2048;     // cross-attention out-projection + norm2 as the FFN kernel's prologue
-                if (!ffn_pro) MMT_TRY(tc_ln(b.att16, D, w.ca_out_w, w.ca_out_b, D, w.n2_w, w.n2_b));
-                if (M >= 2048) {
-                    FfnParams f = ffn_params(M, d.d_ff);
-                    f.b1 = w.l1_b; f.bias = w.l2_b; f.res = b.x; f.gamma = w.n3_w; f.beta = w.n3_b; f.out_f32 = b.x; f.out_b16 = b.x16;
-                    if (getenv("MMT_FFN_DEBUG")) {     // phase stamps of the layer-3 FFN launch (printed by run_decode)
-                        if (!e->ffn_dbg) { MMT_CUDA(cudaMallocManaged(&e->ffn_dbg, 4096 * 16 * sizeof(long long))); memset(e->ffn_dbg, 0, 4096 * 16 * sizeof(long long)); }
-                        f.dbg = l == 3 ? e->ffn_dbg : nullptr;
-                    }
-                    if (ffn_pro) {
-                        const FfnPro pr{e->Wb(w.ca_out_w), plo(w.ca_out_w), w.ca_out_b, w.n2_w, w.n2_b, b.x};
-                        MMT_TRY(launch_ffn(e, f, b.att16, D, e->Wb(w.l1_w), dlo(w.l1_w), e->Wb(w.l2_w), dlo(w.l2_w), TC_EPI_LN, s, pdl_u, &pr));
-                    } else
-                    MMT_TRY(launch_ffn(e, f, b.x16, D, e->Wb(w.l1_w), dlo(w.l1_w), e->Wb(w.l2_w), dlo(w.l2_w), TC_EPI_LN, s, pdl_u));
-                } else {   // few rows: split F over the grid, reduce the partials in the LayerNorm kernel
-                    FfnParams f = ffn_params(M, d.d_ff);
-                    f.b1 = w.l1_b; f.splits = MAX_SPLITS; f.out_f32 = b.part; f.part_stride = Nw * D;
-                    if ((int64_t)f.splits * Nw > b.part_rows) MMT_FAIL("decode: FFN partial buffer too small for this wave (plan_decoder)");
-                    MMT_TRY(launch_ffn(e, f, b.x16, D, e->Wb(w.l1_w), dlo(w.l1_w), e->Wb(w.l2_w), dlo(w.l2_w), TC_EPI_STORE, s, pdl_u));
-                    MMT_TRY(ln(b.part, f.splits, w.l2_b, w.n3_w, w.n3_b));
-                }
-            } else {
-                MMT_TRY(gemm(b.att, D, w.ca_out_w, nullptr, b.part, D, D, 0, 1));
-                MMT_TRY(ln(b.part, 1, w.ca_out_b, w.n2_w, w.n2_b));
-                MMT_TRY(gemm(b.x, D, w.l1_w, w.l1_b, b.h, d.d_ff, D, 1, 1));
-                int splits = pick_splits(M, D, d.d_ff);
-                if ((int64_t)splits * Nw > b.part_rows) MMT_FAIL("decode: FFN partial buffer too small for this wave (plan_decoder)");
-                MMT_TRY(gemm(b.h, d.d_ff, w.l2_w, nullptr, b.part, D, d.d_ff, 0, splits));
-                MMT_TRY(ln(b.part, splits, w.l2_b, w.n3_w, w.n3_b));
-            }
+            MMT_TRY(decode_cross_tail_layer(o, w, l, bf16));
         }
     }
     SampleParams sp;
@@ -2131,6 +2162,50 @@ int32_t mmt_decode_cross_attention(mmt_engine* e, const mmt_decode_args* a, int3
         return check_launch(e, "bf16_to_f32", s);
     }
     MMT_CUDA(cudaMemcpyAsync(d_out, b.att, (size_t)N * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    return 0;
+}
+
+int32_t mmt_decode_layer_tail(mmt_engine* e, int32_t layer, const float* d_x, const float* d_att_self, const float* d_att_cross,
+                              int64_t R, int32_t precision, float* d_x1, float* d_qc, float* d_x2, float* d_out, void* stream) {
+    if (!e || !d_x || !d_att_self || !d_att_cross || !d_x1 || !d_qc || !d_out) MMT_FAIL("null argument");
+    const mmt_model_desc& d = e->desc;
+    if (layer < 0 || layer >= d.n_dec_layers) MMT_FAIL("mmt_decode_layer_tail: layer out of range");
+    if (R <= 0 || R > 0x7fffffff) MMT_FAIL("mmt_decode_layer_tail: R must be in [1, 2^31)");
+    if (precision != MMT_PREC_FP32 && precision != MMT_PREC_BF16) MMT_FAIL("bad precision");
+    const bool bf16 = precision == MMT_PREC_BF16;
+    cudaStream_t s = (cudaStream_t)stream;
+    EngineCall call(e, s);
+    // the buffers of a one-layer decode wave of R sequences, planned like run_decode's
+    mmt_model_desc d1 = d;
+    d1.n_dec_layers = 1;
+    Arena ar;
+    DecBuffers b;
+    plan_decoder(ar, d1, R, 1, 1, 1, b, bf16, e->fused_decode_rows);
+    MMT_TRY(ensure_arena(e, ar.off));
+    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
+    plan_decoder(ar, d1, R, 1, 1, 1, b, bf16, e->fused_decode_rows);
+    const int64_t n_el = R * D;
+    const unsigned blocks = (unsigned)((n_el + 255) / 256);
+    const size_t bytes = (size_t)n_el * sizeof(float);
+    // an attention output enters the step as att16 (bf16 mode) or att (fp32)
+    auto load_att = [&](const float* src) -> int {
+        if (bf16) {
+            f32_to_bf16<<<blocks, 256, 0, s>>>(src, n_el, b.att16);
+            return check_launch(e, "f32_to_bf16", s);
+        }
+        MMT_CUDA(cudaMemcpyAsync(b.att, src, bytes, cudaMemcpyDeviceToDevice, s));
+        return 0;
+    };
+    const DecOps o{e, b, R, false, s};
+    const LayerW& w = e->dec[layer];
+    MMT_CUDA(cudaMemcpyAsync(b.x, d_x, bytes, cudaMemcpyDeviceToDevice, s));
+    MMT_TRY(load_att(d_att_self));
+    MMT_TRY(decode_self_tail_layer(o, w, bf16));
+    MMT_CUDA(cudaMemcpyAsync(d_x1, b.x, bytes, cudaMemcpyDeviceToDevice, s));
+    MMT_CUDA(cudaMemcpyAsync(d_qc, b.qc, bytes, cudaMemcpyDeviceToDevice, s));
+    MMT_TRY(load_att(d_att_cross));
+    MMT_TRY(decode_cross_tail_layer(o, w, layer, bf16, d_x2));
+    MMT_CUDA(cudaMemcpyAsync(d_out, b.x, bytes, cudaMemcpyDeviceToDevice, s));
     return 0;
 }
 

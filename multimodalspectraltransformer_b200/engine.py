@@ -360,6 +360,25 @@ class Engine:
             t.record_stream(torch.cuda.current_stream(self.dev_index))
         return out
 
+    def decode_layer_tail(self, layer, x, att_self, att_cross, precision="bf16"):
+        """The rest of decoder layer ``layer`` of the un-fused decode step after its attentions, on R rows (test hook):
+        x, att_self, att_cross (R,128) -> (x1, qc, x2, out), f32 (R,128): x1 = norm1(x + out_proj(att_self)), qc its
+        cross-attention query, x2 = norm2(x1 + ca_out_proj(att_cross)), out = norm3(x2 + FFN(x2)).  x2 is None where the
+        step keeps it inside the FFN kernel (bf16, R >= 2048, FFN prologue on)."""
+        t = [v.to(self.device, torch.float32).contiguous() for v in (x, att_self, att_cross)]
+        R = t[0].shape[0]
+        if any(tuple(v.shape) != (R, self.desc.d_model) for v in t):
+            raise ValueError("x, att_self and att_cross must be (R, 128)")
+        x1, qc, out = (torch.empty_like(t[0]) for _ in range(3))
+        x2 = torch.full_like(t[0], float("nan"))
+        _lib.check(self.L.mmt_decode_layer_tail(self.h, layer, *[v.data_ptr() for v in t], R, _PREC[precision], x1.data_ptr(),
+                                                qc.data_ptr(), x2.data_ptr(), out.data_ptr(), self._stream()))
+        for v in t:
+            v.record_stream(torch.cuda.current_stream(self.dev_index))
+        if bool(torch.isnan(x2).all()):
+            x2 = None
+        return x1, qc, x2, out
+
     def encoder_layer(self, stack, layer, x, *, key_bias=None, row_start=None, cnt=None, kidx=None, nk=None, S=None,
                       precision="bf16"):
         """Layer ``layer`` of encoder stack ``stack`` (0-4 the modality stacks, 5 encoder_cross) on the rows x (R,128),

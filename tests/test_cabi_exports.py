@@ -38,6 +38,11 @@ def test_library_loads_and_weight_table_matches_reference_state_dict():
             numel *= s
         assert L.mmt_weight_numel(ctypes.byref(d), i) == numel
         assert L.mmt_weight_offset(ctypes.byref(d), i) % 64 == 0
+    # every weight has its own slot: sorted by offset, each ends before the next begins, the last within the total
+    slots = sorted((L.mmt_weight_offset(ctypes.byref(d), i), L.mmt_weight_numel(ctypes.byref(d), i), names[i]) for i in range(n))
+    for (o0, n0, a), (o1, _, b) in zip(slots, slots[1:]):
+        assert o0 >= 0 and o0 + n0 <= o1, (a, b)
+    assert slots[-1][0] + slots[-1][1] <= L.mmt_weight_total(ctypes.byref(d))
     assert L.mmt_memory_len(ctypes.byref(d), _lib.mode_bits("1H_13C_HSQC_COSY_IR_MF_MW")) == 582
     assert L.mmt_memory_len(ctypes.byref(d), _lib.mode_bits("HSQC_MF_MW")) == 518
     assert L.mmt_mask_is_float(_lib.mode_bits("HSQC_MF_MW")) == 1

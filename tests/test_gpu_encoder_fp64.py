@@ -22,6 +22,7 @@ import torch
 import torch.nn.functional as F
 
 from test_gpu_large_wave import SCALE as SCALE8, U16, _tolerance, bf16, outside
+from test_gpu_trained_weights import with_weights
 
 D = 128
 LAYER = {0: 1, 1: 4, 2: 2, 3: 5, 4: 3, 5: 3}      # which layer of each stack the kernel tests use
@@ -32,29 +33,19 @@ def _heads(stack):
     return 4 if stack == 5 else 16
 
 
-def _setup():
-    from test_gpu_parity import setup
-    return setup()
+def _engine(weights, **env):
+    from test_gpu_trained_weights import engine_with
+    return engine_with(weights, **env)
 
 
-_ENGINES = {}
-
-
-def _engine(**env):
-    key = tuple(sorted(env.items()))
-    if key not in _ENGINES:
-        from test_gpu_parity import _engine_with_env
-        _ENGINES[key] = _engine_with_env(**env)
-    return _ENGINES[key]
-
-
-def _layer_params(stack, layer, dev="cuda"):
-    sd = _setup()["model"].state_dict()
+def _layer_params(stack, layer, weights):
+    from test_gpu_trained_weights import state_dict_for
+    sd = state_dict_for(weights)
     p = f"{STACKS[stack]}.layers.{layer}."
     names = ("self_attn.in_proj_weight", "self_attn.in_proj_bias", "self_attn.out_proj.weight", "self_attn.out_proj.bias",
              "linear1.weight", "linear1.bias", "linear2.weight", "linear2.bias", "norm1.weight", "norm1.bias",
              "norm2.weight", "norm2.bias")
-    return {n: sd[p + n].detach().to(dev, torch.float32) for n in names}
+    return {n: sd[p + n] for n in names}
 
 
 # --------------------------------------------------------------------------------------------------------- references
@@ -231,19 +222,20 @@ def _seq_rows(view, t):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", list(CASES))
-@pytest.mark.parametrize("variant", list(VARIANTS))
-def test_encoder_attention_vs_fp64(variant, case):
+@pytest.mark.parametrize("variant,weights", with_weights(list(VARIANTS)))
+def test_encoder_attention_vs_fp64(variant, case, weights):
     """Every query row of every sequence, element by element: |kernel - fp64| within `attention_bound`.  Sharpness
     guard: the references with the dominant (else last) key dropped or read from the neighbouring row leave the bound on
-    > 90 % of the aimed rows, the one with the +1.0 biases ignored on > 75 % of the rows of the float-mask cases."""
+    > 90 % of the aimed rows, the one with the +1.0 biases ignored on > 75 % of the rows of the float-mask cases.
+    weights: the init or the trained-like weights (non-zero Q / K / V biases)."""
     env, prec, split, rounded = VARIANTS[variant]
     stack = CASES[case][0]
     if variant.startswith("tc5") and stack != 5:
         pytest.skip("attn_encoder_tc5 serves the 32-wide heads only")
     layer = LAYER[stack]
-    prm = _layer_params(stack, layer)
+    prm = _layer_params(stack, layer, weights)
     x, args, view = make_case(case, prm)
-    qkv, att, _ = _engine(**env).encoder_layer(stack, layer, x, precision=prec, **args)
+    qkv, att, _ = _engine(weights, **env).encoder_layer(stack, layer, x, precision=prec, **args)
     nh = view["nh"]
     scale = 1.0 / math.sqrt(D // nh)
     qm = view["qmask"]
@@ -261,7 +253,7 @@ def test_encoder_attention_vs_fp64(variant, case):
         assert not bool(bad.any()), (variant, case, torch.nonzero(bad)[:5].tolist(), worst)
         refs.append(o); tols.append(tol)
     ref, tol = torch.cat(refs), torch.cat(tols)
-    print(f"encoder attention {variant} {case}: max |err| / bound = {worst:.3f}")
+    print(f"encoder attention {variant} {case} {weights}: max |err| / bound = {worst:.3f}")
     # sharpness guards
     aimed = torch.zeros_like(qm)
     for bb in range(B):
@@ -288,17 +280,20 @@ LAYER_TOL = {"bf16": (1e-2, 8e-5), "fp32": (5e-5, 5e-6)}
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", LAYER_CASES)
-@pytest.mark.parametrize("prec", ["bf16", "fp32"])
-def test_encoder_layer_vs_fp64_contract(prec, case):
+@pytest.mark.parametrize("prec,weights", with_weights(["bf16", "fp32"]))
+def test_encoder_layer_vs_fp64_contract(prec, case, weights):
     """The whole layer (QKV projection, attention, out_proj + LN1, fused FFN + LN2), every query row, against
     `layer_ref` in fp64: max |err| and mean |err| bounds (LAYER_TOL, like the fused-FFN test: a handful of bf16 values
     round the other way where the fp32 accumulator sits at a midpoint).  Sharpness guard (bf16): the contract with the hi
-    weight terms alone exceeds the mean bound."""
+    weight terms alone exceeds the mean bound.  weights: the init or the trained-like weights; with the trained ones,
+    references with norm1 and norm2 exchanged, the out_proj bias, the V bias or the Q bias dropped each leave the max or
+    the mean bound."""
+    from test_gpu_trained_weights import with_fault
     stack = CASES[case][0]
     layer = LAYER[stack]
-    prm = _layer_params(stack, layer)
+    prm = _layer_params(stack, layer, weights)
     x, args, view = make_case(case, prm)
-    _, _, out = _engine().encoder_layer(stack, layer, x, precision=prec, **args)
+    _, _, out = _engine(weights).encoder_layer(stack, layer, x, precision=prec, **args)
     qm = view["qmask"]
     ref = layer_ref(x, view["qrows"], view["krows"], view["kbias"], prm, view["nh"], prec)
     err = (_seq_rows(view, out).double() - _seq_rows(view, ref))[qm].abs()
@@ -307,11 +302,18 @@ def test_encoder_layer_vs_fp64_contract(prec, case):
     if prec == "bf16":
         hi = layer_ref(x, view["qrows"], view["krows"], view["kbias"], prm, view["nh"], "bf16_hi")
         mean_hi = float((_seq_rows(view, hi) - _seq_rows(view, ref))[qm].abs().mean())
-    print(f"encoder layer {prec} {case}: max |err| {mx:.3e} mean {mean:.3e} (bounds {LAYER_TOL[prec]}; hi terms only: "
-          f"mean {mean_hi})")
+    print(f"encoder layer {prec} {case} {weights}: max |err| {mx:.3e} mean {mean:.3e} (bounds {LAYER_TOL[prec]}; hi terms "
+          f"only: mean {mean_hi})")
     assert mx < LAYER_TOL[prec][0] and mean < LAYER_TOL[prec][1], (prec, case, mx, mean)
     if prec == "bf16":
         assert mean_hi > 2 * LAYER_TOL[prec][1], (case, mean_hi)
+    if weights == "trained":
+        got = _seq_rows(view, out).double()[qm]
+        for kind in ("swap_n1n2", "drop_out_bias", "drop_v_bias", "drop_q_bias"):
+            faulty = {k[2:]: v for k, v in with_fault({"x." + k: v for k, v in prm.items()}, "x", kind).items()}
+            wrong = layer_ref(x, view["qrows"], view["krows"], view["kbias"], faulty, view["nh"], prec)
+            e = (got - _seq_rows(view, wrong)[qm]).abs()
+            assert float(e.max()) >= LAYER_TOL[prec][0] or float(e.mean()) >= LAYER_TOL[prec][1], (kind, prec, case, float(e.max()), float(e.mean()))
 
 
 # --------------------------------------------------------------------------------------------------------- (c)
@@ -345,16 +347,16 @@ def _contract_stack(P, name, nhead, x, mask, num_layers):
     return xr.reshape(B, S, D).transpose(0, 1)
 
 
-def _references(name):
+def _references(name, weights):
     """fp64 oracle (and bf16 contract) outputs of case `name`, in blocks of 128 spectra, kept for the precisions."""
-    if name in _REFS:
-        return _REFS[name]
+    if (name, weights) in _REFS:
+        return _REFS[name, weights]
     from multimodalspectraltransformer_b200 import synthetic
     from oracle import mmt_oracle as O
-    s = _setup()
+    from test_gpu_trained_weights import state_dict_for
     B, seed, peaks, mode = ENCODES[name]
     data = {k: v.cuda() for k, v in synthetic.make_spectra(B, seed=seed, peaks=peaks).items()}
-    P64 = {k: v.detach().cuda().double() for k, v in s["model"].state_dict().items()}
+    P64 = state_dict_for(weights, torch.float64)
     cfg = O.default_config(training_mode=mode)
     out = {"data": data, "mem": [], "mask": [], "fp": [], "emb": [], "contract": []}
     fused, stack = O.FUSED_SDPA, O.encoder_stack
@@ -374,7 +376,8 @@ def _references(name):
         out[k] = torch.cat(out[k], dim=1)
     out["mask"], out["fp"] = torch.cat(out["mask"]), torch.cat(out["fp"])
     out["avg"] = out["mem"].mean(dim=0)
-    _REFS[name] = out
+    _REFS.clear()              # one case at a time: the references of 1024 spectra are large
+    _REFS[name, weights] = out
     return out
 
 
@@ -388,15 +391,16 @@ def _per_spectrum(got, ref, rel):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("prec", ["fp32", "bf16"])
-@pytest.mark.parametrize("name", list(ENCODES))
-def test_encoder_every_spectrum_vs_fp64(name, prec):
+@pytest.mark.parametrize("name,weights", with_weights(list(ENCODES)))
+def test_encoder_every_spectrum_vs_fp64(weights, name, prec):
     """Memory, avg_memory and fingerprint of every spectrum against oracle.encode in fp64 (fp32 mode: max |err| <
     FP32_ABS; bf16: rms error / rms < BF16_REL, and < BF16_CONTRACT_REL against the fp64 contract run through all 12
     layers); key_bias and pad_mask bit for bit from the oracle's mask; embedding_src against fp64 and bit for bit
     against an encode of the same spectra one batch position further on.  Sharpness guards: every spectrum fails against
-    the neighbouring spectrum's reference, and the spectra of a chunk shifted by one fail."""
-    eng = _engine()
-    r = _references(name)
+    the neighbouring spectrum's reference, and the spectra of a chunk shifted by one fail.  weights: the init or the
+    trained-like weights (the bias and LayerNorm faults this bound sees on the latter: test_gpu_trained_weights)."""
+    eng = _engine(weights)
+    r = _references(name, weights)
     data = r["data"]
     B, _, _, mode = ENCODES[name]
     memory, pad, kb, fp, avg, emb = eng.encode(data, mode, prec, want_embedding_src=True)
@@ -422,10 +426,10 @@ def test_encoder_every_spectrum_vs_fp64(name, prec):
     if rel:
         err_c = _per_spectrum(memory, r["contract"], True)
         worst["contract"] = float(err_c.max())
-        print(f"encoder {name} bf16 on {torch.cuda.get_device_name()}: rms err / rms vs fp64 contract max "
+        print(f"encoder {name} {weights} bf16 on {torch.cuda.get_device_name()}: rms err / rms vs fp64 contract max "
               f"{worst['contract']:.3e} mean {float(err_c.mean()):.3e}")
         assert bool((err_c < BF16_CONTRACT_REL).all()), (name, torch.nonzero(err_c >= BF16_CONTRACT_REL)[:8].flatten().tolist(), worst)
-    print(f"encoder {name} {prec}: worst spectrum {worst} (bound {bound})")
+    print(f"encoder {name} {weights} {prec}: worst spectrum {worst} (bound {bound})")
     assert bool((err < bound).all()), (name, prec, torch.nonzero(err >= bound)[:8].flatten().tolist(), worst)
     assert bool((err_avg < bound).all()) and bool((err_fp < bound).all()), (name, prec, worst)
     # sharpness: the neighbouring spectrum's reference fails for every spectrum; so does a chunk shifted by one

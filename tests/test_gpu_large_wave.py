@@ -17,6 +17,8 @@ import math
 import pytest
 import torch
 
+from test_gpu_trained_weights import with_weights
+
 D, H, DH = 128, 16, 8
 SCALE = 1.0 / math.sqrt(DH)
 U16 = 2.0 ** -8          # unit round-off of bf16 (8 significant bits): |bf16(x) - x| <= 2^-8 |x|
@@ -183,11 +185,6 @@ def test_references_equal_oracle_mha(fused, monkeypatch):
 
 
 # --------------------------------------------------------------------------------------------------------- GPU helpers
-def _setup():
-    from test_gpu_parity import setup
-    return setup()
-
-
 VARIANTS = {                                   # engine knobs (read at creation) and precision of each self-attention path
     "token_major": ({}, "bf16"),
     "head_major": ({"MMT_KV_HEAD_MAJOR": "1"}, "bf16"),
@@ -196,15 +193,16 @@ VARIANTS = {                                   # engine knobs (read at creation)
 }
 
 
-def _engine(**env):
-    from test_gpu_parity import _engine_with_env
-    return _engine_with_env(**env)
+def _engine(weights, **env):
+    from test_gpu_trained_weights import engine_with
+    return engine_with(weights, **env)
 
 
-def _layer_weights(s, layer, which):
-    sd = s["model"].state_dict()
+def _layer_weights(weights, layer, which):
+    from test_gpu_trained_weights import state_dict_for
+    sd = state_dict_for(weights)
     p = f"decoder.layers.{layer}.{which}"
-    return sd[f"{p}.in_proj_weight"].detach().cuda().float(), sd[f"{p}.in_proj_bias"].detach().cuda().float()
+    return sd[f"{p}.in_proj_weight"], sd[f"{p}.in_proj_bias"]
 
 
 def _self_attention_inputs(T, N, seed):
@@ -232,18 +230,18 @@ def _check_rows(N, gen_seed):
 @pytest.mark.gpu
 @pytest.mark.parametrize("layer", [0, 5])
 @pytest.mark.parametrize("N", [1, 5, 129, 4099, 131072])
-@pytest.mark.parametrize("variant", list(VARIANTS))
-def test_paged_self_attention_vs_fp64(variant, N, layer):
+@pytest.mark.parametrize("variant,weights", with_weights(list(VARIANTS)))
+def test_paged_self_attention_vs_fp64(variant, N, layer, weights):
     """Self-attention of the un-fused step for T in {1, 4, 8, 16, 17, 33, 128} positions: 1-8 keys (the 4-key and 8-key
     prefetch edges of the token-major / head-major kernels), an open page with t % 16 in {0, 15}, max_len not a multiple of
     16, all eight pages.  Tolerance: `_tolerance` (bf16 output rounding 2^-8 |o|, K / V elements near a bf16 rounding
     midpoint rounded either way, fp32 round-off; fp32 mode: 2e-6 (1 + max |s|) vmax, i.e. ~1e-6 relative).
-    Sharpness guard: references that drop key t, or read key t from the previous slot, leave the bound on > 90 % of rows."""
-    s = _setup()
+    Sharpness guard: references that drop key t, or read key t from the previous slot, leave the bound on > 90 % of rows.
+    weights: the init or the trained-like weights (non-zero Q / K / V biases)."""
     env, prec = VARIANTS[variant]
-    eng = _engine(**env)
+    eng = _engine(weights, **env)
     bf16_mode = prec == "bf16"
-    W, b = _layer_weights(s, layer, "self_attn")
+    W, b = _layer_weights(weights, layer, "self_attn")
     x = _self_attention_inputs(128, N, seed=N + layer)
     rows = _check_rows(N, N)
     xr = x[:, rows]
@@ -260,7 +258,7 @@ def test_paged_self_attention_vs_fp64(variant, N, layer):
         bad = outside(ref[1:], self_attention_ref(xr, W, b, bf16_mode, wrong=wrong)[1:], tol[1:])
         frac = float(bad.double().mean())
         assert frac > 0.9, (wrong, frac)
-    print(f"self-attention {variant} N={N} layer={layer}: max |err| / bound = {worst:.3f}")
+    print(f"self-attention {variant} N={N} layer={layer} {weights}: max |err| / bound = {worst:.3f}")
 
 
 # --------------------------------------------------------------------------------------------------------- (b)
@@ -314,18 +312,18 @@ def _aim_queries(q, k_rows, attended, n_cand):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("n_cand", [1, 7, 8, 15, 16, 17, 100, 128, 130])
-def test_candidate_cross_attention_vs_fp64(n_cand):
+@pytest.mark.parametrize("n_cand,weights", with_weights([1, 7, 8, 15, 16, 17, 100, 128, 130]))
+def test_candidate_cross_attention_vs_fp64(n_cand, weights):
     """Cross attention of the un-fused step (SIMT kernel below 8 candidates, the mma.sync kernel from 8: 16-candidate
     tiles with tails, 32-key softmax rounds, Q as a two-term bf16 split, P in bf16) against fp64: nk in {1, 31, 32, 33, 64,
     65, 169, 582} of S = 582 rows through a strided memory view (stride_b = 256), S = 902 with every row attended and a
     +1.0 float-mask block, 1,024 spectra for the 128-candidate bench geometry; fp32 mode alongside.  Tolerance: `_tolerance`.
-    Sharpness guard: a reference without the last attended key, and one without the +1.0 biases, leave the bound."""
-    s = _setup()
-    eng = _engine()
-    eng_simt = _engine(MMT_NO_TC_ATTENTION="1") if n_cand >= 8 else None
+    Sharpness guard: a reference without the last attended key, and one without the +1.0 biases, leave the bound.
+    weights: the init or the trained-like weights (non-zero K / V biases)."""
+    eng = _engine(weights)
+    eng_simt = _engine(weights, MMT_NO_TC_ATTENTION="1") if n_cand >= 8 else None
     layer = 3
-    W, b = _layer_weights(s, layer, "multihead_attn")
+    W, b = _layer_weights(weights, layer, "multihead_attn")
     Wkv, bkv = W[D:], b[D:]
     configs = [(582, 1024 if n_cand == 128 else 64, False, True), (902, 16, True, False)]
     for S, Bm, float_mask, strided in configs:
@@ -349,7 +347,7 @@ def test_candidate_cross_attention_vs_fp64(n_cand):
                 bad = outside(out, ref, tol)
                 assert not bool(bad.any()), (n_cand, S, prec, torch.nonzero(bad)[:5].tolist(),
                                              float(((out - ref).abs() / tol).max()))
-                print(f"cross n_cand={n_cand} S={S} {prec}{' simt' if e is eng_simt else ''}: max |err| / bound = "
+                print(f"cross n_cand={n_cand} S={S} {prec}{' simt' if e is eng_simt else ''} {weights}: max |err| / bound = "
                       f"{float(((out - ref).abs() / tol).max()):.3f}")
             # sharpness guards
             seq_b = torch.arange(Bm * n_cand, device="cuda") // n_cand
@@ -385,20 +383,26 @@ MAX_TOL_FP32 = 1e-5
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("geometry", list(GEOMETRIES))
-def test_unfused_step_teacher_forced_logits_vs_fp64_oracle(geometry, monkeypatch):
+@pytest.mark.parametrize("geometry,weights", with_weights(list(GEOMETRIES)))
+def test_unfused_step_teacher_forced_logits_vs_fp64_oracle(geometry, weights, monkeypatch):
     """All 128 positions of the un-fused step, teacher-forced with random targets (row 0 = <SOS>; every candidate differs),
     on an fp32-encoded memory, against oracle.teacher_forced_logits in fp64 on the device.  Checked rows: every candidate of
     spectrum 0, the middle and the last spectrum, and of the spectra with the most and the fewest attended memory rows.
     bf16: row-relative error < 1e-2 everywhere, argmax = the fp64 argmax wherever the fp64 top-2 margin exceeds 2e-2 of the
     row scale, mean error < 3e-3; fp32 mode: max row-relative error < 1e-5, mean < 1e-6 (MEAN_TOL).  The same spectra decoded alone (a small wave:
-    the fused decode_attn path) are measured alongside as the reference point."""
-    s = _setup()
+    the fused decode_attn path) are measured alongside as the reference point.  weights: the init or the trained-like
+    weights; with the trained ones, references with one bias or LayerNorm fault (another layer's norm3 / norm1 gamma,
+    norm2 and norm3 exchanged, norm2 beta, a self / cross out_proj bias or V bias dropped; layers 0, 3, 5) leave the
+    bound on > 90 % of the checked rows."""
+    check_teacher_forced(*GEOMETRIES[geometry], weights, geometry, monkeypatch)
+
+
+def check_teacher_forced(Bm, K, env, precs, weights, geometry, monkeypatch):
     from multimodalspectraltransformer_b200 import synthetic
     from oracle import mmt_oracle as O
-    Bm, K, env, precs = GEOMETRIES[geometry]
+    from test_gpu_trained_weights import DECODER_FAULTS, decoder_fault, state_dict_for
     T = 128
-    eng = _engine(**env)
+    eng = _engine(weights, **env)
     data = {k: v.cuda() for k, v in synthetic.make_spectra(Bm, seed=4000 + Bm).items()}
     mode = "1H_13C_HSQC_COSY_IR_MF_MW"
     memory, pad, kb, *_ = eng.encode(data, mode, "fp32")
@@ -410,29 +414,33 @@ def test_unfused_step_teacher_forced_logits_vs_fp64_oracle(geometry, monkeypatch
     sel = sorted({0, Bm // 2, Bm - 1, int(nk.argmax()), int(nk.argmin())})
     cols = torch.cat([torch.arange(bb * K, (bb + 1) * K) for bb in sel]).cuda()
     monkeypatch.setattr(O, "FUSED_SDPA", False)
-    P64 = {k: v.detach().cuda().double() for k, v in s["model"].state_dict().items()}
+    P64 = state_dict_for(weights, torch.float64)
     ocfg = O.default_config()
-    with torch.no_grad():
-        ref = torch.cat([O.teacher_forced_logits(P64, memory[:, bb:bb + 1].double().expand(-1, K, -1), pad[bb:bb + 1].bool().expand(K, -1),
-                                                 trg[:, bb * K:(bb + 1) * K], ocfg) for bb in sel], dim=1)   # (T, len(sel)*K, V)
+
+    def oracle(P):
+        with torch.no_grad():
+            return torch.cat([O.teacher_forced_logits(P, memory[:, bb:bb + 1].double().expand(-1, K, -1), pad[bb:bb + 1].bool().expand(K, -1),
+                                                      trg[:, bb * K:(bb + 1) * K], ocfg) for bb in sel], dim=1)   # (T, len(sel)*K, V)
+    ref = oracle(P64)
     scale = ref.abs().amax(dim=-1)
     top2 = torch.topk(ref, 2, dim=-1).values
     decided = (top2[..., 0] - top2[..., 1]) > 2 * REL_TOL * scale
-    stats, argmax_ok = {}, {}
+    stats, argmax_ok, first = {}, {}, None
     for prec in precs:
         logits = eng.teacher_forced(memory, kb, trg, n_cand=K, precision=prec)
         got = logits[:, cols].double()
         del logits
+        first = got if first is None else first
         rel = (got - ref).abs().amax(dim=-1) / scale
         stats[prec] = (float(rel.max()), float(rel.mean()))
         argmax_ok[prec] = torch.equal(got.argmax(-1)[decided], ref.argmax(-1)[decided])
     # reference point: the same spectra alone, a small wave on the fused path
     sel_t = torch.tensor(sel, device="cuda")
-    eng_small = _engine() if env else eng
+    eng_small = _engine(weights) if env else eng
     small = eng_small.teacher_forced(memory[:, sel_t], kb[sel_t], trg[:, cols], n_cand=K, precision="bf16").double()
     rel_s = (small - ref).abs().amax(dim=-1) / scale
     stats["fused_bf16"] = (float(rel_s.max()), float(rel_s.mean()))
-    print(f"teacher-forced {geometry} on {torch.cuda.get_device_name()}: " +
+    print(f"teacher-forced {geometry} {weights} on {torch.cuda.get_device_name()}: " +
           ", ".join(f"{k} max {v[0]:.3e} mean {v[1]:.3e}" for k, v in stats.items()))
     for prec in precs:
         mx, mean = stats[prec]
@@ -441,3 +449,8 @@ def test_unfused_step_teacher_forced_logits_vs_fp64_oracle(geometry, monkeypatch
         if prec == "bf16":
             assert argmax_ok[prec], geometry
     assert stats["fused_bf16"][0] < REL_TOL
+    if weights == "trained":       # sharpness: each fault moves > 90 % of the checked rows past the bound
+        for kind, layer in DECODER_FAULTS:
+            wrong = oracle(decoder_fault(P64, kind, layer))
+            frac = float(((first - wrong).abs().amax(dim=-1) / scale >= REL_TOL).double().mean())
+            assert frac > 0.9, (geometry, kind, layer, frac)
