@@ -176,6 +176,16 @@ typedef struct mmt_decode_args {
 int32_t mmt_decode(mmt_engine* e, const mmt_decode_args* a, int64_t* d_tokens, float* d_probs,
                    int32_t* h_steps, void* stream);
 
+/* mmt_decode with the multinomial draws in PER-MEMORY streams: the n_cand candidates of memory column b draw what one
+ * torch.multinomial((n_cand, vocab), 1) call per step would, the columns' calls taken in order, as the reference's
+ * per-spectrum loop does (multinomial_sequence_multi on n_cand duplicates, spectrum after spectrum).  With
+ * B0 = seq_index_base / n_cand and inc = mmt_philox_increment(n_cand*vocab): column b at step t uses offset
+ * philox_offset + ((B0 + b)*max_len + t)*inc, candidate j its elements j*vocab .. of that call.  A caller's generator
+ * ends advanced by Bm_total*max_len*inc.  Fails unless a->sampling is multinomial and seq_index_base is a multiple of
+ * n_cand; N_total is ignored. */
+int32_t mmt_decode_memory_streams(mmt_engine* e, const mmt_decode_args* a, int64_t* d_tokens, float* d_probs,
+                                  int32_t* h_steps, void* stream);
+
 /* Replaces the decoder tail of MultimodalTransformer.forward(..., trg_SMI_input)
  * (models_MMT_v15_4.py:955-976) and the teacher-forced scorers' inner call:
  * d_trg (T,N) i64 -> d_logits (T,N,vocab) f32 (fc_out, before softmax). */
@@ -243,6 +253,19 @@ int32_t mmt_ingest_ir(const double* d_values, const int64_t* d_offsets, int32_t 
  * and joins the strings after ONE device-to-host copy. */
 int32_t mmt_first_eos(const int64_t* d_tokens, int32_t T, int64_t N, int32_t eos, int32_t* d_len, void* stream);
 
+/* Distinct strings per memory column of candidate ids d_tokens (T,N) i64, N = Bm*n_cand: for column b, the distinct
+ * values of tensor_to_smiles(tokens[:, b*n_cand:(b+1)*n_cand], itos) in first-occurrence order (dict.fromkeys), each
+ * with the index of its first candidate and its multiplicity.  A string is the byte concatenation of the itos entries
+ * of the ids before the first `eos`; strings are compared byte by byte.  itos as a table: d_itos_entries (n_itos, 2)
+ * i32 {byte start, byte length} into d_itos_bytes (UTF-8), length -1 where an id has no entry; itos_max_bytes = the
+ * longest entry.  With d_work NULL: *work_bytes = the device workspace these sizes need.  Otherwise runs, synchronises
+ * `stream` once and returns h_result[6] = {distinct strings D, their bytes, offset and size of the output in d_work,
+ * 1 if an id before <EOS> has no itos entry, that id}.  The output (int64 unless noted): col_off[Bm+1], first[D],
+ * count[D], ntok[D] (ids before <EOS>), boff[D+1], then the strings' bytes (u8) -- string d = bytes[boff[d], boff[d+1]). */
+int32_t mmt_distinct_smiles(const int64_t* d_tokens, int32_t T, int64_t N, int32_t n_cand, int64_t eos,
+                            const uint8_t* d_itos_bytes, const int32_t* d_itos_entries, int32_t n_itos, int32_t itos_max_bytes,
+                            void* d_work, int64_t* work_bytes, int64_t* h_result, void* stream);
+
 /* ---- building blocks exported for unit parity tests --------------------------- */
 
 /* fused fc_out + softmax(logits/T) + greedy|multinomial pick on hidden states
@@ -266,6 +289,16 @@ int32_t mmt_exponential(uint64_t philox_seed, uint64_t philox_offset, int64_t el
 int32_t mmt_sample_probs(const float* d_p, int64_t N, int32_t V, uint64_t philox_seed, uint64_t philox_offset,
                          int64_t seq_index_base, int64_t N_total, int32_t sm_count, int32_t max_threads_per_sm,
                          int64_t* d_token, void* stream);
+
+/* The per-memory mapping of mmt_decode_memory_streams at one step, stand-alone: rows n of a call placed at
+ * seq_index_base (a multiple of n_cand) draw as candidate (seq_index_base+n) mod n_cand of column
+ * (seq_index_base+n) / n_cand at step `step` of max_len.  Exactly one of d_x (N,128) hidden states (the decode
+ * step's fused fc_out + softmax(logits/temperature) + pick, d_prob optional) and d_p (N,vocab) caller probabilities
+ * (the stream alone, as mmt_sample_probs; d_prob unused). */
+int32_t mmt_sample_memory_streams(mmt_engine* e, const float* d_x, const float* d_p, int64_t N, int32_t n_cand, int32_t max_len,
+                                  int32_t step, float temperature, uint64_t philox_seed, uint64_t philox_offset,
+                                  int64_t seq_index_base, int32_t rng_sm_count, int32_t rng_max_threads_per_sm,
+                                  int64_t* d_token, float* d_prob, void* stream);
 
 /* C[M,N] = act(A[M,K] . W[N,K]^T + bias) in the requested precision
  * (fp32 SIMT or bf16 tcgen05); act: 0 none, 1 ReLU. */

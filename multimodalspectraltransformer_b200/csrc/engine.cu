@@ -8,6 +8,7 @@
 #include "kernels_attn5.cuh"
 #include "kernels_compact.cuh"
 #include "kernels_beam.cuh"
+#include "kernels_smiles.cuh"
 
 #include <algorithm>
 #include <cstdlib>
@@ -978,6 +979,7 @@ struct DecodeRun {
     int64_t* tokens; float* probs; float* logits;   // outputs, leading dimension N_total
     int64_t ldn = -1;         // >= 0 overrides the leading dimension (0: single-row token / logit buffers, beam search)
     bool serial_first = false;   // the step's first kernel waits for full completion of its predecessor (its prologue reads the block table)
+    bool per_memory_rng = false; // multinomial draws in per-memory streams (torch_rng_row): one (n_cand, V) call per column and step
 };
 
 // Projects the memory of one wave to per-layer cross-attention K/V (head-major) once;
@@ -1299,12 +1301,13 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
     sp.temperature = a.temperature; sp.mode = r.mode;
     int smc = a.rng_sm_count > 0 ? a.rng_sm_count : e->sm_count;
     int mts = a.rng_max_threads_per_sm > 0 ? a.rng_max_threads_per_sm : e->max_threads_per_sm;
-    int64_t Nrng = a.N_total > 0 ? a.N_total : N_total;
+    int64_t Nrng = r.per_memory_rng ? a.n_cand : (a.N_total > 0 ? a.N_total : N_total);
     sp.rng.seed = a.philox_seed; sp.rng.offset = a.philox_offset; sp.rng.numel = Nrng * d.vocab;
     sp.rng.threads = torch_rng_threads(sp.rng.numel, smc, mts);
     sp.rng_inc = torch_rng_increment(sp.rng.numel, smc, mts);
     sp.rng_dev = b.rng_state;
-    sp.seq_index_base = a.seq_index_base + n0;
+    sp.seq_index_base = a.seq_index_base + n0;      // waves and lanes start at column boundaries: n0 is a multiple of n_cand
+    if (r.per_memory_rng) { sp.rng_cand = a.n_cand; sp.rng_col_steps = a.max_len; }
     sp.tokens = r.tokens ? r.tokens + n0 : nullptr; sp.probs = r.probs ? r.probs + n0 : nullptr;
     sp.logits = r.logits ? r.logits + n0 * d.vocab : nullptr;
     sp.target = r.target ? r.target + n0 : nullptr; sp.target_prob = r.target_prob ? r.target_prob + n0 : nullptr;
@@ -1425,6 +1428,7 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
             put((uint64_t)r.mode); put((uint64_t)r.T); put((uint64_t)(r.probs != nullptr)); put((uint64_t)a.S); put((uint64_t)a.Bm);
             put((uint64_t)a.n_cand); put((uint64_t)a.max_len); put(tbits); put((uint64_t)a.precision);
             put((uint64_t)a.seq_index_base); put((uint64_t)a.N_total); put((uint64_t)a.rng_sm_count); put((uint64_t)a.rng_max_threads_per_sm);
+            put((uint64_t)r.per_memory_rng);
             put((uint64_t)(uintptr_t)e->arena); put((uint64_t)e->arena_bytes); put((uint64_t)nl); put((uint64_t)U);
             put((uint64_t)e->fused_decode_rows); put((uint64_t)e->use_pdl); put((uint64_t)(uintptr_t)e->da_dbg);
             for (auto& c : e->graph_cache) if (c.key == key) { exec = c.exec; launches_per_group = c.launches_per_group; c.stamp = ++e->graph_cache_clock; break; }
@@ -1839,6 +1843,19 @@ int32_t mmt_decode(mmt_engine* e, const mmt_decode_args* a, int64_t* d_tokens, f
     return run_decode(e, r, h_steps, (cudaStream_t)stream);
 }
 
+int32_t mmt_decode_memory_streams(mmt_engine* e, const mmt_decode_args* a, int64_t* d_tokens, float* d_probs, int32_t* h_steps, void* stream) {
+    if (!e || !a) MMT_FAIL("null engine / args");
+    if (!d_tokens) MMT_FAIL("decode: d_tokens is required");
+    if (a->sampling != MMT_SAMPLE_MULTINOMIAL) MMT_FAIL("mmt_decode_memory_streams: per-memory RNG streams need multinomial sampling");
+    if (a->n_cand <= 0 || a->seq_index_base < 0 || a->seq_index_base % a->n_cand)
+        MMT_FAIL("mmt_decode_memory_streams: seq_index_base must be a non-negative multiple of n_cand");
+    EngineCall call(e, (cudaStream_t)stream);
+    DecodeRun r;
+    r.a = a; r.mode = a->sampling; r.trg = nullptr; r.T = a->max_len; r.tokens = d_tokens; r.probs = d_probs; r.logits = nullptr;
+    r.per_memory_rng = true;
+    return run_decode(e, r, h_steps, (cudaStream_t)stream);
+}
+
 int32_t mmt_teacher_forced(mmt_engine* e, const mmt_decode_args* a, const int64_t* d_trg, int32_t T, float* d_logits, void* stream) {
     if (!e || !a || !d_trg || !d_logits) MMT_FAIL("null argument");
     if (T < 1) MMT_FAIL("T must be >= 1");
@@ -2016,8 +2033,101 @@ int32_t mmt_sample_probs(const float* d_p, int64_t N, int32_t V, uint64_t philox
     if (Nrng < seq_index_base + N) MMT_FAIL("mmt_sample_probs: N_total smaller than seq_index_base + N");
     RngGeom g;
     g.seed = philox_seed; g.offset = philox_offset; g.numel = Nrng * V; g.threads = torch_rng_threads(g.numel, sm_count, max_threads_per_sm);
-    sample_from_probs<<<(unsigned)((N + 7) / 8), 256, 0, (cudaStream_t)stream>>>(d_p, N, V, g, seq_index_base, d_token);
+    sample_from_probs<<<(unsigned)((N + 7) / 8), 256, 0, (cudaStream_t)stream>>>(d_p, N, V, g, seq_index_base, 0, 0, 0, 0, d_token);
     MMT_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int32_t mmt_sample_memory_streams(mmt_engine* e, const float* d_x, const float* d_p, int64_t N, int32_t n_cand, int32_t max_len,
+                                  int32_t step, float temperature, uint64_t philox_seed, uint64_t philox_offset,
+                                  int64_t seq_index_base, int32_t rng_sm_count, int32_t rng_max_threads_per_sm,
+                                  int64_t* d_token, float* d_prob, void* stream) {
+    if (!e || !d_token || (!d_x) == (!d_p)) MMT_FAIL("mmt_sample_memory_streams: give d_token and exactly one of d_x, d_p");
+    if (n_cand <= 0 || max_len < 1 || step < 0 || step >= max_len) MMT_FAIL("mmt_sample_memory_streams: need n_cand >= 1 and 0 <= step < max_len");
+    if (seq_index_base < 0 || seq_index_base % n_cand) MMT_FAIL("mmt_sample_memory_streams: seq_index_base must be a non-negative multiple of n_cand");
+    if (N <= 0) return 0;
+    EngineCall call(e, (cudaStream_t)stream);
+    cudaStream_t cs = (cudaStream_t)stream;
+    const int V = e->desc.vocab;
+    const int smc = rng_sm_count > 0 ? rng_sm_count : e->sm_count;
+    const int mts = rng_max_threads_per_sm > 0 ? rng_max_threads_per_sm : e->max_threads_per_sm;
+    RngGeom g;
+    g.seed = philox_seed; g.offset = philox_offset; g.numel = (int64_t)n_cand * V; g.threads = torch_rng_threads(g.numel, smc, mts);
+    const uint64_t inc = torch_rng_increment(g.numel, smc, mts);
+    prof_pre(e, cs);
+    if (d_p) {
+        sample_from_probs<<<(unsigned)((N + 7) / 8), 256, 0, cs>>>(d_p, N, V, g, seq_index_base, inc, n_cand, max_len, step, d_token);
+        return check_launch(e, "sample_from_probs", cs);
+    }
+    // fused fc_out + softmax + pick at step `step`, read from a device step counter like the decode step's
+    MMT_TRY(ensure_arena(e, 256));
+    int* ctl = reinterpret_cast<int*>(e->arena);
+    MMT_CUDA(cudaMemcpyAsync(ctl, &step, sizeof(int), cudaMemcpyHostToDevice, cs));
+    SampleParams sp;
+    memset(&sp, 0, sizeof(sp));
+    sp.x = d_x; sp.W = e->W("fc_out.weight"); sp.b = e->W("fc_out.bias"); sp.V = V; sp.N = N; sp.ldn = N;
+    sp.temperature = temperature; sp.mode = MMT_SAMPLE_MULTINOMIAL;
+    sp.rng = g; sp.rng_inc = inc; sp.seq_index_base = seq_index_base; sp.rng_cand = n_cand; sp.rng_col_steps = max_len;
+    sp.tokens = d_token - (int64_t)step * N; sp.probs = d_prob ? d_prob - (int64_t)step * N : nullptr;   // row `step` = the caller's
+    sp.ctl.step = ctl;
+    sp.advance = 0;
+    MMT_TRY(sample_init(e));
+    sp.rows_per_warp = N >= 8192 ? SAMPLE_NR : 1;
+    sample_tokens<<<(unsigned)std::min<int64_t>((N + 8 * sp.rows_per_warp - 1) / (8 * sp.rows_per_warp), (int64_t)e->sm_count * 4), 256, sample_smem_bytes(sp.V), cs>>>(sp);
+    return check_launch(e, "sample_tokens", cs);
+}
+
+int32_t mmt_distinct_smiles(const int64_t* d_tokens, int32_t T, int64_t N, int32_t n_cand, int64_t eos,
+                            const uint8_t* d_itos_bytes, const int32_t* d_itos_entries, int32_t n_itos, int32_t itos_max_bytes,
+                            void* d_work, int64_t* work_bytes, int64_t* h_result, void* stream) {
+    if (!work_bytes) MMT_FAIL("null argument");
+    if (T < 1 || N < 1 || n_cand < 1 || N % n_cand || n_itos < 0 || itos_max_bytes < 0)
+        MMT_FAIL("mmt_distinct_smiles: need T >= 1 and N a positive multiple of n_cand");
+    const int64_t Bm = N / n_cand;
+    int P = 2;
+    while (P < 2 * n_cand) P <<= 1;
+    const bool gtab = P > SMILES_SMEM_SLOTS;
+    // workspace: scratch, then the output (metadata + bytes, at most every candidate's T entries of itos_max_bytes)
+    auto al = [](int64_t x) { return (x + 255) & ~(int64_t)255; };
+    const int64_t o_hash = 0, o_nbytes = o_hash + al(8 * N), o_didx = o_nbytes + al(8 * N), o_dbyte = o_didx + al(8 * (N + 1));
+    const int64_t o_ntok = o_dbyte + al(8 * (N + 1)), o_slot = o_ntok + al(4 * N), o_mult = o_slot + al(4 * N), o_isd = o_mult + al(4 * N);
+    const int64_t o_bad = o_isd + al(4 * N), o_tab = o_bad + 256, o_out = o_tab + (gtab ? al(4 * Bm * P) : 0);
+    const int64_t need = o_out + 8 * (Bm + 1 + 4 * N + 1) + N * T * (int64_t)itos_max_bytes;
+    if (!d_work) { *work_bytes = need; return 0; }
+    if (*work_bytes < need || !d_tokens || !d_itos_entries || (!d_itos_bytes && n_itos) || !h_result)
+        MMT_FAIL("mmt_distinct_smiles: workspace too small or null argument");
+    cudaStream_t s = (cudaStream_t)stream;
+    char* w = static_cast<char*>(d_work);
+    SmilesParams p;
+    p.tokens = d_tokens; p.T = T; p.N = N; p.k = n_cand; p.eos = eos;
+    p.tab_bytes = d_itos_bytes; p.tab = reinterpret_cast<const int2*>(d_itos_entries); p.n_tab = n_itos; p.P = P;
+    p.gtable = gtab ? reinterpret_cast<int*>(w + o_tab) : nullptr;
+    p.hash = reinterpret_cast<uint64_t*>(w + o_hash); p.nbytes = reinterpret_cast<int64_t*>(w + o_nbytes);
+    p.ntok = reinterpret_cast<int32_t*>(w + o_ntok); p.slot = reinterpret_cast<int32_t*>(w + o_slot);
+    p.mult = reinterpret_cast<int32_t*>(w + o_mult); p.isd = reinterpret_cast<int32_t*>(w + o_isd);
+    p.bad = reinterpret_cast<int64_t*>(w + o_bad);
+    int64_t* didx = reinterpret_cast<int64_t*>(w + o_didx);
+    int64_t* dbyte = reinterpret_cast<int64_t*>(w + o_dbyte);
+    int64_t* out = reinterpret_cast<int64_t*>(w + o_out);
+    MMT_CUDA(cudaMemsetAsync(p.bad, 0, 2 * sizeof(int64_t), s));
+    const int threads = (int)std::min<int64_t>(1024, (n_cand + 31) / 32 * 32);
+    smiles_dedup<<<(unsigned)Bm, threads, gtab ? 0 : (size_t)P * sizeof(int), s>>>(p);
+    MMT_CUDA(cudaGetLastError());
+    smiles_scan<<<1, 1024, 0, s>>>(p.isd, p.nbytes, N, didx, dbyte);
+    MMT_CUDA(cudaGetLastError());
+    smiles_emit<<<(unsigned)((N + 255) / 256), 256, 0, s>>>(p, didx, dbyte, Bm, out);
+    MMT_CUDA(cudaGetLastError());
+    int64_t tot[4];
+    MMT_CUDA(cudaMemcpyAsync(tot, didx + N, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    MMT_CUDA(cudaMemcpyAsync(tot + 1, dbyte + N, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    MMT_CUDA(cudaMemcpyAsync(tot + 2, p.bad, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    MMT_CUDA(cudaStreamSynchronize(s));
+    h_result[0] = tot[0];                                    // distinct strings
+    h_result[1] = tot[1];                                    // bytes of the distinct strings
+    h_result[2] = o_out;                                     // output offset in d_work ...
+    h_result[3] = 8 * (Bm + 1 + 4 * tot[0] + 1) + tot[1];   // ... and size
+    h_result[4] = tot[2];                                    // 1: an id before <EOS> has no itos entry ...
+    h_result[5] = tot[3];                                    // ... this one
     return 0;
 }
 

@@ -1366,6 +1366,8 @@ struct SampleParams {
     const uint64_t* rng_dev; // optional {seed, offset} in device memory (overrides rng.seed / rng.offset: keeps a captured
                              // decode graph reusable across calls with a different generator state)
     int64_t seq_index_base;
+    int64_t rng_cand;        // 0: global mapping; > 0: per-memory streams of rng_cand rows, rng_col_steps calls per column
+    int64_t rng_col_steps;   //   (torch_rng_row; rng.threads / rng_inc then describe one (rng_cand, V) call)
     int64_t* tokens;         // [max_len][N] or nullptr
     float* probs;            // [max_len][N] or nullptr
     float* logits;           // [T][N][V] (forced / unit test) or nullptr
@@ -1442,8 +1444,7 @@ __device__ __forceinline__ void sample_rows(const SampleParams& p, const float* 
         if (p.mode == 1) {
             RngGeom g = p.rng;
             if (p.rng_dev) { g.seed = p.rng_dev[0]; g.offset = p.rng_dev[1]; }
-            g.offset += (uint64_t)t * p.rng_inc;
-            int64_t li = (p.seq_index_base + n) * p.V;
+            const int64_t li = torch_rng_row(g, p.rng_inc, p.rng_cand, p.rng_col_steps, p.seq_index_base + n, t, p.V);
             if (ok0) r0v = p0 / torch_exponential_at(g, li + v0);
             if (ok1) r1v = p1 / torch_exponential_at(g, li + v1);
         }
@@ -1562,15 +1563,18 @@ __global__ void __launch_bounds__(256) exponential_fill(RngGeom g, int64_t base,
     if (i < n) q[i] = torch_exponential_at(g, base + i);
 }
 
-// token[n] = first arg-max over v of p[n][v] / q[(base + n) * V + v]   (torch.multinomial(p, 1) on given probabilities)
-__global__ void __launch_bounds__(256) sample_from_probs(const float* p, int64_t N, int V, RngGeom g, int64_t seq_base, int64_t* token) {
+// token[n] = first arg-max over v of p[n][v] / q[li + v]   (torch.multinomial(p, 1) on given probabilities), li and the
+// offset of row seq_base + n at step t from torch_rng_row (n_cand == 0, t == 0: element (seq_base + n) * V, offset g.offset)
+__global__ void __launch_bounds__(256) sample_from_probs(const float* p, int64_t N, int V, RngGeom g, int64_t seq_base, uint64_t inc,
+                                                         int64_t n_cand, int64_t col_steps, int t, int64_t* token) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t n = (int64_t)blockIdx.x * 8 + warp;
     if (n >= N) return;
+    const int64_t li = torch_rng_row(g, inc, n_cand, col_steps, seq_base + n, t, V);
     float best = MMT_NEG_INF;
     int bi = 0x7fffffff;
     for (int v = lane; v < V; v += 32) {
-        const float r = p[n * V + v] / torch_exponential_at(g, (seq_base + n) * V + v);
+        const float r = p[n * V + v] / torch_exponential_at(g, li + v);
         if (r > best) { best = r; bi = v; }
     }
 #pragma unroll

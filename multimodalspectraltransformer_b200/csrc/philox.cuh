@@ -71,4 +71,20 @@ __device__ __forceinline__ float torch_exponential_at(const RngGeom& g, int64_t 
     return -1.0f / 1.0f * lg;
 }
 
+// Generator offset and first q element of row `gi` (index inside the logical call) at step t.
+// n_cand == 0, the global mapping: one torch.multinomial((N_total, V), 1) per step -> offset + t*inc, element gi*V.
+// n_cand > 0, per-memory streams: the n_cand rows of memory column c = gi / n_cand are one torch.multinomial((n_cand, V), 1)
+// per step, the columns' calls taken in order (max_len = col_steps calls per column) -> offset + (c*col_steps + t)*inc,
+// element (gi mod n_cand)*V of that call's n_cand*V tensor (g.threads must be torch_rng_threads(n_cand*V)).
+__host__ __device__ __forceinline__ int64_t torch_rng_row(RngGeom& g, uint64_t inc, int64_t n_cand, int64_t col_steps,
+                                                          int64_t gi, int t, int V) {
+    if (n_cand <= 0) {
+        g.offset += (uint64_t)t * inc;
+        return gi * V;
+    }
+    const int64_t c = gi / n_cand;
+    g.offset += ((uint64_t)c * (uint64_t)col_steps + (uint64_t)t) * inc;
+    return (gi - c * n_cand) * V;
+}
+
 }  // namespace mmt

@@ -219,16 +219,21 @@ class Engine:
         return a, (memory, key_bias)
 
     def decode(self, memory, key_bias, *, n_cand=1, max_len=128, temperature=1.0, sampling="greedy",
-               stop_on_all_pad=False, precision="fp32", seed=0, offset=0, seq_index_base=0, n_total=0):
-        """Returns (tokens (T,N) i64, probs (T,N) f32, steps) with T == max_len rows allocated."""
+               stop_on_all_pad=False, precision="fp32", seed=0, offset=0, seq_index_base=0, n_total=0, per_memory_rng=False):
+        """Returns (tokens (T,N) i64, probs (T,N) f32, steps) with T == max_len rows allocated.  ``per_memory_rng``: the
+        n_cand candidates of each memory column draw as one torch.multinomial((n_cand, V), 1) call per step, the columns'
+        calls in order (``mmt_decode_memory_streams``); multinomial only, seq_index_base a multiple of n_cand."""
         smp = _lib.SAMPLE_GREEDY if sampling == "greedy" else _lib.SAMPLE_MULTINOMIAL
+        if per_memory_rng and (smp != _lib.SAMPLE_MULTINOMIAL or seq_index_base % n_cand):
+            raise ValueError("per_memory_rng needs multinomial sampling and seq_index_base a multiple of n_candidates")
         a, keep = self._decode_args(memory, key_bias, n_cand, max_len, temperature, smp, stop_on_all_pad, precision,
                                     seed, offset, seq_index_base, n_total)
         N = a.Bm * n_cand
         tokens = torch.empty(max_len, N, device=self.device, dtype=torch.int64)
         probs = torch.empty(max_len, N, device=self.device, dtype=torch.float32)
         steps = C.c_int32(max_len)
-        _lib.check(self.L.mmt_decode(self.h, C.byref(a), tokens.data_ptr(), probs.data_ptr(), C.byref(steps), self._stream()))
+        fn = self.L.mmt_decode_memory_streams if per_memory_rng else self.L.mmt_decode
+        _lib.check(fn(self.h, C.byref(a), tokens.data_ptr(), probs.data_ptr(), C.byref(steps), self._stream()))
         for t in keep:
             t.record_stream(torch.cuda.current_stream(self.dev_index))
         return tokens, probs, int(steps.value)
@@ -314,6 +319,19 @@ class Engine:
         _lib.check(self.L.mmt_sample_probs(p.data_ptr(), N, V, seed, offset, seq_index_base, n_total, self.sm_count,
                                            self.max_threads_per_sm, tok.data_ptr(), self._stream()))
         return tok
+
+    def sample_memory_streams(self, *, x=None, p=None, n_cand, max_len, step=0, temperature=1.0, seed, offset,
+                              seq_index_base=0):
+        """Per-memory RNG streams at one step (test hook): from hidden states x (N,128) through the fused sampler ->
+        (ids, probabilities), or from probabilities p (N,V) -> (ids, None)."""
+        src = (x if p is None else p).to(self.device, torch.float32).contiguous()
+        N = src.shape[0]
+        tok = torch.empty(N, device=self.device, dtype=torch.int64)
+        pr = torch.empty(N, device=self.device, dtype=torch.float32) if p is None else None
+        _lib.check(self.L.mmt_sample_memory_streams(self.h, src.data_ptr() if p is None else None, src.data_ptr() if p is not None else None,
+                                                    N, n_cand, max_len, step, float(temperature), seed, offset, seq_index_base,
+                                                    0, 0, tok.data_ptr(), pr.data_ptr() if pr is not None else None, self._stream()))
+        return tok, pr
 
     def linear(self, A, W, bias=None, act=0, precision="fp32"):
         A = A.to(self.device, torch.float32).contiguous()

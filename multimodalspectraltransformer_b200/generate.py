@@ -23,6 +23,11 @@ Extensions (keyword-only, default = reference behaviour):
                    reference's 128x tensor duplication (cross-attention K/V shared);
   seq_index_base / n_total  place the call inside a larger logical batch so sharded
                    runs draw the Philox numbers of the unsharded run.
+  per_memory_rng=True  the n_candidates rows of each memory column draw what a separate
+                   torch.multinomial((n_candidates, V), 1) per step would, the columns'
+                   calls in order: one call over many spectra draws the ids of the
+                   reference's per-spectrum loop (seq_index_base must be a multiple of
+                   n_candidates; n_total is then the whole call's sequence count).
 """
 from __future__ import annotations
 
@@ -118,7 +123,18 @@ def duplicate_dict(data_dict, n_times):
 
 
 # ------------------------------------------------------------------- decoder
-def _decode(model, memory, src_padding_mask, config, sampling, stop_on_all_pad, n_candidates, seq_index_base, n_total):
+def _philox_advance(eng, n_candidates, n_total, max_len, per_memory_rng):
+    """Generator offset consumed by one call: max_len torch.multinomial calls over all n_total sequences, or -- per-memory
+    streams -- max_len calls over n_candidates rows for each of the n_total / n_candidates columns."""
+    if per_memory_rng:
+        return (n_total // n_candidates) * max_len * eng.philox_increment(n_candidates)
+    return eng.philox_increment(n_total) * max_len
+
+
+def _decode(model, memory, src_padding_mask, config, sampling, stop_on_all_pad, n_candidates, seq_index_base, n_total,
+            per_memory_rng=False):
+    if per_memory_rng and (sampling != "multinomial" or seq_index_base % n_candidates):
+        raise ValueError("per_memory_rng needs multinomial sampling and seq_index_base a multiple of n_candidates")
     model.eval()                                    # the reference flips eval() and leaves it
     eng = _engine.engine_for(model, config)
     prec = _engine.default_precision(config)
@@ -132,10 +148,9 @@ def _decode(model, memory, src_padding_mask, config, sampling, stop_on_all_pad, 
     tokens, probs, steps = eng.decode(memory, bias, n_cand=n_candidates, max_len=int(config.max_len),
                                       temperature=float(config.temperature), sampling=sampling,
                                       stop_on_all_pad=stop_on_all_pad, precision=prec,
-                                      seq_index_base=seq_index_base, n_total=n_total, **kw)
-    if gen is not None:   # consume exactly what max_len torch.multinomial calls would have
-        inc = eng.philox_increment(n_total if n_total else N)
-        gen.set_offset(offset + inc * int(config.max_len))
+                                      seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng, **kw)
+    if gen is not None:   # consume exactly what the torch.multinomial calls would have
+        gen.set_offset(offset + _philox_advance(eng, n_candidates, n_total if n_total else N, int(config.max_len), per_memory_rng))
     return tokens, probs, steps
 
 
@@ -155,27 +170,32 @@ def greedy_sequence_2(model, stoi, itos, memory, src_padding_mask, config, *, n_
     return tokens[:steps], probs[:steps]
 
 
-def multinomial_sequence(model, stoi, memory, src_padding_mask, config, *, n_candidates=1, seq_index_base=0, n_total=0):
+def multinomial_sequence(model, stoi, memory, src_padding_mask, config, *, n_candidates=1, seq_index_base=0, n_total=0,
+                         per_memory_rng=False):
     """-> ((T,N) i64, (N,T) f32): probabilities transposed, always max_len steps."""
     _check_sos(stoi)
-    tokens, probs, _ = _decode(model, memory, src_padding_mask, config, "multinomial", False, n_candidates, seq_index_base, n_total)
+    tokens, probs, _ = _decode(model, memory, src_padding_mask, config, "multinomial", False, n_candidates, seq_index_base, n_total,
+                               per_memory_rng)
     return tokens, probs.transpose(0, 1)
 
 
-def multinomial_sequence_multi(model, memory, src_padding_mask, stoi, config, *, n_candidates=1, seq_index_base=0, n_total=0):
+def multinomial_sequence_multi(model, memory, src_padding_mask, stoi, config, *, n_candidates=1, seq_index_base=0, n_total=0,
+                               per_memory_rng=False):
     """-> ((T,N) i64, (T,N) f32); the reference's .squeeze() drops the N axis of the
     probabilities when N == 1 (run_batch_gen_val_MMT_v15_4.py:149)."""
     _check_sos(stoi)
-    tokens, probs, _ = _decode(model, memory, src_padding_mask, config, "multinomial", False, n_candidates, seq_index_base, n_total)
+    tokens, probs, _ = _decode(model, memory, src_padding_mask, config, "multinomial", False, n_candidates, seq_index_base, n_total,
+                               per_memory_rng)
     if probs.shape[1] == 1:
         probs = probs.squeeze(1)
     return tokens, probs
 
 
-def multinomial_sequence_multi_2(model, memory, src_padding_mask, stoi, config, *, n_candidates=1, seq_index_base=0, n_total=0):
+def multinomial_sequence_multi_2(model, memory, src_padding_mask, stoi, config, *, n_candidates=1, seq_index_base=0, n_total=0,
+                                 per_memory_rng=False):
     """mrtf variant: probabilities lose their first row -> ((T,N), (T-1,N))."""
     tokens, probs = multinomial_sequence_multi(model, memory, src_padding_mask, stoi, config, n_candidates=n_candidates,
-                                               seq_index_base=seq_index_base, n_total=n_total)
+                                               seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng)
     return tokens, probs[1:]
 
 

@@ -109,14 +109,18 @@ class PendingTokens:
 
 
 def generate_sharded(model, data_dict, config, stoi, *, n_candidates=1, sampling="multinomial", gather_probs=False,
-                     group=None, async_gather=False):
+                     group=None, async_gather=False, per_memory_rng=False):
     """Encode + decode this rank's spectra and all-gather the ids.
 
     Returns (tokens (T, B*n_candidates) i64 -- identical on every rank and identical to the single-GPU run --, probs or
     None, local (lo, hi)); with ``async_gather=True`` a :class:`PendingTokens` instead, whose collective overlaps
-    whatever the caller launches next (greedy early-exit trimming is then the caller's business)."""
+    whatever the caller launches next (greedy early-exit trimming is then the caller's business).  ``per_memory_rng``:
+    every spectrum's candidates draw in their own stream (generate.multinomial_sequence_multi), so the result also
+    equals the reference's per-spectrum loop."""
     from . import generate as G
     from .engine import engine_for
+    if per_memory_rng and sampling == "greedy":
+        raise ValueError("per_memory_rng needs multinomial sampling")
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     B = next(iter(data_dict.values())).shape[0]
@@ -134,7 +138,7 @@ def generate_sharded(model, data_dict, config, stoi, *, n_candidates=1, sampling
             tok, pr, _ = G._decode(model, memory, mask, config, "greedy", False, n_candidates, 0, 0)
         else:
             tok, pr, _ = G._decode(model, memory, mask, config, "multinomial", False, n_candidates,
-                                   lo * n_candidates, B * n_candidates)
+                                   lo * n_candidates, B * n_candidates, per_memory_rng)
         packed = eng.pack_tokens_seqmajor(tok)                                   # (n_local, T) u8
     else:
         packed = torch.zeros(0, T, dtype=torch.uint8, device=eng.device)
@@ -143,7 +147,7 @@ def generate_sharded(model, data_dict, config, stoi, *, n_candidates=1, sampling
             # an empty shard draws nothing, but the unsharded run's T multinomial calls would have advanced this device's
             # generator: keep every rank's Philox offset in step so later sharded calls still reproduce the 1-GPU draws
             gen = torch.cuda.default_generators[eng.dev_index]
-            gen.set_offset(int(gen.get_offset()) + eng.philox_increment(B * n_candidates) * T)
+            gen.set_offset(int(gen.get_offset()) + G._philox_advance(eng, n_candidates, B * n_candidates, T, per_memory_rng))
     n_total = B * n_candidates
     cur = torch.cuda.current_stream(eng.device)
     if world > 1:
