@@ -186,6 +186,23 @@ int32_t mmt_decode(mmt_engine* e, const mmt_decode_args* a, int64_t* d_tokens, f
 int32_t mmt_decode_memory_streams(mmt_engine* e, const mmt_decode_args* a, int64_t* d_tokens, float* d_probs,
                                   int32_t* h_steps, void* stream);
 
+/* mmt_decode (per_memory_rng == 0) or mmt_decode_memory_streams (per_memory_rng != 0) that stops computing a sequence
+ * once it has emitted `eos`: same arguments, preconditions and draws (every sequence keeps its Philox elements, a
+ * caller's generator is advanced by the same amount).  With L_n the position of the first `eos` the plain call writes
+ * for sequence n (max_len if none):
+ *   d_tokens / d_probs  (max_len, N): bit-identical to the plain call at t <= L_n; <PAD> (0) / 0.0f after L_n and at
+ *                       t >= *h_steps
+ *   d_len   out (N) i32: L_n (mmt_first_eos of the plain call's ids)
+ *   h_steps out host int or NULL: positions up to the one at which every sequence had finished (greedy with
+ *           stop_on_all_pad: finished or emitted <PAD>), else max_len
+ *   h_rows  out host (max_len) i64 or NULL: decode-step rows computed at each position, summed over waves and lanes
+ *           (0 where no step ran)
+ * Large (un-fused) waves drop finished rows at 8-position group boundaries, from counts the host reads one group
+ * behind the launches; small waves keep their rows and only stop early.  Fails when `eos` is outside [0, vocab). */
+int32_t mmt_decode_until_eos(mmt_engine* e, const mmt_decode_args* a, int32_t per_memory_rng, int64_t eos,
+                             int64_t* d_tokens, float* d_probs, int32_t* d_len, int32_t* h_steps, int64_t* h_rows,
+                             void* stream);
+
 /* Replaces the decoder tail of MultimodalTransformer.forward(..., trg_SMI_input)
  * (models_MMT_v15_4.py:955-976) and the teacher-forced scorers' inner call:
  * d_trg (T,N) i64 -> d_logits (T,N,vocab) f32 (fc_out, before softmax). */

@@ -9,6 +9,7 @@
 #include "kernels_compact.cuh"
 #include "kernels_beam.cuh"
 #include "kernels_smiles.cuh"
+#include "kernels_retire.cuh"
 
 #include <algorithm>
 #include <cstdlib>
@@ -122,10 +123,12 @@ static int ensure_arena(mmt_engine* e, size_t bytes) {
 // ---------------------------------------------------------------------------
 // launch helpers
 // ---------------------------------------------------------------------------
-static int launch_gemm(mmt_engine* e, GemmParams& p, int ngroups, int maxM, cudaStream_t s) {
+// tile_rows > 0 picks the tile shape for that many rows instead of maxM (a compacted decode wave keeps the shape of its
+// starting size: the two shapes need not round alike)
+static int launch_gemm(mmt_engine* e, GemmParams& p, int ngroups, int maxM, cudaStream_t s, int64_t tile_rows = 0) {
     if (maxM <= 0) return 0;
     if (p.splits < 1) p.splits = 1;
-    if (maxM >= 1024) {
+    if ((tile_rows > 0 ? tile_rows : maxM) >= 1024) {
         dim3 grid((p.N + 127) / 128, (maxM + 127) / 128, ngroups * p.splits);
         prof_pre(e, s);
         gemm_nt_f32<128, 128, 8, 8><<<grid, 256, 0, s>>>(p);
@@ -924,10 +927,19 @@ struct DecBuffers {
     uint64_t* rng_state;   // {philox seed, offset of step 0} of this call (read by the sampler from device memory)
     // bf16 operand copies (tensor-core mode)
     __nv_bfloat16 *x16, *att16, *h16, *mem16;
+    // stop at <EOS> (mmt_decode_until_eos, kernels_retire.cuh), nullptr / 0 otherwise.  plan_rows: the wave's starting size,
+    // which fixes every kernel-variant decision of the un-fused step through its compactions (bit identity with the plain
+    // call).  orig / col_start / col_count: the compacted wave's row -> sequence map and per-column rows (nullptr until the
+    // first compaction).  eos_len: first-<EOS> step per sequence of the lane.  rt_*: compaction storage.
+    int64_t plan_rows;
+    const int *orig, *col_start, *col_count;
+    int* eos_len;
+    int *rt_orig[2], *rt_bt, *rt_src, *rt_col_start, *rt_col_count;
 };
 constexpr int MAX_SPLITS = 32;
 
-static void plan_decoder(Arena& a, const mmt_model_desc& d, int64_t Nw, int Bmw, int S, int max_len, DecBuffers& b, bool bf16, int fused_rows, int kv_copies = 1) {
+static void plan_decoder(Arena& a, const mmt_model_desc& d, int64_t Nw, int Bmw, int S, int max_len, DecBuffers& b, bool bf16, int fused_rows, int kv_copies = 1,
+                         bool retire = false) {
     const int L = d.n_dec_layers;
     const int pps = (max_len + PAGE_TOKENS - 1) / PAGE_TOKENS;
     b.x = a.get<float>(Nw * D);
@@ -959,6 +971,12 @@ static void plan_decoder(Arena& a, const mmt_model_desc& d, int64_t Nw, int Bmw,
         b.h16 = nullptr;   // fused FFN: no hidden activation in HBM
         b.mem16 = a.get<__nv_bfloat16>(R * D);
     }
+    b.plan_rows = 0; b.orig = b.col_start = b.col_count = nullptr; b.eos_len = nullptr;
+    b.rt_orig[0] = b.rt_orig[1] = b.rt_bt = b.rt_src = b.rt_col_start = b.rt_col_count = nullptr;
+    if (retire) {
+        b.rt_orig[0] = a.get<int>(Nw); b.rt_orig[1] = a.get<int>(Nw); b.rt_bt = a.get<int>(Nw * pps); b.rt_src = a.get<int>(Nw);
+        b.rt_col_start = a.get<int>(Bmw); b.rt_col_count = a.get<int>(Bmw);
+    }
 }
 
 // Page map of a wave: page j of sequence n is physical page j * Nw + n ("slot-major").  At position t every sequence reads its
@@ -980,6 +998,9 @@ struct DecodeRun {
     int64_t ldn = -1;         // >= 0 overrides the leading dimension (0: single-row token / logit buffers, beam search)
     bool serial_first = false;   // the step's first kernel waits for full completion of its predecessor (its prologue reads the block table)
     bool per_memory_rng = false; // multinomial draws in per-memory streams (torch_rng_row): one (n_cand, V) call per column and step
+    int64_t eos = -1;            // >= 0: stop at this id (mmt_decode_until_eos): finished sequences retire from large waves
+    int32_t* len = nullptr;      //   out (N) first-<EOS> positions
+    int64_t* h_rows = nullptr;   //   out (T), optional: rows computed per position
 };
 
 // Projects the memory of one wave to per-layer cross-attention K/V (head-major) once;
@@ -1042,7 +1063,7 @@ static int decode_self_attention_layer(mmt_engine* e, const LayerW& w, const Dec
         GemmParams p = gemm_params(3 * D, D, 3 * D, 0);
         p.g[0].A = b.x; p.g[0].lda = D; p.g[0].W = w.in_w; p.g[0].bias = w.in_b; p.g[0].C = b.qkv; p.g[0].M = M;
         p.splits = 1; p.part_stride = Nw * D;
-        MMT_TRY(launch_gemm(e, p, 1, M, s));
+        MMT_TRY(launch_gemm(e, p, 1, M, s, b.plan_rows));
     }
     prof_pre(e, s);
     const unsigned sa_blocks = (unsigned)((Nw * (H / 4) + 7) / 8);     // a warp per (sequence, 4 heads)
@@ -1065,15 +1086,16 @@ static int decode_cross_attention_layer(mmt_engine* e, const mmt_decode_args& a,
     const unsigned attn_blocks = (unsigned)((Nw * H + 7) / 8);
     prof_pre(e, s);
     if (bf16 && a.n_cand >= 8 && e->use_tc_attention)
-        launch_args(decode_cross_attention_tc, dim3(H, Bmw), dim3(256), dx_smem_bytes(a.S), s, pdl_u, (const float*)b.qc, reinterpret_cast<const __nv_bfloat16*>(ckv), (int64_t)a.S, (const int*)b.nk, (const int*)b.row_start, (const float*)b.kbias_c, (int)a.n_cand, H, scale, (float*)nullptr, b.att16);
-    else if (bf16) launch_args(decode_cross_attention<8, __nv_bfloat16>, dim3(attn_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qc, reinterpret_cast<const __nv_bfloat16*>(ckv), (int64_t)a.S, (const int*)b.nk, (const int*)b.row_start, (const float*)b.kbias_c, (int)a.n_cand, Nw, H, scale, (float*)nullptr, b.att16);
-    else decode_cross_attention<8, float><<<attn_blocks, 256, 0, s>>>(b.qc, reinterpret_cast<const float*>(ckv), a.S, b.nk, b.row_start, b.kbias_c, a.n_cand, Nw, H, scale, b.att, b.att16);
+        launch_args(decode_cross_attention_tc, dim3(H, Bmw), dim3(256), dx_smem_bytes(a.S), s, pdl_u, (const float*)b.qc, reinterpret_cast<const __nv_bfloat16*>(ckv), (int64_t)a.S, (const int*)b.nk, (const int*)b.row_start, (const float*)b.kbias_c, (int)a.n_cand, H, scale, (float*)nullptr, b.att16, b.col_start, b.col_count);
+    else if (bf16) launch_args(decode_cross_attention<8, __nv_bfloat16>, dim3(attn_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qc, reinterpret_cast<const __nv_bfloat16*>(ckv), (int64_t)a.S, (const int*)b.nk, (const int*)b.row_start, (const float*)b.kbias_c, (int)a.n_cand, Nw, H, scale, (float*)nullptr, b.att16, b.orig);
+    else decode_cross_attention<8, float><<<attn_blocks, 256, 0, s>>>(b.qc, reinterpret_cast<const float*>(ckv), a.S, b.nk, b.row_start, b.kbias_c, a.n_cand, Nw, H, scale, b.att, b.att16, b.orig);
     return check_launch(e, "decode_cross_attention", s);
 }
 
 // Launches of the decode step over the Nw rows of one wave; the residual stream is b.x (fp32) with its bf16 copy b.x16.
 struct DecOps {
     mmt_engine* e; const DecBuffers& b; int64_t Nw; bool pdl_u; cudaStream_t s;
+    int64_t plan() const { return b.plan_rows > 0 ? b.plan_rows : Nw; }     // rows that decide the kernel variants
     // x = LN(x + bias + sum_s part[s]) (separate kernel; fp32 mode and split-K FFN2)
     int ln(const float* part, int splits, const float* bias, const float* gamma, const float* beta) const {
         LnParams q;
@@ -1088,7 +1110,7 @@ struct DecOps {
         GemmParams p = gemm_params(N, K, N, act);
         p.g[0].A = A; p.g[0].lda = lda; p.g[0].W = W; p.g[0].bias = bias; p.g[0].C = C; p.g[0].M = (int)Nw;
         p.splits = splits; p.part_stride = Nw * D;
-        return launch_gemm(e, p, 1, (int)Nw, s);
+        return launch_gemm(e, p, 1, (int)Nw, s, plan());
     }
     // The four attention projections of the un-fused step run on the hi term of the bf16 weight split alone, like the small-wave
     // kernel's (decode_attn keeps only the hi terms in shared memory): one weight slab per stage -> 68 KB instead of 100 KB of
@@ -1125,7 +1147,7 @@ static int decode_self_tail_layer(const DecOps& o, const LayerW& w, bool bf16) {
         // out-proj + LN1 and the cross-attention query projection as one launch -- for waves up to 24,576 rows: the chained
         // kernel holds 192 KB of shared memory (one CTA per SM instead of three), which costs more than the saved launch
         // once there are several tiles per SM (measured: 1383 -> 1357 us per position at 16,384 rows, 4851 -> 4901 at 65,536)
-        if (o.e->use_gemm_chain && o.Nw <= 24576) {
+        if (o.e->use_gemm_chain && o.plan() <= 24576) {
             const TcChain ch{o.e->Wb(w.ca_in_w), o.plo(w.ca_in_w), w.ca_in_b, b.qc, D};
             MMT_TRY(o.tc_ln(b.att16, D, w.out_w, w.out_b, D, w.n1_w, w.n1_b, &ch));
         } else {
@@ -1153,9 +1175,9 @@ static int decode_cross_tail_layer(const DecOps& o, const LayerW& w, int l, bool
         return 0;
     };
     if (bf16) {
-        const bool ffn_pro = e->use_ffn_prologue && M >= 2048;     // cross-attention out-projection + norm2 as the FFN kernel's prologue
+        const bool ffn_pro = e->use_ffn_prologue && o.plan() >= 2048;     // cross-attention out-projection + norm2 as the FFN kernel's prologue
         if (!ffn_pro) { MMT_TRY(o.tc_ln(b.att16, D, w.ca_out_w, w.ca_out_b, D, w.n2_w, w.n2_b)); MMT_TRY(keep_x2()); }
-        if (M >= 2048) {
+        if (o.plan() >= 2048) {
             FfnParams f = ffn_params(M, F);
             f.b1 = w.l1_b; f.bias = w.l2_b; f.res = b.x; f.gamma = w.n3_w; f.beta = w.n3_b; f.out_f32 = b.x; f.out_b16 = b.x16;
             if (getenv("MMT_FFN_DEBUG")) {     // phase stamps of the layer-3 FFN launch (printed by run_decode)
@@ -1179,7 +1201,7 @@ static int decode_cross_tail_layer(const DecOps& o, const LayerW& w, int l, bool
         MMT_TRY(o.ln(b.part, 1, w.ca_out_b, w.n2_w, w.n2_b));
         MMT_TRY(keep_x2());
         MMT_TRY(o.gemm(b.x, D, w.l1_w, w.l1_b, b.h, F, D, 1, 1));
-        int splits = pick_splits(M, D, F);
+        int splits = pick_splits((int)o.plan(), D, F);
         if ((int64_t)splits * o.Nw > b.part_rows) MMT_FAIL("decode: FFN partial buffer too small for this wave (plan_decoder)");
         MMT_TRY(o.gemm(b.h, F, w.l2_w, nullptr, b.part, D, F, 0, splits));
         MMT_TRY(o.ln(b.part, splits, w.l2_b, w.n3_w, w.n3_b));
@@ -1203,13 +1225,14 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
     // fused kernels per layer replace the chain of projection / attention / LayerNorm launches
     // (kernels_decode.cuh); the previous layer's FFN2 split-K partials + norm3 are folded into the
     // next kernel's prologue (the sampler's for the last layer).
-    const bool fused = e->fused_decode_rows > 0 && Nw <= e->fused_decode_rows;
+    const int64_t P = b.plan_rows > 0 ? b.plan_rows : Nw;     // a compacted wave keeps the variants of its starting size
+    const bool fused = e->fused_decode_rows > 0 && P <= e->fused_decode_rows;
     const bool pdl = fused && e->use_pdl && !e->profiling;
     // un-fused tensor-core step: the same attribute through the chain of 31 launches (every kernel of the chain waits with
     // griddepcontrol.wait before it touches its predecessor's output; the LayerNorm-only kernel has no hook and is launched plainly)
     // Only for moderate waves: measured 50.2 -> 45.2 ms for a beam search over 2560 slots, but 1426 -> 1473 us per position at
     // 16,384 sequences, where the early-scheduled CTAs take SM resources from a predecessor that is throughput-bound.
-    const bool pdl_u = !fused && bf16 && e->use_pdl && !e->profiling && Nw <= e->pdl_rows;
+    const bool pdl_u = !fused && bf16 && e->use_pdl && !e->profiling && P <= e->pdl_rows;
     const DecOps o{e, b, Nw, pdl_u, s};
     int ffn_splits = 1;
     if (fused) {
@@ -1281,8 +1304,8 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
         }
     } else {
         prof_pre(e, s);
-        if (r.trg) launch_args(decode_embed, dim3((unsigned)((Nw + 3) / 4)), dim3(128), 0, s, pdl_u, r.trg + n0, 0, 3, Nw, ldn, e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, step, b.x, b.x16);
-        else launch_args(decode_embed, dim3((unsigned)((Nw + 3) / 4)), dim3(128), 0, s, pdl_u, (const int64_t*)(r.tokens + n0), 1, 3, Nw, ldn, e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, step, b.x, b.x16);
+        if (r.trg) launch_args(decode_embed, dim3((unsigned)((Nw + 3) / 4)), dim3(128), 0, s, pdl_u, r.trg + n0, 0, 3, Nw, ldn, e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, step, b.x, b.x16, b.orig);
+        else launch_args(decode_embed, dim3((unsigned)((Nw + 3) / 4)), dim3(128), 0, s, pdl_u, (const int64_t*)(r.tokens + n0), 1, 3, Nw, ldn, e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, step, b.x, b.x16, b.orig);
         MMT_TRY(check_launch(e, "decode_embed", s));
 
         for (int l = 0; l < d.n_dec_layers; ++l) {
@@ -1313,6 +1336,7 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
     sp.target = r.target ? r.target + n0 : nullptr; sp.target_prob = r.target_prob ? r.target_prob + n0 : nullptr;
     sp.ctl.step = b.ctl; sp.ctl.done_ctas = b.ctl + 1; sp.ctl.nonpad = (r.mode == 0) ? b.ctl + 8 : nullptr;
     sp.advance = 1;
+    if (b.eos_len) { sp.orig = b.orig; sp.eos_len = b.eos_len; sp.live = b.ctl + 8 + 128; sp.eos = r.eos; }
     if (fused && ffn_splits > 0) {   // norm3 of the last layer over the FFN2 partials (the cluster variant has applied it)
         const LayerW& pw = e->dec[d.n_dec_layers - 1];
         sp.part = b.part; sp.splits = ffn_splits; sp.part_stride = Nw * D;
@@ -1320,7 +1344,7 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
     }
     prof_pre(e, s);
     {   // rows per CTA and pass: 2 when the input is still spread over FFN2 partials, else 8; at most four resident waves of CTAs
-        sp.rows_per_warp = Nw >= 8192 ? SAMPLE_NR : 1;       // small waves: one row per warp (latency), large: four (shared-memory traffic)
+        sp.rows_per_warp = P >= 8192 ? SAMPLE_NR : 1;       // small waves: one row per warp (latency), large: four (shared-memory traffic)
         const int rpc = sp.part ? 2 : 8 * sp.rows_per_warp;
         const int64_t groups = (Nw + rpc - 1) / rpc;
         MMT_TRY(sample_init(e));
@@ -1377,13 +1401,19 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     // Single-wave sampling runs write ids / probabilities into engine-owned staging buffers (copied to the caller's
     // tensors at the end): nothing a captured decode-step graph touches then depends on the caller's allocations, so the
     // instantiated graph is reused across calls (capture + instantiation of ~400 nodes costs ~1.2 ms with the GPU idle).
-    const bool staged = e->use_graph && e->use_graph_cache && !e->profiling && n_waves == 1 && r.mode != 2 && !r.trg;   // forced inputs are the caller's tensor: nothing to cache across calls
+    // (A retiring call's large waves capture graphs specific to its sequences' lengths, which are not cached; its small
+    // waves never compact, so their one graph is cached like the plain call's.)
+    const bool retire = r.eos >= 0;
+    const bool small_wave = e->fused_decode_rows > 0 && (int64_t)Bm_wave * a.n_cand <= e->fused_decode_rows;
+    const bool staged = e->use_graph && e->use_graph_cache && !e->profiling && n_waves == 1 && r.mode != 2 && !r.trg && (!retire || small_wave);   // forced inputs are the caller's tensor: nothing to cache across calls
     Arena ar;
     DecBuffers lb[MAX_LANES];
     int64_t* st_tokens = nullptr; float* st_probs = nullptr;
+    int* eos_all = nullptr;                  // retiring call: first-<EOS> step of every sequence (max_len until it emits)
     auto plan_all = [&]() {
-        for (int i = 0; i < NL; ++i) plan_decoder(ar, d, (int64_t)Bm_lane * a.n_cand, Bm_lane, a.S, a.max_len, lb[i], bf16, e->fused_decode_rows);
+        for (int i = 0; i < NL; ++i) plan_decoder(ar, d, (int64_t)Bm_lane * a.n_cand, Bm_lane, a.S, a.max_len, lb[i], bf16, e->fused_decode_rows, 1, retire);
         if (staged) { st_tokens = ar.get<int64_t>((size_t)a.max_len * N_total); st_probs = ar.get<float>((size_t)a.max_len * N_total); }
+        if (retire) eos_all = ar.get<int>(N_total);
     };
     ar.plan = true;
     plan_all();
@@ -1396,6 +1426,12 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     const bool early = (r.mode == 0) && a.stop_on_all_pad && n_waves == 1;
     int steps_done = r.T;
     std::vector<int64_t> nonpad_total(r.T, 0);
+    std::vector<int64_t> live_total(r.T, 0), rows_at(r.T, 0);     // retiring call
+    if (retire) {
+        fill_i32<<<(unsigned)((N_total + 255) / 256), 256, 0, s>>>(eos_all, N_total, a.max_len);
+        MMT_CUDA(cudaGetLastError());
+        for (int i = 0; i < 2; ++i) if (!e->poll_ev[i]) MMT_CUDA(cudaEventCreateWithFlags(&e->poll_ev[i], cudaEventDisableTiming));
+    }
     for (int wv = 0; wv < n_waves; ++wv) {
         const int wb0 = wv * Bm_wave;
         const int Bmw = std::min(Bm_wave, a.Bm - wb0);
@@ -1413,12 +1449,16 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
             init_block_table<<<(unsigned)((lane[i].Nw * pps + 255) / 256), 256, 0, s>>>(b.block_table, lane[i].Nw, pps);
             MMT_TRY(check_launch(e, "init_block_table", s));
             MMT_TRY(decode_prepare_wave(e, a, lane[i].b0, lane[i].Bm, b, bf16, s));
+            if (retire) { b.plan_rows = lane[i].Nw; b.orig = b.col_start = b.col_count = nullptr; b.eos_len = eos_all + lane[i].n0; }
         }
+        int64_t rows[MAX_LANES];              // rows of each lane's wave (a retiring call's large waves shrink)
+        for (int i = 0; i < nl; ++i) rows[i] = lane[i].Nw;
         // One decode step is the same kernel sequence at every position (the step counter lives on
         // the device), so a group of U consecutive steps of every lane is captured once per wave into a CUDA
         // graph (programmatic-dependent-launch edges included) and replayed T / U times.
         int U = 1;
         for (int u = 2; u <= e->graph_steps; ++u) if (r.T % u == 0) U = u;
+        if (retire) U = std::min(r.T, 8);     // groups of 8 positions (a shorter last group runs without a graph)
         cudaGraphExec_t exec = nullptr;
         int64_t launches_per_group = 0;
         std::vector<uint64_t> key;            // every value baked into the graph's nodes
@@ -1428,12 +1468,13 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
             put((uint64_t)r.mode); put((uint64_t)r.T); put((uint64_t)(r.probs != nullptr)); put((uint64_t)a.S); put((uint64_t)a.Bm);
             put((uint64_t)a.n_cand); put((uint64_t)a.max_len); put(tbits); put((uint64_t)a.precision);
             put((uint64_t)a.seq_index_base); put((uint64_t)a.N_total); put((uint64_t)a.rng_sm_count); put((uint64_t)a.rng_max_threads_per_sm);
-            put((uint64_t)r.per_memory_rng);
+            put((uint64_t)r.per_memory_rng); put((uint64_t)r.eos);
             put((uint64_t)(uintptr_t)e->arena); put((uint64_t)e->arena_bytes); put((uint64_t)nl); put((uint64_t)U);
             put((uint64_t)e->fused_decode_rows); put((uint64_t)e->use_pdl); put((uint64_t)(uintptr_t)e->da_dbg);
             for (auto& c : e->graph_cache) if (c.key == key) { exec = c.exec; launches_per_group = c.launches_per_group; c.stamp = ++e->graph_cache_clock; break; }
         }
-        if (e->use_graph && !e->profiling && !exec) {
+        // capture U steps of the lanes that still have rows into `exec`
+        auto capture = [&]() -> int {
             if (bf16) MMT_TRY(tc_init(e));
             for (int i = 0; i < nl; ++i) {
                 if (!e->cap_stream[i]) MMT_CUDA(cudaStreamCreateWithFlags(&e->cap_stream[i], cudaStreamNonBlocking));
@@ -1445,11 +1486,12 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
             cudaError_t fe = cudaSuccess;
             if (nl > 1) {                                 // fork the other lanes' branches off the capture origin
                 fe = cudaEventRecord(e->lane_ev[0], e->cap_stream[0]);
-                for (int i = 1; i < nl && fe == cudaSuccess; ++i) fe = cudaStreamWaitEvent(e->cap_stream[i], e->lane_ev[0], 0);
+                for (int i = 1; i < nl && fe == cudaSuccess; ++i) if (rows[i] > 0) fe = cudaStreamWaitEvent(e->cap_stream[i], e->lane_ev[0], 0);
             }
             for (int u = 0; u < U && !rc && fe == cudaSuccess; ++u)
-                for (int i = 0; i < nl && !rc; ++i) rc = decode_step(e, rs, lane[i].n0, lane[i].Nw, lane[i].Bm, lb[i], bf16, e->cap_stream[i]);
+                for (int i = 0; i < nl && !rc; ++i) if (rows[i] > 0) rc = decode_step(e, rs, lane[i].n0, rows[i], lane[i].Bm, lb[i], bf16, e->cap_stream[i]);
             for (int i = 1; i < nl && fe == cudaSuccess; ++i) {   // join
+                if (rows[i] == 0) continue;
                 fe = cudaEventRecord(e->lane_ev[i], e->cap_stream[i]);
                 if (fe == cudaSuccess) fe = cudaStreamWaitEvent(e->cap_stream[0], e->lane_ev[i], 0);
             }
@@ -1463,6 +1505,10 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
             ce = cudaGraphInstantiate(&exec, graph, 0);
             cudaGraphDestroy(graph);
             if (ce != cudaSuccess) MMT_FAIL(std::string("cudaGraphInstantiate failed: ") + cudaGetErrorString(ce));
+            return 0;
+        };
+        if (e->use_graph && !e->profiling && !exec) {
+            MMT_TRY(capture());
             if (staged) {
                 if (e->graph_cache.size() >= 4) {      // evict the least recently used entry
                     size_t lru = 0;
@@ -1472,10 +1518,75 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
                 }
                 e->graph_cache.push_back({key, exec, launches_per_group, ++e->graph_cache_clock});
             }
-        } else if (!exec) {
+        } else if (!exec && !retire) {
             U = 1;
         }
         struct ExecGuard { cudaGraphExec_t x; ~ExecGuard() { if (x) cudaGraphExecDestroy(x); } } guard{staged ? nullptr : exec};
+        if (retire) {
+            // Groups of U positions; after group g is enqueued, its per-step counts are copied back (poll g) and the host
+            // reads poll g - 1, whose group the GPU has finished while it runs group g.  A large lane whose live rows at the
+            // end of group g - 1 are at most 7/8 of its wave is compacted to those rows before group g + 1 (rows finished
+            // during group g ride along once, masked), and the group graph is captured again for the smaller wave.
+            // Small (fused) waves are latency chains that fewer rows do not shorten: they only stop once all have finished.
+            const bool pad_stop = n_waves == 1 && r.mode == 0 && a.stop_on_all_pad;
+            int g = 0, tpoll[2] = {0, 0};
+            bool stop = false;
+            for (int t = 0; t < r.T && !stop;) {
+                const int n = std::min(U, r.T - t);
+                if (exec && n == U) { MMT_CUDA(cudaGraphLaunch(exec, s)); e->launches += launches_per_group; }
+                else for (int q = 0; q < n; ++q) for (int i = 0; i < nl; ++i) if (rows[i] > 0) MMT_TRY(decode_step(e, rs, lane[i].n0, rows[i], lane[i].Bm, lb[i], bf16, s));
+                for (int q = t; q < t + n; ++q) for (int i = 0; i < nl; ++i) rows_at[q] += rows[i];
+                t += n;
+                for (int i = 0; i < nl; ++i)       // nonpad [0, 128) | live [128, 256)
+                    MMT_CUDA(cudaMemcpyAsync(e->h_pinned + (g & 1) * 1024 + i * 256, lb[i].ctl + 8, 256 * sizeof(int), cudaMemcpyDeviceToHost, s));
+                MMT_CUDA(cudaEventRecord(e->poll_ev[g & 1], s));
+                tpoll[g & 1] = t - 1;
+                ++g;
+                if (g < 2 || t >= r.T) continue;
+                const int k = (g - 2) & 1, tp = tpoll[k];
+                MMT_CUDA(cudaEventSynchronize(e->poll_ev[k]));
+                const int32_t* cnt = e->h_pinned + k * 1024;
+                for (int q = 0; q <= tp && !stop; ++q) {
+                    int64_t live = 0, nonpad = 0;
+                    for (int i = 0; i < nl; ++i) { live += cnt[i * 256 + 128 + q]; nonpad += cnt[i * 256 + q]; }
+                    stop = live == 0 || (pad_stop && nonpad == 0);
+                }
+                if (stop) break;
+                bool changed = false;
+                for (int i = 0; i < nl; ++i) {
+                    const int64_t live = cnt[i * 256 + 128 + tp];
+                    if (rows[i] == 0 || lb[i].plan_rows <= e->fused_decode_rows || live * 8 > rows[i] * 7) continue;
+                    DecBuffers& b = lb[i];
+                    if (live > 0) {
+                        int* orig_new = b.orig == b.rt_orig[0] ? b.rt_orig[1] : b.rt_orig[0];
+                        MMT_CUDA(cudaMemsetAsync(b.rt_col_count, 0, lane[i].Bm * sizeof(int), s));
+                        prof_pre(e, s);
+                        retire_scan<<<1, 1024, 0, s>>>(b.orig, b.eos_len, rows[i], tp, b.rt_src);
+                        MMT_TRY(check_launch(e, "retire_scan", s));
+                        prof_pre(e, s);
+                        retire_gather<<<(unsigned)((live + 255) / 256), 256, 0, s>>>(b.rt_src, b.orig, b.block_table, pps, live, a.n_cand, orig_new,
+                                                                                     b.rt_bt, b.rt_col_start, b.rt_col_count);
+                        MMT_TRY(check_launch(e, "retire_gather", s));
+                        std::swap(b.block_table, b.rt_bt);
+                        b.orig = orig_new; b.col_start = b.rt_col_start; b.col_count = b.rt_col_count;
+                    }
+                    rows[i] = live;
+                    changed = true;
+                }
+                if (changed && exec) {
+                    cudaGraphExecDestroy(exec);
+                    exec = guard.x = nullptr;
+                    MMT_TRY(capture());
+                    guard.x = exec;
+                }
+            }
+            // the last poll holds the wave's complete counts
+            MMT_CUDA(cudaEventSynchronize(e->poll_ev[(g - 1) & 1]));
+            const int32_t* cnt = e->h_pinned + ((g - 1) & 1) * 1024;
+            for (int i = 0; i < nl; ++i)
+                for (int q = 0; q < r.T; ++q) { nonpad_total[q] += cnt[i * 256 + q]; live_total[q] += cnt[i * 256 + 128 + q]; }
+            continue;
+        }
         // greedy early exit (validate_generate_MMT_v15_4.py:763): the per-step non-PAD counts are polled one
         // group behind the launches, so the host never drains the stream inside the loop
         if (early) for (int i = 0; i < 2; ++i) if (!e->poll_ev[i]) MMT_CUDA(cudaEventCreateWithFlags(&e->poll_ev[i], cudaEventDisableTiming));
@@ -1519,8 +1630,16 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
         MMT_CUDA(cudaMemcpyAsync(r.tokens, st_tokens, (size_t)r.T * N_total * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
         if (r.probs) MMT_CUDA(cudaMemcpyAsync(r.probs, st_probs, (size_t)r.T * N_total * sizeof(float), cudaMemcpyDeviceToDevice, s));
     }
-    if ((r.mode == 0) && a.stop_on_all_pad && n_waves > 1)
+    if ((r.mode == 0) && a.stop_on_all_pad && n_waves > 1 && !retire)
         for (int q = 0; q < r.T; ++q) if (nonpad_total[q] == 0) { steps_done = q + 1; break; }
+    if (retire) {   // every sequence finished (or, greedy stop_on_all_pad, finished or emitted <PAD>) at step q
+        for (int q = 0; q < r.T; ++q)
+            if (live_total[q] == 0 || ((r.mode == 0) && a.stop_on_all_pad && nonpad_total[q] == 0)) { steps_done = q + 1; break; }
+        prof_pre(e, s);
+        retire_fill<<<(unsigned)(((int64_t)r.T * N_total + 255) / 256), 256, 0, s>>>(r.tokens, r.probs, r.T, N_total, eos_all, steps_done, r.len);
+        MMT_TRY(check_launch(e, "retire_fill", s));
+        if (r.h_rows) for (int q = 0; q < r.T; ++q) r.h_rows[q] = rows_at[q];
+    }
     if (h_steps) *h_steps = steps_done;
     if (e->ffn_dbg) {  // MMT_FFN_DEBUG: un-fused FFN launch of layer 3, last position
         MMT_CUDA(cudaStreamSynchronize(s));
@@ -1753,7 +1872,7 @@ int32_t mmt_create(const mmt_model_desc* desc, const float* h_weights, int64_t n
     if (cudaMalloc(&e->w16lo, n_floats * sizeof(__nv_bfloat16)) != cudaSuccess) return fail("cudaMalloc bf16 weights (low term) failed");
     f32_to_bf16_split<<<(unsigned)((n_floats + 255) / 256), 256>>>(e->w32, n_floats, e->w16, e->w16lo);
     if (cudaDeviceSynchronize() != cudaSuccess) return fail(std::string("bf16 weight conversion failed: ") + cudaGetErrorString(cudaGetLastError()));
-    if (cudaMallocHost(&e->h_pinned, 1024 * sizeof(int32_t)) != cudaSuccess) return fail("cudaMallocHost failed");
+    if (cudaMallocHost(&e->h_pinned, 2048 * sizeof(int32_t)) != cudaSuccess) return fail("cudaMallocHost failed");
     for (int k = 0; k < 6; ++k) {
         e->enc[k].resize(desc->n_enc_layers);
         for (int l = 0; l < desc->n_enc_layers; ++l) fill_layer(e, e->enc[k][l], std::string(kEncNames[k]) + ".layers." + std::to_string(l), false);
@@ -1853,6 +1972,24 @@ int32_t mmt_decode_memory_streams(mmt_engine* e, const mmt_decode_args* a, int64
     DecodeRun r;
     r.a = a; r.mode = a->sampling; r.trg = nullptr; r.T = a->max_len; r.tokens = d_tokens; r.probs = d_probs; r.logits = nullptr;
     r.per_memory_rng = true;
+    return run_decode(e, r, h_steps, (cudaStream_t)stream);
+}
+
+int32_t mmt_decode_until_eos(mmt_engine* e, const mmt_decode_args* a, int32_t per_memory_rng, int64_t eos, int64_t* d_tokens, float* d_probs,
+                             int32_t* d_len, int32_t* h_steps, int64_t* h_rows, void* stream) {
+    if (!e || !a) MMT_FAIL("null engine / args");
+    if (!d_tokens || !d_len) MMT_FAIL("mmt_decode_until_eos: d_tokens and d_len are required");
+    if (a->sampling != MMT_SAMPLE_GREEDY && a->sampling != MMT_SAMPLE_MULTINOMIAL) MMT_FAIL("bad sampling mode");
+    if (per_memory_rng) {
+        if (a->sampling != MMT_SAMPLE_MULTINOMIAL) MMT_FAIL("mmt_decode_until_eos: per-memory RNG streams need multinomial sampling");
+        if (a->n_cand <= 0 || a->seq_index_base < 0 || a->seq_index_base % a->n_cand)
+            MMT_FAIL("mmt_decode_until_eos: seq_index_base must be a non-negative multiple of n_cand");
+    }
+    if (eos < 0 || eos >= e->desc.vocab) MMT_FAIL("mmt_decode_until_eos: eos must be in [0, vocab)");
+    EngineCall call(e, (cudaStream_t)stream);
+    DecodeRun r;
+    r.a = a; r.mode = a->sampling; r.trg = nullptr; r.T = a->max_len; r.tokens = d_tokens; r.probs = d_probs; r.logits = nullptr;
+    r.per_memory_rng = per_memory_rng != 0; r.eos = eos; r.len = d_len; r.h_rows = h_rows;
     return run_decode(e, r, h_steps, (cudaStream_t)stream);
 }
 

@@ -867,19 +867,20 @@ struct StepCtl {
     int* nonpad;        // [max_len] count of non-<PAD> picks per step
 };
 
-// x[n] = E_tok[token_in(t, n)] + E_pos[t]        (validate_generate_MMT_v15_4.py:746-747)
+// x[n] = E_tok[token_in(t, n)] + E_pos[t]        (validate_generate_MMT_v15_4.py:746-747); orig (compacted wave) or nullptr
 __global__ void __launch_bounds__(128) decode_embed(const int64_t* tokens, int tok_shift, int sos, int64_t N, int64_t ldn,
                                                     const float* E_tok, const float* E_pos, int vocab,
-                                                    const int* step, float* x, __nv_bfloat16* x_bf16) {
+                                                    const int* step, float* x, __nv_bfloat16* x_bf16, const int* orig) {
     pdl_launch_dependents();
     pdl_wait();
     const int t = *step;
     const int64_t n = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
     if (n >= N) return;
     const int lane = threadIdx.x & 31;
+    const int64_t col = orig ? orig[n] : n;      // compacted wave (kernels_retire.cuh): row n is sequence orig[n]
     int64_t tok;
-    if (tok_shift) tok = (t == 0) ? sos : tokens[(int64_t)(t - 1) * ldn + n];
-    else tok = tokens[(int64_t)t * ldn + n];
+    if (tok_shift) tok = (t == 0) ? sos : tokens[(int64_t)(t - 1) * ldn + col];
+    else tok = tokens[(int64_t)t * ldn + col];
     if (tok < 0 || tok >= vocab) tok = 0;
     float4 a = *reinterpret_cast<const float4*>(E_tok + tok * D + lane * 4);
     float4 b = *reinterpret_cast<const float4*>(E_pos + (int64_t)t * D + lane * 4);
@@ -1168,7 +1169,7 @@ template <int DH, typename KVT>
 __global__ void __launch_bounds__(256) decode_cross_attention(const float* q_in, const KVT* kv, int64_t rows_total,
                                                               const int* nk, const int* row_start, const float* kbias_c,
                                                               int n_cand, int64_t N, int H, float scale, float* out,
-                                                              __nv_bfloat16* out16) {
+                                                              __nv_bfloat16* out16, const int* orig) {
     static_assert(DH == 8, "8-element key rows");
     typedef KvRow<KVT> KV;
     pdl_launch_dependents();
@@ -1178,7 +1179,7 @@ __global__ void __launch_bounds__(256) decode_cross_attention(const float* q_in,
     const int lane = threadIdx.x & 31;
     const int64_t n = w / H;
     const int h = (int)(w % H);
-    const int64_t b = n / n_cand;
+    const int64_t b = (orig ? orig[n] : n) / n_cand;      // compacted wave: row n is sequence orig[n]
     const int cnt = nk[b];
     const int64_t r0 = row_start[b];
     // one contiguous K/V block per spectrum: [K|V][H][S][DH], S = rows reserved per spectrum (r0 = b * S)
@@ -1239,13 +1240,18 @@ __host__ __device__ inline size_t dx_smem_bytes(int key_bound) {
 }
 __global__ void __launch_bounds__(256) decode_cross_attention_tc(const float* q_in, const __nv_bfloat16* kv, int64_t rows_total,
                                                                  const int* nk, const int* row_start, const float* kbias_c,
-                                                                 int n_cand, int H, float scale, float* out, __nv_bfloat16* out16) {
+                                                                 int n_cand, int H, float scale, float* out, __nv_bfloat16* out16,
+                                                                 const int* col_start, const int* col_count) {
     extern __shared__ __align__(16) unsigned char dx_smem[];
     constexpr int DH = 8;
     constexpr float LOG2E = 1.4426950408889634f;
     pdl_launch_dependents();
     const int h = blockIdx.x;
     const int64_t b = blockIdx.y;
+    // compacted wave (kernels_retire.cuh): column b's candidates are rows col_start[b] .. + col_count[b]
+    const int nc = col_count ? col_count[b] : n_cand;
+    const int64_t row0 = col_count ? (int64_t)col_start[b] : b * n_cand;
+    if (nc == 0) return;
     const int cnt = nk[b];
     const int64_t r0 = row_start[b];
     const int nkp_max = dx_keys_padded((int)rows_total), nkp = dx_keys_padded(cnt);
@@ -1277,14 +1283,14 @@ __global__ void __launch_bounds__(256) decode_cross_attention_tc(const float* q_
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
     const int gq = lane >> 2, tq = lane & 3;
     const float qscale = scale * LOG2E;
-    for (int tile = warp; tile * 16 < n_cand; tile += nwarps) {
+    for (int tile = warp; tile * 16 < nc; tile += nwarps) {
         const int c_lo = tile * 16 + gq, c_hi = c_lo + 8;
-        const int64_t n_lo = b * n_cand + c_lo, n_hi = b * n_cand + c_hi;
+        const int64_t n_lo = row0 + c_lo, n_hi = row0 + c_hi;
         uint32_t qh[2], ql[2];
         {
             float2 a = make_float2(0.f, 0.f), c = a;
-            if (c_lo < n_cand) a = *reinterpret_cast<const float2*>(q_in + n_lo * D + h * DH + 2 * tq);
-            if (c_hi < n_cand) c = *reinterpret_cast<const float2*>(q_in + n_hi * D + h * DH + 2 * tq);
+            if (c_lo < nc) a = *reinterpret_cast<const float2*>(q_in + n_lo * D + h * DH + 2 * tq);
+            if (c_hi < nc) c = *reinterpret_cast<const float2*>(q_in + n_hi * D + h * DH + 2 * tq);
             split_pair(a.x * qscale, a.y * qscale, qh[0], ql[0]);
             split_pair(c.x * qscale, c.y * qscale, qh[1], ql[1]);
         }
@@ -1335,12 +1341,12 @@ __global__ void __launch_bounds__(256) decode_cross_attention_tc(const float* q_
         l_lo += __shfl_xor_sync(0xffffffffu, l_lo, 1); l_lo += __shfl_xor_sync(0xffffffffu, l_lo, 2);
         l_hi += __shfl_xor_sync(0xffffffffu, l_hi, 1); l_hi += __shfl_xor_sync(0xffffffffu, l_hi, 2);
         const int col = h * DH + 2 * tq;
-        if (c_lo < n_cand) {
+        if (c_lo < nc) {
             const float o0 = acc[0] / l_lo, o1 = acc[1] / l_lo;
             if (out) *reinterpret_cast<float2*>(out + n_lo * D + col) = make_float2(o0, o1);
             if (out16) *reinterpret_cast<__nv_bfloat162*>(out16 + n_lo * D + col) = __floats2bfloat162_rn(o0, o1);
         }
-        if (c_hi < n_cand) {
+        if (c_hi < nc) {
             const float o0 = acc[2] / l_hi, o1 = acc[3] / l_hi;
             if (out) *reinterpret_cast<float2*>(out + n_hi * D + col) = make_float2(o0, o1);
             if (out16) *reinterpret_cast<__nv_bfloat162*>(out16 + n_hi * D + col) = __floats2bfloat162_rn(o0, o1);
@@ -1379,6 +1385,10 @@ struct SampleParams {
     const float* part; int splits; int64_t part_stride;
     const float* pbias; const float* pgamma; const float* pbeta; float eps;
     int rows_per_warp;       // dense input: 1 or SAMPLE_NR rows per warp (0 = 1)
+    // stop at <EOS> (mmt_decode_until_eos), all nullptr otherwise: row r is sequence orig[r] of the launch (compacted wave,
+    // kernels_retire.cuh; nullptr = r), whose first-<EOS> step eos_len[] holds (max_len until it emits `eos`).  A
+    // finished sequence writes <PAD> / 0 and counts as <PAD>; live[t] counts the sequences not finished after step t.
+    const int* orig; int* eos_len; int* live; int64_t eos;
 };
 
 // CTA = 8 warps.  Rows are taken in groups of `rpc` per CTA, grid-stride: a CTA stages fc_out once and keeps sampling
@@ -1394,7 +1404,8 @@ constexpr int SAMPLE_NR = 4;             // rows per warp (dense input)
 constexpr int SAMPLE_ROWS = 8 * SAMPLE_NR;
 
 template <int NR>
-__device__ __forceinline__ void sample_rows(const SampleParams& p, const float* Ws, const float (*xs)[D], int r0, int64_t n0, int t, int lane, int& my_nonpad) {
+__device__ __forceinline__ void sample_rows(const SampleParams& p, const float* Ws, const float (*xs)[D], int r0, int64_t n0, int t, int lane, int& my_nonpad,
+                                            int& my_live) {
     const int v0 = lane, v1 = lane + 32;
     float a0[NR], a1[NR];
 #pragma unroll
@@ -1420,6 +1431,7 @@ __device__ __forceinline__ void sample_rows(const SampleParams& p, const float* 
     for (int r = 0; r < NR; ++r) {
         const int64_t n = n0 + r;
         if (n >= p.N) break;
+        const int64_t no = p.orig ? p.orig[n] : n;        // the sequence's own column and Philox row
         float lg0 = ok0 ? a0[r] + b0 : MMT_NEG_INF;
         float lg1 = ok1 ? a1[r] + b1 : MMT_NEG_INF;
         if (p.logits) {
@@ -1444,7 +1456,7 @@ __device__ __forceinline__ void sample_rows(const SampleParams& p, const float* 
         if (p.mode == 1) {
             RngGeom g = p.rng;
             if (p.rng_dev) { g.seed = p.rng_dev[0]; g.offset = p.rng_dev[1]; }
-            const int64_t li = torch_rng_row(g, p.rng_inc, p.rng_cand, p.rng_col_steps, p.seq_index_base + n, t, p.V);
+            const int64_t li = torch_rng_row(g, p.rng_inc, p.rng_cand, p.rng_col_steps, p.seq_index_base + no, t, p.V);
             if (ok0) r0v = p0 / torch_exponential_at(g, li + v0);
             if (ok1) r1v = p1 / torch_exponential_at(g, li + v1);
         }
@@ -1461,9 +1473,15 @@ __device__ __forceinline__ void sample_rows(const SampleParams& p, const float* 
             if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; bp = op; }
         }
         if (lane == 0) {
-            if (p.tokens) p.tokens[(int64_t)t * p.ldn + n] = bi;
-            if (p.probs) p.probs[(int64_t)t * p.ldn + n] = bp;
-            my_nonpad += (bi != 0);
+            bool fin = false;
+            if (p.eos_len) {
+                fin = t > p.eos_len[no];
+                if (!fin && bi == p.eos) p.eos_len[no] = t;
+                my_live += !fin && bi != p.eos;
+            }
+            if (p.tokens) p.tokens[(int64_t)t * p.ldn + no] = fin ? 0 : bi;
+            if (p.probs) p.probs[(int64_t)t * p.ldn + no] = fin ? 0.f : bp;
+            my_nonpad += !fin && bi != 0;
         }
     }
 }
@@ -1474,7 +1492,7 @@ __global__ void __launch_bounds__(256) sample_tokens(const __grid_constant__ Sam
     extern __shared__ float Ws[];
     __shared__ __align__(16) float xs[SAMPLE_ROWS][D];
     __shared__ __align__(16) float psum[8][D];
-    __shared__ int s_nonpad;
+    __shared__ int s_nonpad, s_live;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     pdl_launch_dependents();
     // fc_out weights -> padded smem rows (independent of the step: issued before anything else)
@@ -1483,12 +1501,12 @@ __global__ void __launch_bounds__(256) sample_tokens(const __grid_constant__ Sam
         float* dst = Ws + (i / (D / 4)) * (D + 1) + (i % (D / 4)) * 4;
         dst[0] = w.x; dst[1] = w.y; dst[2] = w.z; dst[3] = w.w;
     }
-    if (threadIdx.x == 0) s_nonpad = 0;
+    if (threadIdx.x == 0) { s_nonpad = 0; s_live = 0; }
     pdl_wait();
     const int t = p.ctl.step ? *p.ctl.step : 0;
     const bool nr4 = p.rows_per_warp == SAMPLE_NR;
     const int rpc = p.part ? 2 : (nr4 ? SAMPLE_ROWS : 8);       // rows per CTA and pass
-    int my_nonpad = 0;
+    int my_nonpad = 0, my_live = 0;
     for (int64_t base = (int64_t)blockIdx.x * rpc; base < p.N; base += (int64_t)gridDim.x * rpc) {
         if (p.part) {   // ---- input rows -> xs: four warps per row over the FFN2 partials
             const int wpr = 4;
@@ -1523,7 +1541,7 @@ __global__ void __launch_bounds__(256) sample_tokens(const __grid_constant__ Sam
                 *reinterpret_cast<float4*>(&xs[warp][lane * 4]) = v;
             }
             __syncthreads();
-            if (warp < rpc && base + warp < p.N) sample_rows<1>(p, Ws, xs, warp, base + warp, t, lane, my_nonpad);
+            if (warp < rpc && base + warp < p.N) sample_rows<1>(p, Ws, xs, warp, base + warp, t, lane, my_nonpad, my_live);
         } else if (nr4) {   // ---- dense input: each warp stages and samples its own four rows
 #pragma unroll
             for (int r = 0; r < SAMPLE_NR; ++r) {
@@ -1531,20 +1549,22 @@ __global__ void __launch_bounds__(256) sample_tokens(const __grid_constant__ Sam
                 if (n < p.N) *reinterpret_cast<float4*>(&xs[warp * SAMPLE_NR + r][lane * 4]) = *reinterpret_cast<const float4*>(p.x + n * D + lane * 4);
             }
             __syncthreads();      // (also orders the Ws staging of the first pass)
-            if (base + warp * SAMPLE_NR < p.N) sample_rows<SAMPLE_NR>(p, Ws, xs, warp * SAMPLE_NR, base + warp * SAMPLE_NR, t, lane, my_nonpad);
+            if (base + warp * SAMPLE_NR < p.N) sample_rows<SAMPLE_NR>(p, Ws, xs, warp * SAMPLE_NR, base + warp * SAMPLE_NR, t, lane, my_nonpad, my_live);
         } else {            // ---- dense input, small waves: one row per warp (more CTAs, shorter chain)
             const int64_t n = base + warp;
             if (n < p.N) *reinterpret_cast<float4*>(&xs[warp][lane * 4]) = *reinterpret_cast<const float4*>(p.x + n * D + lane * 4);
             __syncthreads();
-            if (n < p.N) sample_rows<1>(p, Ws, xs, warp, n, t, lane, my_nonpad);
+            if (n < p.N) sample_rows<1>(p, Ws, xs, warp, n, t, lane, my_nonpad, my_live);
         }
         __syncthreads();          // xs / psum are rewritten by the next group
     }
-    if (p.advance || p.ctl.nonpad) {
+    if (p.advance || p.ctl.nonpad || p.live) {
         if (my_nonpad) atomicAdd(&s_nonpad, my_nonpad);
+        if (my_live) atomicAdd(&s_live, my_live);
         __syncthreads();
         if (threadIdx.x == 0) {   // one global atomic per CTA, not per sequence
             if (p.ctl.nonpad && s_nonpad) atomicAdd(p.ctl.nonpad + t, s_nonpad);
+            if (p.live && s_live) atomicAdd(p.live + t, s_live);
             if (p.advance) {
                 __threadfence();
                 int done = atomicAdd(p.ctl.done_ctas, 1);

@@ -238,6 +238,32 @@ class Engine:
             t.record_stream(torch.cuda.current_stream(self.dev_index))
         return tokens, probs, int(steps.value)
 
+    def decode_until_eos(self, memory, key_bias, *, eos, n_cand=1, max_len=128, temperature=1.0, sampling="greedy",
+                         stop_on_all_pad=False, precision="fp32", seed=0, offset=0, seq_index_base=0, n_total=0,
+                         per_memory_rng=False):
+        """``decode`` that stops computing a sequence once it has emitted ``eos`` (``mmt_decode_until_eos``).  Returns
+        (tokens (T,N) i64, probs (T,N) f32, steps, lengths (N,) i32, rows (T,) i64 on the host): ids and probabilities
+        equal ``decode``'s up to and including each sequence's first ``eos`` and are <PAD> / 0 after it (and from
+        ``steps`` on); ``lengths`` = position of that first ``eos`` (max_len if none); ``rows`` = decode-step rows
+        computed at each position."""
+        smp = _lib.SAMPLE_GREEDY if sampling == "greedy" else _lib.SAMPLE_MULTINOMIAL
+        if per_memory_rng and (smp != _lib.SAMPLE_MULTINOMIAL or seq_index_base % n_cand):
+            raise ValueError("per_memory_rng needs multinomial sampling and seq_index_base a multiple of n_candidates")
+        a, keep = self._decode_args(memory, key_bias, n_cand, max_len, temperature, smp, stop_on_all_pad, precision,
+                                    seed, offset, seq_index_base, n_total)
+        N = a.Bm * n_cand
+        tokens = torch.empty(max_len, N, device=self.device, dtype=torch.int64)
+        probs = torch.empty(max_len, N, device=self.device, dtype=torch.float32)
+        lengths = torch.empty(N, device=self.device, dtype=torch.int32)
+        rows = torch.zeros(max_len, dtype=torch.int64)
+        steps = C.c_int32(max_len)
+        _lib.check(self.L.mmt_decode_until_eos(self.h, C.byref(a), int(per_memory_rng), int(eos), tokens.data_ptr(),
+                                               probs.data_ptr(), lengths.data_ptr(), C.byref(steps), rows.data_ptr(),
+                                               self._stream()))
+        for t in keep:
+            t.record_stream(torch.cuda.current_stream(self.dev_index))
+        return tokens, probs, int(steps.value), lengths, rows
+
     def teacher_forced(self, memory, key_bias, trg, *, n_cand=1, precision="fp32"):
         """trg (T,N) i64 -> logits (T,N,V)."""
         trg = trg.to(self.device, torch.int64).contiguous()

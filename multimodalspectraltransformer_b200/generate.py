@@ -28,6 +28,11 @@ Extensions (keyword-only, default = reference behaviour):
                    calls in order: one call over many spectra draws the ids of the
                    reference's per-spectrum loop (seq_index_base must be a multiple of
                    n_candidates; n_total is then the whole call's sequence count).
+  stop_at_eos=True  stop computing a sequence once it has emitted stoi["<EOS>"]: ids and
+                   probabilities equal the default's up to and including that <EOS> and are
+                   <PAD> / 0 after it; shapes and generator advance are unchanged (greedy
+                   also stops once every sequence has finished).  Every consumer of the ids
+                   (tensor_to_smiles*, distinct_smiles) ignores what follows <EOS>.
 """
 from __future__ import annotations
 
@@ -66,6 +71,12 @@ def _check_sos(stoi):
     if sos != 3:
         raise ValueError("the engine hard-codes <SOS> = 3 (stoi.json)")
     return sos
+
+
+def _eos_id(stoi):
+    if "<EOS>" not in stoi:
+        raise ValueError("stop_at_eos needs an <EOS> entry in stoi")
+    return int(stoi["<EOS>"])
 
 
 def _philox_state(dev_index):
@@ -132,7 +143,8 @@ def _philox_advance(eng, n_candidates, n_total, max_len, per_memory_rng):
 
 
 def _decode(model, memory, src_padding_mask, config, sampling, stop_on_all_pad, n_candidates, seq_index_base, n_total,
-            per_memory_rng=False):
+            per_memory_rng=False, eos=None):
+    """eos: None, or the id at which a sequence stops being computed (Engine.decode_until_eos)."""
     if per_memory_rng and (sampling != "multinomial" or seq_index_base % n_candidates):
         raise ValueError("per_memory_rng needs multinomial sampling and seq_index_base a multiple of n_candidates")
     model.eval()                                    # the reference flips eval() and leaves it
@@ -145,57 +157,65 @@ def _decode(model, memory, src_padding_mask, config, sampling, stop_on_all_pad, 
     if sampling == "multinomial":
         gen, seed, offset = _philox_state(eng.dev_index)
         kw = dict(seed=seed, offset=offset)
-    tokens, probs, steps = eng.decode(memory, bias, n_cand=n_candidates, max_len=int(config.max_len),
-                                      temperature=float(config.temperature), sampling=sampling,
-                                      stop_on_all_pad=stop_on_all_pad, precision=prec,
-                                      seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng, **kw)
+    if eos is not None:
+        kw["eos"] = eos
+    run = eng.decode if eos is None else eng.decode_until_eos
+    tokens, probs, steps = run(memory, bias, n_cand=n_candidates, max_len=int(config.max_len),
+                               temperature=float(config.temperature), sampling=sampling,
+                               stop_on_all_pad=stop_on_all_pad, precision=prec,
+                               seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng, **kw)[:3]
     if gen is not None:   # consume exactly what the torch.multinomial calls would have
         gen.set_offset(offset + _philox_advance(eng, n_candidates, n_total if n_total else N, int(config.max_len), per_memory_rng))
     return tokens, probs, steps
 
 
-def greedy_sequence(model, stoi, itos, memory, src_padding_mask, config, *, n_candidates=1):
+def greedy_sequence(model, stoi, itos, memory, src_padding_mask, config, *, n_candidates=1, stop_at_eos=False):
     """-> ((T,N) i64 tokens without <SOS>, (T-1,N) f32 probs).  T < max_len only when one
-    step emitted <PAD> for every sequence.  NB the reference fails for N == 1
-    (SURVEY.md B.6); this returns the shapes its N > 1 code path would."""
+    step emitted <PAD> for every sequence (stop_at_eos: or every sequence had emitted <EOS>).  NB the reference
+    fails for N == 1 (SURVEY.md B.6); this returns the shapes its N > 1 code path would."""
     _check_sos(stoi)
-    tokens, probs, steps = _decode(model, memory, src_padding_mask, config, "greedy", True, n_candidates, 0, 0)
+    eos = _eos_id(stoi) if stop_at_eos else None
+    tokens, probs, steps = _decode(model, memory, src_padding_mask, config, "greedy", True, n_candidates, 0, 0, eos=eos)
     return tokens[:steps], probs[1:steps]
 
 
-def greedy_sequence_2(model, stoi, itos, memory, src_padding_mask, config, *, n_candidates=1):
+def greedy_sequence_2(model, stoi, itos, memory, src_padding_mask, config, *, n_candidates=1, stop_at_eos=False):
     """mrtf variant: probabilities are NOT sliced -> ((T,N), (T,N))."""
     _check_sos(stoi)
-    tokens, probs, steps = _decode(model, memory, src_padding_mask, config, "greedy", True, n_candidates, 0, 0)
+    eos = _eos_id(stoi) if stop_at_eos else None
+    tokens, probs, steps = _decode(model, memory, src_padding_mask, config, "greedy", True, n_candidates, 0, 0, eos=eos)
     return tokens[:steps], probs[:steps]
 
 
 def multinomial_sequence(model, stoi, memory, src_padding_mask, config, *, n_candidates=1, seq_index_base=0, n_total=0,
-                         per_memory_rng=False):
+                         per_memory_rng=False, stop_at_eos=False):
     """-> ((T,N) i64, (N,T) f32): probabilities transposed, always max_len steps."""
     _check_sos(stoi)
+    eos = _eos_id(stoi) if stop_at_eos else None
     tokens, probs, _ = _decode(model, memory, src_padding_mask, config, "multinomial", False, n_candidates, seq_index_base, n_total,
-                               per_memory_rng)
+                               per_memory_rng, eos=eos)
     return tokens, probs.transpose(0, 1)
 
 
 def multinomial_sequence_multi(model, memory, src_padding_mask, stoi, config, *, n_candidates=1, seq_index_base=0, n_total=0,
-                               per_memory_rng=False):
+                               per_memory_rng=False, stop_at_eos=False):
     """-> ((T,N) i64, (T,N) f32); the reference's .squeeze() drops the N axis of the
     probabilities when N == 1 (run_batch_gen_val_MMT_v15_4.py:149)."""
     _check_sos(stoi)
+    eos = _eos_id(stoi) if stop_at_eos else None
     tokens, probs, _ = _decode(model, memory, src_padding_mask, config, "multinomial", False, n_candidates, seq_index_base, n_total,
-                               per_memory_rng)
+                               per_memory_rng, eos=eos)
     if probs.shape[1] == 1:
         probs = probs.squeeze(1)
     return tokens, probs
 
 
 def multinomial_sequence_multi_2(model, memory, src_padding_mask, stoi, config, *, n_candidates=1, seq_index_base=0, n_total=0,
-                                 per_memory_rng=False):
+                                 per_memory_rng=False, stop_at_eos=False):
     """mrtf variant: probabilities lose their first row -> ((T,N), (T-1,N))."""
     tokens, probs = multinomial_sequence_multi(model, memory, src_padding_mask, stoi, config, n_candidates=n_candidates,
-                                               seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng)
+                                               seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng,
+                                               stop_at_eos=stop_at_eos)
     return tokens, probs[1:]
 
 

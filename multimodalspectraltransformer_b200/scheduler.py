@@ -109,18 +109,20 @@ class PendingTokens:
 
 
 def generate_sharded(model, data_dict, config, stoi, *, n_candidates=1, sampling="multinomial", gather_probs=False,
-                     group=None, async_gather=False, per_memory_rng=False):
+                     group=None, async_gather=False, per_memory_rng=False, stop_at_eos=False):
     """Encode + decode this rank's spectra and all-gather the ids.
 
     Returns (tokens (T, B*n_candidates) i64 -- identical on every rank and identical to the single-GPU run --, probs or
     None, local (lo, hi)); with ``async_gather=True`` a :class:`PendingTokens` instead, whose collective overlaps
     whatever the caller launches next (greedy early-exit trimming is then the caller's business).  ``per_memory_rng``:
     every spectrum's candidates draw in their own stream (generate.multinomial_sequence_multi), so the result also
-    equals the reference's per-spectrum loop."""
+    equals the reference's per-spectrum loop.  ``stop_at_eos``: sequences stop being computed at stoi["<EOS>"]
+    (generate.multinomial_sequence_multi); retirement is per sequence, so the result is still shard invariant."""
     from . import generate as G
     from .engine import engine_for
     if per_memory_rng and sampling == "greedy":
         raise ValueError("per_memory_rng needs multinomial sampling")
+    eos = G._eos_id(stoi) if stop_at_eos else None
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     B = next(iter(data_dict.values())).shape[0]
@@ -135,10 +137,10 @@ def generate_sharded(model, data_dict, config, stoi, *, n_candidates=1, sampling
         memory, mask, *_ = G.run_model(model, local, config)
         if sampling == "greedy":
             # stop_on_all_pad is a whole-batch property: decide it after the gather
-            tok, pr, _ = G._decode(model, memory, mask, config, "greedy", False, n_candidates, 0, 0)
+            tok, pr, _ = G._decode(model, memory, mask, config, "greedy", False, n_candidates, 0, 0, eos=eos)
         else:
             tok, pr, _ = G._decode(model, memory, mask, config, "multinomial", False, n_candidates,
-                                   lo * n_candidates, B * n_candidates, per_memory_rng)
+                                   lo * n_candidates, B * n_candidates, per_memory_rng, eos=eos)
         packed = eng.pack_tokens_seqmajor(tok)                                   # (n_local, T) u8
     else:
         packed = torch.zeros(0, T, dtype=torch.uint8, device=eng.device)
