@@ -918,8 +918,10 @@ static int encode_chunk(mmt_engine* e, const mmt_spectra& in, int b0, int Bc, in
 struct DecBuffers {
     float *x, *qkv, *att, *part, *qc, *h;
     int64_t part_rows;                 // capacity of `part` in rows of D floats
-    char* kv_pool; int* block_table;   // paged self-attention cache, 6 pools of kv_esz-byte elements
+    char* kv_pool; int* block_table;   // paged self-attention cache, a pool of kv_esz-byte elements per layer (layer_pool)
     int64_t pool_pages;                // pages per layer pool (Nw * pps; twice that for the beam search's copy-on-write parity)
+    int kv_first;                      // first layer with a pool: 1 when every wave of the run takes layer 0 from the table
+    uint8_t* hist; int hist_ld;        // layer 0 on the position x token table: token history [col][hist_ld] (nullptr otherwise)
     char* cross_kv;                    // projected memory [layer][K|V][head][row][dh], kv_esz-byte elements
     size_t kv_esz;                     // 4 (fp32 check mode) | 2 (bf16 tensor-core mode)
     int *nk, *row_start; int64_t* row_off; float* kbias_c;
@@ -938,8 +940,9 @@ struct DecBuffers {
 };
 constexpr int MAX_SPLITS = 32;
 
+// l0_table: the run's un-fused waves take layer 0 from the table (token history); l0_pool: a wave may need layer 0's pages
 static void plan_decoder(Arena& a, const mmt_model_desc& d, int64_t Nw, int Bmw, int S, int max_len, DecBuffers& b, bool bf16, int fused_rows, int kv_copies = 1,
-                         bool retire = false) {
+                         bool retire = false, bool l0_table = false, bool l0_pool = true) {
     const int L = d.n_dec_layers;
     const int pps = (max_len + PAGE_TOKENS - 1) / PAGE_TOKENS;
     b.x = a.get<float>(Nw * D);
@@ -954,7 +957,10 @@ static void plan_decoder(Arena& a, const mmt_model_desc& d, int64_t Nw, int Bmw,
     b.h = a.get<float>(bf16 ? 0 : Nw * d.d_ff);
     b.kv_esz = bf16 ? 2 : 4;
     b.pool_pages = (int64_t)kv_copies * Nw * pps;
-    b.kv_pool = a.get<char>((size_t)L * b.pool_pages * 2 * PAGE_TOKENS * D * b.kv_esz);
+    b.kv_first = l0_pool ? 0 : 1;
+    b.kv_pool = a.get<char>((size_t)(L - b.kv_first) * b.pool_pages * 2 * PAGE_TOKENS * D * b.kv_esz);
+    b.hist_ld = pps * PAGE_TOKENS;
+    b.hist = l0_table ? a.get<uint8_t>((size_t)Nw * b.hist_ld) : nullptr;
     b.block_table = a.get<int>(Nw * pps);
     int64_t R = (int64_t)Bmw * S;
     b.cross_kv = a.get<char>((size_t)L * 2 * R * D * b.kv_esz);
@@ -977,6 +983,11 @@ static void plan_decoder(Arena& a, const mmt_model_desc& d, int64_t Nw, int Bmw,
         b.rt_orig[0] = a.get<int>(Nw); b.rt_orig[1] = a.get<int>(Nw); b.rt_bt = a.get<int>(Nw * pps); b.rt_src = a.get<int>(Nw);
         b.rt_col_start = a.get<int>(Bmw); b.rt_col_count = a.get<int>(Bmw);
     }
+}
+
+// layer l's cache pages (nullptr: layer 0 of a run that takes it from the table throughout)
+static char* layer_pool(const DecBuffers& b, int l) {
+    return l < b.kv_first ? nullptr : b.kv_pool + (size_t)(l - b.kv_first) * b.pool_pages * 2 * PAGE_TOKENS * D * b.kv_esz;
 }
 
 // Page map of a wave: page j of sequence n is physical page j * Nw + n ("slot-major").  At position t every sequence reads its
@@ -1041,17 +1052,76 @@ static int decode_prepare_wave(mmt_engine* e, const mmt_decode_args& a, int b0, 
     return 0;
 }
 
+// Decoder layer 0's input at position t is E_tok[tok] + E_pos[t]: its Q and K | V rows depend on the pair (t, tok) alone.
+// The table holds them for every pair (128 x 43 = 5,504 rows: Q 2.8 MB fp32, K | V 2.8 MB bf16, small enough to stay in
+// L2), made by the step's own layer-0 projection -- the same bf16 input rows, tcgen05 GEMM call, bias add and bf16
+// rounding -- so that the large-wave step reads layer 0 from it bit for bit instead of projecting, appending and re-reading
+// 67 MB of cache per position.  Built once, outside any capture (a fixed allocation: cached step graphs stay valid).
+static int ensure_l0_table(mmt_engine* e, cudaStream_t s) {
+    if (e->l0_qtab) return 0;
+    cudaStreamCaptureStatus cs;
+    MMT_CUDA(cudaStreamIsCapturing(s, &cs));
+    if (cs != cudaStreamCaptureStatusNone) MMT_FAIL("decode: the layer-0 table is built by the first large bf16 decode, which cannot run under stream capture");
+    const mmt_model_desc& d = e->desc;
+    const LayerW& w = e->dec[0];
+    const int64_t rows = (int64_t)d.max_len * d.vocab;
+    __nv_bfloat16* x16 = nullptr;
+    float* qkv = nullptr;
+    float* qtab = nullptr;
+    __nv_bfloat16* kvtab = nullptr;
+    auto release = [&]() { cudaFree(x16); cudaFree(qkv); cudaFree(qtab); cudaFree(kvtab); };
+    if (cudaMalloc(&x16, rows * D * sizeof(__nv_bfloat16)) != cudaSuccess || cudaMalloc(&qkv, rows * 3 * D * sizeof(float)) != cudaSuccess ||
+        cudaMalloc(&qtab, rows * D * sizeof(float)) != cudaSuccess || cudaMalloc(&kvtab, rows * 2 * D * sizeof(__nv_bfloat16)) != cudaSuccess) {
+        release();
+        MMT_FAIL("decode: cudaMalloc of the layer-0 table failed");
+    }
+    int rc = 0;
+    prof_pre(e, s);
+    l0_table_rows<<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, rows, x16);
+    rc = check_launch(e, "l0_table_rows", s);
+    if (!rc) {     // decode_self_attention_layer's projection, every column to fp32
+        TcGemmParams p = tc_params((int)rows, 3 * D, D);
+        p.bias = w.in_b; p.out_f32 = qkv; p.ld_f32 = 3 * D;
+        rc = launch_tc(e, p, x16, D, e->Wb(w.in_w), TC_EPI_STORE, s, e->dec_proj_single ? nullptr : e->Wlo(w.in_w));
+    }
+    if (!rc) {
+        prof_pre(e, s);
+        l0_table_split<<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(qkv, rows, qtab, kvtab);
+        rc = check_launch(e, "l0_table_split", s);
+    }
+    cudaError_t se = cudaStreamSynchronize(s);
+    cudaFree(x16); cudaFree(qkv);
+    x16 = nullptr; qkv = nullptr;
+    if (rc || se != cudaSuccess) {
+        release();
+        if (rc) return rc;
+        MMT_FAIL(std::string("decode: layer-0 table build failed: ") + cudaGetErrorString(se));
+    }
+    e->l0_qtab = qtab; e->l0_kvtab = kvtab;
+    return 0;
+}
+
 // Un-fused step, one decoder layer: the QKV projection of the new position (x16 / x at step *b.ctl) and its self-attention
 // over the layer's cache `pool` -> att16 (bf16) | att (fp32).  bf16: tcgen05 projection whose epilogue appends K | V to the
 // token-major (default) or head-major pages, or (MMT_NO_KV_EPILOGUE) the attention kernel appends them; fp32: SIMT GEMM.
 // decode_step and the unit hook mmt_decode_self_attention both run this.
+// l0_table (layer 0 of the un-fused bf16 token-major step, b.hist set): no projection and no cache; the attention reads the
+// rows of the sequence's (position, token) pairs from the engine's layer-0 table (ensure_l0_table, TmTable).
 static int decode_self_attention_layer(mmt_engine* e, const LayerW& w, const DecBuffers& b, char* pool, int pps, int64_t Nw, bool bf16,
-                                       bool pdl_u, cudaStream_t s) {
+                                       bool pdl_u, cudaStream_t s, bool l0_table = false) {
     const int H = e->desc.n_heads, dh = D / H;
     const float scale = 1.0f / sqrtf((float)dh);
     const int* step = b.ctl;
     const int M = (int)Nw;
     if (dh != 8) MMT_FAIL("decoder head dim must be 8");
+    const unsigned tm_blocks = (unsigned)((Nw * (H / 8) + 7) / 8);      // token-major / table: a warp per (sequence, 8 heads)
+    if (l0_table) {
+        if (!b.hist || !e->l0_qtab) MMT_FAIL("decode: layer-0 table path without its table or token history");
+        const TmTable src{e->l0_qtab, e->l0_kvtab, b.hist, b.hist_ld, (int)e->desc.vocab, b.orig};
+        prof_pre(e, s);
+        launch_args(decode_self_attention_tm<8, TmTable>, dim3(tm_blocks), dim3(256), 0, s, pdl_u, src, Nw, H, scale, step, b.att16);
+        return check_launch(e, "decode_self_attention_l0", s);
+    }
     if (bf16) {   // K | V columns of the projection land in the cache pages directly; the fp32 row keeps only Q
         TcGemmParams p = tc_params(M, 3 * D, D);
         // (with the K | V columns going to the cache, the Q columns form a dense [N][D] buffer: a 512-byte row every 512
@@ -1068,7 +1138,7 @@ static int decode_self_attention_layer(mmt_engine* e, const LayerW& w, const Dec
     prof_pre(e, s);
     const unsigned sa_blocks = (unsigned)((Nw * (H / 4) + 7) / 8);     // a warp per (sequence, 4 heads)
     if (bf16 && e->use_kv_epilogue && e->kv_tok_major && H % 8 == 0)      // token-major pages: a warp per (sequence, 8 heads)
-        launch_args(decode_self_attention_tm<8>, dim3((unsigned)((Nw * (H / 8) + 7) / 8)), dim3(256), 0, s, pdl_u, (const float*)b.qkv, (const __nv_bfloat16*)reinterpret_cast<__nv_bfloat16*>(pool), (const int*)b.block_table, pps, Nw, H, scale, step, b.att16);
+        launch_args(decode_self_attention_tm<8, TmPaged>, dim3(tm_blocks), dim3(256), 0, s, pdl_u, TmPaged{b.qkv, reinterpret_cast<const __nv_bfloat16*>(pool), b.block_table, pps}, Nw, H, scale, step, b.att16);
     else if (bf16 && e->use_kv_epilogue) launch_args(decode_self_attention_g8<8, __nv_bfloat16, false>, dim3(sa_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qkv, reinterpret_cast<__nv_bfloat16*>(pool), (const int*)b.block_table, pps, Nw, H, scale, step, (float*)nullptr, b.att16);
     else if (bf16) launch_args(decode_self_attention_g8<8, __nv_bfloat16>, dim3(sa_blocks), dim3(256), 0, s, pdl_u, (const float*)b.qkv, reinterpret_cast<__nv_bfloat16*>(pool), (const int*)b.block_table, pps, Nw, H, scale, step, (float*)nullptr, b.att16);
     else decode_self_attention_g8<8, float><<<sa_blocks, 256, 0, s>>>(b.qkv, reinterpret_cast<float*>(pool), b.block_table, pps, Nw, H, scale, step, b.att, b.att16);
@@ -1277,7 +1347,8 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
                 q.b1 = w.l1_b; q.b2 = w.l2_b; q.n3_w = w.n3_w; q.n3_b = w.n3_b; q.x_out = b.x;
             }
             q.in_w = w.in_w; q.in_b = w.in_b; q.out_w = w.out_w; q.out_b = w.out_b; q.n1_w = w.n1_w; q.n1_b = w.n1_b;
-            q.kv_pool = b.kv_pool + (size_t)l * b.pool_pages * 2 * PAGE_TOKENS * D * b.kv_esz; q.block_table = b.block_table; q.pps = pps;
+            q.kv_pool = layer_pool(b, l); q.block_table = b.block_table; q.pps = pps;
+            if (!q.kv_pool) MMT_FAIL("decode: fused step without layer-0 cache pages (run_decode planned every wave on the layer-0 table)");
             q.step = step;
             q.in_w16 = e->Wb(w.in_w); q.out_w16 = e->Wb(w.out_w); q.cq_w16 = e->Wb(w.ca_in_w); q.co_w16 = e->Wb(w.ca_out_w);
             q.cq_w = w.ca_in_w; q.cq_b = w.ca_in_b; q.co_w = w.ca_out_w; q.co_b = w.ca_out_b; q.n2_w = w.n2_w; q.n2_b = w.n2_b;
@@ -1303,16 +1374,19 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
             }
         }
     } else {
+        // layer 0 on the position x token table (b.hist, see run_decode): the embedding's bf16 copy has no reader (it was the
+        // layer-0 projection's operand), the token goes to the history instead
+        const bool l0_table = b.hist != nullptr;
+        __nv_bfloat16* x16 = l0_table ? nullptr : b.x16;
         prof_pre(e, s);
-        if (r.trg) launch_args(decode_embed, dim3((unsigned)((Nw + 3) / 4)), dim3(128), 0, s, pdl_u, r.trg + n0, 0, 3, Nw, ldn, e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, step, b.x, b.x16, b.orig);
-        else launch_args(decode_embed, dim3((unsigned)((Nw + 3) / 4)), dim3(128), 0, s, pdl_u, (const int64_t*)(r.tokens + n0), 1, 3, Nw, ldn, e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, step, b.x, b.x16, b.orig);
+        if (r.trg) launch_args(decode_embed, dim3((unsigned)((Nw + 3) / 4)), dim3(128), 0, s, pdl_u, r.trg + n0, 0, 3, Nw, ldn, e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, step, b.x, x16, b.orig, b.hist, b.hist_ld);
+        else launch_args(decode_embed, dim3((unsigned)((Nw + 3) / 4)), dim3(128), 0, s, pdl_u, (const int64_t*)(r.tokens + n0), 1, 3, Nw, ldn, e->W("embed_trg.weight"), e->W("pe_trg.weight"), (int)d.vocab, step, b.x, x16, b.orig, b.hist, b.hist_ld);
         MMT_TRY(check_launch(e, "decode_embed", s));
 
         for (int l = 0; l < d.n_dec_layers; ++l) {
             const LayerW& w = e->dec[l];
-            char* pool = b.kv_pool + (size_t)l * b.pool_pages * 2 * PAGE_TOKENS * D * b.kv_esz;
             const char* ckv = b.cross_kv + (size_t)l * 2 * R * D * b.kv_esz;
-            MMT_TRY(decode_self_attention_layer(e, w, b, pool, pps, Nw, bf16, pdl_u, s));
+            MMT_TRY(decode_self_attention_layer(e, w, b, layer_pool(b, l), pps, Nw, bf16, pdl_u, s, l == 0 && l0_table));
             MMT_TRY(decode_self_tail_layer(o, w, bf16));
             MMT_TRY(decode_cross_attention_layer(e, a, b, ckv, Nw, Bmw, bf16, pdl_u, s));
             MMT_TRY(decode_cross_tail_layer(o, w, l, bf16));
@@ -1406,12 +1480,27 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     const bool retire = r.eos >= 0;
     const bool small_wave = e->fused_decode_rows > 0 && (int64_t)Bm_wave * a.n_cand <= e->fused_decode_rows;
     const bool staged = e->use_graph && e->use_graph_cache && !e->profiling && n_waves == 1 && r.mode != 2 && !r.trg && (!retire || small_wave);   // forced inputs are the caller's tensor: nothing to cache across calls
+    // Layer 0 on the position x token table: the un-fused bf16 step with token-major pages (the fused small-wave step and the
+    // other page layouts keep the cache).  Layer 0's pages are only planned if some wave of the run is a fused one.
+    bool l0_table = false, l0_pool = true;
+    if (bf16 && e->use_l0_table && e->use_kv_epilogue && e->kv_tok_major && d.n_heads % 8 == 0 && d.vocab <= 256) {
+        bool any_fused = false;
+        for (int wb0 = 0; wb0 < a.Bm; wb0 += Bm_wave)
+            for (int i = 0; i < NL; ++i) {
+                const int Bmw = std::min(Bm_wave, a.Bm - wb0), lo = std::min(i * Bm_lane, Bmw), hi = std::min(lo + Bm_lane, Bmw);
+                if (hi <= lo) continue;
+                if (e->fused_decode_rows > 0 && (int64_t)(hi - lo) * a.n_cand <= e->fused_decode_rows) any_fused = true;
+                else l0_table = true;
+            }
+        l0_pool = any_fused;
+    }
+    if (l0_table) MMT_TRY(ensure_l0_table(e, s));
     Arena ar;
     DecBuffers lb[MAX_LANES];
     int64_t* st_tokens = nullptr; float* st_probs = nullptr;
     int* eos_all = nullptr;                  // retiring call: first-<EOS> step of every sequence (max_len until it emits)
     auto plan_all = [&]() {
-        for (int i = 0; i < NL; ++i) plan_decoder(ar, d, (int64_t)Bm_lane * a.n_cand, Bm_lane, a.S, a.max_len, lb[i], bf16, e->fused_decode_rows, 1, retire);
+        for (int i = 0; i < NL; ++i) plan_decoder(ar, d, (int64_t)Bm_lane * a.n_cand, Bm_lane, a.S, a.max_len, lb[i], bf16, e->fused_decode_rows, 1, retire, l0_table, l0_pool);
         if (staged) { st_tokens = ar.get<int64_t>((size_t)a.max_len * N_total); st_probs = ar.get<float>((size_t)a.max_len * N_total); }
         if (retire) eos_all = ar.get<int>(N_total);
     };
@@ -1858,6 +1947,7 @@ int32_t mmt_create(const mmt_model_desc* desc, const float* h_weights, int64_t n
     if (getenv("MMT_NO_GEMM_CHAIN")) e->use_gemm_chain = false;
     if (getenv("MMT_NO_FFN_WIDE")) e->use_ffn_wide = false;
     if (getenv("MMT_NO_KV_EPILOGUE")) e->use_kv_epilogue = false;
+    if (getenv("MMT_NO_L0_TABLE")) e->use_l0_table = false;
     if (getenv("MMT_KV_HEAD_MAJOR")) e->kv_tok_major = false;
     if (getenv("MMT_CLUSTER_FFN")) e->use_cluster_ffn = true;
     if (getenv("MMT_NO_FFN_PROLOGUE")) e->use_ffn_prologue = false;
@@ -1891,6 +1981,8 @@ void mmt_destroy(mmt_engine* e) {
     if (e->w16) cudaFree(e->w16);
     if (e->w16lo) cudaFree(e->w16lo);
     if (e->arena) cudaFree(e->arena);
+    if (e->l0_qtab) cudaFree(e->l0_qtab);
+    if (e->l0_kvtab) cudaFree(e->l0_kvtab);
     if (e->h_pinned) cudaFreeHost(e->h_pinned);
     for (auto& c : e->graph_cache) cudaGraphExecDestroy(c.exec);
     for (int i = 0; i < 5; ++i) if (e->enc_stream[i]) cudaStreamDestroy(e->enc_stream[i]);

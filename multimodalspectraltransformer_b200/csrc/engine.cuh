@@ -124,6 +124,9 @@ struct mmt_engine {
     bool use_ffn_prologue = true;      // un-fused decode step, >= 2048 rows: cross-attention out-projection + norm2 inside the FFN kernel (MMT_NO_FFN_PROLOGUE=1 disables)
     bool use_cluster_ffn = false;      // MMT_CLUSTER_FFN=1: small bf16 waves run the FFN inside decode_attn, launched as clusters of 4 CTAs (parity-tested; measured equal to the separate fused-FFN kernel in the bench, profiles/r02_cluster_probe.md)
     bool kv_tok_major = true;          // un-fused bf16 step with the KV epilogue: token-major cache pages + decode_self_attention_tm (MMT_KV_HEAD_MAJOR=1: head-major pages + decode_self_attention_g8)
+    bool use_l0_table = true;          // un-fused bf16 token-major step: decoder layer 0's Q / K | V from the position x token table (MMT_NO_L0_TABLE=1: the paged cache like layers 1-5)
+    float* l0_qtab = nullptr;          // that table (built at the first decode that uses it): Q [pos][tok][D] fp32
+    __nv_bfloat16* l0_kvtab = nullptr; //   and K | V [pos][tok][2 D] bf16
     bool use_kv_epilogue = true;       // un-fused bf16 step: the QKV projection's epilogue writes K | V of the new position into the cache pages (MMT_NO_KV_EPILOGUE=1: the attention kernel appends)
     bool use_ffn_wide = true;          // hi-term FFN with the LayerNorm epilogue: 128-column chunks (MMT_NO_FFN_WIDE=1: 64)
     bool use_gemm_chain = true;        // un-fused decode step: out-proj + LN1 + cross-attention query projection as one launch (MMT_NO_GEMM_CHAIN=1 disables)

@@ -867,10 +867,13 @@ struct StepCtl {
     int* nonpad;        // [max_len] count of non-<PAD> picks per step
 };
 
-// x[n] = E_tok[token_in(t, n)] + E_pos[t]        (validate_generate_MMT_v15_4.py:746-747); orig (compacted wave) or nullptr
+// x[n] = E_tok[token_in(t, n)] + E_pos[t]        (validate_generate_MMT_v15_4.py:746-747); orig (compacted wave) or nullptr.
+// hist (layer 0 on the position x token table, vocab <= 256): the token also goes to hist[col * hist_ld + t], the history
+// decode_self_attention_tm<TmTable> reads -- indexed by the sequence's column, so a compaction moves nothing.
 __global__ void __launch_bounds__(128) decode_embed(const int64_t* tokens, int tok_shift, int sos, int64_t N, int64_t ldn,
                                                     const float* E_tok, const float* E_pos, int vocab,
-                                                    const int* step, float* x, __nv_bfloat16* x_bf16, const int* orig) {
+                                                    const int* step, float* x, __nv_bfloat16* x_bf16, const int* orig,
+                                                    uint8_t* hist, int hist_ld) {
     pdl_launch_dependents();
     pdl_wait();
     const int t = *step;
@@ -882,6 +885,7 @@ __global__ void __launch_bounds__(128) decode_embed(const int64_t* tokens, int t
     if (tok_shift) tok = (t == 0) ? sos : tokens[(int64_t)(t - 1) * ldn + col];
     else tok = tokens[(int64_t)t * ldn + col];
     if (tok < 0 || tok >= vocab) tok = 0;
+    if (hist && lane == 0) hist[col * hist_ld + t] = (uint8_t)tok;
     float4 a = *reinterpret_cast<const float4*>(E_tok + tok * D + lane * 4);
     float4 b = *reinterpret_cast<const float4*>(E_pos + (int64_t)t * D + lane * 4);
     float4 o = make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
@@ -1075,9 +1079,37 @@ __global__ void __launch_bounds__(256) decode_self_attention_g8(const float* qkv
 // one load instruction covers 4 tokens x 128 contiguous bytes.  Online softmax, two keys per lane in flight and two more
 // prefetched; the 8 output dimensions are reduce-scattered over the 4 lanes of a head (lane kl keeps dimensions 2 kl,
 // 2 kl + 1), so a warp stores 128 consecutive bytes.  K / V of position t are already in the cache (kernels_tc.cuh).
-template <int DH>
-__global__ void __launch_bounds__(256) decode_self_attention_tm(const float* qd, const __nv_bfloat16* kv_pool, const int* block_table,
-                                                                int pages_per_seq, int64_t N, int H, float scale,
+// The row source Src gives, per sequence, the query row of position t and the K | V row of key j (512 bytes: K of every
+// head, then V -- the token-major page row): TmPaged (the cache) or TmTable (decoder layer 0).
+struct TmPaged {     // query: the QKV projection's dense [N][D] Q output; key j: slot j % 16 of page block_table[n][j / 16]
+    const float* qd; const __nv_bfloat16* kv_pool; const int* block_table; int pps;
+    struct Seq {
+        const float* q; const __nv_bfloat16* pool; const int* bt;
+        __device__ __forceinline__ const float* q_row(int) const { return q; }
+        __device__ __forceinline__ const __nv_bfloat16* kv_row(int j) const {
+            return pool + (int64_t)bt[j / PAGE_TOKENS] * (2 * PAGE_TOKENS * D) + (j % PAGE_TOKENS) * (2 * D);
+        }
+    };
+    __device__ __forceinline__ Seq seq(int64_t n) const { return {qd + n * D, kv_pool, block_table + n * pps}; }
+};
+// Decoder layer 0: its input at position j is E_tok[tok_j] + E_pos[j], so its Q and K | V rows depend on (j, tok_j) alone.
+// qtab [pos][tok][D] fp32 and kvtab [pos][tok][2 D] bf16 hold them for every pair (built once per engine, engine.cu
+// ensure_l0_table, by the same projection as the step's); tok_j comes from the sequence's token history (decode_embed),
+// row hist_ld * col, col = orig[n] in a compacted wave.  Plain cached loads: rows shared by many sequences (every
+// sequence's key 0 is the same <SOS> row) stay in L1.
+struct TmTable {
+    const float* qtab; const __nv_bfloat16* kvtab; const uint8_t* hist; int hist_ld; int vocab; const int* orig;
+    struct Seq {
+        const float* qtab; const __nv_bfloat16* kvtab; const uint8_t* hist; int vocab;
+        __device__ __forceinline__ const float* q_row(int t) const { return qtab + ((int64_t)t * vocab + hist[t]) * D; }
+        __device__ __forceinline__ const __nv_bfloat16* kv_row(int j) const { return kvtab + ((int64_t)j * vocab + hist[j]) * (2 * D); }
+    };
+    __device__ __forceinline__ Seq seq(int64_t n) const {
+        return {qtab, kvtab, hist + (int64_t)(orig ? orig[n] : n) * hist_ld, vocab};
+    }
+};
+template <int DH, class Src>
+__global__ void __launch_bounds__(256) decode_self_attention_tm(const Src src, int64_t N, int H, float scale,
                                                                 const int* step, __nv_bfloat16* out16) {
     static_assert(DH == 8, "8-element key rows");
     typedef KvRow<__nv_bfloat16> KV;
@@ -1090,9 +1122,8 @@ __global__ void __launch_bounds__(256) decode_self_attention_tm(const float* qd,
     const int lane = threadIdx.x & 31, h8 = lane >> 2, kl = lane & 3;
     const int64_t n = w / HG;
     const int h = (int)(w % HG) * 8 + h8;
-    constexpr int PAGE_ELEMS = 2 * PAGE_TOKENS * D;
-    const int* bt = block_table + n * pages_per_seq;
-    const float* row = qd + n * D + h * DH;
+    const typename Src::Seq sq = src.seq(n);
+    const float* row = sq.q_row(t) + h * DH;
     float q[DH], acc[DH];
     {
         const float4 a = *reinterpret_cast<const float4*>(row), b = *reinterpret_cast<const float4*>(row + 4);
@@ -1102,7 +1133,7 @@ __global__ void __launch_bounds__(256) decode_self_attention_tm(const float* qd,
 #pragma unroll
     for (int d = 0; d < DH; ++d) acc[d] = 0.f;
     float m = MMT_NEG_INF, l = 0.f;
-    auto row_ptr = [&](int j) { return kv_pool + (int64_t)bt[j / PAGE_TOKENS] * PAGE_ELEMS + (j % PAGE_TOKENS) * (2 * D) + h * DH; };
+    auto row_ptr = [&](int j) { return sq.kv_row(j) + h * DH; };
     typename KV::Raw rk0, rk1, rv0, rv1;
     if (kl <= t) {
         const __nv_bfloat16* p0 = row_ptr(kl);
@@ -1161,6 +1192,35 @@ __global__ void __launch_bounds__(256) decode_self_attention_tm(const float* qd,
     }
     const __nv_bfloat162 o = __floats2bfloat162_rn(acc[0] / l, acc[1] / l);
     *reinterpret_cast<__nv_bfloat162*>(out16 + n * D + h * DH + 2 * kl) = o;
+}
+
+// Layer-0 table (TmTable), input rows: row r = t * vocab + tok is bf16(E_tok[tok] + E_pos[t]), decode_embed's arithmetic
+__global__ void __launch_bounds__(128) l0_table_rows(const float* E_tok, const float* E_pos, int vocab, int64_t rows, __nv_bfloat16* out) {
+    const int64_t r = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (r >= rows) return;
+    const int lane = threadIdx.x & 31;
+    const int64_t t = r / vocab, tok = r % vocab;
+    const float4 a = *reinterpret_cast<const float4*>(E_tok + tok * D + lane * 4);
+    const float4 b = *reinterpret_cast<const float4*>(E_pos + t * D + lane * 4);
+    const float4 o = make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
+    __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
+    *reinterpret_cast<uint2*>(out + r * D + lane * 4) = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
+}
+
+// Layer-0 table: the projected rows [rows][Q | K | V] (fp32, bias added) -> qtab [rows][D] fp32 and kvtab [rows][K | V] bf16,
+// rounded like the KV-append epilogue (kernels_tc.cuh pack_bf16x4)
+__global__ void __launch_bounds__(128) l0_table_split(const float* qkv, int64_t rows, float* qtab, __nv_bfloat16* kvtab) {
+    const int64_t r = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (r >= rows) return;
+    const int lane = threadIdx.x & 31;
+    const float* src = qkv + r * (3 * D);
+    *reinterpret_cast<float4*>(qtab + r * D + lane * 4) = *reinterpret_cast<const float4*>(src + lane * 4);
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {
+        const float4 v = *reinterpret_cast<const float4*>(src + D + c * D + lane * 4);
+        __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
+        *reinterpret_cast<uint2*>(kvtab + r * (2 * D) + c * D + lane * 4) = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
+    }
 }
 
 // Cross-attention of the new position over the (compacted) projected memory;
