@@ -203,6 +203,35 @@ int32_t mmt_decode_until_eos(mmt_engine* e, const mmt_decode_args* a, int32_t pe
                              int64_t* d_tokens, float* d_probs, int32_t* d_len, int32_t* h_steps, int64_t* h_rows,
                              void* stream);
 
+/* Per-memory-column sampling controls for multinomial decoding.  Each non-NULL array holds `count` (== the call's
+ * columns) host values; column b (one spectrum, all its n_cand candidates) samples at every step as follows:
+ *   p = softmax(logits / temperature[b])            (bit-identical to the plain call's p where temperature[b] equals it)
+ *   rank: token i before j iff p_i > p_j, or p_i == p_j and i < j
+ *   top-k: keep rank < top_k[b]                     (0 or vocab: off)
+ *   top-p: of the top-k survivors keep the rank-0 token and every i with before_i < top_p[b] * mass, mass = fp32 sum of
+ *          the survivors' p, before_i = that of the survivors ranked before i, both summed in ascending token index
+ *          (top_p[b] == 1: off, not evaluated)
+ *   draw:  the first arg-max of p_i / q_i over the kept tokens, q the Exp(1) variates of the plain call (either RNG
+ *          mapping), so a draw the plain call makes inside the kept set is unchanged; the generator advance is the plain
+ *          call's whatever the controls
+ *   reported probability: p of the chosen token, NOT renormalised over the kept set (equal to the plain call's wherever
+ *          the draw is, and comparable across columns with different truncation).
+ * Ranges, checked on the host: temperature > 0 and finite, top_k in [0, vocab], top_p in (0, 1]. */
+typedef struct mmt_sampling_controls {
+    int64_t        count;           /* entries in each non-NULL array */
+    const float*   h_temperature;   /* (count) host, or NULL: a->temperature for every column */
+    const int32_t* h_top_k;         /* (count) host, or NULL: off */
+    const float*   h_top_p;         /* (count) host, or NULL: off */
+} mmt_sampling_controls;
+
+/* mmt_decode / mmt_decode_memory_streams (eos < 0) or mmt_decode_until_eos (eos >= 0; d_len, h_steps, h_rows as there,
+ * ignored when eos < 0) with per-column sampling controls (count == a->Bm).  Multinomial only.  Neutral controls (every
+ * temperature a->temperature, top-k and top-p off) give the plain call's output bit for bit.  The values are copied to
+ * the device before the first step and are not part of a cached decode graph. */
+int32_t mmt_decode_controlled(mmt_engine* e, const mmt_decode_args* a, int32_t per_memory_rng, int64_t eos,
+                              const mmt_sampling_controls* c, int64_t* d_tokens, float* d_probs, int32_t* d_len,
+                              int32_t* h_steps, int64_t* h_rows, void* stream);
+
 /* Replaces the decoder tail of MultimodalTransformer.forward(..., trg_SMI_input)
  * (models_MMT_v15_4.py:955-976) and the teacher-forced scorers' inner call:
  * d_trg (T,N) i64 -> d_logits (T,N,vocab) f32 (fc_out, before softmax). */
@@ -316,6 +345,18 @@ int32_t mmt_sample_memory_streams(mmt_engine* e, const float* d_x, const float* 
                                   int32_t step, float temperature, uint64_t philox_seed, uint64_t philox_offset,
                                   int64_t seq_index_base, int32_t rng_sm_count, int32_t rng_max_threads_per_sm,
                                   int64_t* d_token, float* d_prob, void* stream);
+
+/* The controlled pick (mmt_sampling_controls) at step `step` of max_len, stand-alone, for N rows; row n belongs to control
+ * column n / n_cand (c->count == ceil(N / n_cand)).  Exactly one of d_x (N,128) hidden states (the decode step's fc_out +
+ * softmax(logits / temperature) + pick; d_logits_out (N,vocab) optional) and d_p (N,vocab) caller probabilities
+ * (temperatures ignored).  RNG: per_memory_rng as mmt_sample_memory_streams, else the global mapping of mmt_sample
+ * (rows seq_index_base .. of an N_total-row call, step `step` at offset philox_offset + step * increment).
+ * d_prob (N) optional: p of the chosen token; d_kept (N,vocab) u8 optional: 1 where the token is kept. */
+int32_t mmt_sample_controlled(mmt_engine* e, const float* d_x, const float* d_p, int64_t N, int32_t n_cand,
+                              const mmt_sampling_controls* c, int32_t per_memory_rng, int32_t max_len, int32_t step,
+                              uint64_t philox_seed, uint64_t philox_offset, int64_t seq_index_base, int64_t N_total,
+                              int32_t rng_sm_count, int32_t rng_max_threads_per_sm,
+                              int64_t* d_token, float* d_prob, float* d_logits_out, uint8_t* d_kept, void* stream);
 
 /* C[M,N] = act(A[M,K] . W[N,K]^T + bias) in the requested precision
  * (fp32 SIMT or bf16 tcgen05); act: 0 none, 1 ReLU. */

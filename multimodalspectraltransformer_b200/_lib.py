@@ -23,8 +23,8 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 EXPORTS = [
     "mmt_abi_version", "mmt_last_error", "mmt_weight_count", "mmt_weight_name", "mmt_weight_numel",
     "mmt_weight_offset", "mmt_weight_total", "mmt_create", "mmt_destroy", "mmt_memory_len",
-    "mmt_mask_is_float", "mmt_encode", "mmt_spectra_equal", "mmt_decode", "mmt_decode_memory_streams", "mmt_decode_until_eos", "mmt_teacher_forced", "mmt_teacher_forced_scores", "mmt_beam_search", "mmt_philox_increment",
-    "mmt_pack_tokens_u8", "mmt_unpack_tokens_u8", "mmt_pack_tokens_u8_seqmajor", "mmt_unpack_tokens_u8_seqmajor", "mmt_first_eos", "mmt_distinct_smiles", "mmt_ingest_peaks", "mmt_ingest_ir", "mmt_sample", "mmt_exponential", "mmt_sample_probs", "mmt_sample_memory_streams", "mmt_linear", "mmt_ffn",
+    "mmt_mask_is_float", "mmt_encode", "mmt_spectra_equal", "mmt_decode", "mmt_decode_memory_streams", "mmt_decode_until_eos", "mmt_decode_controlled", "mmt_teacher_forced", "mmt_teacher_forced_scores", "mmt_beam_search", "mmt_philox_increment",
+    "mmt_pack_tokens_u8", "mmt_unpack_tokens_u8", "mmt_pack_tokens_u8_seqmajor", "mmt_unpack_tokens_u8_seqmajor", "mmt_first_eos", "mmt_distinct_smiles", "mmt_ingest_peaks", "mmt_ingest_ir", "mmt_sample", "mmt_exponential", "mmt_sample_probs", "mmt_sample_memory_streams", "mmt_sample_controlled", "mmt_linear", "mmt_ffn",
     "mmt_decode_self_attention", "mmt_decode_cross_attention", "mmt_decode_layer_tail", "mmt_encoder_layer", "mmt_launch_count",
     "mmt_profile_enable", "mmt_profile_report",
 ]
@@ -57,6 +57,10 @@ class DecodeArgs(C.Structure):
         ("seq_index_base", C.c_int64), ("N_total", C.c_int64),
         ("rng_sm_count", C.c_int32), ("rng_max_threads_per_sm", C.c_int32),
     ]
+
+
+class SamplingControls(C.Structure):
+    _fields_ = [("count", C.c_int64), ("h_temperature", C.c_void_p), ("h_top_k", C.c_void_p), ("h_top_p", C.c_void_p)]
 
 
 def mode_bits(training_mode: str) -> int:
@@ -154,6 +158,11 @@ def lib():
     L.mmt_decode_memory_streams.argtypes = [vp, C.POINTER(DecodeArgs), vp, vp, C.POINTER(i32), vp]; L.mmt_decode_memory_streams.restype = i32
     L.mmt_decode_until_eos.argtypes = [vp, C.POINTER(DecodeArgs), i32, i64, vp, vp, vp, C.POINTER(i32), vp, vp]
     L.mmt_decode_until_eos.restype = i32
+    SC = C.POINTER(SamplingControls)
+    L.mmt_decode_controlled.argtypes = [vp, C.POINTER(DecodeArgs), i32, i64, SC, vp, vp, vp, C.POINTER(i32), vp, vp]
+    L.mmt_decode_controlled.restype = i32
+    L.mmt_sample_controlled.argtypes = [vp, vp, vp, i64, i32, SC, i32, i32, i32, u64, u64, i64, i64, i32, i32, vp, vp, vp, vp, vp]
+    L.mmt_sample_controlled.restype = i32
     L.mmt_spectra_equal.argtypes = [vp, C.POINTER(Spectra), C.POINTER(Spectra), i32, C.c_uint32, C.POINTER(C.c_int32), vp]; L.mmt_spectra_equal.restype = i32
     L.mmt_teacher_forced.argtypes = [vp, C.POINTER(DecodeArgs), vp, i32, vp, vp]; L.mmt_teacher_forced.restype = i32
     L.mmt_teacher_forced_scores.argtypes = [vp, C.POINTER(DecodeArgs), vp, vp, i32, vp, vp, vp, vp]; L.mmt_teacher_forced_scores.restype = i32

@@ -221,7 +221,8 @@ static TcGemmParams tc_params(int M, int N, int K) {
 // sample_tokens keeps fc_out in dynamic shared memory (33 KB at the 64-row maximum, next to 20 KB of static row buffers)
 static int sample_init(mmt_engine* e) {
     if (e->sample_ready) return 0;
-    MMT_CUDA(cudaFuncSetAttribute(sample_tokens, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem_bytes(VOCAB_MAX)));
+    MMT_CUDA(cudaFuncSetAttribute(sample_tokens<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem_bytes(VOCAB_MAX)));
+    MMT_CUDA(cudaFuncSetAttribute(sample_tokens<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem_bytes(VOCAB_MAX)));
     e->sample_ready = true;
     return 0;
 }
@@ -1012,6 +1013,10 @@ struct DecodeRun {
     int64_t eos = -1;            // >= 0: stop at this id (mmt_decode_until_eos): finished sequences retire from large waves
     int32_t* len = nullptr;      //   out (N) first-<EOS> positions
     int64_t* h_rows = nullptr;   //   out (T), optional: rows computed per position
+    // per-column sampling controls (mmt_decode_controlled), multinomial only: validated host arrays (Bm) that run_decode
+    // copies to the device arrays the sampler reads (the values stay out of the captured graph); nullptr otherwise
+    const float* h_temp = nullptr; const int32_t* h_topk = nullptr; const float* h_topp = nullptr;
+    const float* ctl_temp = nullptr; const int32_t* ctl_topk = nullptr; const float* ctl_topp = nullptr;
 };
 
 // Projects the memory of one wave to per-layer cross-attention K/V (head-major) once;
@@ -1411,6 +1416,10 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
     sp.ctl.step = b.ctl; sp.ctl.done_ctas = b.ctl + 1; sp.ctl.nonpad = (r.mode == 0) ? b.ctl + 8 : nullptr;
     sp.advance = 1;
     if (b.eos_len) { sp.orig = b.orig; sp.eos_len = b.eos_len; sp.live = b.ctl + 8 + 128; sp.eos = r.eos; }
+    if (r.ctl_temp) {      // the lane's columns start at column n0 / n_cand
+        const int64_t c0 = n0 / a.n_cand;
+        sp.ctl_temp = r.ctl_temp + c0; sp.ctl_topk = r.ctl_topk + c0; sp.ctl_topp = r.ctl_topp + c0; sp.ctl_cand = a.n_cand;
+    }
     if (fused && ffn_splits > 0) {   // norm3 of the last layer over the FFN2 partials (the cluster variant has applied it)
         const LayerW& pw = e->dec[d.n_dec_layers - 1];
         sp.part = b.part; sp.splits = ffn_splits; sp.part_stride = Nw * D;
@@ -1422,9 +1431,10 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
         const int rpc = sp.part ? 2 : 8 * sp.rows_per_warp;
         const int64_t groups = (Nw + rpc - 1) / rpc;
         MMT_TRY(sample_init(e));
-        launch_kernel(sample_tokens, dim3((unsigned)std::min<int64_t>(groups, (int64_t)e->sm_count * 4)), dim3(256), sample_smem_bytes(sp.V), s, pdl || pdl_u, sp);
+        launch_kernel(r.ctl_temp ? sample_tokens<true> : sample_tokens<false>, dim3((unsigned)std::min<int64_t>(groups, (int64_t)e->sm_count * 4)), dim3(256),
+                      sample_smem_bytes(sp.V), s, pdl || pdl_u, sp);
     }
-    MMT_TRY(check_launch(e, "sample_tokens", s));
+    MMT_TRY(check_launch(e, r.ctl_temp ? "sample_tokens_controlled" : "sample_tokens", s));
     return 0;
 }
 
@@ -1499,10 +1509,13 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     DecBuffers lb[MAX_LANES];
     int64_t* st_tokens = nullptr; float* st_probs = nullptr;
     int* eos_all = nullptr;                  // retiring call: first-<EOS> step of every sequence (max_len until it emits)
+    const bool controlled = r.h_temp != nullptr;
+    float *ctl_temp = nullptr, *ctl_topp = nullptr; int32_t* ctl_topk = nullptr;   // (Bm) per-column sampling controls
     auto plan_all = [&]() {
         for (int i = 0; i < NL; ++i) plan_decoder(ar, d, (int64_t)Bm_lane * a.n_cand, Bm_lane, a.S, a.max_len, lb[i], bf16, e->fused_decode_rows, 1, retire, l0_table, l0_pool);
         if (staged) { st_tokens = ar.get<int64_t>((size_t)a.max_len * N_total); st_probs = ar.get<float>((size_t)a.max_len * N_total); }
         if (retire) eos_all = ar.get<int>(N_total);
+        if (controlled) { ctl_temp = ar.get<float>(a.Bm); ctl_topk = ar.get<int32_t>(a.Bm); ctl_topp = ar.get<float>(a.Bm); }
     };
     ar.plan = true;
     plan_all();
@@ -1511,6 +1524,12 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     plan_all();
     DecodeRun rs = r;                        // the run as the kernels see it
     if (staged) { rs.tokens = st_tokens; rs.probs = r.probs ? st_probs : nullptr; }
+    if (controlled) {     // device copies at fixed arena addresses: a cached decode graph serves calls with other values
+        MMT_CUDA(cudaMemcpyAsync(ctl_temp, r.h_temp, (size_t)a.Bm * sizeof(float), cudaMemcpyHostToDevice, s));
+        MMT_CUDA(cudaMemcpyAsync(ctl_topk, r.h_topk, (size_t)a.Bm * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        MMT_CUDA(cudaMemcpyAsync(ctl_topp, r.h_topp, (size_t)a.Bm * sizeof(float), cudaMemcpyHostToDevice, s));
+        rs.ctl_temp = ctl_temp; rs.ctl_topk = ctl_topk; rs.ctl_topp = ctl_topp;
+    }
     const int pps = (a.max_len + PAGE_TOKENS - 1) / PAGE_TOKENS;
     const bool early = (r.mode == 0) && a.stop_on_all_pad && n_waves == 1;
     int steps_done = r.T;
@@ -1557,7 +1576,7 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
             put((uint64_t)r.mode); put((uint64_t)r.T); put((uint64_t)(r.probs != nullptr)); put((uint64_t)a.S); put((uint64_t)a.Bm);
             put((uint64_t)a.n_cand); put((uint64_t)a.max_len); put(tbits); put((uint64_t)a.precision);
             put((uint64_t)a.seq_index_base); put((uint64_t)a.N_total); put((uint64_t)a.rng_sm_count); put((uint64_t)a.rng_max_threads_per_sm);
-            put((uint64_t)r.per_memory_rng); put((uint64_t)r.eos);
+            put((uint64_t)r.per_memory_rng); put((uint64_t)r.eos); put((uint64_t)controlled);   // controls: their presence, never their values
             put((uint64_t)(uintptr_t)e->arena); put((uint64_t)e->arena_bytes); put((uint64_t)nl); put((uint64_t)U);
             put((uint64_t)e->fused_decode_rows); put((uint64_t)e->use_pdl); put((uint64_t)(uintptr_t)e->da_dbg);
             for (auto& c : e->graph_cache) if (c.key == key) { exec = c.exec; launches_per_group = c.launches_per_group; c.stamp = ++e->graph_cache_clock; break; }
@@ -2085,6 +2104,45 @@ int32_t mmt_decode_until_eos(mmt_engine* e, const mmt_decode_args* a, int32_t pe
     return run_decode(e, r, h_steps, (cudaStream_t)stream);
 }
 
+// The caller's sampling controls for Bm columns, checked on the host, as full host arrays (absent ones: temperature
+// `t_default`, top-k 0, top-p 1).
+static int host_controls(const mmt_sampling_controls* c, int64_t Bm, float t_default, int V, std::vector<float>& temp,
+                         std::vector<int32_t>& topk, std::vector<float>& topp, const char* who) {
+    if (!c) MMT_FAIL(std::string(who) + ": sampling controls are required");
+    if ((c->h_temperature || c->h_top_k || c->h_top_p) && c->count != Bm)
+        MMT_FAIL(std::string(who) + ": sampling controls hold " + std::to_string(c->count) + " columns, the call has " + std::to_string(Bm));
+    temp.assign(Bm, t_default); topk.assign(Bm, 0); topp.assign(Bm, 1.f);
+    for (int64_t b = 0; b < Bm; ++b) {
+        if (c->h_temperature) temp[b] = c->h_temperature[b];
+        if (c->h_top_k) topk[b] = c->h_top_k[b];
+        if (c->h_top_p) topp[b] = c->h_top_p[b];
+        if (!(temp[b] > 0.f) || !std::isfinite(temp[b])) MMT_FAIL(std::string(who) + ": temperature must be > 0 and finite (column " + std::to_string(b) + ")");
+        if (topk[b] < 0 || topk[b] > V) MMT_FAIL(std::string(who) + ": top_k must be in [0, vocab] (column " + std::to_string(b) + ")");
+        if (!(topp[b] > 0.f && topp[b] <= 1.f)) MMT_FAIL(std::string(who) + ": top_p must be in (0, 1] (column " + std::to_string(b) + ")");
+    }
+    return 0;
+}
+
+int32_t mmt_decode_controlled(mmt_engine* e, const mmt_decode_args* a, int32_t per_memory_rng, int64_t eos, const mmt_sampling_controls* c,
+                              int64_t* d_tokens, float* d_probs, int32_t* d_len, int32_t* h_steps, int64_t* h_rows, void* stream) {
+    if (!e || !a) MMT_FAIL("null engine / args");
+    if (!d_tokens) MMT_FAIL("mmt_decode_controlled: d_tokens is required");
+    if (a->sampling != MMT_SAMPLE_MULTINOMIAL) MMT_FAIL("mmt_decode_controlled: sampling controls need multinomial sampling");
+    if (per_memory_rng && (a->n_cand <= 0 || a->seq_index_base < 0 || a->seq_index_base % a->n_cand))
+        MMT_FAIL("mmt_decode_controlled: seq_index_base must be a non-negative multiple of n_cand");
+    if (eos >= 0 && (eos >= e->desc.vocab || !d_len)) MMT_FAIL("mmt_decode_controlled: eos must be in [0, vocab) and d_len given");
+    if (a->Bm <= 0 || a->n_cand <= 0) MMT_FAIL("decode: empty batch");
+    std::vector<float> temp, topp; std::vector<int32_t> topk;
+    MMT_TRY(host_controls(c, a->Bm, a->temperature, e->desc.vocab, temp, topk, topp, "mmt_decode_controlled"));
+    EngineCall call(e, (cudaStream_t)stream);
+    DecodeRun r;
+    r.a = a; r.mode = a->sampling; r.trg = nullptr; r.T = a->max_len; r.tokens = d_tokens; r.probs = d_probs; r.logits = nullptr;
+    r.per_memory_rng = per_memory_rng != 0;
+    if (eos >= 0) { r.eos = eos; r.len = d_len; r.h_rows = h_rows; }
+    r.h_temp = temp.data(); r.h_topk = topk.data(); r.h_topp = topp.data();
+    return run_decode(e, r, h_steps, (cudaStream_t)stream);
+}
+
 int32_t mmt_teacher_forced(mmt_engine* e, const mmt_decode_args* a, const int64_t* d_trg, int32_t T, float* d_logits, void* stream) {
     if (!e || !a || !d_trg || !d_logits) MMT_FAIL("null argument");
     if (T < 1) MMT_FAIL("T must be >= 1");
@@ -2236,7 +2294,7 @@ int32_t mmt_sample(mmt_engine* e, const float* d_x, int64_t N, float temperature
     prof_pre(e, cs);
     MMT_TRY(sample_init(e));
     sp.rows_per_warp = N >= 8192 ? SAMPLE_NR : 1;
-    sample_tokens<<<(unsigned)std::min<int64_t>((N + 8 * sp.rows_per_warp - 1) / (8 * sp.rows_per_warp), (int64_t)e->sm_count * 4), 256, sample_smem_bytes(sp.V), cs>>>(sp);
+    sample_tokens<false><<<(unsigned)std::min<int64_t>((N + 8 * sp.rows_per_warp - 1) / (8 * sp.rows_per_warp), (int64_t)e->sm_count * 4), 256, sample_smem_bytes(sp.V), cs>>>(sp);
     return check_launch(e, "sample_tokens", cs);
 }
 
@@ -2302,8 +2360,69 @@ int32_t mmt_sample_memory_streams(mmt_engine* e, const float* d_x, const float* 
     sp.advance = 0;
     MMT_TRY(sample_init(e));
     sp.rows_per_warp = N >= 8192 ? SAMPLE_NR : 1;
-    sample_tokens<<<(unsigned)std::min<int64_t>((N + 8 * sp.rows_per_warp - 1) / (8 * sp.rows_per_warp), (int64_t)e->sm_count * 4), 256, sample_smem_bytes(sp.V), cs>>>(sp);
+    sample_tokens<false><<<(unsigned)std::min<int64_t>((N + 8 * sp.rows_per_warp - 1) / (8 * sp.rows_per_warp), (int64_t)e->sm_count * 4), 256, sample_smem_bytes(sp.V), cs>>>(sp);
     return check_launch(e, "sample_tokens", cs);
+}
+
+int32_t mmt_sample_controlled(mmt_engine* e, const float* d_x, const float* d_p, int64_t N, int32_t n_cand, const mmt_sampling_controls* c,
+                              int32_t per_memory_rng, int32_t max_len, int32_t step, uint64_t philox_seed, uint64_t philox_offset,
+                              int64_t seq_index_base, int64_t N_total, int32_t rng_sm_count, int32_t rng_max_threads_per_sm,
+                              int64_t* d_token, float* d_prob, float* d_logits_out, uint8_t* d_kept, void* stream) {
+    if (!e || !d_token || (!d_x) == (!d_p)) MMT_FAIL("mmt_sample_controlled: give d_token and exactly one of d_x, d_p");
+    if (n_cand <= 0 || max_len < 1 || step < 0 || step >= max_len) MMT_FAIL("mmt_sample_controlled: need n_cand >= 1 and 0 <= step < max_len");
+    if (per_memory_rng && (seq_index_base < 0 || seq_index_base % n_cand))
+        MMT_FAIL("mmt_sample_controlled: seq_index_base must be a non-negative multiple of n_cand");
+    if (d_p && d_logits_out) MMT_FAIL("mmt_sample_controlled: d_logits_out needs d_x");
+    const int V = e->desc.vocab;
+    if (N <= 0) return 0;
+    const int64_t Nrng = N_total > 0 ? N_total : N;
+    if (!per_memory_rng && (seq_index_base < 0 || Nrng < seq_index_base + N)) MMT_FAIL("mmt_sample_controlled: N_total smaller than seq_index_base + N");
+    const int64_t Bm = (N + n_cand - 1) / n_cand;
+    std::vector<float> temp, topp; std::vector<int32_t> topk;
+    MMT_TRY(host_controls(c, Bm, 1.f, V, temp, topk, topp, "mmt_sample_controlled"));
+    EngineCall call(e, (cudaStream_t)stream);
+    cudaStream_t cs = (cudaStream_t)stream;
+    const int smc = rng_sm_count > 0 ? rng_sm_count : e->sm_count;
+    const int mts = rng_max_threads_per_sm > 0 ? rng_max_threads_per_sm : e->max_threads_per_sm;
+    RngGeom g;
+    g.seed = philox_seed; g.offset = philox_offset; g.numel = (per_memory_rng ? (int64_t)n_cand : Nrng) * V; g.threads = torch_rng_threads(g.numel, smc, mts);
+    const uint64_t inc = torch_rng_increment(g.numel, smc, mts);
+    // workspace: step counter, then the controls
+    const size_t o_temp = 256, o_topk = o_temp + (size_t)Bm * 4, o_topp = o_topk + (size_t)Bm * 4;
+    MMT_TRY(ensure_arena(e, o_topp + (size_t)Bm * 4));
+    char* ws = reinterpret_cast<char*>(e->arena);
+    float* ctl_temp = reinterpret_cast<float*>(ws + o_temp); int32_t* ctl_topk = reinterpret_cast<int32_t*>(ws + o_topk);
+    float* ctl_topp = reinterpret_cast<float*>(ws + o_topp);
+    MMT_CUDA(cudaMemcpyAsync(ctl_temp, temp.data(), (size_t)Bm * 4, cudaMemcpyHostToDevice, cs));
+    MMT_CUDA(cudaMemcpyAsync(ctl_topk, topk.data(), (size_t)Bm * 4, cudaMemcpyHostToDevice, cs));
+    MMT_CUDA(cudaMemcpyAsync(ctl_topp, topp.data(), (size_t)Bm * 4, cudaMemcpyHostToDevice, cs));
+    prof_pre(e, cs);
+    if (d_p) {
+        if (V > 64) MMT_FAIL("mmt_sample_controlled: vocab > 64");
+        sample_probs_controlled<<<(unsigned)((N + 7) / 8), 256, 0, cs>>>(d_p, N, V, g, seq_index_base, inc, per_memory_rng ? n_cand : 0, max_len, step,
+                                                                          n_cand, ctl_topk, ctl_topp, d_token, d_prob, d_kept);
+        return check_launch(e, "sample_probs_controlled", cs);
+    }
+    int* ctl = reinterpret_cast<int*>(ws);
+    MMT_CUDA(cudaMemcpyAsync(ctl, &step, sizeof(int), cudaMemcpyHostToDevice, cs));
+    SampleParams sp;
+    memset(&sp, 0, sizeof(sp));
+    sp.x = d_x; sp.W = e->W("fc_out.weight"); sp.b = e->W("fc_out.bias"); sp.V = V; sp.N = N; sp.ldn = N;
+    sp.temperature = 1.f; sp.mode = MMT_SAMPLE_MULTINOMIAL;
+    sp.rng = g; sp.rng_inc = inc; sp.seq_index_base = seq_index_base;
+    if (per_memory_rng) { sp.rng_cand = n_cand; sp.rng_col_steps = max_len; }
+    // row `step` of each output = the caller's buffer
+    sp.tokens = d_token - (int64_t)step * N; sp.probs = d_prob ? d_prob - (int64_t)step * N : nullptr;
+    sp.logits = d_logits_out ? d_logits_out - (int64_t)step * N * V : nullptr;
+    sp.kept = d_kept ? d_kept - (int64_t)step * N * V : nullptr;
+    sp.ctl_temp = ctl_temp; sp.ctl_topk = ctl_topk; sp.ctl_topp = ctl_topp; sp.ctl_cand = n_cand;
+    sp.ctl.step = ctl;
+    sp.advance = 0;
+    MMT_TRY(sample_init(e));
+    sp.rows_per_warp = N >= 8192 ? SAMPLE_NR : 1;
+    sample_tokens<true><<<(unsigned)std::min<int64_t>((N + 8 * sp.rows_per_warp - 1) / (8 * sp.rows_per_warp), (int64_t)e->sm_count * 4), 256,
+                               sample_smem_bytes(sp.V), cs>>>(sp);
+    return check_launch(e, "sample_tokens_controlled", cs);
 }
 
 int32_t mmt_distinct_smiles(const int64_t* d_tokens, int32_t T, int64_t N, int32_t n_cand, int64_t eos,

@@ -1449,6 +1449,11 @@ struct SampleParams {
     // kernels_retire.cuh; nullptr = r), whose first-<EOS> step eos_len[] holds (max_len until it emits `eos`).  A
     // finished sequence writes <PAD> / 0 and counts as <PAD>; live[t] counts the sequences not finished after step t.
     const int* orig; int* eos_len; int* live; int64_t eos;
+    // per-column sampling controls (sample_tokens_controlled, multinomial only): row r, sequence no = orig[r] (or r) of the
+    // launch, belongs to column no / ctl_cand, which samples at temperature ctl_temp[c] from the kept set of top-k ctl_topk[c]
+    // and top-p ctl_topp[c] (sample_kept).  kept: optional [T][N][V] u8 copy of the kept set (unit test).
+    const float* ctl_temp; const int* ctl_topk; const float* ctl_topp; int64_t ctl_cand;
+    uint8_t* kept;
 };
 
 // CTA = 8 warps.  Rows are taken in groups of `rpc` per CTA, grid-stride: a CTA stages fc_out once and keeps sampling
@@ -1463,7 +1468,47 @@ struct SampleParams {
 constexpr int SAMPLE_NR = 4;             // rows per warp (dense input)
 constexpr int SAMPLE_ROWS = 8 * SAMPLE_NR;
 
-template <int NR>
+// Kept set of one row under top-k / top-p; the warp holds the row's probabilities two tokens per lane (token lane in p0,
+// lane + 32 in p1; V <= 64, p = 0 past V), keep0 / keep1 come in as "token exists" and leave as "token kept".
+// Token i ranks before j iff p_i > p_j, or p_i == p_j and i < j.  top-k (0 < k < V) keeps rank < k.  top-p (top_p < 1)
+// then keeps, among those survivors, the rank-0 token and every i with before_i < top_p * mass: mass is the fp32 sum of
+// the survivors' p, before_i that of the survivors ranked before i, both summed in ascending token index (HF order:
+// top-k first, the nucleus over the renormalised survivors).  Every j ranked before a survivor is a survivor, so before_i
+// is the sum over all j ranked before i.  Both controls off: nothing is evaluated.
+__device__ __forceinline__ void sample_kept(float p0, float p1, int V, int k, float top_p, int lane, bool& keep0, bool& keep1) {
+    const bool use_k = k > 0 && k < V, use_p = top_p < 1.f;
+    if (!use_k && !use_p) return;
+    const int v0 = lane, v1 = lane + 32;
+    int rk0 = 0, rk1 = 0;
+    float bf0 = 0.f, bf1 = 0.f, tot = 0.f;
+    for (int j = 0; j < V; ++j) {      // p_j broadcast in index order
+        const float pj = __shfl_sync(0xffffffffu, j < 32 ? p0 : p1, j & 31);
+        const bool b0 = pj > p0 || (pj == p0 && j < v0);
+        const bool b1 = pj > p1 || (pj == p1 && j < v1);
+        rk0 += b0; rk1 += b1;
+        if (b0) bf0 += pj;
+        if (b1) bf1 += pj;
+        tot += pj;
+    }
+    if (use_k) { keep0 = keep0 && rk0 < k; keep1 = keep1 && rk1 < k; }
+    if (!use_p) return;
+    float mass = tot;                  // no top-k: every token survives
+    if (use_k) {
+        mass = 0.f;
+        for (int j = 0; j < V; ++j) {
+            const float pj = __shfl_sync(0xffffffffu, j < 32 ? p0 : p1, j & 31);
+            const int kj = __shfl_sync(0xffffffffu, (int)(j < 32 ? keep0 : keep1), j & 31);
+            if (kj) mass += pj;
+        }
+    }
+    const float lim = top_p * mass;
+    keep0 = keep0 && (rk0 == 0 || bf0 < lim);
+    keep1 = keep1 && (rk1 == 0 || bf1 < lim);
+}
+
+// CTL: the controlled variant (per-column temperature / top-k / top-p, SampleParams::ctl_*); the plain instantiation is
+// the decode step's sampler as it always was
+template <int NR, bool CTL>
 __device__ __forceinline__ void sample_rows(const SampleParams& p, const float* Ws, const float (*xs)[D], int r0, int64_t n0, int t, int lane, int& my_nonpad,
                                             int& my_live) {
     const int v0 = lane, v1 = lane + 32;
@@ -1500,8 +1545,9 @@ __device__ __forceinline__ void sample_rows(const SampleParams& p, const float* 
             if (ok1) out[v1] = lg1;
         }
         if (p.mode == 2) continue;
-        float z0 = ok0 ? lg0 / p.temperature : MMT_NEG_INF;
-        float z1 = ok1 ? lg1 / p.temperature : MMT_NEG_INF;
+        const int64_t col = CTL ? no / p.ctl_cand : 0;      // the row's control column
+        float z0 = ok0 ? lg0 / (CTL ? p.ctl_temp[col] : p.temperature) : MMT_NEG_INF;
+        float z1 = ok1 ? lg1 / (CTL ? p.ctl_temp[col] : p.temperature) : MMT_NEG_INF;
         float mx = warp_max(fmaxf(z0, z1));
         float e0 = ok0 ? expf(z0 - mx) : 0.f;
         float e1 = ok1 ? expf(z1 - mx) : 0.f;
@@ -1512,6 +1558,15 @@ __device__ __forceinline__ void sample_rows(const SampleParams& p, const float* 
             const float a = __shfl_sync(0xffffffffu, p0, (int)(tg & 31)), b = __shfl_sync(0xffffffffu, p1, (int)(tg & 31));
             if (lane == 0) p.target_prob[(int64_t)t * p.ldn + n] = (tg < 0 || tg >= p.V) ? 0.f : (tg < 32 ? a : b);
         }
+        bool k0 = ok0, k1 = ok1;       // candidates of the arg-max
+        if constexpr (CTL) {
+            sample_kept(p0, p1, p.V, p.ctl_topk[col], p.ctl_topp[col], lane, k0, k1);
+            if (p.kept) {
+                uint8_t* out = p.kept + ((int64_t)t * p.ldn + n) * p.V;
+                if (ok0) out[v0] = k0;
+                if (ok1) out[v1] = k1;
+            }
+        }
         float r0v = p0, r1v = p1;
         if (p.mode == 1) {
             RngGeom g = p.rng;
@@ -1520,11 +1575,12 @@ __device__ __forceinline__ void sample_rows(const SampleParams& p, const float* 
             if (ok0) r0v = p0 / torch_exponential_at(g, li + v0);
             if (ok1) r1v = p1 / torch_exponential_at(g, li + v1);
         }
-        // argmax with lowest-index ties (torch argmax / multinomial)
-        float best = ok0 ? r0v : MMT_NEG_INF;
-        int bi = ok0 ? v0 : 0x7fffffff;
+        // argmax with lowest-index ties (torch argmax / multinomial); the controlled variant over the kept set, reporting
+        // the chosen token's p (not renormalised)
+        float best = k0 ? r0v : MMT_NEG_INF;
+        int bi = k0 ? v0 : 0x7fffffff;
         float bp = p0;
-        if (ok1 && (r1v > best)) { best = r1v; bi = v1; bp = p1; }
+        if (k1 && (r1v > best)) { best = r1v; bi = v1; bp = p1; }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
             float ob = __shfl_xor_sync(0xffffffffu, best, o);
@@ -1548,6 +1604,8 @@ __device__ __forceinline__ void sample_rows(const SampleParams& p, const float* 
 
 // dynamic shared memory: fc_out as V padded rows (sample_smem_bytes)
 __host__ __device__ constexpr size_t sample_smem_bytes(int V) { return (size_t)V * (D + 1) * sizeof(float); }
+// CTL: per-column temperature / top-k / top-p (mmt_decode_controlled, mmt_sample_controlled)
+template <bool CTL>
 __global__ void __launch_bounds__(256) sample_tokens(const __grid_constant__ SampleParams p) {
     extern __shared__ float Ws[];
     __shared__ __align__(16) float xs[SAMPLE_ROWS][D];
@@ -1601,7 +1659,7 @@ __global__ void __launch_bounds__(256) sample_tokens(const __grid_constant__ Sam
                 *reinterpret_cast<float4*>(&xs[warp][lane * 4]) = v;
             }
             __syncthreads();
-            if (warp < rpc && base + warp < p.N) sample_rows<1>(p, Ws, xs, warp, base + warp, t, lane, my_nonpad, my_live);
+            if (warp < rpc && base + warp < p.N) sample_rows<1, CTL>(p, Ws, xs, warp, base + warp, t, lane, my_nonpad, my_live);
         } else if (nr4) {   // ---- dense input: each warp stages and samples its own four rows
 #pragma unroll
             for (int r = 0; r < SAMPLE_NR; ++r) {
@@ -1609,12 +1667,12 @@ __global__ void __launch_bounds__(256) sample_tokens(const __grid_constant__ Sam
                 if (n < p.N) *reinterpret_cast<float4*>(&xs[warp * SAMPLE_NR + r][lane * 4]) = *reinterpret_cast<const float4*>(p.x + n * D + lane * 4);
             }
             __syncthreads();      // (also orders the Ws staging of the first pass)
-            if (base + warp * SAMPLE_NR < p.N) sample_rows<SAMPLE_NR>(p, Ws, xs, warp * SAMPLE_NR, base + warp * SAMPLE_NR, t, lane, my_nonpad, my_live);
+            if (base + warp * SAMPLE_NR < p.N) sample_rows<SAMPLE_NR, CTL>(p, Ws, xs, warp * SAMPLE_NR, base + warp * SAMPLE_NR, t, lane, my_nonpad, my_live);
         } else {            // ---- dense input, small waves: one row per warp (more CTAs, shorter chain)
             const int64_t n = base + warp;
             if (n < p.N) *reinterpret_cast<float4*>(&xs[warp][lane * 4]) = *reinterpret_cast<const float4*>(p.x + n * D + lane * 4);
             __syncthreads();
-            if (n < p.N) sample_rows<1>(p, Ws, xs, warp, n, t, lane, my_nonpad, my_live);
+            if (n < p.N) sample_rows<1, CTL>(p, Ws, xs, warp, n, t, lane, my_nonpad, my_live);
         }
         __syncthreads();          // xs / psum are rewritten by the next group
     }
@@ -1664,6 +1722,44 @@ __global__ void __launch_bounds__(256) sample_from_probs(const float* p, int64_t
         if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
     }
     if (lane == 0) token[n] = bi;
+}
+
+// sample_from_probs restricted to the kept set of each row (sample_kept; V <= 64): row n belongs to column n / ctl_cand,
+// whose top-k / top-p are topk / topp[column].  prob (optional) = p of the chosen token, kept (optional) (N,V) u8.
+__global__ void __launch_bounds__(256) sample_probs_controlled(const float* p, int64_t N, int V, RngGeom g, int64_t seq_base, uint64_t inc,
+                                                               int64_t n_cand, int64_t col_steps, int t, int64_t ctl_cand, const int* topk,
+                                                               const float* topp, int64_t* token, float* prob, uint8_t* kept) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t n = (int64_t)blockIdx.x * 8 + warp;
+    if (n >= N) return;
+    const int v0 = lane, v1 = lane + 32;
+    const bool ok0 = v0 < V, ok1 = v1 < V;
+    const float p0 = ok0 ? p[n * V + v0] : 0.f, p1 = ok1 ? p[n * V + v1] : 0.f;
+    bool k0 = ok0, k1 = ok1;
+    sample_kept(p0, p1, V, topk[n / ctl_cand], topp[n / ctl_cand], lane, k0, k1);
+    if (kept) {
+        if (ok0) kept[n * V + v0] = k0;
+        if (ok1) kept[n * V + v1] = k1;
+    }
+    const int64_t li = torch_rng_row(g, inc, n_cand, col_steps, seq_base + n, t, V);
+    float best = k0 ? p0 / torch_exponential_at(g, li + v0) : MMT_NEG_INF;
+    int bi = k0 ? v0 : 0x7fffffff;
+    float bp = p0;
+    if (k1) {
+        const float r1 = p1 / torch_exponential_at(g, li + v1);
+        if (r1 > best) { best = r1; bi = v1; bp = p1; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const float ob = __shfl_xor_sync(0xffffffffu, best, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        const float op = __shfl_xor_sync(0xffffffffu, bp, o);
+        if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; bp = op; }
+    }
+    if (lane == 0) {
+        token[n] = bi;
+        if (prob) prob[n] = bp;
+    }
 }
 
 // len[n] = index of the first `eos` in column n of tokens (T, N), or T when there is none

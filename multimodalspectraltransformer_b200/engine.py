@@ -8,6 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import weakref
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -54,6 +55,55 @@ def _normalize_state_dict(state_dict):
 def default_precision(config) -> str:
     """``config.precision`` ("fp32" check mode | "bf16" tensor-core mode); fp32 when unset."""
     return str(getattr(config, "precision", "fp32"))
+
+
+def control_arrays(n_cols, vocab, temperature, top_k=0, top_p=1.0):
+    """Per-column sampling controls for ``n_cols`` memory columns (spectra), each a scalar or a length-``n_cols``
+    sequence / tensor, checked: temperature > 0 and finite, top_k an integer in [0, vocab] (0 or vocab: off), top_p in
+    (0, 1] (1: off).  -> (temperature f32, top_k i32, top_p f32) numpy arrays of ``n_cols``; raises ValueError."""
+    def column(name, v):
+        a = np.asarray(v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else v)
+        if a.ndim == 0:
+            a = np.full(n_cols, a)
+        if a.ndim != 1 or a.shape[0] != n_cols:
+            raise ValueError(f"{name} must be a scalar or hold one value per spectrum ({n_cols}), got shape {a.shape}")
+        if not (np.issubdtype(a.dtype, np.number) or a.dtype == np.bool_):
+            raise ValueError(f"{name} must be numeric")
+        return a
+    t = column("temperature", temperature).astype(np.float32)
+    if not bool(np.all(np.isfinite(t) & (t > 0))):
+        raise ValueError("temperature must be > 0 and finite")
+    k = column("top_k", top_k)
+    if not np.issubdtype(k.dtype, np.integer):
+        if not bool(np.all(np.isfinite(k) & (k == np.round(k)))):
+            raise ValueError("top_k must be an integer")
+    k = k.astype(np.float64)
+    if not bool(np.all((k >= 0) & (k <= vocab))):
+        raise ValueError(f"top_k must be in [0, {vocab}]")
+    p = column("top_p", top_p).astype(np.float32)
+    if not bool(np.all((p > 0) & (p <= 1))):
+        raise ValueError("top_p must be in (0, 1]")
+    return np.ascontiguousarray(t), np.ascontiguousarray(k.astype(np.int32)), np.ascontiguousarray(p)
+
+
+def sampling_controls(n_cols, vocab, temperature, top_k=0, top_p=1.0, *, sampling="multinomial"):
+    """``control_arrays``, then -> (temperature, None) when the controls are neutral -- one temperature for every column,
+    top-k and top-p off: the plain decode call -- else (the first column's temperature, the arrays).  Controls that are not
+    neutral need multinomial sampling (ValueError for greedy).  The defaults (a scalar temperature, top_k=0, top_p=1.0)
+    return at once: the plain call checks its temperature as it always has."""
+    if isinstance(temperature, (int, float)) and isinstance(top_k, int) and isinstance(top_p, (int, float)) and top_k == 0 and top_p == 1:
+        return float(temperature), None
+    t, k, p = control_arrays(n_cols, vocab, temperature, top_k, top_p)
+    if bool(np.all(t == t[0])) and bool(np.all((k == 0) | (k == vocab))) and bool(np.all(p == 1)):
+        return float(t[0]), None
+    if sampling != "multinomial":
+        raise ValueError("temperature per spectrum, top_k and top_p need multinomial sampling")
+    return float(t[0]), (t, k, p)
+
+
+def _controls_struct(ctl):
+    t, k, p = ctl
+    return _lib.SamplingControls(count=len(t), h_temperature=t.ctypes.data, h_top_k=k.ctypes.data, h_top_p=p.ctypes.data)
 
 
 class Engine:
@@ -219,10 +269,18 @@ class Engine:
         return a, (memory, key_bias)
 
     def decode(self, memory, key_bias, *, n_cand=1, max_len=128, temperature=1.0, sampling="greedy",
-               stop_on_all_pad=False, precision="fp32", seed=0, offset=0, seq_index_base=0, n_total=0, per_memory_rng=False):
+               stop_on_all_pad=False, precision="fp32", seed=0, offset=0, seq_index_base=0, n_total=0, per_memory_rng=False,
+               top_k=0, top_p=1.0):
         """Returns (tokens (T,N) i64, probs (T,N) f32, steps) with T == max_len rows allocated.  ``per_memory_rng``: the
         n_cand candidates of each memory column draw as one torch.multinomial((n_cand, V), 1) call per step, the columns'
-        calls in order (``mmt_decode_memory_streams``); multinomial only, seq_index_base a multiple of n_cand."""
+        calls in order (``mmt_decode_memory_streams``); multinomial only, seq_index_base a multiple of n_cand.
+        ``temperature`` / ``top_k`` / ``top_p``: a scalar or one value per memory column (``control_arrays``); controls
+        that are not neutral run ``decode_controlled``."""
+        temperature, ctl = sampling_controls(memory.shape[1], self.vocab, temperature, top_k, top_p, sampling=sampling)
+        if ctl is not None:
+            return self.decode_controlled(memory, key_bias, n_cand=n_cand, max_len=max_len, temperature=ctl[0], top_k=ctl[1],
+                                          top_p=ctl[2], precision=precision, seed=seed, offset=offset,
+                                          seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng)[:3]
         smp = _lib.SAMPLE_GREEDY if sampling == "greedy" else _lib.SAMPLE_MULTINOMIAL
         if per_memory_rng and (smp != _lib.SAMPLE_MULTINOMIAL or seq_index_base % n_cand):
             raise ValueError("per_memory_rng needs multinomial sampling and seq_index_base a multiple of n_candidates")
@@ -240,12 +298,17 @@ class Engine:
 
     def decode_until_eos(self, memory, key_bias, *, eos, n_cand=1, max_len=128, temperature=1.0, sampling="greedy",
                          stop_on_all_pad=False, precision="fp32", seed=0, offset=0, seq_index_base=0, n_total=0,
-                         per_memory_rng=False):
+                         per_memory_rng=False, top_k=0, top_p=1.0):
         """``decode`` that stops computing a sequence once it has emitted ``eos`` (``mmt_decode_until_eos``).  Returns
         (tokens (T,N) i64, probs (T,N) f32, steps, lengths (N,) i32, rows (T,) i64 on the host): ids and probabilities
         equal ``decode``'s up to and including each sequence's first ``eos`` and are <PAD> / 0 after it (and from
         ``steps`` on); ``lengths`` = position of that first ``eos`` (max_len if none); ``rows`` = decode-step rows
-        computed at each position."""
+        computed at each position.  Sampling controls as ``decode``."""
+        temperature, ctl = sampling_controls(memory.shape[1], self.vocab, temperature, top_k, top_p, sampling=sampling)
+        if ctl is not None:
+            return self.decode_controlled(memory, key_bias, eos=eos, n_cand=n_cand, max_len=max_len, temperature=ctl[0],
+                                          top_k=ctl[1], top_p=ctl[2], precision=precision, seed=seed, offset=offset,
+                                          seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng)
         smp = _lib.SAMPLE_GREEDY if sampling == "greedy" else _lib.SAMPLE_MULTINOMIAL
         if per_memory_rng and (smp != _lib.SAMPLE_MULTINOMIAL or seq_index_base % n_cand):
             raise ValueError("per_memory_rng needs multinomial sampling and seq_index_base a multiple of n_candidates")
@@ -262,6 +325,35 @@ class Engine:
                                                self._stream()))
         for t in keep:
             t.record_stream(torch.cuda.current_stream(self.dev_index))
+        return tokens, probs, int(steps.value), lengths, rows
+
+    def decode_controlled(self, memory, key_bias, *, n_cand=1, max_len=128, temperature=1.0, top_k=0, top_p=1.0, eos=None,
+                          precision="fp32", seed=0, offset=0, seq_index_base=0, n_total=0, per_memory_rng=False):
+        """Multinomial decode with per-column sampling controls (``mmt_decode_controlled``), also when they are neutral:
+        at temperature[b] (a scalar or one per memory column), from the kept set of top_k[b] / top_p[b]
+        (``mmt_sampling_controls``: HF order, ties by lower index).  The reported probabilities are softmax(logits /
+        temperature[b]) of the chosen token, NOT renormalised over the kept set: where a draw equals the plain call's, so
+        does its probability, and probabilities stay comparable across columns.  The generator advance is the plain
+        call's.  -> (tokens, probs, steps), and with ``eos`` (``decode_until_eos``) also (lengths, rows)."""
+        if per_memory_rng and seq_index_base % n_cand:
+            raise ValueError("per_memory_rng needs seq_index_base a multiple of n_candidates")
+        ctl = control_arrays(memory.shape[1], self.vocab, temperature, top_k, top_p)
+        a, keep = self._decode_args(memory, key_bias, n_cand, max_len, float(ctl[0][0]), _lib.SAMPLE_MULTINOMIAL, False,
+                                    precision, seed, offset, seq_index_base, n_total)
+        N = a.Bm * n_cand
+        tokens = torch.empty(max_len, N, device=self.device, dtype=torch.int64)
+        probs = torch.empty(max_len, N, device=self.device, dtype=torch.float32)
+        lengths = torch.empty(N, device=self.device, dtype=torch.int32) if eos is not None else None
+        rows = torch.zeros(max_len, dtype=torch.int64)
+        steps = C.c_int32(max_len)
+        c = _controls_struct(ctl)
+        _lib.check(self.L.mmt_decode_controlled(self.h, C.byref(a), int(per_memory_rng), -1 if eos is None else int(eos), C.byref(c),
+                                                tokens.data_ptr(), probs.data_ptr(), lengths.data_ptr() if lengths is not None else None,
+                                                C.byref(steps), rows.data_ptr(), self._stream()))
+        for t in keep:
+            t.record_stream(torch.cuda.current_stream(self.dev_index))
+        if eos is None:
+            return tokens, probs, int(steps.value)
         return tokens, probs, int(steps.value), lengths, rows
 
     def teacher_forced(self, memory, key_bias, trg, *, n_cand=1, precision="fp32"):
@@ -358,6 +450,25 @@ class Engine:
                                                     N, n_cand, max_len, step, float(temperature), seed, offset, seq_index_base,
                                                     0, 0, tok.data_ptr(), pr.data_ptr() if pr is not None else None, self._stream()))
         return tok, pr
+
+    def sample_controlled(self, *, x=None, p=None, n_cand=1, temperature=1.0, top_k=0, top_p=1.0, per_memory_rng=False,
+                          max_len=1, step=0, seed=0, offset=0, seq_index_base=0, n_total=0, want_logits=False, want_kept=False):
+        """The controlled pick at one step (``mmt_sample_controlled``, test hook): rows n of x (N,128) hidden states or
+        of p (N,V) probabilities, control column n // n_cand (controls: a scalar or one per column).
+        -> (ids (N,), probabilities (N,) of the chosen token, logits (N,V) | None, kept (N,V) u8 | None)."""
+        src = (x if p is None else p).to(self.device, torch.float32).contiguous()
+        N = src.shape[0]
+        ctl = control_arrays((N + n_cand - 1) // n_cand, self.vocab, temperature, top_k, top_p)
+        tok = torch.empty(N, device=self.device, dtype=torch.int64)
+        pr = torch.empty(N, device=self.device, dtype=torch.float32)
+        lg = torch.empty(N, self.vocab, device=self.device, dtype=torch.float32) if want_logits and p is None else None
+        kept = torch.empty(N, self.vocab, device=self.device, dtype=torch.uint8) if want_kept else None
+        c = _controls_struct(ctl)
+        _lib.check(self.L.mmt_sample_controlled(self.h, src.data_ptr() if p is None else None, src.data_ptr() if p is not None else None,
+                                                N, n_cand, C.byref(c), int(per_memory_rng), max_len, step, seed, offset, seq_index_base,
+                                                n_total, 0, 0, tok.data_ptr(), pr.data_ptr(), lg.data_ptr() if lg is not None else None,
+                                                kept.data_ptr() if kept is not None else None, self._stream()))
+        return tok, pr, lg, kept
 
     def linear(self, A, W, bias=None, act=0, precision="fp32"):
         A = A.to(self.device, torch.float32).contiguous()

@@ -33,6 +33,14 @@ Extensions (keyword-only, default = reference behaviour):
                    <PAD> / 0 after it; shapes and generator advance are unchanged (greedy
                    also stops once every sequence has finished).  Every consumer of the ids
                    (tensor_to_smiles*, distinct_smiles) ignores what follows <EOS>.
+  temperature=None, top_k=0, top_p=1.0  multinomial sampling controls per spectrum, each a
+                   scalar or one value per spectrum (a spectrum's candidates share them):
+                   softmax(logits / temperature) (None: config.temperature at call time), then
+                   the draw restricted to the top_k most probable tokens (0 or vocab: off) and,
+                   of those, the nucleus of mass top_p (1: off), HF order.  A draw the default
+                   call makes inside the kept set is unchanged; the reported probability is the
+                   chosen token's softmax(logits / temperature), not renormalised.  Neutral
+                   controls run the default call; greedy sampling refuses any other.
 """
 from __future__ import annotations
 
@@ -142,11 +150,26 @@ def _philox_advance(eng, n_candidates, n_total, max_len, per_memory_rng):
     return eng.philox_increment(n_total) * max_len
 
 
+def _vocab(model, config):
+    return _engine._desc_from(getattr(model, "config", config), _engine._normalize_state_dict(model.state_dict())).vocab
+
+
+def _controls(model, config, n_cols, sampling, temperature, top_k, top_p):
+    """Checked sampling controls for n_cols spectra (engine.sampling_controls), before any engine exists."""
+    if temperature is None:
+        temperature = float(config.temperature)
+    return _engine.sampling_controls(n_cols, _vocab(model, config), temperature, top_k, top_p, sampling=sampling)
+
+
 def _decode(model, memory, src_padding_mask, config, sampling, stop_on_all_pad, n_candidates, seq_index_base, n_total,
-            per_memory_rng=False, eos=None):
-    """eos: None, or the id at which a sequence stops being computed (Engine.decode_until_eos)."""
+            per_memory_rng=False, eos=None, temperature=None, top_k=0, top_p=1.0):
+    """eos: None, or the id at which a sequence stops being computed (Engine.decode_until_eos).  temperature / top_k /
+    top_p: sampling controls per memory column (module docstring)."""
     if per_memory_rng and (sampling != "multinomial" or seq_index_base % n_candidates):
         raise ValueError("per_memory_rng needs multinomial sampling and seq_index_base a multiple of n_candidates")
+    temperature, ctl = _controls(model, config, memory.size(1), sampling, temperature, top_k, top_p)
+    if ctl is not None:
+        temperature, top_k, top_p = ctl
     model.eval()                                    # the reference flips eval() and leaves it
     eng = _engine.engine_for(model, config)
     prec = _engine.default_precision(config)
@@ -160,8 +183,10 @@ def _decode(model, memory, src_padding_mask, config, sampling, stop_on_all_pad, 
     if eos is not None:
         kw["eos"] = eos
     run = eng.decode if eos is None else eng.decode_until_eos
+    if ctl is not None:
+        kw.update(top_k=top_k, top_p=top_p)
     tokens, probs, steps = run(memory, bias, n_cand=n_candidates, max_len=int(config.max_len),
-                               temperature=float(config.temperature), sampling=sampling,
+                               temperature=temperature, sampling=sampling,
                                stop_on_all_pad=stop_on_all_pad, precision=prec,
                                seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng, **kw)[:3]
     if gen is not None:   # consume exactly what the torch.multinomial calls would have
@@ -188,34 +213,34 @@ def greedy_sequence_2(model, stoi, itos, memory, src_padding_mask, config, *, n_
 
 
 def multinomial_sequence(model, stoi, memory, src_padding_mask, config, *, n_candidates=1, seq_index_base=0, n_total=0,
-                         per_memory_rng=False, stop_at_eos=False):
+                         per_memory_rng=False, stop_at_eos=False, temperature=None, top_k=0, top_p=1.0):
     """-> ((T,N) i64, (N,T) f32): probabilities transposed, always max_len steps."""
     _check_sos(stoi)
     eos = _eos_id(stoi) if stop_at_eos else None
     tokens, probs, _ = _decode(model, memory, src_padding_mask, config, "multinomial", False, n_candidates, seq_index_base, n_total,
-                               per_memory_rng, eos=eos)
+                               per_memory_rng, eos=eos, temperature=temperature, top_k=top_k, top_p=top_p)
     return tokens, probs.transpose(0, 1)
 
 
 def multinomial_sequence_multi(model, memory, src_padding_mask, stoi, config, *, n_candidates=1, seq_index_base=0, n_total=0,
-                               per_memory_rng=False, stop_at_eos=False):
+                               per_memory_rng=False, stop_at_eos=False, temperature=None, top_k=0, top_p=1.0):
     """-> ((T,N) i64, (T,N) f32); the reference's .squeeze() drops the N axis of the
     probabilities when N == 1 (run_batch_gen_val_MMT_v15_4.py:149)."""
     _check_sos(stoi)
     eos = _eos_id(stoi) if stop_at_eos else None
     tokens, probs, _ = _decode(model, memory, src_padding_mask, config, "multinomial", False, n_candidates, seq_index_base, n_total,
-                               per_memory_rng, eos=eos)
+                               per_memory_rng, eos=eos, temperature=temperature, top_k=top_k, top_p=top_p)
     if probs.shape[1] == 1:
         probs = probs.squeeze(1)
     return tokens, probs
 
 
 def multinomial_sequence_multi_2(model, memory, src_padding_mask, stoi, config, *, n_candidates=1, seq_index_base=0, n_total=0,
-                                 per_memory_rng=False, stop_at_eos=False):
+                                 per_memory_rng=False, stop_at_eos=False, temperature=None, top_k=0, top_p=1.0):
     """mrtf variant: probabilities lose their first row -> ((T,N), (T-1,N))."""
     tokens, probs = multinomial_sequence_multi(model, memory, src_padding_mask, stoi, config, n_candidates=n_candidates,
                                                seq_index_base=seq_index_base, n_total=n_total, per_memory_rng=per_memory_rng,
-                                               stop_at_eos=stop_at_eos)
+                                               stop_at_eos=stop_at_eos, temperature=temperature, top_k=top_k, top_p=top_p)
     return tokens, probs[1:]
 
 

@@ -109,7 +109,7 @@ class PendingTokens:
 
 
 def generate_sharded(model, data_dict, config, stoi, *, n_candidates=1, sampling="multinomial", gather_probs=False,
-                     group=None, async_gather=False, per_memory_rng=False, stop_at_eos=False):
+                     group=None, async_gather=False, per_memory_rng=False, stop_at_eos=False, temperature=None, top_k=0, top_p=1.0):
     """Encode + decode this rank's spectra and all-gather the ids.
 
     Returns (tokens (T, B*n_candidates) i64 -- identical on every rank and identical to the single-GPU run --, probs or
@@ -117,7 +117,9 @@ def generate_sharded(model, data_dict, config, stoi, *, n_candidates=1, sampling
     whatever the caller launches next (greedy early-exit trimming is then the caller's business).  ``per_memory_rng``:
     every spectrum's candidates draw in their own stream (generate.multinomial_sequence_multi), so the result also
     equals the reference's per-spectrum loop.  ``stop_at_eos``: sequences stop being computed at stoi["<EOS>"]
-    (generate.multinomial_sequence_multi); retirement is per sequence, so the result is still shard invariant."""
+    (generate.multinomial_sequence_multi); retirement is per sequence, so the result is still shard invariant.
+    ``temperature`` / ``top_k`` / ``top_p``: sampling controls, a scalar or one value per spectrum of ``data_dict``
+    (generate.multinomial_sequence_multi); each rank takes its spectra's values."""
     from . import generate as G
     from .engine import engine_for
     if per_memory_rng and sampling == "greedy":
@@ -126,7 +128,10 @@ def generate_sharded(model, data_dict, config, stoi, *, n_candidates=1, sampling
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     B = next(iter(data_dict.values())).shape[0]
+    temperature, ctl = G._controls(model, config, B, sampling, temperature, top_k, top_p)
     local, lo, hi = shard_dict(data_dict, world, rank)
+    if ctl is not None:
+        temperature, top_k, top_p = (a[lo:hi] for a in ctl)
     per = (B + world - 1) // world
     T = int(config.max_len)
     eng = engine_for(model, config)
@@ -140,7 +145,8 @@ def generate_sharded(model, data_dict, config, stoi, *, n_candidates=1, sampling
             tok, pr, _ = G._decode(model, memory, mask, config, "greedy", False, n_candidates, 0, 0, eos=eos)
         else:
             tok, pr, _ = G._decode(model, memory, mask, config, "multinomial", False, n_candidates,
-                                   lo * n_candidates, B * n_candidates, per_memory_rng, eos=eos)
+                                   lo * n_candidates, B * n_candidates, per_memory_rng, eos=eos,
+                                   temperature=temperature, top_k=top_k, top_p=top_p)
         packed = eng.pack_tokens_seqmajor(tok)                                   # (n_local, T) u8
     else:
         packed = torch.zeros(0, T, dtype=torch.uint8, device=eng.device)
