@@ -263,6 +263,44 @@ int32_t mmt_teacher_forced_scores(mmt_engine* e, const mmt_decode_args* a, const
 int32_t mmt_beam_search(mmt_engine* e, const mmt_decode_args* a, int32_t beam_size, int32_t gen_len, int32_t eos,
                         int64_t* d_seq, int32_t* d_len, double* d_score, float* d_probs, int32_t* h_steps, void* stream);
 
+/* Sampling without replacement by stochastic beam search (Kool, van Hoof & Welling, ICML 2019): per memory column b the
+ * k = a->n_cand (1..128) slots hold k DISTINCT sequences that are an exact sample without replacement from the engine's
+ * ancestral-sampling distribution at temperature tau_b (the leaves of the tree of <SOS>-prefixes: sequences ending in
+ * `eos` or holding max_len tokens), in the order of a Gumbel-top-k: slot 0 is an ancestral sample, slot 1 a sample from
+ * the rest, ...  Per step, each live slot of rank r perturbs its children's log-probabilities phi + log p_i
+ * (p = softmax(logits / tau_b) in fp32, as the multinomial sampler computes it) with -log E_i, E_i the Exp(1) variate at
+ * element r * V + i of one torch exponential_ call of k * V elements at generator offset
+ * philox_offset + ((seq_index_base / k + b) * max_len + t) * increment(k * V) (per-memory streams); children's keys
+ * are conditioned on the parent's key in double; the k largest keys of all children and carried finished slots become
+ * the new slots (ties: parent rank, then token id).  Slots without a sequence (fewer than k leaves exist) are empty.
+ * Uses a->n_cand, max_len, philox_seed / philox_offset, seq_index_base (a multiple of n_cand), N_total (0, or a multiple
+ * of n_cand: the caller advances its generator by (N_total or Bm * n_cand) / n_cand * max_len * increment(k * V)),
+ * rng_sm_count / rng_max_threads_per_sm and precision; a->sampling is ignored.  h_temperature: (Bm) host, or NULL for
+ * a->temperature everywhere; each > 0 and finite.  Slot n = column * n_cand + rank:
+ *   d_tokens   out (max_len, N) i64  ids without <SOS>, <PAD> after <EOS> and in empty slots
+ *   d_probs    out (max_len, N) f32  p of each chosen token, 0 after <EOS>
+ *   d_len      out (N) i32           generated tokens including <EOS> (0: empty slot)
+ *   d_log_prob out (N) f64           sum of log((double)p) (-inf: empty slot)
+ *   d_key      out (N) f64           Gumbel key, descending within a column (-inf: empty slot)
+ *   h_steps    out host int or NULL: steps executed (fewer than max_len once every slot has finished).
+ * Synchronises `stream` every 16 steps and between waves. */
+int32_t mmt_sample_without_replacement(mmt_engine* e, const mmt_decode_args* a, const float* h_temperature, int32_t eos,
+                                       int64_t* d_tokens, float* d_probs, int32_t* d_len, double* d_log_prob, double* d_key,
+                                       int32_t* h_steps, void* stream);
+
+/* One selection step of mmt_sample_without_replacement on given logits and state (unit-test hook): Bm columns of k
+ * slots, V tokens, step `step` of T.  In: d_logits (Bm*k, V) f32, slot state d_phi / d_key (Bm*k) f64 (-inf: empty),
+ * d_len (Bm*k) i32, d_hist (Bm*k, T) u8 token ids, d_probs (Bm*k, T) f32; h_temperature (Bm) host.  Out: the new state
+ * in the *_out buffers (positions past `step` of hist / probs copied from the input); d_p_out (Bm*k, V) f32 optional:
+ * softmax(logits / tau) of every live, unfinished slot (other rows untouched).  RNG as above with seq_index_base / k
+ * the global index of column 0. */
+int32_t mmt_sbs_select_step(mmt_engine* e, const float* d_logits, int32_t Bm, int32_t k, int32_t V, int32_t T, int32_t step, int32_t eos,
+                            const float* h_temperature, uint64_t philox_seed, uint64_t philox_offset, int64_t seq_index_base,
+                            int32_t rng_sm_count, int32_t rng_max_threads_per_sm,
+                            const double* d_phi, const double* d_key, const int32_t* d_len, const uint8_t* d_hist, const float* d_probs,
+                            double* d_phi_out, double* d_key_out, int32_t* d_len_out, uint8_t* d_hist_out, float* d_probs_out, float* d_p_out,
+                            void* stream);
+
 /* Offset increment torch applies to its Philox generator for one
  * exponential_() over `numel` elements (DistributionTemplates.h calc_execution_policy). */
 uint64_t mmt_philox_increment(int64_t numel, int32_t sm_count, int32_t max_threads_per_sm);

@@ -23,7 +23,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 EXPORTS = [
     "mmt_abi_version", "mmt_last_error", "mmt_weight_count", "mmt_weight_name", "mmt_weight_numel",
     "mmt_weight_offset", "mmt_weight_total", "mmt_create", "mmt_destroy", "mmt_memory_len",
-    "mmt_mask_is_float", "mmt_encode", "mmt_spectra_equal", "mmt_decode", "mmt_decode_memory_streams", "mmt_decode_until_eos", "mmt_decode_controlled", "mmt_teacher_forced", "mmt_teacher_forced_scores", "mmt_beam_search", "mmt_philox_increment",
+    "mmt_mask_is_float", "mmt_encode", "mmt_spectra_equal", "mmt_decode", "mmt_decode_memory_streams", "mmt_decode_until_eos", "mmt_decode_controlled", "mmt_teacher_forced", "mmt_teacher_forced_scores", "mmt_beam_search", "mmt_sample_without_replacement", "mmt_sbs_select_step", "mmt_philox_increment",
     "mmt_pack_tokens_u8", "mmt_unpack_tokens_u8", "mmt_pack_tokens_u8_seqmajor", "mmt_unpack_tokens_u8_seqmajor", "mmt_first_eos", "mmt_distinct_smiles", "mmt_ingest_peaks", "mmt_ingest_ir", "mmt_sample", "mmt_exponential", "mmt_sample_probs", "mmt_sample_memory_streams", "mmt_sample_controlled", "mmt_linear", "mmt_ffn",
     "mmt_decode_self_attention", "mmt_decode_cross_attention", "mmt_decode_layer_tail", "mmt_encoder_layer", "mmt_launch_count",
     "mmt_profile_enable", "mmt_profile_report",
@@ -167,6 +167,11 @@ def lib():
     L.mmt_teacher_forced.argtypes = [vp, C.POINTER(DecodeArgs), vp, i32, vp, vp]; L.mmt_teacher_forced.restype = i32
     L.mmt_teacher_forced_scores.argtypes = [vp, C.POINTER(DecodeArgs), vp, vp, i32, vp, vp, vp, vp]; L.mmt_teacher_forced_scores.restype = i32
     L.mmt_beam_search.argtypes = [vp, C.POINTER(DecodeArgs), i32, i32, i32, vp, vp, vp, vp, C.POINTER(C.c_int32), vp]; L.mmt_beam_search.restype = i32
+    L.mmt_sample_without_replacement.argtypes = [vp, C.POINTER(DecodeArgs), vp, i32, vp, vp, vp, vp, vp, C.POINTER(C.c_int32), vp]
+    L.mmt_sample_without_replacement.restype = i32
+    L.mmt_sbs_select_step.argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, u64, u64, i64, i32, i32,
+                                      vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.mmt_sbs_select_step.restype = i32
     L.mmt_philox_increment.argtypes = [i64, i32, i32]; L.mmt_philox_increment.restype = u64
     L.mmt_pack_tokens_u8.argtypes = [vp, i64, vp, vp]; L.mmt_pack_tokens_u8.restype = i32
     L.mmt_unpack_tokens_u8.argtypes = [vp, i64, vp, vp]; L.mmt_unpack_tokens_u8.restype = i32

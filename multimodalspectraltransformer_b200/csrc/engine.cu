@@ -8,12 +8,14 @@
 #include "kernels_attn5.cuh"
 #include "kernels_compact.cuh"
 #include "kernels_beam.cuh"
+#include "kernels_sbs.cuh"
 #include "kernels_smiles.cuh"
 #include "kernels_retire.cuh"
 
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 
 namespace mmt {
 thread_local std::string g_last_error;
@@ -1438,6 +1440,12 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
     return 0;
 }
 
+// Sequences a decode wave may hold (MMT_MAX_WAVE_SEQS, else by precision and device memory; see run_decode).
+static int64_t max_wave_sequences(const mmt_engine* e, int precision) {
+    return e->max_wave_seqs > 0 ? e->max_wave_seqs
+                                : (precision == MMT_PREC_BF16 ? (int64_t)e->sm_count * (e->total_mem >= ((size_t)128 << 30) ? 8 : 4) * 128 : 32768);
+}
+
 static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaStream_t s) {
     const mmt_model_desc& d = e->desc;
     const mmt_decode_args& a = *r.a;
@@ -1457,8 +1465,7 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     // 4 + 3 rounds instead of 2 x 3.46 -> 2 x 4.)
     // (second half of round 2: EIGHT full rounds -- 151,552 rows, 59.6 GB of pool -- where the device has the memory (>= 128 GB):
     // the whole 1024 x 128 job is then one wave and 128 x 31 kernel boundaries disappear, 951 -> 940 ms per decode.)
-    const int64_t max_wave_seqs = e->max_wave_seqs > 0 ? e->max_wave_seqs
-                                  : (a.precision == MMT_PREC_BF16 ? (int64_t)e->sm_count * (e->total_mem >= ((size_t)128 << 30) ? 8 : 4) * 128 : 32768);
+    const int64_t max_wave_seqs = max_wave_sequences(e, a.precision);
     int Bm_wave = (int)std::max<int64_t>(1, std::min<int64_t>(a.Bm, max_wave_seqs / a.n_cand));
     const int n_waves = (a.Bm + Bm_wave - 1) / Bm_wave;
     if (a.precision != MMT_PREC_FP32 && a.precision != MMT_PREC_BF16) MMT_FAIL("decode: bad precision");
@@ -1782,67 +1789,49 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     return 0;
 }
 
-// Batched beam search (reference validate_generate_MMT_v15_4.py:995-1086): the K beams of every memory column are K
-// slots of one KV-cached wave; per step one decoder step over all slots (forced-token mode, single-row token / logit
-// buffers), then beam_select + beam_copy_pages (kernels_beam.cuh).  The per-step kernel sequence is position
-// independent (step counter and page parity live on the device), so groups of steps replay as one CUDA graph.
-static int run_beam(mmt_engine* e, const mmt_decode_args& a0, int K, int T, int eos, int64_t* d_seq, int32_t* d_len,
-                    double* d_score, float* d_probs, int32_t* h_steps, cudaStream_t s) {
+// Wave loop shared by the batched beam search (run_beam) and the stochastic beam search (run_sbs): the K slots of every
+// memory column are K rows of one KV-cached wave; per step one decoder step over all slots (forced-token mode,
+// single-row token / logit buffers), then the search's `select` kernel and beam_copy_pages (kernels_beam.cuh).  The
+// per-step kernel sequence is position independent (step counter and page parity live on the device), so groups of
+// steps replay as one CUDA graph.  `select` adds the slots still open after step t to ctl[8 + t]: once a step leaves
+// none open, the remaining steps are fixed points and the wave stops at the next poll.
+struct BeamWave { int b0, Bmw; int64_t n0, Nw; };
+struct BeamLoop {
+    int K, T, Bm_wave;
+    DecBuffers* b;
+    float* logits; int64_t* cur_tok; int *copy_src, *copy_dst;
+    std::function<int(const BeamWave&, cudaStream_t)> init;     // state of the wave's slots (before the memory projection)
+    std::function<int(const BeamWave&, cudaStream_t)> select;   // one selection step (captured)
+    std::function<int(const BeamWave&, cudaStream_t)> finish;   // optional: after the wave's last step
+    // optional: every value the step graph of a wave bakes in besides the arena's addresses -> the graph is kept in
+    // the engine's graph cache and serves later calls with the same key
+    std::function<void(const BeamWave&, std::vector<uint64_t>&)> graph_key;
+};
+
+static int beam_wave_loop(mmt_engine* e, const mmt_decode_args& a, bool bf16, const BeamLoop& L, int32_t* h_steps, cudaStream_t s) {
     const mmt_model_desc& d = e->desc;
-    if (a0.Bm <= 0 || a0.S <= 0) MMT_FAIL("beam: empty batch");
-    if (K < 1 || K > BEAM_MAX || K > d.vocab) MMT_FAIL("beam: beam_size must be in [1, min(32, vocab)]");
-    if (T < 1 || T > d.max_len || T > 128) MMT_FAIL("beam: gen_len must be in [1, min(128, pe_trg rows)]");
-    if (eos < 0 || eos >= d.vocab) MMT_FAIL("beam: bad <EOS> id");
-    if ((a0.stride_s % 4) || (a0.stride_b % 4) || ((uintptr_t)a0.d_memory % 16)) MMT_FAIL("beam: memory must be 16-byte aligned with strides that are multiples of 4 floats");
-    if (a0.precision != MMT_PREC_FP32 && a0.precision != MMT_PREC_BF16) MMT_FAIL("beam: bad precision");
-    const bool bf16 = a0.precision == MMT_PREC_BF16;
-    mmt_decode_args a = a0;
-    a.n_cand = K; a.max_len = T; a.temperature = 1.f; a.sampling = MMT_SAMPLE_GREEDY; a.stop_on_all_pad = 0;
-    const int pps = (T + PAGE_TOKENS - 1) / PAGE_TOKENS;
-    const int Bm_wave = (int)std::max<int64_t>(1, std::min<int64_t>(a.Bm, 8192 / K));
-    const int n_waves = (a.Bm + Bm_wave - 1) / Bm_wave;
-    const int64_t Nw_max = (int64_t)Bm_wave * K;
-    Arena ar;
-    DecBuffers b;
-    float* logits = nullptr; int64_t* cur_tok = nullptr; int *copy_src = nullptr, *copy_dst = nullptr;
-    auto plan_all = [&]() {
-        plan_decoder(ar, d, Nw_max, Bm_wave, a.S, T, b, bf16, e->fused_decode_rows, 2);
-        logits = ar.get<float>((size_t)Nw_max * d.vocab);
-        cur_tok = ar.get<int64_t>((size_t)Nw_max);
-        copy_src = ar.get<int>((size_t)Nw_max); copy_dst = ar.get<int>((size_t)Nw_max);
-    };
-    ar.plan = true;
-    plan_all();
-    MMT_TRY(ensure_arena(e, ar.off));
-    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
-    plan_all();
+    DecBuffers& b = *L.b;
+    const int K = L.K, T = L.T;
+    const int n_waves = (a.Bm + L.Bm_wave - 1) / L.Bm_wave;
     if (bf16) MMT_TRY(tc_init(e));
     int steps_max = 0;
     for (int wv = 0; wv < n_waves; ++wv) {
-        const int b0 = wv * Bm_wave, Bmw = std::min(Bm_wave, a.Bm - b0);
-        const int64_t n0 = (int64_t)b0 * K, Nw = (int64_t)Bmw * K;
-        // the wave addresses its slots from 0: pools of a smaller last wave keep the planned (larger) layer stride
-        BeamParams bp;
-        memset(&bp, 0, sizeof(bp));
-        bp.logits = logits; bp.V = d.vocab; bp.K = K; bp.T = T; bp.eos = eos; bp.pps = pps; bp.Nw = Nw; bp.step = b.ctl;
-        bp.score = d_score + n0; bp.len = d_len + n0; bp.hist = d_seq + n0 * (T + 1); bp.probs = d_probs + n0 * T;
-        bp.cur_tok = cur_tok; bp.block_table = b.block_table; bp.copy_src = copy_src; bp.copy_dst = copy_dst; bp.unfinished = b.ctl + 8;
+        BeamWave w;
+        w.b0 = wv * L.Bm_wave; w.Bmw = std::min(L.Bm_wave, a.Bm - w.b0);
+        w.n0 = (int64_t)w.b0 * K; w.Nw = (int64_t)w.Bmw * K;
         MMT_CUDA(cudaMemsetAsync(b.ctl, 0, (8 + 256) * sizeof(int), s));
-        prof_pre(e, s);
-        beam_init<<<(unsigned)((Nw + 255) / 256), 256, 0, s>>>(bp, 3);
-        MMT_TRY(check_launch(e, "beam_init", s));
-        MMT_TRY(decode_prepare_wave(e, a, b0, Bmw, b, bf16, s));
+        MMT_TRY(L.init(w, s));
+        MMT_TRY(decode_prepare_wave(e, a, w.b0, w.Bmw, b, bf16, s));
         DecodeRun r;
-        r.a = &a; r.mode = 2; r.trg = cur_tok; r.T = T; r.tokens = nullptr; r.probs = nullptr; r.logits = logits;
+        r.a = &a; r.mode = 2; r.trg = L.cur_tok; r.T = T; r.tokens = nullptr; r.probs = nullptr; r.logits = L.logits;
         r.ldn = 0; r.serial_first = true;
+        // the wave addresses its slots from 0: pools of a smaller last wave keep the planned (larger) layer stride
         const size_t page_bytes = (size_t)2 * PAGE_TOKENS * D * b.kv_esz;
         auto one_step = [&](cudaStream_t cs) -> int {
-            MMT_TRY(decode_step(e, r, 0, Nw, Bmw, b, bf16, cs));
+            MMT_TRY(decode_step(e, r, 0, w.Nw, w.Bmw, b, bf16, cs));
+            MMT_TRY(L.select(w, cs));
             prof_pre(e, cs);
-            beam_select<<<Bmw, 256, 0, cs>>>(bp);
-            MMT_TRY(check_launch(e, "beam_select", cs));
-            prof_pre(e, cs);
-            beam_copy_pages<<<dim3((unsigned)Nw, d.n_dec_layers), 256, 0, cs>>>(b.kv_pool, (size_t)b.pool_pages * page_bytes, (int)page_bytes, copy_src, copy_dst);
+            beam_copy_pages<<<dim3((unsigned)w.Nw, d.n_dec_layers), 256, 0, cs>>>(b.kv_pool, (size_t)b.pool_pages * page_bytes, (int)page_bytes, L.copy_src, L.copy_dst);
             MMT_TRY(check_launch(e, "beam_copy_pages", cs));
             return 0;
         };
@@ -1850,7 +1839,15 @@ static int run_beam(mmt_engine* e, const mmt_decode_args& a0, int K, int T, int 
         for (int u = 2; u <= e->graph_steps; ++u) if (T % u == 0) U = u;
         cudaGraphExec_t exec = nullptr;
         int64_t launches_per_group = 0;
-        if (e->use_graph && !e->profiling) {
+        std::vector<uint64_t> key;
+        const bool cached = L.graph_key && e->use_graph && e->use_graph_cache && !e->profiling;
+        if (cached) {
+            L.graph_key(w, key);
+            for (uint64_t v : {(uint64_t)U, (uint64_t)(uintptr_t)e->arena, (uint64_t)e->arena_bytes, (uint64_t)e->fused_decode_rows,
+                               (uint64_t)e->use_pdl, (uint64_t)(uintptr_t)e->da_dbg}) key.push_back(v);
+            for (auto& c : e->graph_cache) if (c.key == key) { exec = c.exec; launches_per_group = c.launches_per_group; c.stamp = ++e->graph_cache_clock; break; }
+        }
+        if (e->use_graph && !e->profiling && !exec) {
             if (!e->cap_stream[0]) MMT_CUDA(cudaStreamCreateWithFlags(&e->cap_stream[0], cudaStreamNonBlocking));
             const int64_t l0 = e->launches;
             MMT_CUDA(cudaStreamBeginCapture(e->cap_stream[0], cudaStreamCaptureModeRelaxed));
@@ -1865,11 +1862,19 @@ static int run_beam(mmt_engine* e, const mmt_decode_args& a0, int K, int T, int 
             ce = cudaGraphInstantiate(&exec, graph, 0);
             cudaGraphDestroy(graph);
             if (ce != cudaSuccess) MMT_FAIL(std::string("cudaGraphInstantiate failed: ") + cudaGetErrorString(ce));
-        } else {
+            if (cached) {
+                if (e->graph_cache.size() >= 4) {      // evict the least recently used entry
+                    size_t lru = 0;
+                    for (size_t i = 1; i < e->graph_cache.size(); ++i) if (e->graph_cache[i].stamp < e->graph_cache[lru].stamp) lru = i;
+                    cudaGraphExecDestroy(e->graph_cache[lru].exec);
+                    e->graph_cache.erase(e->graph_cache.begin() + lru);
+                }
+                e->graph_cache.push_back({key, exec, launches_per_group, ++e->graph_cache_clock});
+            }
+        } else if (!exec) {
             U = 1;
         }
-        struct ExecGuard { cudaGraphExec_t x; ~ExecGuard() { if (x) cudaGraphExecDestroy(x); } } guard{exec};
-        // every beam of every item finished -> the remaining steps are fixed points of the reference's loop
+        struct ExecGuard { cudaGraphExec_t x; ~ExecGuard() { if (x) cudaGraphExecDestroy(x); } } guard{cached ? nullptr : exec};
         const int poll_every = U >= 16 ? U : (16 / U) * U;
         int steps_done = T;
         for (int t = 0; t < T; t += U) {
@@ -1884,11 +1889,142 @@ static int run_beam(mmt_engine* e, const mmt_decode_args& a0, int K, int T, int 
                 if (stop) break;
             }
         }
+        if (L.finish) MMT_TRY(L.finish(w, s));
         steps_max = std::max(steps_max, steps_done);
         if (n_waves > 1) MMT_CUDA(cudaStreamSynchronize(s));   // the next wave reuses the pools
     }
     if (h_steps) *h_steps = steps_max;
     return 0;
+}
+
+// Batched beam search (reference validate_generate_MMT_v15_4.py:995-1086) on beam_wave_loop: beam_init + beam_select.
+static int run_beam(mmt_engine* e, const mmt_decode_args& a0, int K, int T, int eos, int64_t* d_seq, int32_t* d_len,
+                    double* d_score, float* d_probs, int32_t* h_steps, cudaStream_t s) {
+    const mmt_model_desc& d = e->desc;
+    if (a0.Bm <= 0 || a0.S <= 0) MMT_FAIL("beam: empty batch");
+    if (K < 1 || K > BEAM_MAX || K > d.vocab) MMT_FAIL("beam: beam_size must be in [1, min(32, vocab)]");
+    if (T < 1 || T > d.max_len || T > 128) MMT_FAIL("beam: gen_len must be in [1, min(128, pe_trg rows)]");
+    if (eos < 0 || eos >= d.vocab) MMT_FAIL("beam: bad <EOS> id");
+    if ((a0.stride_s % 4) || (a0.stride_b % 4) || ((uintptr_t)a0.d_memory % 16)) MMT_FAIL("beam: memory must be 16-byte aligned with strides that are multiples of 4 floats");
+    if (a0.precision != MMT_PREC_FP32 && a0.precision != MMT_PREC_BF16) MMT_FAIL("beam: bad precision");
+    const bool bf16 = a0.precision == MMT_PREC_BF16;
+    mmt_decode_args a = a0;
+    a.n_cand = K; a.max_len = T; a.temperature = 1.f; a.sampling = MMT_SAMPLE_GREEDY; a.stop_on_all_pad = 0;
+    const int pps = (T + PAGE_TOKENS - 1) / PAGE_TOKENS;
+    BeamLoop L;
+    L.K = K; L.T = T;
+    L.Bm_wave = (int)std::max<int64_t>(1, std::min<int64_t>(a.Bm, 8192 / K));
+    const int64_t Nw_max = (int64_t)L.Bm_wave * K;
+    Arena ar;
+    DecBuffers b;
+    L.b = &b;
+    auto plan_all = [&]() {
+        plan_decoder(ar, d, Nw_max, L.Bm_wave, a.S, T, b, bf16, e->fused_decode_rows, 2);
+        L.logits = ar.get<float>((size_t)Nw_max * d.vocab);
+        L.cur_tok = ar.get<int64_t>((size_t)Nw_max);
+        L.copy_src = ar.get<int>((size_t)Nw_max); L.copy_dst = ar.get<int>((size_t)Nw_max);
+    };
+    ar.plan = true;
+    plan_all();
+    MMT_TRY(ensure_arena(e, ar.off));
+    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
+    plan_all();
+    auto params = [&](const BeamWave& w) {
+        BeamParams bp;
+        memset(&bp, 0, sizeof(bp));
+        bp.logits = L.logits; bp.V = d.vocab; bp.K = K; bp.T = T; bp.eos = eos; bp.pps = pps; bp.Nw = w.Nw; bp.step = b.ctl;
+        bp.score = d_score + w.n0; bp.len = d_len + w.n0; bp.hist = d_seq + w.n0 * (T + 1); bp.probs = d_probs + w.n0 * T;
+        bp.cur_tok = L.cur_tok; bp.block_table = b.block_table; bp.copy_src = L.copy_src; bp.copy_dst = L.copy_dst; bp.unfinished = b.ctl + 8;
+        return bp;
+    };
+    L.init = [&](const BeamWave& w, cudaStream_t cs) -> int {
+        prof_pre(e, cs);
+        beam_init<<<(unsigned)((w.Nw + 255) / 256), 256, 0, cs>>>(params(w), 3);
+        return check_launch(e, "beam_init", cs);
+    };
+    L.select = [&](const BeamWave& w, cudaStream_t cs) -> int {
+        prof_pre(e, cs);
+        beam_select<<<w.Bmw, 256, 0, cs>>>(params(w));
+        return check_launch(e, "beam_select", cs);
+    };
+    return beam_wave_loop(e, a, bf16, L, h_steps, s);
+}
+
+// Stochastic beam search (kernels_sbs.cuh) on beam_wave_loop.  Waves: two page parities, so at most half the decode
+// wave of the precision (max_wave_sequences / 2 slots), in whole columns.  Slot state lives in the arena (both
+// parities) and the column temperatures are copied there before the first step, so a wave's step graph -- kept in the
+// graph cache -- serves later calls with other temperatures, generator states and outputs; sbs_finish writes the
+// caller's tensors after the wave's last step.
+static int run_sbs(mmt_engine* e, const mmt_decode_args& a0, const float* h_temp, int eos, int64_t* d_tokens, float* d_probs,
+                   int32_t* d_len, double* d_log_prob, double* d_key, int32_t* h_steps, cudaStream_t s) {
+    const mmt_model_desc& d = e->desc;
+    const int K = a0.n_cand, T = a0.max_len, V = d.vocab;
+    const bool bf16 = a0.precision == MMT_PREC_BF16;
+    mmt_decode_args a = a0;
+    a.temperature = 1.f; a.sampling = MMT_SAMPLE_GREEDY; a.stop_on_all_pad = 0; a.seq_index_base = 0; a.N_total = 0;
+    const int pps = (T + PAGE_TOKENS - 1) / PAGE_TOKENS;
+    BeamLoop L;
+    L.K = K; L.T = T;
+    L.Bm_wave = (int)std::max<int64_t>(1, std::min<int64_t>(a.Bm, max_wave_sequences(e, a.precision) / 2 / K));
+    const int64_t Nw_max = (int64_t)L.Bm_wave * K;
+    Arena ar;
+    DecBuffers b;
+    L.b = &b;
+    double *phi[2], *key[2]; int* len[2]; uint8_t* hist[2]; float* probs[2]; float* temp = nullptr;
+    auto plan_all = [&]() {
+        plan_decoder(ar, d, Nw_max, L.Bm_wave, a.S, T, b, bf16, e->fused_decode_rows, 2);
+        L.logits = ar.get<float>((size_t)Nw_max * V);
+        L.cur_tok = ar.get<int64_t>((size_t)Nw_max);
+        L.copy_src = ar.get<int>((size_t)Nw_max); L.copy_dst = ar.get<int>((size_t)Nw_max);
+        for (int i = 0; i < 2; ++i) {
+            phi[i] = ar.get<double>((size_t)Nw_max); key[i] = ar.get<double>((size_t)Nw_max); len[i] = ar.get<int>((size_t)Nw_max);
+            hist[i] = ar.get<uint8_t>((size_t)Nw_max * T); probs[i] = ar.get<float>((size_t)Nw_max * T);
+        }
+        temp = ar.get<float>((size_t)a.Bm);
+    };
+    ar.plan = true;
+    plan_all();
+    MMT_TRY(ensure_arena(e, ar.off));
+    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
+    plan_all();
+    MMT_CUDA(cudaFuncSetAttribute(sbs_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbs_smem_bytes(SBS_MAX, VOCAB_MAX)));
+    MMT_CUDA(cudaMemcpyAsync(temp, h_temp, (size_t)a.Bm * sizeof(float), cudaMemcpyHostToDevice, s));
+    const int smc = a.rng_sm_count > 0 ? a.rng_sm_count : e->sm_count;
+    const int mts = a.rng_max_threads_per_sm > 0 ? a.rng_max_threads_per_sm : e->max_threads_per_sm;
+    auto params = [&](const BeamWave& w) {
+        SbsParams sp;
+        memset(&sp, 0, sizeof(sp));
+        sp.logits = L.logits; sp.V = V; sp.K = K; sp.T = T; sp.eos = eos; sp.pps = pps; sp.Nw = w.Nw; sp.step = b.ctl;
+        sp.temp = temp + w.b0;
+        sp.rng.numel = (int64_t)K * V; sp.rng.threads = torch_rng_threads(sp.rng.numel, smc, mts);
+        sp.rng_inc = torch_rng_increment(sp.rng.numel, smc, mts);
+        sp.rng_dev = b.rng_state;
+        sp.col_base = a0.seq_index_base / K + w.b0;
+        for (int i = 0; i < 2; ++i) { sp.phi[i] = phi[i]; sp.key[i] = key[i]; sp.len[i] = len[i]; sp.hist[i] = hist[i]; sp.probs[i] = probs[i]; }
+        sp.cur_tok = L.cur_tok; sp.block_table = b.block_table; sp.copy_src = L.copy_src; sp.copy_dst = L.copy_dst; sp.unfinished = b.ctl + 8;
+        return sp;
+    };
+    L.init = [&](const BeamWave& w, cudaStream_t cs) -> int {
+        set_u64x2<<<1, 1, 0, cs>>>(b.rng_state, a0.philox_seed, a0.philox_offset);
+        prof_pre(e, cs);
+        sbs_init<<<(unsigned)((w.Nw + 255) / 256), 256, 0, cs>>>(params(w), 3);
+        return check_launch(e, "sbs_init", cs);
+    };
+    L.select = [&](const BeamWave& w, cudaStream_t cs) -> int {
+        prof_pre(e, cs);
+        sbs_select<<<w.Bmw, SBS_THREADS, sbs_smem_bytes(K, V), cs>>>(params(w));
+        return check_launch(e, "sbs_select", cs);
+    };
+    L.finish = [&](const BeamWave& w, cudaStream_t cs) -> int {
+        prof_pre(e, cs);
+        sbs_finish<<<(unsigned)((w.Nw * T + 255) / 256), 256, 0, cs>>>(params(w), w.n0, (int64_t)a.Bm * K, d_tokens, d_probs, d_len, d_log_prob, d_key);
+        return check_launch(e, "sbs_finish", cs);
+    };
+    L.graph_key = [&](const BeamWave& w, std::vector<uint64_t>& k) {
+        for (uint64_t v : {(uint64_t)0x5B5, (uint64_t)K, (uint64_t)T, (uint64_t)eos, (uint64_t)a.S, (uint64_t)w.Bmw, (uint64_t)a.precision,
+                           (uint64_t)(a0.seq_index_base / K + w.b0), (uint64_t)smc, (uint64_t)mts, (uint64_t)w.b0}) k.push_back(v);
+    };
+    return beam_wave_loop(e, a, bf16, L, h_steps, s);
 }
 
 }  // namespace mmt
@@ -2157,6 +2293,94 @@ int32_t mmt_beam_search(mmt_engine* e, const mmt_decode_args* a, int32_t beam_si
     if (!e || !a || !d_seq || !d_len || !d_score || !d_probs) MMT_FAIL("null argument");
     EngineCall call(e, (cudaStream_t)stream);
     return run_beam(e, *a, beam_size, gen_len, eos, d_seq, d_len, d_score, d_probs, h_steps, (cudaStream_t)stream);
+}
+
+// Column temperatures of a stochastic beam search: h_temperature (Bm) or a->temperature for every column, checked.
+static int sbs_temperatures(const float* h_temperature, int64_t Bm, float t_default, std::vector<float>& temp, const char* who) {
+    temp.assign(Bm, t_default);
+    for (int64_t b = 0; b < Bm; ++b) {
+        if (h_temperature) temp[b] = h_temperature[b];
+        if (!(temp[b] > 0.f) || !std::isfinite(temp[b])) MMT_FAIL(std::string(who) + ": temperature must be > 0 and finite (column " + std::to_string(b) + ")");
+    }
+    return 0;
+}
+
+int32_t mmt_sample_without_replacement(mmt_engine* e, const mmt_decode_args* a, const float* h_temperature, int32_t eos,
+                                       int64_t* d_tokens, float* d_probs, int32_t* d_len, double* d_log_prob, double* d_key,
+                                       int32_t* h_steps, void* stream) {
+    const char* who = "mmt_sample_without_replacement";
+    if (!e || !a) MMT_FAIL("null engine / args");
+    if (!d_tokens || !d_probs || !d_len || !d_log_prob || !d_key) MMT_FAIL(std::string(who) + ": every output is required");
+    if (a->Bm <= 0 || a->S <= 0) MMT_FAIL(std::string(who) + ": empty batch");
+    const int64_t K = a->n_cand;
+    if (K < 1 || K > SBS_MAX) MMT_FAIL(std::string(who) + ": n_cand must be in [1, 128]");
+    if (a->max_len < 1 || a->max_len > e->desc.max_len || a->max_len > 128) MMT_FAIL(std::string(who) + ": max_len must be in [1, min(128, pe_trg rows)]");
+    if (eos < 0 || eos >= e->desc.vocab) MMT_FAIL(std::string(who) + ": eos must be in [0, vocab)");
+    if (a->seq_index_base < 0 || a->seq_index_base % K) MMT_FAIL(std::string(who) + ": seq_index_base must be a non-negative multiple of n_cand");
+    if (a->N_total < 0 || (a->N_total > 0 && (a->N_total % K || a->N_total < a->seq_index_base + a->Bm * K)))
+        MMT_FAIL(std::string(who) + ": N_total must be 0 or a multiple of n_cand covering seq_index_base + Bm * n_cand");
+    if ((a->stride_s % 4) || (a->stride_b % 4) || ((uintptr_t)a->d_memory % 16)) MMT_FAIL(std::string(who) + ": memory must be 16-byte aligned with strides that are multiples of 4 floats");
+    if (a->precision != MMT_PREC_FP32 && a->precision != MMT_PREC_BF16) MMT_FAIL(std::string(who) + ": bad precision");
+    std::vector<float> temp;
+    MMT_TRY(sbs_temperatures(h_temperature, a->Bm, a->temperature, temp, who));
+    EngineCall call(e, (cudaStream_t)stream);
+    return run_sbs(e, *a, temp.data(), eos, d_tokens, d_probs, d_len, d_log_prob, d_key, h_steps, (cudaStream_t)stream);
+}
+
+int32_t mmt_sbs_select_step(mmt_engine* e, const float* d_logits, int32_t Bm, int32_t k, int32_t V, int32_t T, int32_t step, int32_t eos,
+                            const float* h_temperature, uint64_t philox_seed, uint64_t philox_offset, int64_t seq_index_base,
+                            int32_t rng_sm_count, int32_t rng_max_threads_per_sm,
+                            const double* d_phi, const double* d_key, const int32_t* d_len, const uint8_t* d_hist, const float* d_probs,
+                            double* d_phi_out, double* d_key_out, int32_t* d_len_out, uint8_t* d_hist_out, float* d_probs_out, float* d_p_out, void* stream) {
+    const char* who = "mmt_sbs_select_step";
+    if (!e || !d_logits || !d_phi || !d_key || !d_len || !d_hist || !d_probs || !d_phi_out || !d_key_out || !d_len_out || !d_hist_out || !d_probs_out || !h_temperature)
+        MMT_FAIL("null argument");
+    if (Bm < 1) MMT_FAIL(std::string(who) + ": empty batch");
+    if (k < 1 || k > SBS_MAX) MMT_FAIL(std::string(who) + ": k must be in [1, 128]");
+    if (V < 1 || V > VOCAB_MAX) MMT_FAIL(std::string(who) + ": V must be in [1, 64]");
+    if (T < 1 || T > 128 || step < 0 || step >= T) MMT_FAIL(std::string(who) + ": need 1 <= T <= 128 and 0 <= step < T");
+    if (eos < 0 || eos >= V) MMT_FAIL(std::string(who) + ": eos must be in [0, V)");
+    if (seq_index_base < 0 || seq_index_base % k) MMT_FAIL(std::string(who) + ": seq_index_base must be a non-negative multiple of k");
+    std::vector<float> temp;
+    MMT_TRY(sbs_temperatures(h_temperature, Bm, 1.f, temp, who));
+    EngineCall call(e, (cudaStream_t)stream);
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t N = (int64_t)Bm * k;
+    const int pps = (T + PAGE_TOKENS - 1) / PAGE_TOKENS;
+    Arena ar;
+    int* ctl = nullptr; float* d_temp = nullptr; int64_t* cur_tok = nullptr; int *bt = nullptr, *cs = nullptr, *cd = nullptr;
+    auto plan_all = [&]() {
+        ctl = ar.get<int>(1); d_temp = ar.get<float>(Bm); cur_tok = ar.get<int64_t>(N);
+        bt = ar.get<int>(N * pps); cs = ar.get<int>(N); cd = ar.get<int>(N);
+    };
+    ar.plan = true;
+    plan_all();
+    MMT_TRY(ensure_arena(e, ar.off));
+    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
+    plan_all();
+    const int t1 = step + 1;      // the step counter as the sampler leaves it
+    MMT_CUDA(cudaMemcpyAsync(ctl, &t1, sizeof(int), cudaMemcpyHostToDevice, s));
+    MMT_CUDA(cudaMemcpyAsync(d_temp, temp.data(), (size_t)Bm * sizeof(float), cudaMemcpyHostToDevice, s));
+    MMT_CUDA(cudaMemsetAsync(bt, 0, (size_t)N * pps * sizeof(int), s));
+    MMT_CUDA(cudaMemcpyAsync(d_hist_out, d_hist, (size_t)N * T, cudaMemcpyDeviceToDevice, s));
+    MMT_CUDA(cudaMemcpyAsync(d_probs_out, d_probs, (size_t)N * T * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    SbsParams sp;
+    memset(&sp, 0, sizeof(sp));
+    sp.logits = d_logits; sp.V = V; sp.K = k; sp.T = T; sp.eos = eos; sp.pps = pps; sp.Nw = N; sp.step = ctl; sp.temp = d_temp;
+    const int smc = rng_sm_count > 0 ? rng_sm_count : e->sm_count;
+    const int mts = rng_max_threads_per_sm > 0 ? rng_max_threads_per_sm : e->max_threads_per_sm;
+    sp.rng.seed = philox_seed; sp.rng.offset = philox_offset; sp.rng.numel = (int64_t)k * V;
+    sp.rng.threads = torch_rng_threads(sp.rng.numel, smc, mts); sp.rng_inc = torch_rng_increment(sp.rng.numel, smc, mts);
+    sp.col_base = seq_index_base / k;
+    const int rd = step & 1, wr = rd ^ 1;
+    sp.phi[rd] = const_cast<double*>(d_phi); sp.key[rd] = const_cast<double*>(d_key); sp.len[rd] = const_cast<int*>(d_len);
+    sp.hist[rd] = const_cast<uint8_t*>(d_hist); sp.probs[rd] = const_cast<float*>(d_probs);
+    sp.phi[wr] = d_phi_out; sp.key[wr] = d_key_out; sp.len[wr] = d_len_out; sp.hist[wr] = d_hist_out; sp.probs[wr] = d_probs_out;
+    sp.cur_tok = cur_tok; sp.block_table = bt; sp.copy_src = cs; sp.copy_dst = cd; sp.p_out = d_p_out;
+    MMT_CUDA(cudaFuncSetAttribute(sbs_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbs_smem_bytes(SBS_MAX, VOCAB_MAX)));
+    prof_pre(e, s);
+    sbs_select<<<Bm, SBS_THREADS, sbs_smem_bytes(k, V), s>>>(sp);
+    return check_launch(e, "sbs_select", s);
 }
 
 int32_t mmt_spectra_equal(mmt_engine* e, const mmt_spectra* a, const mmt_spectra* b, int32_t B, uint32_t mode_bits, int32_t* h_equal, void* stream) {

@@ -408,7 +408,53 @@ class Engine:
             t.record_stream(torch.cuda.current_stream(self.dev_index))
         return seq, ln, score, probs, int(steps.value)
 
+    def sample_without_replacement(self, memory, key_bias, *, n_cand, max_len, temperature=1.0, eos=2, seed=0, offset=0,
+                                   seq_index_base=0, n_total=0, precision="fp32"):
+        """Stochastic beam search (``mmt_sample_without_replacement``): ``n_cand`` distinct sequences per memory column,
+        an exact sample without replacement from the decoder's sampling distribution at ``temperature`` (a scalar or one
+        per memory column), slot 0 first.  The generator state (seed, offset) is read, not advanced.
+        -> (tokens (T,N) i64, probs (T,N) f32, lengths (N,) i32, log_prob (N,) f64, key (N,) f64, steps)."""
+        temp = control_arrays(memory.shape[1], self.vocab, temperature)[0]
+        a, keep = self._decode_args(memory, key_bias, n_cand, max_len, float(temp[0]), _lib.SAMPLE_MULTINOMIAL, False,
+                                    precision, seed, offset, seq_index_base, n_total)
+        N = a.Bm * n_cand
+        tokens = torch.empty(max_len, N, device=self.device, dtype=torch.int64)
+        probs = torch.empty(max_len, N, device=self.device, dtype=torch.float32)
+        lengths = torch.empty(N, device=self.device, dtype=torch.int32)
+        log_prob = torch.empty(N, device=self.device, dtype=torch.float64)
+        key = torch.empty(N, device=self.device, dtype=torch.float64)
+        steps = C.c_int32(max_len)
+        _lib.check(self.L.mmt_sample_without_replacement(self.h, C.byref(a), temp.ctypes.data, int(eos), tokens.data_ptr(),
+                                                         probs.data_ptr(), lengths.data_ptr(), log_prob.data_ptr(),
+                                                         key.data_ptr(), C.byref(steps), self._stream()))
+        for t in keep:
+            t.record_stream(torch.cuda.current_stream(self.dev_index))
+        return tokens, probs, lengths, log_prob, key, int(steps.value)
+
     # ------------------------------------------------------------ unit hooks
+    def sbs_select_step(self, logits, phi, key, lengths, hist, probs, *, k, step, eos, temperature, seed, offset,
+                        seq_index_base=0):
+        """One selection step of ``sample_without_replacement`` on given logits (Bm*k, V) and slot state: phi / key
+        (Bm*k,) f64 (-inf: empty slot), lengths (Bm*k,) i32, hist (Bm*k, T) u8 ids, probs (Bm*k, T) f32
+        (``mmt_sbs_select_step``, test hook).  -> the new (phi, key, lengths, hist, probs) and p (Bm*k, V) f32, the
+        softmax the step computed for every live, unfinished slot (0 in other rows)."""
+        dev = self.device
+        lg = logits.to(dev, torch.float32).contiguous()
+        N, V = lg.shape
+        st = [phi.to(dev, torch.float64).contiguous(), key.to(dev, torch.float64).contiguous(),
+              lengths.to(dev, torch.int32).contiguous(), hist.to(dev, torch.uint8).contiguous(),
+              probs.to(dev, torch.float32).contiguous()]
+        T = st[3].shape[1]
+        temp = control_arrays(N // k, V, temperature)[0]
+        out = [torch.empty_like(t) for t in st]
+        p = torch.zeros(N, V, device=dev, dtype=torch.float32)
+        _lib.check(self.L.mmt_sbs_select_step(self.h, lg.data_ptr(), N // k, k, V, T, step, eos, temp.ctypes.data, seed, offset,
+                                              seq_index_base, 0, 0, *[t.data_ptr() for t in st], *[t.data_ptr() for t in out],
+                                              p.data_ptr(), self._stream()))
+        for t in st + [lg]:
+            t.record_stream(torch.cuda.current_stream(self.dev_index))
+        return tuple(out) + (p,)
+
     def sample(self, x, temperature=1.0, sampling="greedy", seed=0, offset=0, seq_index_base=0, n_total=0,
                want_logits=False):
         x = x.to(self.device, torch.float32).contiguous()

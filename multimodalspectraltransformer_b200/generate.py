@@ -9,6 +9,7 @@ running on the B200 engine.
     greedy_sequence_2            mmt_result_test_functions_15_4.py:984-1032
     multinomial_sequence_multi_2 mmt_result_test_functions_15_4.py:791-829
     beam_search                  validate_generate_MMT_v15_4.py:995-1086
+    sample_without_replacement   (extension) k distinct candidates per spectrum by stochastic beam search
     predict_prop_correct_max_sequence(_2)   validate_generate_MMT_v15_4.py:309-509
     predict_prop_correct_max_sequence_3     mmt_result_test_functions_15_4.py:340-400
 
@@ -268,6 +269,46 @@ def beam_search(model, stoi, memory, src_padding_mask, config, beam_size):
                                                precision=_engine.default_precision(config))
     seq, ln, score, probs = seq.cpu().tolist(), ln.cpu().tolist(), score.cpu().tolist(), probs.cpu().tolist()
     return [[(score[i][k], seq[i][k][:ln[i][k]], probs[i][k][:ln[i][k] - 1]) for k in range(len(seq[i]))] for i in range(N)]
+
+
+def sample_without_replacement(model, stoi, memory, src_padding_mask, config, *, n_candidates, temperature=None,
+                               seq_index_base=0, n_total=0):
+    """``n_candidates`` DISTINCT sequences per spectrum in one call: stochastic beam search (Kool, van Hoof & Welling,
+    ICML 2019) on the KV-cached decoder, an exact sample without replacement from the sequences ``multinomial_sequence``
+    draws (cut at <EOS>) at ``temperature`` (a scalar or one per spectrum; None: config.temperature at call time), for
+    ``config.max_len`` steps.  Candidate n = spectrum * n_candidates + slot; within a spectrum the slots are ordered by
+    their Gumbel key, so slot 0 is an ordinary sample and slot j a sample from what slots 0..j-1 left.
+    -> (tokens (T,N) i64 without <SOS>, <PAD> after <EOS>; probs (T,N) f32 of each chosen token, 0 after <EOS>;
+        log_prob (N,) f64 = sum of log(probs); key (N,) f64, descending per spectrum).  Fewer than n_candidates
+    possible sequences (tiny max_len): the remaining slots are empty (<PAD> only, log_prob = key = -inf).
+    The noise follows torch's CUDA generator in per-memory streams (``per_memory_rng``): seq_index_base (a multiple of
+    n_candidates) / n_total place the call inside a larger logical batch; the generator advances by
+    (n_total or N) / n_candidates * max_len exponential_ calls of n_candidates x vocab elements."""
+    _check_sos(stoi)
+    if "<EOS>" not in stoi:
+        raise ValueError("sample_without_replacement needs an <EOS> entry in stoi")
+    eos = int(stoi["<EOS>"])
+    if isinstance(n_candidates, bool) or not isinstance(n_candidates, int) or not 1 <= n_candidates <= 128:
+        raise ValueError(f"n_candidates must be an integer in [1, 128], got {n_candidates!r}")
+    k = n_candidates
+    Bm = memory.size(1)
+    if not isinstance(seq_index_base, int) or seq_index_base < 0 or seq_index_base % k:
+        raise ValueError("seq_index_base must be a non-negative multiple of n_candidates")
+    if n_total and (n_total % k or n_total < seq_index_base + Bm * k):
+        raise ValueError("n_total must be a multiple of n_candidates covering seq_index_base + the call's sequences")
+    if temperature is None:
+        temperature = float(config.temperature)
+    temperature = _engine.control_arrays(Bm, _vocab(model, config), temperature)[0]
+    max_len = int(config.max_len)
+    model.eval()
+    eng = _engine.engine_for(model, config)
+    bias = _mask_to_bias(src_padding_mask.to(eng.device))
+    gen, seed, offset = _philox_state(eng.dev_index)
+    tokens, probs, _, log_prob, key, _ = eng.sample_without_replacement(
+        memory, bias, n_cand=k, max_len=max_len, temperature=temperature, eos=eos, seed=seed, offset=offset,
+        seq_index_base=seq_index_base, n_total=n_total, precision=_engine.default_precision(config))
+    gen.set_offset(offset + _philox_advance(eng, k, n_total if n_total else Bm * k, max_len, True))
+    return tokens, probs, log_prob, key
 
 
 # ------------------------------------------------------------- teacher-forced scorers
