@@ -122,6 +122,30 @@ static int ensure_arena(mmt_engine* e, size_t bytes) {
     return 0;
 }
 
+// A call's workspace in the arena: `plan` lays out its buffers with ar.get, once to measure them, and -- after the arena
+// has grown to fit -- once more to place them.
+template <typename F>
+static int plan_arena(mmt_engine* e, Arena& ar, F&& plan) {
+    ar = Arena();
+    plan();
+    MMT_TRY(ensure_arena(e, ar.off));
+    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
+    plan();
+    return 0;
+}
+
+// torch's Philox launch geometry for a draw of `numel` elements, on the call's device description (sm_count /
+// max_threads_per_sm > 0) or the engine's device; *inc = the generator advance of one such draw
+static RngGeom rng_geom(const mmt_engine* e, uint64_t seed, uint64_t offset, int64_t numel, int sm_count, int max_threads_per_sm,
+                        uint64_t* inc) {
+    const int smc = sm_count > 0 ? sm_count : e->sm_count;
+    const int mts = max_threads_per_sm > 0 ? max_threads_per_sm : e->max_threads_per_sm;
+    RngGeom g;
+    g.seed = seed; g.offset = offset; g.numel = numel; g.threads = torch_rng_threads(numel, smc, mts);
+    *inc = torch_rng_increment(numel, smc, mts);
+    return g;
+}
+
 // ---------------------------------------------------------------------------
 // launch helpers
 // ---------------------------------------------------------------------------
@@ -218,17 +242,27 @@ static TcGemmParams tc_params(int M, int N, int K) {
     return p;
 }
 
-// A [M,K] bf16 (row pitch lda), W [N,K] bf16 (dense), optional low-order weight term Wlo; the
-// rest of `p` is filled by the caller
-// sample_tokens keeps fc_out in dynamic shared memory (33 KB at the 64-row maximum, next to 20 KB of static row buffers)
-static int sample_init(mmt_engine* e) {
-    if (e->sample_ready) return 0;
-    MMT_CUDA(cudaFuncSetAttribute(sample_tokens<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem_bytes(VOCAB_MAX)));
-    MMT_CUDA(cudaFuncSetAttribute(sample_tokens<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem_bytes(VOCAB_MAX)));
-    e->sample_ready = true;
-    return 0;
+// sample_tokens over sp.N rows (sample_tokens<true> with per-column controls).  `plan_rows` fixes the variant: a decode
+// wave's starting size (a compacted wave keeps it), else N.
+static int launch_sample(mmt_engine* e, SampleParams& sp, int64_t plan_rows, bool controlled, bool pdl, cudaStream_t s) {
+    if (!e->sample_ready) {   // fc_out sits in dynamic shared memory (33 KB at the 64-row maximum, next to 20 KB of static row buffers)
+        MMT_CUDA(cudaFuncSetAttribute(sample_tokens<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem_bytes(VOCAB_MAX)));
+        MMT_CUDA(cudaFuncSetAttribute(sample_tokens<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem_bytes(VOCAB_MAX)));
+        e->sample_ready = true;
+    }
+    // rows per CTA and pass: 2 when the input is still spread over FFN2 partials, else 8 warps' rows; at most four resident
+    // waves of CTAs.  Small waves take one row per warp (latency), large ones four (shared-memory traffic).
+    sp.rows_per_warp = plan_rows >= 8192 ? SAMPLE_NR : 1;
+    const int rpc = sp.part ? 2 : 8 * sp.rows_per_warp;
+    const int64_t groups = (sp.N + rpc - 1) / rpc;
+    prof_pre(e, s);
+    launch_kernel(controlled ? sample_tokens<true> : sample_tokens<false>, dim3((unsigned)std::min<int64_t>(groups, (int64_t)e->sm_count * 4)),
+                  dim3(256), sample_smem_bytes(sp.V), s, pdl, sp);
+    return check_launch(e, controlled ? "sample_tokens_controlled" : "sample_tokens", s);
 }
 
+// A [M,K] bf16 (row pitch lda), W [N,K] bf16 (dense), optional low-order weight term Wlo; the
+// rest of `p` is filled by the caller
 struct TcChain { const __nv_bfloat16 *W, *Wlo; const float* bias; float* out; int64_t ld; };
 static int launch_tc(mmt_engine* e, TcGemmParams& p, const __nv_bfloat16* A, int64_t lda, const __nv_bfloat16* W, int epi, cudaStream_t s,
                      const __nv_bfloat16* Wlo = nullptr, bool pdl = false, const TcChain* chain = nullptr) {
@@ -601,9 +635,7 @@ static int encode_chunk_compact(mmt_engine* e, const mmt_spectra& in, int b0, in
             Xc16 = ATT16 = nullptr;
         }
     };
-    a.plan = true; plan();
-    MMT_TRY(ensure_arena(e, a.off));
-    a.plan = false; a.base = e->arena; a.cap = e->arena_bytes; a.off = 0; plan();
+    MMT_TRY(plan_arena(e, a, plan));
     float* key_bias = d_key_bias ? d_key_bias + (int64_t)b0 * L.S_total : key_bias_l;
     uint8_t* pad_mask = d_pad_mask ? d_pad_mask + (int64_t)b0 * L.S_total : pad_mask_l;
 
@@ -785,11 +817,7 @@ static int encode_chunk(mmt_engine* e, const mmt_spectra& in, int b0, int Bc, in
     const int P = d.pad_points;
     Arena a;
     EncBuffers b;
-    a.plan = true;
-    plan_encoder(a, L, Bc, d.d_ff, b, d_key_bias == nullptr, d_pad_mask == nullptr, bf16);
-    MMT_TRY(ensure_arena(e, a.off));
-    a.plan = false; a.base = e->arena; a.cap = e->arena_bytes; a.off = 0;
-    plan_encoder(a, L, Bc, d.d_ff, b, d_key_bias == nullptr, d_pad_mask == nullptr, bf16);
+    MMT_TRY(plan_arena(e, a, [&]() { plan_encoder(a, L, Bc, d.d_ff, b, d_key_bias == nullptr, d_pad_mask == nullptr, bf16); }));
     float* key_bias = d_key_bias ? d_key_bias + (int64_t)b0 * L.S_total : b.key_bias;
     uint8_t* pad_mask = d_pad_mask ? d_pad_mask + (int64_t)b0 * L.S_total : b.pad_mask;
 
@@ -1286,6 +1314,9 @@ static int decode_cross_tail_layer(const DecOps& o, const LayerW& w, int l, bool
     return 0;
 }
 
+// A wave (or lane) planned for `rows` sequences takes the fused row-local step (MMT_FUSED_DECODE_ROWS)
+static bool fused_wave(const mmt_engine* e, int64_t rows) { return e->fused_decode_rows > 0 && rows <= e->fused_decode_rows; }
+
 static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw, int Bmw, DecBuffers& b, bool bf16, cudaStream_t s) {
     const mmt_model_desc& d = e->desc;
     const mmt_decode_args& a = *r.a;
@@ -1303,7 +1334,7 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
     // (kernels_decode.cuh); the previous layer's FFN2 split-K partials + norm3 are folded into the
     // next kernel's prologue (the sampler's for the last layer).
     const int64_t P = b.plan_rows > 0 ? b.plan_rows : Nw;     // a compacted wave keeps the variants of its starting size
-    const bool fused = e->fused_decode_rows > 0 && P <= e->fused_decode_rows;
+    const bool fused = fused_wave(e, P);
     const bool pdl = fused && e->use_pdl && !e->profiling;
     // un-fused tensor-core step: the same attribute through the chain of 31 launches (every kernel of the chain waits with
     // griddepcontrol.wait before it touches its predecessor's output; the LayerNorm-only kernel has no hook and is launched plainly)
@@ -1403,12 +1434,8 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
     memset(&sp, 0, sizeof(sp));
     sp.x = b.x; sp.W = e->W("fc_out.weight"); sp.b = e->W("fc_out.bias"); sp.V = d.vocab; sp.N = Nw; sp.ldn = ldn;
     sp.temperature = a.temperature; sp.mode = r.mode;
-    int smc = a.rng_sm_count > 0 ? a.rng_sm_count : e->sm_count;
-    int mts = a.rng_max_threads_per_sm > 0 ? a.rng_max_threads_per_sm : e->max_threads_per_sm;
-    int64_t Nrng = r.per_memory_rng ? a.n_cand : (a.N_total > 0 ? a.N_total : N_total);
-    sp.rng.seed = a.philox_seed; sp.rng.offset = a.philox_offset; sp.rng.numel = Nrng * d.vocab;
-    sp.rng.threads = torch_rng_threads(sp.rng.numel, smc, mts);
-    sp.rng_inc = torch_rng_increment(sp.rng.numel, smc, mts);
+    const int64_t Nrng = r.per_memory_rng ? a.n_cand : (a.N_total > 0 ? a.N_total : N_total);
+    sp.rng = rng_geom(e, a.philox_seed, a.philox_offset, Nrng * d.vocab, a.rng_sm_count, a.rng_max_threads_per_sm, &sp.rng_inc);
     sp.rng_dev = b.rng_state;
     sp.seq_index_base = a.seq_index_base + n0;      // waves and lanes start at column boundaries: n0 is a multiple of n_cand
     if (r.per_memory_rng) { sp.rng_cand = a.n_cand; sp.rng_col_steps = a.max_len; }
@@ -1427,23 +1454,150 @@ static int decode_step(mmt_engine* e, const DecodeRun& r, int64_t n0, int64_t Nw
         sp.part = b.part; sp.splits = ffn_splits; sp.part_stride = Nw * D;
         sp.pbias = pw.l2_b; sp.pgamma = pw.n3_w; sp.pbeta = pw.n3_b; sp.eps = 1e-5f;
     }
-    prof_pre(e, s);
-    {   // rows per CTA and pass: 2 when the input is still spread over FFN2 partials, else 8; at most four resident waves of CTAs
-        sp.rows_per_warp = P >= 8192 ? SAMPLE_NR : 1;       // small waves: one row per warp (latency), large: four (shared-memory traffic)
-        const int rpc = sp.part ? 2 : 8 * sp.rows_per_warp;
-        const int64_t groups = (Nw + rpc - 1) / rpc;
-        MMT_TRY(sample_init(e));
-        launch_kernel(r.ctl_temp ? sample_tokens<true> : sample_tokens<false>, dim3((unsigned)std::min<int64_t>(groups, (int64_t)e->sm_count * 4)), dim3(256),
-                      sample_smem_bytes(sp.V), s, pdl || pdl_u, sp);
-    }
-    MMT_TRY(check_launch(e, r.ctl_temp ? "sample_tokens_controlled" : "sample_tokens", s));
-    return 0;
+    return launch_sample(e, sp, P, r.ctl_temp != nullptr, pdl || pdl_u, s);
 }
 
 // Sequences a decode wave may hold (MMT_MAX_WAVE_SEQS, else by precision and device memory; see run_decode).
 static int64_t max_wave_sequences(const mmt_engine* e, int precision) {
     return e->max_wave_seqs > 0 ? e->max_wave_seqs
                                 : (precision == MMT_PREC_BF16 ? (int64_t)e->sm_count * (e->total_mem >= ((size_t)128 << 30) ? 8 : 4) * 128 : 32768);
+}
+
+// ---------------------------------------------------------------------------
+// step graphs and lanes of the decode drivers
+// ---------------------------------------------------------------------------
+// A decode step is the same kernel sequence at every position (the step counter and page parity live on the device), so
+// the drivers capture a group of U consecutive steps once into a CUDA graph (programmatic-dependent-launch edges included)
+// and replay it.  The group spans 1..4 lanes, independent parts of a wave whose steps are parallel branches of the graph.
+// A graph with a key -- the caller's tag and every value its nodes bake in -- is kept in the engine's graph cache (4
+// entries, the least recently used evicted) and serves later calls with the same key; one without belongs to the
+// StepGraph and is destroyed with it.
+struct StepGraph {
+    mmt_engine* e;
+    int lanes, U;
+    std::vector<uint64_t> key;        // empty: not cached
+    cudaGraphExec_t exec = nullptr;
+    int64_t launches = 0;             // kernel launches one replay stands for
+    StepGraph(mmt_engine* e_, int lanes_, int U_) : e(e_), lanes(lanes_), U(U_) {}
+    StepGraph(const StepGraph&) = delete;
+    StepGraph& operator=(const StepGraph&) = delete;
+    ~StepGraph() { if (key.empty() && exec) cudaGraphExecDestroy(exec); }
+
+    // look the graph up under `k` and the values every step graph bakes in
+    void find(std::vector<uint64_t> k) {
+        for (uint64_t v : {(uint64_t)lanes, (uint64_t)U, (uint64_t)(uintptr_t)e->arena, (uint64_t)e->arena_bytes,
+                           (uint64_t)e->fused_decode_rows, (uint64_t)e->use_pdl, (uint64_t)(uintptr_t)e->da_dbg}) k.push_back(v);
+        key = std::move(k);
+        for (auto& c : e->graph_cache)
+            if (c.key == key) { exec = c.exec; launches = c.launches_per_group; c.stamp = ++e->graph_cache_clock; return; }
+    }
+
+    // (re)capture U steps of the lanes in `active` (bit i: lane i); step(i, stream) enqueues one step of lane i
+    int capture(unsigned active, const std::function<int(int, cudaStream_t)>& step) {
+        if (key.empty() && exec) cudaGraphExecDestroy(exec);
+        exec = nullptr;
+        for (int i = 0; i < lanes; ++i) {     // capture-only streams: the caller's stream may be the legacy default stream
+            if (!e->cap_stream[i]) MMT_CUDA(cudaStreamCreateWithFlags(&e->cap_stream[i], cudaStreamNonBlocking));
+            if (!e->lane_ev[i]) MMT_CUDA(cudaEventCreateWithFlags(&e->lane_ev[i], cudaEventDisableTiming));
+        }
+        const int64_t l0 = e->launches;
+        MMT_CUDA(cudaStreamBeginCapture(e->cap_stream[0], cudaStreamCaptureModeRelaxed));
+        int rc = 0;
+        cudaError_t fe = cudaSuccess;
+        if (lanes > 1) {                      // fork the other lanes' branches off the capture origin
+            fe = cudaEventRecord(e->lane_ev[0], e->cap_stream[0]);
+            for (int i = 1; i < lanes && fe == cudaSuccess; ++i) if (active >> i & 1) fe = cudaStreamWaitEvent(e->cap_stream[i], e->lane_ev[0], 0);
+        }
+        for (int u = 0; u < U && !rc && fe == cudaSuccess; ++u)
+            for (int i = 0; i < lanes && !rc; ++i) if (active >> i & 1) rc = step(i, e->cap_stream[i]);
+        for (int i = 1; i < lanes && fe == cudaSuccess; ++i) {   // join
+            if (!(active >> i & 1)) continue;
+            fe = cudaEventRecord(e->lane_ev[i], e->cap_stream[i]);
+            if (fe == cudaSuccess) fe = cudaStreamWaitEvent(e->cap_stream[0], e->lane_ev[i], 0);
+        }
+        cudaGraph_t graph = nullptr;
+        cudaError_t ce = cudaStreamEndCapture(e->cap_stream[0], &graph);
+        launches = e->launches - l0;
+        e->launches = l0;
+        if (rc) { if (graph) cudaGraphDestroy(graph); return 1; }
+        if (fe != cudaSuccess) { if (graph) cudaGraphDestroy(graph); MMT_FAIL(std::string("step graph lane fork/join failed: ") + cudaGetErrorString(fe)); }
+        if (ce != cudaSuccess) MMT_FAIL(std::string("step graph capture failed: ") + cudaGetErrorString(ce));
+        ce = cudaGraphInstantiate(&exec, graph, 0);
+        cudaGraphDestroy(graph);
+        if (ce != cudaSuccess) { exec = nullptr; MMT_FAIL(std::string("cudaGraphInstantiate failed: ") + cudaGetErrorString(ce)); }
+        if (!key.empty()) {
+            if (e->graph_cache.size() >= 4) {
+                size_t lru = 0;
+                for (size_t i = 1; i < e->graph_cache.size(); ++i) if (e->graph_cache[i].stamp < e->graph_cache[lru].stamp) lru = i;
+                cudaGraphExecDestroy(e->graph_cache[lru].exec);
+                e->graph_cache.erase(e->graph_cache.begin() + lru);
+            }
+            e->graph_cache.push_back({key, exec, launches, ++e->graph_cache_clock});
+        }
+        return 0;
+    }
+
+    int replay(cudaStream_t s) {
+        MMT_CUDA(cudaGraphLaunch(exec, s));
+        e->launches += launches;
+        return 0;
+    }
+};
+
+// steps per graph group: the largest divisor of T up to MMT_GRAPH_STEPS
+static int step_group(const mmt_engine* e, int T) {
+    int U = 1;
+    for (int u = 2; u <= e->graph_steps; ++u) if (T % u == 0) U = u;
+    return U;
+}
+
+// Lanes of the decode wave of spectra [wb0, wb0 + Bmw): lane i takes the wave's spectra [i * Bm_lane, (i + 1) * Bm_lane);
+// lanes left empty by a short wave are dropped.  Returns the number of lanes.
+constexpr int MAX_LANES = 4;
+struct Lane { int b0, Bm; int64_t n0, Nw; };
+static int wave_lanes(int wb0, int Bmw, int NL, int Bm_lane, int n_cand, Lane* lane) {
+    int nl = 0;
+    for (int i = 0; i < NL; ++i) {
+        const int lo = std::min(i * Bm_lane, Bmw), hi = std::min(lo + Bm_lane, Bmw);
+        if (hi > lo) lane[nl++] = {wb0 + lo, hi - lo, (int64_t)(wb0 + lo) * n_cand, (int64_t)(hi - lo) * n_cand};
+    }
+    return nl;
+}
+
+// MMT_FFN_DEBUG / MMT_DA_DEBUG: print the phase timestamps the kernels of the last decode recorded (SM cycles).
+// `rows`: sequences of that decode's first wave.
+static int print_debug_phases(mmt_engine* e, int64_t rows, cudaStream_t s) {
+    if (e->ffn_dbg) {  // un-fused FFN launch of layer 3, last position
+        MMT_CUDA(cudaStreamSynchronize(s));
+        for (int bshow : {0, 64, 127}) {
+            const long long* d = e->ffn_dbg + bshow * 16;
+            fprintf(stderr, "ffn_fused_tc<LN> CTA %d: setup %lld | first acc1 %lld | first convert %lld | chunks 8..15:", bshow, d[1] - d[0], d[2] - d[1], d[3] - d[2]);
+            for (int i = 9; i <= 15; ++i) fprintf(stderr, " %lld", d[i] - d[i - 1]);
+            fprintf(stderr, " | start->acc2 %lld | tmem->stage %lld | LN rows %lld | total %lld\n", d[4] - d[0], d[5] - d[4], d[6] - d[5], d[7] - d[0]);
+        }
+    }
+    if (e->da_dbg) {   // the last decode_attn launch of layer 3
+        MMT_CUDA(cudaStreamSynchronize(s));
+        const int blocks = (int)std::min<int64_t>(4096, (rows + DA_R - 1) / DA_R);
+        for (int bshow : {0, blocks / 2, blocks - 1}) {
+            fprintf(stderr, "decode_attn phases, CTA %d:", bshow);
+            const int last = e->da_dbg[bshow * 16 + 14] ? 14 : 10;     // cluster variant: 10 gather | 11 GEMM1 | 12 GEMM2 | 13 scatter | 14 norm3
+            for (int i = 1; i <= last; ++i) fprintf(stderr, " %lld", e->da_dbg[bshow * 16 + i] - e->da_dbg[bshow * 16 + i - 1]);
+            fprintf(stderr, "  total %lld\n", e->da_dbg[bshow * 16 + last] - e->da_dbg[bshow * 16]);
+        }
+        for (int bshow : {1, blocks / 2}) {
+            const long long* d = e->da_dbg + (1024 + bshow) * 16;
+            fprintf(stderr, "decode_attn warp 5, CTA %d: self [K+scores %lld | V+acc %lld | reduce %lld | sync %lld]  cross [loop %lld | reduce %lld | sync %lld]\n", bshow,
+                    d[1] - d[0], d[2] - d[1], d[3] - d[2], d[4] - d[3], d[6] - d[5], d[7] - d[6], d[8] - d[7]);
+        }
+        for (int bshow : {0, 33}) {
+            const long long* d = e->da_dbg + (2048 + bshow) * 16;
+            fprintf(stderr, "ffn_fused phases, CTA %d:", bshow);
+            for (int i = 1; i <= 7; ++i) fprintf(stderr, " %lld", d[i] - d[i - 1]);
+            fprintf(stderr, "  total %lld\n", d[7] - d[0]);
+        }
+    }
+    return 0;
 }
 
 static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaStream_t s) {
@@ -1473,20 +1627,17 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     // Lanes: a small wave is a latency chain of ~13 dependent kernels per position that leaves most of the GPU
     // idle, so the wave's spectra are split into independent lanes whose chains run concurrently (parallel
     // branches of the same CUDA graph, own KV pools / step counters); every sequence is independent (SURVEY 8e).
-    constexpr int MAX_LANES = 4;
+    const int64_t Nwave = (int64_t)Bm_wave * a.n_cand;
+    const bool small_wave = fused_wave(e, Nwave);
     int NL = 1;
-    {
-        const int64_t Nwave = (int64_t)Bm_wave * a.n_cand;
-        const bool fused = e->fused_decode_rows > 0 && Nwave <= e->fused_decode_rows;
-        if (fused && e->use_graph && !e->profiling) {
-            NL = std::min(std::min(e->decode_lanes, MAX_LANES), Bm_wave);
-            while (NL > 1 && Nwave / NL < 32) --NL;
-        } else if (!fused && bf16 && e->use_graph && !e->profiling && Nwave >= 4096) {
-            // Large waves: the step alternates HBM-bound kernels (self-attention over the KV pages) with tensor-bound ones
-            // (the FFN), each leaving the other resource idle.  Two lanes -- independent halves of the wave as parallel
-            // branches of the step graph -- let one half's attention stream pages while the other half's FFN runs.
-            NL = std::min(std::min(e->decode_lanes_large, MAX_LANES), Bm_wave);
-        }
+    if (small_wave && e->use_graph && !e->profiling) {
+        NL = std::min(std::min(e->decode_lanes, MAX_LANES), Bm_wave);
+        while (NL > 1 && Nwave / NL < 32) --NL;
+    } else if (!small_wave && bf16 && e->use_graph && !e->profiling && Nwave >= 4096) {
+        // Large waves: the step alternates HBM-bound kernels (self-attention over the KV pages) with tensor-bound ones
+        // (the FFN), each leaving the other resource idle.  Two lanes -- independent halves of the wave as parallel
+        // branches of the step graph -- let one half's attention stream pages while the other half's FFN runs.
+        NL = std::min(std::min(e->decode_lanes_large, MAX_LANES), Bm_wave);
     }
     const int Bm_lane = (Bm_wave + NL - 1) / NL;
     // Single-wave sampling runs write ids / probabilities into engine-owned staging buffers (copied to the caller's
@@ -1495,20 +1646,17 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     // (A retiring call's large waves capture graphs specific to its sequences' lengths, which are not cached; its small
     // waves never compact, so their one graph is cached like the plain call's.)
     const bool retire = r.eos >= 0;
-    const bool small_wave = e->fused_decode_rows > 0 && (int64_t)Bm_wave * a.n_cand <= e->fused_decode_rows;
     const bool staged = e->use_graph && e->use_graph_cache && !e->profiling && n_waves == 1 && r.mode != 2 && !r.trg && (!retire || small_wave);   // forced inputs are the caller's tensor: nothing to cache across calls
     // Layer 0 on the position x token table: the un-fused bf16 step with token-major pages (the fused small-wave step and the
     // other page layouts keep the cache).  Layer 0's pages are only planned if some wave of the run is a fused one.
     bool l0_table = false, l0_pool = true;
     if (bf16 && e->use_l0_table && e->use_kv_epilogue && e->kv_tok_major && d.n_heads % 8 == 0 && d.vocab <= 256) {
         bool any_fused = false;
-        for (int wb0 = 0; wb0 < a.Bm; wb0 += Bm_wave)
-            for (int i = 0; i < NL; ++i) {
-                const int Bmw = std::min(Bm_wave, a.Bm - wb0), lo = std::min(i * Bm_lane, Bmw), hi = std::min(lo + Bm_lane, Bmw);
-                if (hi <= lo) continue;
-                if (e->fused_decode_rows > 0 && (int64_t)(hi - lo) * a.n_cand <= e->fused_decode_rows) any_fused = true;
-                else l0_table = true;
-            }
+        for (int wb0 = 0; wb0 < a.Bm; wb0 += Bm_wave) {
+            Lane lane[MAX_LANES];
+            const int nl = wave_lanes(wb0, std::min(Bm_wave, a.Bm - wb0), NL, Bm_lane, a.n_cand, lane);
+            for (int i = 0; i < nl; ++i) (fused_wave(e, lane[i].Nw) ? any_fused : l0_table) = true;
+        }
         l0_pool = any_fused;
     }
     if (l0_table) MMT_TRY(ensure_l0_table(e, s));
@@ -1518,17 +1666,12 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
     int* eos_all = nullptr;                  // retiring call: first-<EOS> step of every sequence (max_len until it emits)
     const bool controlled = r.h_temp != nullptr;
     float *ctl_temp = nullptr, *ctl_topp = nullptr; int32_t* ctl_topk = nullptr;   // (Bm) per-column sampling controls
-    auto plan_all = [&]() {
+    MMT_TRY(plan_arena(e, ar, [&]() {
         for (int i = 0; i < NL; ++i) plan_decoder(ar, d, (int64_t)Bm_lane * a.n_cand, Bm_lane, a.S, a.max_len, lb[i], bf16, e->fused_decode_rows, 1, retire, l0_table, l0_pool);
         if (staged) { st_tokens = ar.get<int64_t>((size_t)a.max_len * N_total); st_probs = ar.get<float>((size_t)a.max_len * N_total); }
         if (retire) eos_all = ar.get<int>(N_total);
         if (controlled) { ctl_temp = ar.get<float>(a.Bm); ctl_topk = ar.get<int32_t>(a.Bm); ctl_topp = ar.get<float>(a.Bm); }
-    };
-    ar.plan = true;
-    plan_all();
-    MMT_TRY(ensure_arena(e, ar.off));
-    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
-    plan_all();
+    }));
     DecodeRun rs = r;                        // the run as the kernels see it
     if (staged) { rs.tokens = st_tokens; rs.probs = r.probs ? st_probs : nullptr; }
     if (controlled) {     // device copies at fixed arena addresses: a cached decode graph serves calls with other values
@@ -1538,24 +1681,23 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
         rs.ctl_temp = ctl_temp; rs.ctl_topk = ctl_topk; rs.ctl_topp = ctl_topp;
     }
     const int pps = (a.max_len + PAGE_TOKENS - 1) / PAGE_TOKENS;
-    const bool early = (r.mode == 0) && a.stop_on_all_pad && n_waves == 1;
-    int steps_done = r.T;
-    std::vector<int64_t> nonpad_total(r.T, 0);
-    std::vector<int64_t> live_total(r.T, 0), rows_at(r.T, 0);     // retiring call
+    // Per-step counts the host reads back, ctl[8 + t] of every lane: non-<PAD> picks (greedy) and, in a retiring call,
+    // the sequences not finished after step t.  Greedy stop_on_all_pad ends the call after the first step at which every
+    // sequence of every wave has emitted <PAD> (validate_generate_MMT_v15_4.py:763); a retiring call ends after the first
+    // step that leaves none unfinished.
+    const bool pad_stop = r.mode == 0 && a.stop_on_all_pad;
+    const bool counts = retire || pad_stop;
+    std::vector<int64_t> nonpad_total(r.T, 0), live_total(r.T, 0), rows_at(r.T, 0);
     if (retire) {
         fill_i32<<<(unsigned)((N_total + 255) / 256), 256, 0, s>>>(eos_all, N_total, a.max_len);
         MMT_CUDA(cudaGetLastError());
-        for (int i = 0; i < 2; ++i) if (!e->poll_ev[i]) MMT_CUDA(cudaEventCreateWithFlags(&e->poll_ev[i], cudaEventDisableTiming));
     }
-    for (int wv = 0; wv < n_waves; ++wv) {
-        const int wb0 = wv * Bm_wave;
-        const int Bmw = std::min(Bm_wave, a.Bm - wb0);
-        struct Lane { int b0, Bm; int64_t n0, Nw; } lane[MAX_LANES];
-        int nl = 0;
-        for (int i = 0; i < NL; ++i) {
-            const int lo = std::min(i * Bm_lane, Bmw), hi = std::min(lo + Bm_lane, Bmw);
-            if (hi > lo) { lane[nl].b0 = wb0 + lo; lane[nl].Bm = hi - lo; lane[nl].n0 = (int64_t)(wb0 + lo) * a.n_cand; lane[nl].Nw = (int64_t)(hi - lo) * a.n_cand; ++nl; }
-        }
+    if (counts) for (int i = 0; i < 2; ++i) if (!e->poll_ev[i]) MMT_CUDA(cudaEventCreateWithFlags(&e->poll_ev[i], cudaEventDisableTiming));
+    if (bf16) MMT_TRY(tc_init(e));
+    for (int wb0 = 0; wb0 < a.Bm; wb0 += Bm_wave) {
+        Lane lane[MAX_LANES];
+        const int nl = wave_lanes(wb0, std::min(Bm_wave, a.Bm - wb0), NL, Bm_lane, a.n_cand, lane);
+        int64_t rows[MAX_LANES];              // rows of each lane's wave (a retiring call's large waves shrink)
         for (int i = 0; i < nl; ++i) {
             DecBuffers& b = lb[i];
             MMT_CUDA(cudaMemsetAsync(b.ctl, 0, (8 + 256) * sizeof(int), s));
@@ -1565,228 +1707,109 @@ static int run_decode(mmt_engine* e, const DecodeRun& r, int32_t* h_steps, cudaS
             MMT_TRY(check_launch(e, "init_block_table", s));
             MMT_TRY(decode_prepare_wave(e, a, lane[i].b0, lane[i].Bm, b, bf16, s));
             if (retire) { b.plan_rows = lane[i].Nw; b.orig = b.col_start = b.col_count = nullptr; b.eos_len = eos_all + lane[i].n0; }
+            rows[i] = lane[i].Nw;
         }
-        int64_t rows[MAX_LANES];              // rows of each lane's wave (a retiring call's large waves shrink)
-        for (int i = 0; i < nl; ++i) rows[i] = lane[i].Nw;
-        // One decode step is the same kernel sequence at every position (the step counter lives on
-        // the device), so a group of U consecutive steps of every lane is captured once per wave into a CUDA
-        // graph (programmatic-dependent-launch edges included) and replayed T / U times.
-        int U = 1;
-        for (int u = 2; u <= e->graph_steps; ++u) if (r.T % u == 0) U = u;
-        if (retire) U = std::min(r.T, 8);     // groups of 8 positions (a shorter last group runs without a graph)
-        cudaGraphExec_t exec = nullptr;
-        int64_t launches_per_group = 0;
-        std::vector<uint64_t> key;            // every value baked into the graph's nodes
+        auto step = [&](int i, cudaStream_t cs) { return decode_step(e, rs, lane[i].n0, rows[i], lane[i].Bm, lb[i], bf16, cs); };
+        auto active = [&]() { unsigned m = 0; for (int i = 0; i < nl; ++i) if (rows[i] > 0) m |= 1u << i; return m; };
+        // a retiring call's groups are 8 positions (a shorter last group runs without the graph)
+        int U = retire ? std::min(r.T, 8) : step_group(e, r.T);
+        StepGraph graph(e, nl, U);
         if (staged) {
-            auto put = [&](uint64_t v) { key.push_back(v); };
             uint32_t tbits; memcpy(&tbits, &a.temperature, 4);
-            put((uint64_t)r.mode); put((uint64_t)r.T); put((uint64_t)(r.probs != nullptr)); put((uint64_t)a.S); put((uint64_t)a.Bm);
-            put((uint64_t)a.n_cand); put((uint64_t)a.max_len); put(tbits); put((uint64_t)a.precision);
-            put((uint64_t)a.seq_index_base); put((uint64_t)a.N_total); put((uint64_t)a.rng_sm_count); put((uint64_t)a.rng_max_threads_per_sm);
-            put((uint64_t)r.per_memory_rng); put((uint64_t)r.eos); put((uint64_t)controlled);   // controls: their presence, never their values
-            put((uint64_t)(uintptr_t)e->arena); put((uint64_t)e->arena_bytes); put((uint64_t)nl); put((uint64_t)U);
-            put((uint64_t)e->fused_decode_rows); put((uint64_t)e->use_pdl); put((uint64_t)(uintptr_t)e->da_dbg);
-            for (auto& c : e->graph_cache) if (c.key == key) { exec = c.exec; launches_per_group = c.launches_per_group; c.stamp = ++e->graph_cache_clock; break; }
+            graph.find({0xDEC, (uint64_t)r.mode, (uint64_t)r.T, (uint64_t)(r.probs != nullptr), (uint64_t)a.S, (uint64_t)a.Bm,
+                        (uint64_t)a.n_cand, (uint64_t)a.max_len, tbits, (uint64_t)a.precision, (uint64_t)a.seq_index_base,
+                        (uint64_t)a.N_total, (uint64_t)a.rng_sm_count, (uint64_t)a.rng_max_threads_per_sm, (uint64_t)r.per_memory_rng,
+                        (uint64_t)r.eos, (uint64_t)controlled});   // controls: their presence, never their values
         }
-        // capture U steps of the lanes that still have rows into `exec`
-        auto capture = [&]() -> int {
-            if (bf16) MMT_TRY(tc_init(e));
-            for (int i = 0; i < nl; ++i) {
-                if (!e->cap_stream[i]) MMT_CUDA(cudaStreamCreateWithFlags(&e->cap_stream[i], cudaStreamNonBlocking));
-                if (!e->lane_ev[i]) MMT_CUDA(cudaEventCreateWithFlags(&e->lane_ev[i], cudaEventDisableTiming));
-            }
-            const int64_t l0 = e->launches;
-            MMT_CUDA(cudaStreamBeginCapture(e->cap_stream[0], cudaStreamCaptureModeRelaxed));
-            int rc = 0;
-            cudaError_t fe = cudaSuccess;
-            if (nl > 1) {                                 // fork the other lanes' branches off the capture origin
-                fe = cudaEventRecord(e->lane_ev[0], e->cap_stream[0]);
-                for (int i = 1; i < nl && fe == cudaSuccess; ++i) if (rows[i] > 0) fe = cudaStreamWaitEvent(e->cap_stream[i], e->lane_ev[0], 0);
-            }
-            for (int u = 0; u < U && !rc && fe == cudaSuccess; ++u)
-                for (int i = 0; i < nl && !rc; ++i) if (rows[i] > 0) rc = decode_step(e, rs, lane[i].n0, rows[i], lane[i].Bm, lb[i], bf16, e->cap_stream[i]);
-            for (int i = 1; i < nl && fe == cudaSuccess; ++i) {   // join
-                if (rows[i] == 0) continue;
-                fe = cudaEventRecord(e->lane_ev[i], e->cap_stream[i]);
-                if (fe == cudaSuccess) fe = cudaStreamWaitEvent(e->cap_stream[0], e->lane_ev[i], 0);
-            }
-            cudaGraph_t graph = nullptr;
-            cudaError_t ce = cudaStreamEndCapture(e->cap_stream[0], &graph);
-            launches_per_group = e->launches - l0;
-            e->launches = l0;
-            if (rc) { if (graph) cudaGraphDestroy(graph); return 1; }
-            if (fe != cudaSuccess) { if (graph) cudaGraphDestroy(graph); MMT_FAIL(std::string("decode lane fork/join failed: ") + cudaGetErrorString(fe)); }
-            if (ce != cudaSuccess) MMT_FAIL(std::string("decode step capture failed: ") + cudaGetErrorString(ce));
-            ce = cudaGraphInstantiate(&exec, graph, 0);
-            cudaGraphDestroy(graph);
-            if (ce != cudaSuccess) MMT_FAIL(std::string("cudaGraphInstantiate failed: ") + cudaGetErrorString(ce));
+        if (e->use_graph && !e->profiling && !graph.exec) MMT_TRY(graph.capture(active(), step));
+        else if (!graph.exec && !retire) U = 1;
+        // Polls: after a group is enqueued, its per-step counts are copied back (poll n) and the host reads poll n - 1,
+        // whose groups the GPU has finished while it runs this one, so the loop never drains the stream.  A retiring wave
+        // polls every group, the single wave of a greedy stop_on_all_pad call every ~16 steps (a multiple of U); other
+        // waves do not poll, and only a call that needs the counts reads them once the wave is done.
+        const bool wave_pad_stop = pad_stop && n_waves == 1;
+        const int poll_every = retire ? U : wave_pad_stop ? (U >= 16 ? U : (16 / U) * U) : 0;
+        int n_polls = 0, polled_t[2] = {0, 0};
+        const int32_t* cnt = nullptr;         // the poll the host read last: lane i's nonpad at [i * 256 + t], live at [i * 256 + 128 + t]
+        auto post = [&](int t) -> int {
+            for (int i = 0; i < nl; ++i)
+                MMT_CUDA(cudaMemcpyAsync(e->h_pinned + (n_polls & 1) * 1024 + i * 256, lb[i].ctl + 8, 256 * sizeof(int), cudaMemcpyDeviceToHost, s));
+            MMT_CUDA(cudaEventRecord(e->poll_ev[n_polls & 1], s));
+            polled_t[n_polls & 1] = t;
+            ++n_polls;
             return 0;
         };
-        if (e->use_graph && !e->profiling && !exec) {
-            MMT_TRY(capture());
-            if (staged) {
-                if (e->graph_cache.size() >= 4) {      // evict the least recently used entry
-                    size_t lru = 0;
-                    for (size_t i = 1; i < e->graph_cache.size(); ++i) if (e->graph_cache[i].stamp < e->graph_cache[lru].stamp) lru = i;
-                    cudaGraphExecDestroy(e->graph_cache[lru].exec);
-                    e->graph_cache.erase(e->graph_cache.begin() + lru);
-                }
-                e->graph_cache.push_back({key, exec, launches_per_group, ++e->graph_cache_clock});
-            }
-        } else if (!exec && !retire) {
-            U = 1;
-        }
-        struct ExecGuard { cudaGraphExec_t x; ~ExecGuard() { if (x) cudaGraphExecDestroy(x); } } guard{staged ? nullptr : exec};
-        if (retire) {
-            // Groups of U positions; after group g is enqueued, its per-step counts are copied back (poll g) and the host
-            // reads poll g - 1, whose group the GPU has finished while it runs group g.  A large lane whose live rows at the
-            // end of group g - 1 are at most 7/8 of its wave is compacted to those rows before group g + 1 (rows finished
-            // during group g ride along once, masked), and the group graph is captured again for the smaller wave.
-            // Small (fused) waves are latency chains that fewer rows do not shorten: they only stop once all have finished.
-            const bool pad_stop = n_waves == 1 && r.mode == 0 && a.stop_on_all_pad;
-            int g = 0, tpoll[2] = {0, 0};
-            bool stop = false;
-            for (int t = 0; t < r.T && !stop;) {
-                const int n = std::min(U, r.T - t);
-                if (exec && n == U) { MMT_CUDA(cudaGraphLaunch(exec, s)); e->launches += launches_per_group; }
-                else for (int q = 0; q < n; ++q) for (int i = 0; i < nl; ++i) if (rows[i] > 0) MMT_TRY(decode_step(e, rs, lane[i].n0, rows[i], lane[i].Bm, lb[i], bf16, s));
-                for (int q = t; q < t + n; ++q) for (int i = 0; i < nl; ++i) rows_at[q] += rows[i];
-                t += n;
-                for (int i = 0; i < nl; ++i)       // nonpad [0, 128) | live [128, 256)
-                    MMT_CUDA(cudaMemcpyAsync(e->h_pinned + (g & 1) * 1024 + i * 256, lb[i].ctl + 8, 256 * sizeof(int), cudaMemcpyDeviceToHost, s));
-                MMT_CUDA(cudaEventRecord(e->poll_ev[g & 1], s));
-                tpoll[g & 1] = t - 1;
-                ++g;
-                if (g < 2 || t >= r.T) continue;
-                const int k = (g - 2) & 1, tp = tpoll[k];
-                MMT_CUDA(cudaEventSynchronize(e->poll_ev[k]));
-                const int32_t* cnt = e->h_pinned + k * 1024;
-                for (int q = 0; q <= tp && !stop; ++q) {
-                    int64_t live = 0, nonpad = 0;
-                    for (int i = 0; i < nl; ++i) { live += cnt[i * 256 + 128 + q]; nonpad += cnt[i * 256 + q]; }
-                    stop = live == 0 || (pad_stop && nonpad == 0);
-                }
-                if (stop) break;
-                bool changed = false;
-                for (int i = 0; i < nl; ++i) {
-                    const int64_t live = cnt[i * 256 + 128 + tp];
-                    if (rows[i] == 0 || lb[i].plan_rows <= e->fused_decode_rows || live * 8 > rows[i] * 7) continue;
-                    DecBuffers& b = lb[i];
-                    if (live > 0) {
-                        int* orig_new = b.orig == b.rt_orig[0] ? b.rt_orig[1] : b.rt_orig[0];
-                        MMT_CUDA(cudaMemsetAsync(b.rt_col_count, 0, lane[i].Bm * sizeof(int), s));
-                        prof_pre(e, s);
-                        retire_scan<<<1, 1024, 0, s>>>(b.orig, b.eos_len, rows[i], tp, b.rt_src);
-                        MMT_TRY(check_launch(e, "retire_scan", s));
-                        prof_pre(e, s);
-                        retire_gather<<<(unsigned)((live + 255) / 256), 256, 0, s>>>(b.rt_src, b.orig, b.block_table, pps, live, a.n_cand, orig_new,
-                                                                                     b.rt_bt, b.rt_col_start, b.rt_col_count);
-                        MMT_TRY(check_launch(e, "retire_gather", s));
-                        std::swap(b.block_table, b.rt_bt);
-                        b.orig = orig_new; b.col_start = b.rt_col_start; b.col_count = b.rt_col_count;
-                    }
-                    rows[i] = live;
-                    changed = true;
-                }
-                if (changed && exec) {
-                    cudaGraphExecDestroy(exec);
-                    exec = guard.x = nullptr;
-                    MMT_TRY(capture());
-                    guard.x = exec;
-                }
-            }
-            // the last poll holds the wave's complete counts
-            MMT_CUDA(cudaEventSynchronize(e->poll_ev[(g - 1) & 1]));
-            const int32_t* cnt = e->h_pinned + ((g - 1) & 1) * 1024;
-            for (int i = 0; i < nl; ++i)
-                for (int q = 0; q < r.T; ++q) { nonpad_total[q] += cnt[i * 256 + q]; live_total[q] += cnt[i * 256 + 128 + q]; }
-            continue;
-        }
-        // greedy early exit (validate_generate_MMT_v15_4.py:763): the per-step non-PAD counts are polled one
-        // group behind the launches, so the host never drains the stream inside the loop
-        if (early) for (int i = 0; i < 2; ++i) if (!e->poll_ev[i]) MMT_CUDA(cudaEventCreateWithFlags(&e->poll_ev[i], cudaEventDisableTiming));
-        const int poll_every = U >= 16 ? U : (16 / U) * U;    // steps between polls (multiple of U, >= ~16)
-        int n_polls = 0, checked_polls = 0;
-        bool stop = false;
-        auto check_poll = [&](int k) -> int {       // inspect poll k (covers steps < (k+1)*poll_every, capped at T)
+        auto read = [&](int k) -> int {
             MMT_CUDA(cudaEventSynchronize(e->poll_ev[k & 1]));
-            const int upto = std::min(r.T, (k + 1) * poll_every);
-            const int32_t* cnt = e->h_pinned + (k & 1) * 512;
-            for (int q = 0; q < upto; ++q) {
-                int tot = 0;
-                for (int i = 0; i < nl; ++i) tot += cnt[i * 128 + q];
-                if (tot == 0) { steps_done = q + 1; stop = true; break; }
-            }
+            cnt = e->h_pinned + (k & 1) * 1024;
             return 0;
         };
-        for (int t = 0; t < r.T && !stop; t += U) {
-            if (exec) { MMT_CUDA(cudaGraphLaunch(exec, s)); e->launches += launches_per_group; }
-            else for (int i = 0; i < nl; ++i) MMT_TRY(decode_step(e, rs, lane[i].n0, lane[i].Nw, lane[i].Bm, lb[i], bf16, s));
-            const int done = t + U;
-            if (early && (done % poll_every == 0 || done == r.T)) {
-                if (n_polls - checked_polls >= 2) { MMT_TRY(check_poll(checked_polls)); ++checked_polls; }
-                if (stop) break;
-                for (int i = 0; i < nl; ++i)
-                    MMT_CUDA(cudaMemcpyAsync(e->h_pinned + (n_polls & 1) * 512 + i * 128, lb[i].ctl + 8, r.T * sizeof(int), cudaMemcpyDeviceToHost, s));
-                MMT_CUDA(cudaEventRecord(e->poll_ev[n_polls & 1], s));
-                ++n_polls;
-                if (n_polls - checked_polls >= 2) { MMT_TRY(check_poll(checked_polls)); ++checked_polls; }
+        auto total = [&](int field, int q) { int64_t v = 0; for (int i = 0; i < nl; ++i) v += cnt[i * 256 + field + q]; return v; };
+        bool stop = false;
+        for (int t = 0; t < r.T && !stop;) {
+            const int n = std::min(U, r.T - t);
+            if (graph.exec && n == U) MMT_TRY(graph.replay(s));
+            else for (int q = 0; q < n; ++q) for (int i = 0; i < nl; ++i) if (rows[i] > 0) MMT_TRY(step(i, s));
+            for (int q = t; q < t + n; ++q) for (int i = 0; i < nl; ++i) rows_at[q] += rows[i];
+            t += n;
+            if (!poll_every || (t % poll_every && t < r.T)) continue;
+            MMT_TRY(post(t));
+            if (n_polls < 2 || t >= r.T) continue;
+            MMT_TRY(read(n_polls - 2));
+            const int tp = polled_t[n_polls & 1] - 1;      // the last step poll n - 2 covers
+            for (int q = 0; q <= tp && !stop; ++q) stop = (retire && total(128, q) == 0) || (wave_pad_stop && total(0, q) == 0);
+            if (stop || !retire) continue;
+            // A large lane whose live rows after step tp are at most 7/8 of its wave is compacted to those rows before the
+            // next group (rows finished during the group the GPU runs ride along once, masked), and the group graph is
+            // captured again for the smaller wave.  Small (fused) waves are latency chains that fewer rows do not shorten:
+            // they only stop once all have finished.
+            bool changed = false;
+            for (int i = 0; i < nl; ++i) {
+                const int64_t live = cnt[i * 256 + 128 + tp];
+                if (rows[i] == 0 || fused_wave(e, lb[i].plan_rows) || live * 8 > rows[i] * 7) continue;
+                DecBuffers& b = lb[i];
+                if (live > 0) {
+                    int* orig_new = b.orig == b.rt_orig[0] ? b.rt_orig[1] : b.rt_orig[0];
+                    MMT_CUDA(cudaMemsetAsync(b.rt_col_count, 0, lane[i].Bm * sizeof(int), s));
+                    prof_pre(e, s);
+                    retire_scan<<<1, 1024, 0, s>>>(b.orig, b.eos_len, rows[i], tp, b.rt_src);
+                    MMT_TRY(check_launch(e, "retire_scan", s));
+                    prof_pre(e, s);
+                    retire_gather<<<(unsigned)((live + 255) / 256), 256, 0, s>>>(b.rt_src, b.orig, b.block_table, pps, live, a.n_cand, orig_new,
+                                                                                 b.rt_bt, b.rt_col_start, b.rt_col_count);
+                    MMT_TRY(check_launch(e, "retire_gather", s));
+                    std::swap(b.block_table, b.rt_bt);
+                    b.orig = orig_new; b.col_start = b.rt_col_start; b.col_count = b.rt_col_count;
+                }
+                rows[i] = live;
+                changed = true;
             }
+            if (changed && graph.exec) MMT_TRY(graph.capture(active(), step));
         }
-        while (early && !stop && checked_polls < n_polls) { MMT_TRY(check_poll(checked_polls)); ++checked_polls; }
-        if ((r.mode == 0) && a.stop_on_all_pad && n_waves > 1) {
-            for (int i = 0; i < nl; ++i)
-                MMT_CUDA(cudaMemcpyAsync(e->h_pinned + i * 128, lb[i].ctl + 8, r.T * sizeof(int), cudaMemcpyDeviceToHost, s));
-            MMT_CUDA(cudaStreamSynchronize(s));
-            for (int i = 0; i < nl; ++i) for (int q = 0; q < r.T; ++q) nonpad_total[q] += e->h_pinned[i * 128 + q];
+        if (counts) {     // the wave's counts: the poll that stopped it, else one taken after its last step
+            if (!stop) {
+                if (!poll_every) MMT_TRY(post(r.T));
+                MMT_TRY(read(n_polls - 1));
+            }
+            for (int q = 0; q < r.T; ++q) { nonpad_total[q] += total(0, q); live_total[q] += total(128, q); }
         }
     }
     if (staged) {
         MMT_CUDA(cudaMemcpyAsync(r.tokens, st_tokens, (size_t)r.T * N_total * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
         if (r.probs) MMT_CUDA(cudaMemcpyAsync(r.probs, st_probs, (size_t)r.T * N_total * sizeof(float), cudaMemcpyDeviceToDevice, s));
     }
-    if ((r.mode == 0) && a.stop_on_all_pad && n_waves > 1 && !retire)
-        for (int q = 0; q < r.T; ++q) if (nonpad_total[q] == 0) { steps_done = q + 1; break; }
-    if (retire) {   // every sequence finished (or, greedy stop_on_all_pad, finished or emitted <PAD>) at step q
-        for (int q = 0; q < r.T; ++q)
-            if (live_total[q] == 0 || ((r.mode == 0) && a.stop_on_all_pad && nonpad_total[q] == 0)) { steps_done = q + 1; break; }
+    // steps a wave never launched count zero: a wave that stopped early ends the call no later than its stop
+    int steps_done = r.T;
+    for (int q = 0; q < r.T; ++q)
+        if ((retire && live_total[q] == 0) || (pad_stop && nonpad_total[q] == 0)) { steps_done = q + 1; break; }
+    if (retire) {
         prof_pre(e, s);
         retire_fill<<<(unsigned)(((int64_t)r.T * N_total + 255) / 256), 256, 0, s>>>(r.tokens, r.probs, r.T, N_total, eos_all, steps_done, r.len);
         MMT_TRY(check_launch(e, "retire_fill", s));
         if (r.h_rows) for (int q = 0; q < r.T; ++q) r.h_rows[q] = rows_at[q];
     }
     if (h_steps) *h_steps = steps_done;
-    if (e->ffn_dbg) {  // MMT_FFN_DEBUG: un-fused FFN launch of layer 3, last position
-        MMT_CUDA(cudaStreamSynchronize(s));
-        for (int bshow : {0, 64, 127}) {
-            const long long* d = e->ffn_dbg + bshow * 16;
-            fprintf(stderr, "ffn_fused_tc<LN> CTA %d: setup %lld | first acc1 %lld | first convert %lld | chunks 8..15:", bshow, d[1] - d[0], d[2] - d[1], d[3] - d[2]);
-            for (int i = 9; i <= 15; ++i) fprintf(stderr, " %lld", d[i] - d[i - 1]);
-            fprintf(stderr, " | start->acc2 %lld | tmem->stage %lld | LN rows %lld | total %lld\n", d[4] - d[0], d[5] - d[4], d[6] - d[5], d[7] - d[0]);
-        }
-    }
-    if (e->da_dbg) {   // MMT_DA_DEBUG: phase timestamps (SM cycles) of the last decode_attn launch of layer 3
-        MMT_CUDA(cudaStreamSynchronize(s));
-        const int blocks = (int)std::min<int64_t>(4096, (std::min<int64_t>(N_total, max_wave_seqs) + DA_R - 1) / DA_R);
-        for (int bshow : {0, blocks / 2, blocks - 1}) {
-            fprintf(stderr, "decode_attn phases, CTA %d:", bshow);
-            const int last = e->da_dbg[bshow * 16 + 14] ? 14 : 10;     // cluster variant: 10 gather | 11 GEMM1 | 12 GEMM2 | 13 scatter | 14 norm3
-            for (int i = 1; i <= last; ++i) fprintf(stderr, " %lld", e->da_dbg[bshow * 16 + i] - e->da_dbg[bshow * 16 + i - 1]);
-            fprintf(stderr, "  total %lld\n", e->da_dbg[bshow * 16 + last] - e->da_dbg[bshow * 16]);
-        }
-        for (int bshow : {1, blocks / 2}) {
-            const long long* d = e->da_dbg + (1024 + bshow) * 16;
-            fprintf(stderr, "decode_attn warp 5, CTA %d: self [K+scores %lld | V+acc %lld | reduce %lld | sync %lld]  cross [loop %lld | reduce %lld | sync %lld]\n", bshow,
-                    d[1] - d[0], d[2] - d[1], d[3] - d[2], d[4] - d[3], d[6] - d[5], d[7] - d[6], d[8] - d[7]);
-        }
-        for (int bshow : {0, 33}) {
-            const long long* d = e->da_dbg + (2048 + bshow) * 16;
-            fprintf(stderr, "ffn_fused phases, CTA %d:", bshow);
-            for (int i = 1; i <= 7; ++i) fprintf(stderr, " %lld", d[i] - d[i - 1]);
-            fprintf(stderr, "  total %lld\n", d[7] - d[0]);
-        }
-    }
-    return 0;
+    return print_debug_phases(e, std::min<int64_t>(N_total, max_wave_seqs), s);
 }
 
 // Wave loop shared by the batched beam search (run_beam) and the stochastic beam search (run_sbs): the K slots of every
@@ -1803,8 +1826,8 @@ struct BeamLoop {
     std::function<int(const BeamWave&, cudaStream_t)> init;     // state of the wave's slots (before the memory projection)
     std::function<int(const BeamWave&, cudaStream_t)> select;   // one selection step (captured)
     std::function<int(const BeamWave&, cudaStream_t)> finish;   // optional: after the wave's last step
-    // optional: every value the step graph of a wave bakes in besides the arena's addresses -> the graph is kept in
-    // the engine's graph cache and serves later calls with the same key
+    // optional: a tag and every value the step graph of a wave bakes in besides those StepGraph::find adds -> the graph
+    // is kept in the engine's graph cache and serves later calls with the same key
     std::function<void(const BeamWave&, std::vector<uint64_t>&)> graph_key;
 };
 
@@ -1835,50 +1858,20 @@ static int beam_wave_loop(mmt_engine* e, const mmt_decode_args& a, bool bf16, co
             MMT_TRY(check_launch(e, "beam_copy_pages", cs));
             return 0;
         };
-        int U = 1;
-        for (int u = 2; u <= e->graph_steps; ++u) if (T % u == 0) U = u;
-        cudaGraphExec_t exec = nullptr;
-        int64_t launches_per_group = 0;
-        std::vector<uint64_t> key;
-        const bool cached = L.graph_key && e->use_graph && e->use_graph_cache && !e->profiling;
-        if (cached) {
+        int U = step_group(e, T);
+        StepGraph graph(e, 1, U);
+        if (L.graph_key && e->use_graph && e->use_graph_cache && !e->profiling) {
+            std::vector<uint64_t> key;
             L.graph_key(w, key);
-            for (uint64_t v : {(uint64_t)U, (uint64_t)(uintptr_t)e->arena, (uint64_t)e->arena_bytes, (uint64_t)e->fused_decode_rows,
-                               (uint64_t)e->use_pdl, (uint64_t)(uintptr_t)e->da_dbg}) key.push_back(v);
-            for (auto& c : e->graph_cache) if (c.key == key) { exec = c.exec; launches_per_group = c.launches_per_group; c.stamp = ++e->graph_cache_clock; break; }
+            graph.find(std::move(key));
         }
-        if (e->use_graph && !e->profiling && !exec) {
-            if (!e->cap_stream[0]) MMT_CUDA(cudaStreamCreateWithFlags(&e->cap_stream[0], cudaStreamNonBlocking));
-            const int64_t l0 = e->launches;
-            MMT_CUDA(cudaStreamBeginCapture(e->cap_stream[0], cudaStreamCaptureModeRelaxed));
-            int rc = 0;
-            for (int u = 0; u < U && !rc; ++u) rc = one_step(e->cap_stream[0]);
-            cudaGraph_t graph = nullptr;
-            cudaError_t ce = cudaStreamEndCapture(e->cap_stream[0], &graph);
-            launches_per_group = e->launches - l0;
-            e->launches = l0;
-            if (rc) { if (graph) cudaGraphDestroy(graph); return 1; }
-            if (ce != cudaSuccess) MMT_FAIL(std::string("beam step capture failed: ") + cudaGetErrorString(ce));
-            ce = cudaGraphInstantiate(&exec, graph, 0);
-            cudaGraphDestroy(graph);
-            if (ce != cudaSuccess) MMT_FAIL(std::string("cudaGraphInstantiate failed: ") + cudaGetErrorString(ce));
-            if (cached) {
-                if (e->graph_cache.size() >= 4) {      // evict the least recently used entry
-                    size_t lru = 0;
-                    for (size_t i = 1; i < e->graph_cache.size(); ++i) if (e->graph_cache[i].stamp < e->graph_cache[lru].stamp) lru = i;
-                    cudaGraphExecDestroy(e->graph_cache[lru].exec);
-                    e->graph_cache.erase(e->graph_cache.begin() + lru);
-                }
-                e->graph_cache.push_back({key, exec, launches_per_group, ++e->graph_cache_clock});
-            }
-        } else if (!exec) {
-            U = 1;
-        }
-        struct ExecGuard { cudaGraphExec_t x; ~ExecGuard() { if (x) cudaGraphExecDestroy(x); } } guard{cached ? nullptr : exec};
+        if (e->use_graph && !e->profiling && !graph.exec) MMT_TRY(graph.capture(1, [&](int, cudaStream_t cs) { return one_step(cs); }));
+        else if (!graph.exec) U = 1;
+        // a synchronous poll every ~16 steps (a multiple of U)
         const int poll_every = U >= 16 ? U : (16 / U) * U;
         int steps_done = T;
         for (int t = 0; t < T; t += U) {
-            if (exec) { MMT_CUDA(cudaGraphLaunch(exec, s)); e->launches += launches_per_group; }
+            if (graph.exec) MMT_TRY(graph.replay(s));
             else MMT_TRY(one_step(s));
             const int done = t + U;
             if (done < T && done % poll_every == 0) {
@@ -1918,17 +1911,12 @@ static int run_beam(mmt_engine* e, const mmt_decode_args& a0, int K, int T, int 
     Arena ar;
     DecBuffers b;
     L.b = &b;
-    auto plan_all = [&]() {
+    MMT_TRY(plan_arena(e, ar, [&]() {
         plan_decoder(ar, d, Nw_max, L.Bm_wave, a.S, T, b, bf16, e->fused_decode_rows, 2);
         L.logits = ar.get<float>((size_t)Nw_max * d.vocab);
         L.cur_tok = ar.get<int64_t>((size_t)Nw_max);
         L.copy_src = ar.get<int>((size_t)Nw_max); L.copy_dst = ar.get<int>((size_t)Nw_max);
-    };
-    ar.plan = true;
-    plan_all();
-    MMT_TRY(ensure_arena(e, ar.off));
-    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
-    plan_all();
+    }));
     auto params = [&](const BeamWave& w) {
         BeamParams bp;
         memset(&bp, 0, sizeof(bp));
@@ -1971,7 +1959,7 @@ static int run_sbs(mmt_engine* e, const mmt_decode_args& a0, const float* h_temp
     DecBuffers b;
     L.b = &b;
     double *phi[2], *key[2]; int* len[2]; uint8_t* hist[2]; float* probs[2]; float* temp = nullptr;
-    auto plan_all = [&]() {
+    MMT_TRY(plan_arena(e, ar, [&]() {
         plan_decoder(ar, d, Nw_max, L.Bm_wave, a.S, T, b, bf16, e->fused_decode_rows, 2);
         L.logits = ar.get<float>((size_t)Nw_max * V);
         L.cur_tok = ar.get<int64_t>((size_t)Nw_max);
@@ -1981,23 +1969,17 @@ static int run_sbs(mmt_engine* e, const mmt_decode_args& a0, const float* h_temp
             hist[i] = ar.get<uint8_t>((size_t)Nw_max * T); probs[i] = ar.get<float>((size_t)Nw_max * T);
         }
         temp = ar.get<float>((size_t)a.Bm);
-    };
-    ar.plan = true;
-    plan_all();
-    MMT_TRY(ensure_arena(e, ar.off));
-    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
-    plan_all();
+    }));
     MMT_CUDA(cudaFuncSetAttribute(sbs_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbs_smem_bytes(SBS_MAX, VOCAB_MAX)));
     MMT_CUDA(cudaMemcpyAsync(temp, h_temp, (size_t)a.Bm * sizeof(float), cudaMemcpyHostToDevice, s));
-    const int smc = a.rng_sm_count > 0 ? a.rng_sm_count : e->sm_count;
-    const int mts = a.rng_max_threads_per_sm > 0 ? a.rng_max_threads_per_sm : e->max_threads_per_sm;
+    uint64_t rng_inc;      // the generator state comes from b.rng_state
+    const RngGeom rng = rng_geom(e, 0, 0, (int64_t)K * V, a.rng_sm_count, a.rng_max_threads_per_sm, &rng_inc);
     auto params = [&](const BeamWave& w) {
         SbsParams sp;
         memset(&sp, 0, sizeof(sp));
         sp.logits = L.logits; sp.V = V; sp.K = K; sp.T = T; sp.eos = eos; sp.pps = pps; sp.Nw = w.Nw; sp.step = b.ctl;
         sp.temp = temp + w.b0;
-        sp.rng.numel = (int64_t)K * V; sp.rng.threads = torch_rng_threads(sp.rng.numel, smc, mts);
-        sp.rng_inc = torch_rng_increment(sp.rng.numel, smc, mts);
+        sp.rng = rng; sp.rng_inc = rng_inc;
         sp.rng_dev = b.rng_state;
         sp.col_base = a0.seq_index_base / K + w.b0;
         for (int i = 0; i < 2; ++i) { sp.phi[i] = phi[i]; sp.key[i] = key[i]; sp.len[i] = len[i]; sp.hist[i] = hist[i]; sp.probs[i] = probs[i]; }
@@ -2022,7 +2004,7 @@ static int run_sbs(mmt_engine* e, const mmt_decode_args& a0, const float* h_temp
     };
     L.graph_key = [&](const BeamWave& w, std::vector<uint64_t>& k) {
         for (uint64_t v : {(uint64_t)0x5B5, (uint64_t)K, (uint64_t)T, (uint64_t)eos, (uint64_t)a.S, (uint64_t)w.Bmw, (uint64_t)a.precision,
-                           (uint64_t)(a0.seq_index_base / K + w.b0), (uint64_t)smc, (uint64_t)mts, (uint64_t)w.b0}) k.push_back(v);
+                           (uint64_t)(a0.seq_index_base / K + w.b0), (uint64_t)rng.threads, rng_inc, (uint64_t)w.b0}) k.push_back(v);
     };
     return beam_wave_loop(e, a, bf16, L, h_steps, s);
 }
@@ -2349,15 +2331,10 @@ int32_t mmt_sbs_select_step(mmt_engine* e, const float* d_logits, int32_t Bm, in
     const int pps = (T + PAGE_TOKENS - 1) / PAGE_TOKENS;
     Arena ar;
     int* ctl = nullptr; float* d_temp = nullptr; int64_t* cur_tok = nullptr; int *bt = nullptr, *cs = nullptr, *cd = nullptr;
-    auto plan_all = [&]() {
+    MMT_TRY(plan_arena(e, ar, [&]() {
         ctl = ar.get<int>(1); d_temp = ar.get<float>(Bm); cur_tok = ar.get<int64_t>(N);
         bt = ar.get<int>(N * pps); cs = ar.get<int>(N); cd = ar.get<int>(N);
-    };
-    ar.plan = true;
-    plan_all();
-    MMT_TRY(ensure_arena(e, ar.off));
-    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
-    plan_all();
+    }));
     const int t1 = step + 1;      // the step counter as the sampler leaves it
     MMT_CUDA(cudaMemcpyAsync(ctl, &t1, sizeof(int), cudaMemcpyHostToDevice, s));
     MMT_CUDA(cudaMemcpyAsync(d_temp, temp.data(), (size_t)Bm * sizeof(float), cudaMemcpyHostToDevice, s));
@@ -2367,10 +2344,7 @@ int32_t mmt_sbs_select_step(mmt_engine* e, const float* d_logits, int32_t Bm, in
     SbsParams sp;
     memset(&sp, 0, sizeof(sp));
     sp.logits = d_logits; sp.V = V; sp.K = k; sp.T = T; sp.eos = eos; sp.pps = pps; sp.Nw = N; sp.step = ctl; sp.temp = d_temp;
-    const int smc = rng_sm_count > 0 ? rng_sm_count : e->sm_count;
-    const int mts = rng_max_threads_per_sm > 0 ? rng_max_threads_per_sm : e->max_threads_per_sm;
-    sp.rng.seed = philox_seed; sp.rng.offset = philox_offset; sp.rng.numel = (int64_t)k * V;
-    sp.rng.threads = torch_rng_threads(sp.rng.numel, smc, mts); sp.rng_inc = torch_rng_increment(sp.rng.numel, smc, mts);
+    sp.rng = rng_geom(e, philox_seed, philox_offset, (int64_t)k * V, rng_sm_count, rng_max_threads_per_sm, &sp.rng_inc);
     sp.col_base = seq_index_base / k;
     const int rd = step & 1, wr = rd ^ 1;
     sp.phi[rd] = const_cast<double*>(d_phi); sp.key[rd] = const_cast<double*>(d_key); sp.len[rd] = const_cast<int*>(d_len);
@@ -2505,21 +2479,12 @@ int32_t mmt_sample(mmt_engine* e, const float* d_x, int64_t N, float temperature
     memset(&sp, 0, sizeof(sp));
     sp.x = d_x; sp.W = e->W("fc_out.weight"); sp.b = e->W("fc_out.bias"); sp.V = e->desc.vocab; sp.N = N; sp.ldn = N;
     sp.temperature = temperature; sp.mode = sampling;
-    int smc = rng_sm_count > 0 ? rng_sm_count : e->sm_count;
-    int mts = rng_max_threads_per_sm > 0 ? rng_max_threads_per_sm : e->max_threads_per_sm;
-    int64_t Nrng = N_total > 0 ? N_total : N;
-    sp.rng.seed = philox_seed; sp.rng.offset = philox_offset; sp.rng.numel = Nrng * sp.V;
-    sp.rng.threads = torch_rng_threads(sp.rng.numel, smc, mts);
-    sp.rng_inc = torch_rng_increment(sp.rng.numel, smc, mts);
+    const int64_t Nrng = N_total > 0 ? N_total : N;
+    sp.rng = rng_geom(e, philox_seed, philox_offset, Nrng * sp.V, rng_sm_count, rng_max_threads_per_sm, &sp.rng_inc);
     sp.seq_index_base = seq_index_base;
     sp.tokens = d_token; sp.probs = d_prob; sp.logits = d_logits_out;
     sp.advance = 0;
-    cudaStream_t cs = (cudaStream_t)stream;
-    prof_pre(e, cs);
-    MMT_TRY(sample_init(e));
-    sp.rows_per_warp = N >= 8192 ? SAMPLE_NR : 1;
-    sample_tokens<false><<<(unsigned)std::min<int64_t>((N + 8 * sp.rows_per_warp - 1) / (8 * sp.rows_per_warp), (int64_t)e->sm_count * 4), 256, sample_smem_bytes(sp.V), cs>>>(sp);
-    return check_launch(e, "sample_tokens", cs);
+    return launch_sample(e, sp, N, false, false, (cudaStream_t)stream);
 }
 
 int32_t mmt_exponential(uint64_t philox_seed, uint64_t philox_offset, int64_t elem_base, int64_t n, int64_t numel_total,
@@ -2560,19 +2525,17 @@ int32_t mmt_sample_memory_streams(mmt_engine* e, const float* d_x, const float* 
     EngineCall call(e, (cudaStream_t)stream);
     cudaStream_t cs = (cudaStream_t)stream;
     const int V = e->desc.vocab;
-    const int smc = rng_sm_count > 0 ? rng_sm_count : e->sm_count;
-    const int mts = rng_max_threads_per_sm > 0 ? rng_max_threads_per_sm : e->max_threads_per_sm;
-    RngGeom g;
-    g.seed = philox_seed; g.offset = philox_offset; g.numel = (int64_t)n_cand * V; g.threads = torch_rng_threads(g.numel, smc, mts);
-    const uint64_t inc = torch_rng_increment(g.numel, smc, mts);
-    prof_pre(e, cs);
+    uint64_t inc;
+    const RngGeom g = rng_geom(e, philox_seed, philox_offset, (int64_t)n_cand * V, rng_sm_count, rng_max_threads_per_sm, &inc);
     if (d_p) {
+        prof_pre(e, cs);
         sample_from_probs<<<(unsigned)((N + 7) / 8), 256, 0, cs>>>(d_p, N, V, g, seq_index_base, inc, n_cand, max_len, step, d_token);
         return check_launch(e, "sample_from_probs", cs);
     }
     // fused fc_out + softmax + pick at step `step`, read from a device step counter like the decode step's
-    MMT_TRY(ensure_arena(e, 256));
-    int* ctl = reinterpret_cast<int*>(e->arena);
+    Arena ar;
+    int* ctl = nullptr;
+    MMT_TRY(plan_arena(e, ar, [&]() { ctl = ar.get<int>(1); }));
     MMT_CUDA(cudaMemcpyAsync(ctl, &step, sizeof(int), cudaMemcpyHostToDevice, cs));
     SampleParams sp;
     memset(&sp, 0, sizeof(sp));
@@ -2582,10 +2545,7 @@ int32_t mmt_sample_memory_streams(mmt_engine* e, const float* d_x, const float* 
     sp.tokens = d_token - (int64_t)step * N; sp.probs = d_prob ? d_prob - (int64_t)step * N : nullptr;   // row `step` = the caller's
     sp.ctl.step = ctl;
     sp.advance = 0;
-    MMT_TRY(sample_init(e));
-    sp.rows_per_warp = N >= 8192 ? SAMPLE_NR : 1;
-    sample_tokens<false><<<(unsigned)std::min<int64_t>((N + 8 * sp.rows_per_warp - 1) / (8 * sp.rows_per_warp), (int64_t)e->sm_count * 4), 256, sample_smem_bytes(sp.V), cs>>>(sp);
-    return check_launch(e, "sample_tokens", cs);
+    return launch_sample(e, sp, N, false, false, cs);
 }
 
 int32_t mmt_sample_controlled(mmt_engine* e, const float* d_x, const float* d_p, int64_t N, int32_t n_cand, const mmt_sampling_controls* c,
@@ -2606,28 +2566,21 @@ int32_t mmt_sample_controlled(mmt_engine* e, const float* d_x, const float* d_p,
     MMT_TRY(host_controls(c, Bm, 1.f, V, temp, topk, topp, "mmt_sample_controlled"));
     EngineCall call(e, (cudaStream_t)stream);
     cudaStream_t cs = (cudaStream_t)stream;
-    const int smc = rng_sm_count > 0 ? rng_sm_count : e->sm_count;
-    const int mts = rng_max_threads_per_sm > 0 ? rng_max_threads_per_sm : e->max_threads_per_sm;
-    RngGeom g;
-    g.seed = philox_seed; g.offset = philox_offset; g.numel = (per_memory_rng ? (int64_t)n_cand : Nrng) * V; g.threads = torch_rng_threads(g.numel, smc, mts);
-    const uint64_t inc = torch_rng_increment(g.numel, smc, mts);
-    // workspace: step counter, then the controls
-    const size_t o_temp = 256, o_topk = o_temp + (size_t)Bm * 4, o_topp = o_topk + (size_t)Bm * 4;
-    MMT_TRY(ensure_arena(e, o_topp + (size_t)Bm * 4));
-    char* ws = reinterpret_cast<char*>(e->arena);
-    float* ctl_temp = reinterpret_cast<float*>(ws + o_temp); int32_t* ctl_topk = reinterpret_cast<int32_t*>(ws + o_topk);
-    float* ctl_topp = reinterpret_cast<float*>(ws + o_topp);
+    uint64_t inc;
+    const RngGeom g = rng_geom(e, philox_seed, philox_offset, (per_memory_rng ? (int64_t)n_cand : Nrng) * V, rng_sm_count, rng_max_threads_per_sm, &inc);
+    Arena ar;      // workspace: step counter, then the controls
+    int* ctl = nullptr; float *ctl_temp = nullptr, *ctl_topp = nullptr; int32_t* ctl_topk = nullptr;
+    MMT_TRY(plan_arena(e, ar, [&]() { ctl = ar.get<int>(1); ctl_temp = ar.get<float>(Bm); ctl_topk = ar.get<int32_t>(Bm); ctl_topp = ar.get<float>(Bm); }));
     MMT_CUDA(cudaMemcpyAsync(ctl_temp, temp.data(), (size_t)Bm * 4, cudaMemcpyHostToDevice, cs));
     MMT_CUDA(cudaMemcpyAsync(ctl_topk, topk.data(), (size_t)Bm * 4, cudaMemcpyHostToDevice, cs));
     MMT_CUDA(cudaMemcpyAsync(ctl_topp, topp.data(), (size_t)Bm * 4, cudaMemcpyHostToDevice, cs));
-    prof_pre(e, cs);
     if (d_p) {
         if (V > 64) MMT_FAIL("mmt_sample_controlled: vocab > 64");
+        prof_pre(e, cs);
         sample_probs_controlled<<<(unsigned)((N + 7) / 8), 256, 0, cs>>>(d_p, N, V, g, seq_index_base, inc, per_memory_rng ? n_cand : 0, max_len, step,
                                                                           n_cand, ctl_topk, ctl_topp, d_token, d_prob, d_kept);
         return check_launch(e, "sample_probs_controlled", cs);
     }
-    int* ctl = reinterpret_cast<int*>(ws);
     MMT_CUDA(cudaMemcpyAsync(ctl, &step, sizeof(int), cudaMemcpyHostToDevice, cs));
     SampleParams sp;
     memset(&sp, 0, sizeof(sp));
@@ -2642,11 +2595,7 @@ int32_t mmt_sample_controlled(mmt_engine* e, const float* d_x, const float* d_p,
     sp.ctl_temp = ctl_temp; sp.ctl_topk = ctl_topk; sp.ctl_topp = ctl_topp; sp.ctl_cand = n_cand;
     sp.ctl.step = ctl;
     sp.advance = 0;
-    MMT_TRY(sample_init(e));
-    sp.rows_per_warp = N >= 8192 ? SAMPLE_NR : 1;
-    sample_tokens<true><<<(unsigned)std::min<int64_t>((N + 8 * sp.rows_per_warp - 1) / (8 * sp.rows_per_warp), (int64_t)e->sm_count * 4), 256,
-                               sample_smem_bytes(sp.V), cs>>>(sp);
-    return check_launch(e, "sample_tokens_controlled", cs);
+    return launch_sample(e, sp, N, true, false, cs);
 }
 
 int32_t mmt_distinct_smiles(const int64_t* d_tokens, int32_t T, int64_t N, int32_t n_cand, int64_t eos,
@@ -2788,10 +2737,7 @@ int32_t mmt_decode_self_attention(mmt_engine* e, int32_t layer, const float* d_x
     d1.n_dec_layers = 1;
     Arena ar;
     DecBuffers b;
-    plan_decoder(ar, d1, N, 1, 1, T, b, bf16, e->fused_decode_rows);
-    MMT_TRY(ensure_arena(e, ar.off));
-    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
-    plan_decoder(ar, d1, N, 1, 1, T, b, bf16, e->fused_decode_rows);
+    MMT_TRY(plan_arena(e, ar, [&]() { plan_decoder(ar, d1, N, 1, 1, T, b, bf16, e->fused_decode_rows); }));
     const int pps = (T + PAGE_TOKENS - 1) / PAGE_TOKENS;
     // unwritten cache slots hold NaN: a key read before it was appended poisons the output instead of passing unnoticed
     MMT_CUDA(cudaMemsetAsync(b.kv_pool, 0xff, (size_t)b.pool_pages * 2 * PAGE_TOKENS * D * b.kv_esz, s));
@@ -2831,10 +2777,7 @@ int32_t mmt_decode_cross_attention(mmt_engine* e, const mmt_decode_args* a, int3
     // one wave of all Bm memories, planned like run_decode's (self-attention cache of a single position)
     Arena ar;
     DecBuffers b;
-    plan_decoder(ar, d, N, a->Bm, a->S, 1, b, bf16, e->fused_decode_rows);
-    MMT_TRY(ensure_arena(e, ar.off));
-    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
-    plan_decoder(ar, d, N, a->Bm, a->S, 1, b, bf16, e->fused_decode_rows);
+    MMT_TRY(plan_arena(e, ar, [&]() { plan_decoder(ar, d, N, a->Bm, a->S, 1, b, bf16, e->fused_decode_rows); }));
     MMT_TRY(decode_prepare_wave(e, *a, 0, a->Bm, b, bf16, s));
     MMT_CUDA(cudaMemcpyAsync(b.qc, d_q, (size_t)N * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
     const int64_t R = (int64_t)a->Bm * a->S;
@@ -2862,10 +2805,7 @@ int32_t mmt_decode_layer_tail(mmt_engine* e, int32_t layer, const float* d_x, co
     d1.n_dec_layers = 1;
     Arena ar;
     DecBuffers b;
-    plan_decoder(ar, d1, R, 1, 1, 1, b, bf16, e->fused_decode_rows);
-    MMT_TRY(ensure_arena(e, ar.off));
-    ar.plan = false; ar.base = e->arena; ar.cap = e->arena_bytes; ar.off = 0;
-    plan_decoder(ar, d1, R, 1, 1, 1, b, bf16, e->fused_decode_rows);
+    MMT_TRY(plan_arena(e, ar, [&]() { plan_decoder(ar, d1, R, 1, 1, 1, b, bf16, e->fused_decode_rows); }));
     const int64_t n_el = R * D;
     const unsigned blocks = (unsigned)((n_el + 255) / 256);
     const size_t bytes = (size_t)n_el * sizeof(float);
@@ -2934,9 +2874,7 @@ int32_t mmt_encoder_layer(mmt_engine* e, int32_t stack, int32_t layer, const flo
         else { ATT = a.get<float>((size_t)rows * D); PART = a.get<float>((size_t)rows * D); H = a.get<float>((size_t)rows * d.d_ff); }
         if (!ragged) { kidx = a.get<int>((size_t)B * S); nkd = a.get<int>(B); }
     };
-    a.plan = true; plan();
-    MMT_TRY(ensure_arena(e, a.off));
-    a.plan = false; a.base = e->arena; a.cap = e->arena_bytes; a.off = 0; plan();
+    MMT_TRY(plan_arena(e, a, plan));
     MMT_CUDA(cudaMemcpyAsync(X, d_x, (size_t)rows * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
     EncGroupRun g;
     memset(&g, 0, sizeof(g));
